@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/sec of the fused ShipEnv step on B200, with roofline, CPU baseline and e2e numbers.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One bench "step" = one pass of the hot path over one batch: a rollout of ROLLOUT (1000) consecutive env-steps of
 ENVS (4096) environments in ONE persistent kernel launch, with synthetic uniform{0,1,2} actions resident in HBM
@@ -39,6 +39,7 @@ ENVS = 4096          # BASELINE.json configs[1]
 ROLLOUT = 1000       # env-steps per launch ("1,000 steps")
 N_SCENARIOS = 1024   # SURVEY.md §8(d) config 2
 SEED = 0
+DUMP_OBS_ENVS = 192  # --dump-outputs: observation rows of this many envs (the whole obs tensor is 524 MB)
 METRIC = "env-steps/sec"
 UNIT = "env-steps/s"
 
@@ -310,6 +311,37 @@ def oracle_self_check(env, actions, obs, rew, done, state0, rank, steps=64, n_ch
             "K=%d launch" % (steps, n, ROLLOUT)}
 
 
+class OutputDump(object):
+    """--dump-outputs: what the last timed rollout returned, as float32 .npy files (57 MB in all), so that two builds can
+    be compared output for output: reward.npy and done.npy [ROLLOUT, ENVS] in full, obs.npy [ROLLOUT, DUMP_OBS_ENVS, 32]
+    for a fixed, seeded sample of env indices (in increasing order).  The device buffers are allocated, and the copy
+    kernels used once, before the timed region; after it take() only queues copies into them, so that nothing
+    allocates, loads or waits while the clock sampler still counts; write() runs after the sampler has stopped."""
+
+    def __init__(self, out):
+        import numpy as np
+        import torch
+        obs, rew, done = out
+        idx = np.sort(np.random.RandomState(SEED).choice(obs.shape[1], DUMP_OBS_ENVS, replace=False))
+        self.idx = torch.as_tensor(idx, device=obs.device)
+        self.bufs = {"obs": obs.new_empty(obs.shape[0], DUMP_OBS_ENVS, obs.shape[2]), "reward": torch.empty_like(rew),
+                     "done": torch.empty_like(done)}
+        self.take(out)      # the first copies load their kernels (milliseconds): not in the sampled region
+
+    def take(self, out):
+        import torch
+        obs, rew, done = out
+        torch.index_select(obs, 1, self.idx, out=self.bufs["obs"])
+        self.bufs["reward"].copy_(rew)
+        self.bufs["done"].copy_(done)
+
+    def write(self, dirname):
+        import numpy as np
+        os.makedirs(dirname, exist_ok=True)
+        for name, t in self.bufs.items():
+            np.save(os.path.join(dirname, name + ".npy"), t.float().cpu().numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -321,7 +353,13 @@ def main():
     ap.add_argument("--no-self-check", action="store_true")
     ap.add_argument("--lanes", type=int, default=0)
     ap.add_argument("--window", type=int, default=0, help="steps_in_flight (0 = auto)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last timed rollout's obs "
+                    "(a fixed sample of envs), reward and done to DIR/<name>.npy (rank 0's envs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3 if args.impl == "ours" else 0)
 
     rank = int(os.environ.get("RANK", 0))
@@ -345,6 +383,7 @@ def main():
     gen = torch.Generator(device=dev).manual_seed(SEED + rank)
     actions = torch.randint(0, 3, (ROLLOUT, ENVS), dtype=torch.int32, device=dev, generator=gen)
     out = env.alloc_rollout(ROLLOUT)
+    dump = OutputDump(out) if args.dump_outputs and rank == 0 else None
     reducer = sdist.StatsReducer(dev)
     reduce_mode = os.environ.get("SHIPSIM_BENCH_REDUCE", "full")
 
@@ -383,12 +422,16 @@ def main():
     launches = env.launch_info()["launches"] - l0
     # this rank's statistics as of the last all-reduced rollout (taken before anything else steps the envs)
     local_stats = env.stats_tensor(clear=False).clone()
+    if dump is not None:                    # stream-ordered before anything below launches into `out` again
+        dump.take(out)
     if sampler.nv is not None and sampler.armed_samples() < 5:    # region too short for NVML: extend, untimed
         t_end = time.time() + 0.5
         while time.time() < t_end:          # no collective in here: ranks run different numbers of these
             env.rollout(actions, out=out)
         torch.cuda.synchronize()
     clocks = sampler.stop()
+    if dump is not None:
+        dump.write(args.dump_outputs)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
