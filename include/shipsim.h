@@ -66,6 +66,26 @@ typedef enum shipsim_stat {
     SHIPSIM_STAT_STEPS           /* env-steps executed                                                 */
 } shipsim_stat;
 
+/* Episode log (shipsim_episode_log_bind): one record per finished episode, 8 int32 of metadata + the terminal row. */
+#define SHIPSIM_EPISODE_META 8
+enum {
+    SHIPSIM_EP_K = 0,            /* step index within the caller's shipsim_step / shipsim_step_host call   */
+    SHIPSIM_EP_ENV,              /* local env index                                                          */
+    SHIPSIM_EP_LENGTH,           /* ShipEnv.step_count at episode end (ship_env.py:152)                      */
+    SHIPSIM_EP_RETURN,           /* ShipEnv.cumulative_reward at episode end (ship_env.py:150), float bits   */
+    SHIPSIM_EP_END,              /* why it ended: SHIPSIM_END_* bits, possibly several                       */
+    SHIPSIM_EP_SCENARIO,         /* the finished episode's scenario ...                                      */
+    SHIPSIM_EP_EPISODE,          /* ... and episode number                                                   */
+    SHIPSIM_EP_CALL              /* the handle's sequence number of the step call, taken at enqueue         */
+};
+enum {
+    SHIPSIM_END_COLLISION = 1,   /* game.colliding (ship_env.py:120)          */
+    SHIPSIM_END_ALL_GOALS = 2,   /* no goals left (ship_env.py:122)           */
+    SHIPSIM_END_OOB = 4,         /* out of bounds (ship_env.py:126-129)       */
+    SHIPSIM_END_TIMEOUT = 8,     /* step_count >= MAX_STEPS (ship_env.py:131): the only truncation */
+    SHIPSIM_END_GOAL = 16        /* a goal was taken on the last step         */
+};
+
 /* Knobs.  Mirrors ship_gym/config.py:14-24 (GameConfig / EnvConfig) plus the constants the reference
  * hard-codes; the host layer fills it from those classes.  Zero-initialise, then call
  * shipsim_config_default(). */
@@ -179,6 +199,19 @@ int shipsim_reset(shipsim_t *h, const uint8_t *dev_mask, const int32_t *dev_scen
  * Any output pointer may be NULL to skip it. */
 int shipsim_step(shipsim_t *h, const void *dev_actions, int action_dtype, int32_t K, float *dev_obs,
                  float *dev_reward, uint8_t *dev_done, void *stream);
+
+/* Episode log.  With auto_reset a done env's observation is replaced by the reset observation; with a log bound, the
+ * step kernels first append one record per finished episode: dev_meta[i][SHIPSIM_EPISODE_META] (SHIPSIM_EP_*) and
+ * dev_rows[i][16 * history] = exactly the row an auto_reset = 0 launch writes for that env at that step (terminal
+ * observation; history = the config's 1 or 2).  Slots are reserved with an atomic add on *dev_count (int32, the records
+ * appended so far); a record whose slot is >= capacity is not written, but the count keeps counting, so a caller sees
+ * the loss.  The caller owns the three buffers (device memory; dev_rows and dev_meta may also be page-locked host
+ * memory, written over PCIe without atomics -- dev_count must be device memory) and drains the log by reading it and
+ * zeroing *dev_count on its stream.  SHIPSIM_EP_K includes the chunk offset on the chunked shipsim_step_host path;
+ * SHIPSIM_EP_CALL counts shipsim_step / shipsim_step_host calls of the handle (a replayed CUDA graph repeats the
+ * captured values).  Results with the log on are bit-identical to results with it off.  capacity == 0 unbinds.  Needs
+ * auto_reset (SHIPSIM_ERR_STATE otherwise). */
+int shipsim_episode_log_bind(shipsim_t *h, float *dev_rows, int32_t *dev_meta, int32_t capacity, int32_t *dev_count);
 
 /* Same transition with HOST buffers: host_actions in, rows / rewards / done flags out, waited for (what a CPU-side caller
  * such as the reference's own training scripts sees).  Any output pointer may be NULL.  Buffers should be page-locked

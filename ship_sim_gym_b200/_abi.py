@@ -14,6 +14,10 @@ ACTION_I32, ACTION_I64, ACTION_U8, ACTION_RANDOM = 0, 1, 2, 3
 STATS_LEN = 16
 STAT_NAMES = ("episodes", "return_sum", "length_sum", "goal_steps", "collision", "oob", "timeout", "all_goals", "steps")
 N_GOALS, N_BEAMS, FRAME, STATE_PLANES, MAX_HULL = 5, 10, 16, 8, 32
+# episode log (shipsim_episode_log_bind): columns of a record's metadata, and the SHIPSIM_END_* bits
+EPISODE_META = 8
+EP_K, EP_ENV, EP_LENGTH, EP_RETURN, EP_END, EP_SCENARIO, EP_EPISODE, EP_CALL = range(8)
+END_COLLISION, END_ALL_GOALS, END_OOB, END_TIMEOUT, END_GOAL = 1, 2, 4, 8, 16
 
 # every symbol include/shipsim.h declares (tests check the library exports all of them)
 SYMBOLS = (
@@ -22,7 +26,7 @@ SYMBOLS = (
     "shipsim_step", "shipsim_step_host", "shipsim_stats_read", "shipsim_set_state", "shipsim_get_state",
     "shipsim_launch_count", "shipsim_launch_shape", "shipsim_launch_window", "shipsim_set_max_steps",
     "shipsim_generate_scenarios", "shipsim_read_scenarios", "shipsim_render", "shipsim_assemble_history", "shipsim_expand_delta", "shipsim_host_traffic", "shipsim_host_threads",
-    "shipsim_fresh_maps", "shipsim_fresh_info", "shipsim_mlp_policy_forward", "shipsim_gae",
+    "shipsim_fresh_maps", "shipsim_fresh_info", "shipsim_mlp_policy_forward", "shipsim_gae", "shipsim_episode_log_bind",
 )
 
 
@@ -86,6 +90,7 @@ def load():
     L.shipsim_fresh_info.argtypes = [vp, C.POINTER(i32)]
     L.shipsim_mlp_policy_forward.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.shipsim_gae.argtypes = [vp, vp, vp, i32, i32, C.c_float, C.c_float, vp, vp, vp]
+    L.shipsim_episode_log_bind.argtypes = [vp, vp, vp, i32, vp]
     L.shipsim_launch_count.argtypes = [vp, C.POINTER(i64)]
     L.shipsim_launch_shape.argtypes = [vp, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)]
     L.shipsim_launch_window.argtypes = [vp, C.POINTER(i32)]

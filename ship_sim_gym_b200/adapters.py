@@ -15,6 +15,7 @@ libraries call.  Both sit on one `BatchedShipEnv`, i.e. one GPU; numpy in / nump
 import numpy as np
 import torch
 
+from . import _abi
 from .env import BatchedShipEnv
 
 
@@ -30,10 +31,34 @@ def tile_images(images):
     return grid.reshape(rows * h, cols * w, c)
 
 
-class ShipVecEnv(object):
-    """stable-baselines `VecEnv` over a BatchedShipEnv (auto-reset on, like a SubprocVecEnv worker)."""
+def episode_infos(base, env, ret, length, truncated, rows):
+    """The per-env info dicts of one step, as `Monitor` and the stable-baselines workers fill them: an env whose episode
+    ended gets {'episode': {'r': return, 'l': length}, 'terminal_observation': row, 'TimeLimit.truncated': ended on the
+    step cap alone}; the others keep their entry of `base` ({}).  env / ret / length / truncated: lists with one entry per
+    finished episode (plain Python numbers: this runs once per step on the caller's critical path), rows: its terminal
+    observations."""
+    infos = list(base)
+    for e, r, ln, tr, row in zip(env, ret, length, truncated, rows):
+        infos[e] = {"episode": {"r": r, "l": ln}, "terminal_observation": row, "TimeLimit.truncated": tr}
+    return infos
 
-    def __init__(self, num_envs, game_config=None, env_config=None, as_tensors=False, **kw):
+
+def log_infos(base, meta, rows):
+    """episode_infos from raw episode-log records (int32 meta [n, 8], rows [n, D]; numpy; the rows are copied)."""
+    meta = np.asarray(meta, dtype=np.int32)
+    reasons = meta[:, _abi.EP_END] & (_abi.END_COLLISION | _abi.END_ALL_GOALS | _abi.END_OOB | _abi.END_TIMEOUT)
+    return episode_infos(base, meta[:, _abi.EP_ENV].tolist(), meta[:, _abi.EP_RETURN].view(np.float32).tolist(),
+                         meta[:, _abi.EP_LENGTH].tolist(), (reasons == _abi.END_TIMEOUT).tolist(), np.array(rows, dtype=np.float32))
+
+
+class ShipVecEnv(object):
+    """stable-baselines `VecEnv` over a BatchedShipEnv (auto-reset on, like a SubprocVecEnv worker).
+
+    episode_info=True: the info of an env whose episode ended on this step carries what `Monitor` and the later
+    stable-baselines workers put there -- `episode` {r, l}, `terminal_observation`, `TimeLimit.truncated` -- from the
+    kernels' episode log (BatchedShipEnv.enable_episode_log)."""
+
+    def __init__(self, num_envs, game_config=None, env_config=None, as_tensors=False, episode_info=False, **kw):
         kw["auto_reset"] = True
         self.batch = BatchedShipEnv(num_envs, game_config, env_config, **kw)
         self.num_envs = self.batch.num_envs
@@ -42,6 +67,18 @@ class ShipVecEnv(object):
         self.as_tensors = bool(as_tensors)
         self._pending = None
         self._infos = [{} for _ in range(self.num_envs)]       # ShipEnv.step's info is always {} (ship_env.py:156)
+        self.episode_info = bool(episode_info)
+        if self.episode_info:
+            # numpy callers: the log lives in page-locked host memory, written by the kernel during the step; the step's
+            # own wait makes it readable, and the number of new records is the number of done flags (one per finished
+            # episode), so nothing else is read from the device.  The count is reset only when the log is nearly full.
+            self._np_log = not self.as_tensors and self.batch.history <= 2
+            self._log_cap = 64 * self.num_envs if self._np_log else self.num_envs
+            self.batch.enable_episode_log(self._log_cap, pinned=self._np_log)
+            self._log_used = 0
+            if self._np_log:
+                rows, meta, _, _ = self.batch._eplog
+                self._log_np = (rows.numpy(), meta.numpy())
 
     def _out(self, t):
         return t if self.as_tensors else t.cpu().numpy()
@@ -54,8 +91,18 @@ class ShipVecEnv(object):
             raise RuntimeError("step_async called twice without step_wait")
         if not self.as_tensors and not torch.is_tensor(actions) and self.batch.history <= 2:
             # a numpy caller: one call into the C ABI's host-buffer path (no torch ops; the work is done here)
+            if self.episode_info and self._log_used + self.num_envs > self._log_cap:
+                self.batch._eplog[2].zero_()                # (enqueued ahead of the step on the same stream)
+                self._log_used = 0
             obs, rew, done = self.batch.step_np(np.asarray(actions))
-            self._pending = (obs.copy(), rew.copy(), done.copy(), None)
+            infos = None
+            if self.episode_info:
+                n = int(np.count_nonzero(done))
+                rows, meta = self._log_np
+                lo = self._log_used
+                infos = log_infos(self._infos, meta[lo:lo + n], rows[lo:lo + n]) if n else self._infos
+                self._log_used += n
+            self._pending = (obs.copy(), rew.copy(), done.copy(), infos)
             return
         a = torch.as_tensor(np.asarray(actions) if not torch.is_tensor(actions) else actions)
         self._pending = self.batch.step(a)       # enqueued on the GPU; nothing is waited for here
@@ -63,11 +110,18 @@ class ShipVecEnv(object):
     def step_wait(self):
         if self._pending is None:
             raise RuntimeError("step_wait called before step_async")
-        obs, rew, done, _ = self._pending
+        obs, rew, done, infos = self._pending
         self._pending = None
         if isinstance(obs, np.ndarray):
-            return obs, rew, done, self._infos
-        return self._out(obs), self._out(rew), self._out(done), self._infos
+            return obs, rew, done, infos if infos is not None else self._infos
+        infos = self._infos
+        if self.episode_info:                   # (tensor path: the records are read back from the device once per step)
+            ep = self.batch.episodes()
+            self._log_used = 0
+            if ep["env"].numel():
+                rows = ep["terminal_obs"] if self.as_tensors else ep["terminal_obs"].cpu().numpy()
+                infos = episode_infos(self._infos, *(ep[k].tolist() for k in ("env", "return", "length", "truncated")), rows)
+        return self._out(obs), self._out(rew), self._out(done), infos
 
     def step(self, actions):
         self.step_async(actions)

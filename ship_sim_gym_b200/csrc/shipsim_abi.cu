@@ -137,6 +137,7 @@ struct shipsim_handle {
     HostPool *pool = nullptr;
     int64_t last_h2d = 0, last_d2h = 0;      // bytes the last shipsim_step_host moved over PCIe
     int64_t launches = 0;
+    int32_t calls = 0;                       // shipsim_step / shipsim_step_host calls so far (SHIPSIM_EP_CALL)
     LaunchShape shape{1, kThreads, 0, 1};
 };
 
@@ -694,6 +695,40 @@ extern "C" int shipsim_reset(shipsim_t *h, const uint8_t *dev_mask, const int32_
     return SHIPSIM_OK;
 }
 
+extern "C" int shipsim_episode_log_bind(shipsim_t *h, float *dev_rows, int32_t *dev_meta, int32_t capacity, int32_t *dev_count)
+{
+    if (!h) return fail(SHIPSIM_ERR_ARG, "handle is NULL");
+    StepParams &p = h->p;
+    if (capacity == 0) {
+        p.log_rows = nullptr; p.log_meta = nullptr; p.log_count = nullptr; p.log_cap = 0; p.log_row4 = 0;
+        return SHIPSIM_OK;
+    }
+    if (!h->cfg.auto_reset) return fail(SHIPSIM_ERR_STATE, "the episode log needs auto_reset (without it the caller sees the terminal rows)");
+    if (capacity < 0 || !dev_rows || !dev_meta || !dev_count) return fail(SHIPSIM_ERR_ARG, "NULL buffer or capacity < 0");
+    if (((uintptr_t)dev_rows & 15) || ((uintptr_t)dev_meta & 15) || ((uintptr_t)dev_count & 3))
+        return fail(SHIPSIM_ERR_ARG, "dev_rows / dev_meta must be 16-byte aligned");
+    DeviceGuard g(h->device);
+    // rows and metadata may sit in page-locked host memory (written over PCIe): the kernels need its device alias
+    auto device_alias = [](void *ptr) {
+        cudaPointerAttributes attr{};
+        const bool host = cudaPointerGetAttributes(&attr, ptr) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer;
+        cudaGetLastError();
+        return host ? attr.devicePointer : ptr;
+    };
+    {
+        cudaPointerAttributes attr{};
+        const bool dev = cudaPointerGetAttributes(&attr, dev_count) == cudaSuccess && attr.type == cudaMemoryTypeDevice;
+        cudaGetLastError();
+        if (!dev) return fail(SHIPSIM_ERR_ARG, "dev_count must be device memory (it is the target of device atomics)");
+    }
+    p.log_rows = (float4 *)device_alias(dev_rows);
+    p.log_meta = (int4 *)device_alias(dev_meta);
+    p.log_count = (int *)dev_count;
+    p.log_cap = capacity;
+    p.log_row4 = 4 * h->cfg.history;
+    return SHIPSIM_OK;
+}
+
 static int step_impl(shipsim_t *h, const void *dev_actions, int action_dtype, int32_t K, float *dev_obs, float *dev_reward,
                      uint8_t *dev_done, void *stream, int history)
 {
@@ -723,6 +758,7 @@ static int step_impl(shipsim_t *h, const void *dev_actions, int action_dtype, in
 extern "C" int shipsim_step(shipsim_t *h, const void *dev_actions, int action_dtype, int32_t K, float *dev_obs, float *dev_reward,
                             uint8_t *dev_done, void *stream)
 {
+    if (h) { h->p.log_call = h->calls++; h->p.log_k0 = 0; }
     return step_impl(h, dev_actions, action_dtype, K, dev_obs, dev_reward, dev_done, stream, h ? h->p.history : 1);
 }
 
@@ -733,6 +769,8 @@ extern "C" int shipsim_step_host(shipsim_t *h, const int32_t *host_actions, int3
     if (rc) return rc;
     if (K < 1 || !host_actions) return fail(SHIPSIM_ERR_ARG, "K must be >= 1 and host_actions non-NULL");
     DeviceGuard g(h->device);
+    h->p.log_call = h->calls++;
+    h->p.log_k0 = 0;
     const size_t N = (size_t)h->cfg.num_envs;
     const size_t n = N * K;
     // With HISTORY_SIZE = 2 an observation is [frame of the previous step | frame of this step] (ship_env.py:112-113):
@@ -966,8 +1004,14 @@ extern "C" int shipsim_step_host(shipsim_t *h, const int32_t *host_actions, int3
                     CU(cudaEventRecord(h->act_up, h->aux_stream));
                 }
             } else if (c == 1) CU(cudaStreamWaitEvent(s, h->act_up, 0));
+            h->p.log_k0 = k0;                                       // episode-log records carry the step index within the call
             const int rc2 = step_impl(h, h->d_act + off, SHIPSIM_ACTION_I32, kc, d_chunk, h->d_rew + off, h->d_done + off, stream, hist_c);
+            h->p.log_k0 = 0;
             if (rc2) return rc2;
+            if (frames_only && h->p.log_count && h->cfg.history == 2) {     // the one-frame kernel logged the terminal frame only
+                CU(launch_log_prev_frames(h->p, (const float4 *)d_chunk, prev_frames, k0, kc, s));
+                h->launches++;
+            }
             if (trace) CU(cudaEventRecord(h->trace_mid[c], s));
             if (frames_only) {
                 if (nd < (int)N) {

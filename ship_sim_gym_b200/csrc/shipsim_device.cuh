@@ -99,7 +99,42 @@ struct StepParams {
     float ship_off[kShipVerts];                      // ship_n[j] . ship_l[j]: offset of the hull's plane j (rotation invariant)
     float ship_aabb[4];                                // body-frame l,b,r,t of the hull
     float goal_cull_r2;                              // (max |hull vertex| + goal radius)^2: bounding circle about the body origin
+    // episode log (shipsim_episode_log_bind; log_count == nullptr: off, and the kernels run their log-free instantiation)
+    float4 *log_rows;                                // [log_cap][log_row4]
+    int4 *log_meta;                                  // [log_cap][2] = SHIPSIM_EP_K .. SHIPSIM_EP_CALL
+    int *log_count;
+    int log_cap, log_row4;                           // log_row4 = float4 per record row (4 * the config's history)
+    int log_k0;                                      // added to the step index (the chunk offset of shipsim_step_host)
+    int log_call;                                    // sequence number of the step call
 };
+
+// SHIPSIM_END_* (include/shipsim.h)
+constexpr int kEndCollision = 1, kEndAllGoals = 2, kEndOob = 4, kEndTimeout = 8, kEndGoal = 16;
+
+__device__ __forceinline__ int end_bits(bool colliding, bool all_goals, bool oob, bool timeout, bool goal_reached)
+{
+    return (colliding ? kEndCollision : 0) | (all_goals ? kEndAllGoals : 0) | (oob ? kEndOob : 0) | (timeout ? kEndTimeout : 0)
+           | (goal_reached ? kEndGoal : 0);
+}
+
+// Episode log: one atomic per warp reserves the slots of the lanes in `m` (a ballot; non-zero, warp-uniform), which are
+// handed out in lane order.  Returns this lane's slot (meaningful where its bit of m is set).
+__device__ __forceinline__ unsigned log_reserve(const StepParams &p, int lane, unsigned m)
+{
+    const int src = __ffs(m) - 1;
+    unsigned base = 0u;
+    if (lane == src) base = (unsigned)atomicAdd(p.log_count, __popc(m));
+    base = __shfl_sync(0xffffffffu, base, src);
+    return base + (unsigned)__popc(m & ((1u << lane) - 1u));
+}
+
+// the record's metadata (the caller writes the row: its last `4 * history` float4 of log_rows[slot])
+__device__ __forceinline__ void log_meta(const StepParams &p, unsigned slot, int k, int e, int steps, float ret, int end, int scen, int ep)
+{
+    int4 *m = p.log_meta + (size_t)slot * 2;
+    m[0] = make_int4(p.log_k0 + k, e, steps, __float_as_int(ret));
+    m[1] = make_int4(end, scen, ep, p.log_call);
+}
 
 struct EnvRegs {
     float x, y, th, vx, vy, w, ret;

@@ -52,7 +52,9 @@ constexpr float kDeadGoal = 3.0e19f;        // coordinate of a goal that has bee
 // compiler rebuilt those indices from threadIdx / blockIdx inside the loop: 12 % of the instructions, and an S2R
 // stall that was the hottest sample of the kernel.  The offsets are laundered through an empty asm so that they stay
 // in their registers.)
-template <int G, int HIST, int MINB, int THREADS>
+// LOG: write the episode log (shipsim_episode_log_bind).  The log-free kernel is a separate instantiation: its registers
+// and spills are those of the kernel before the log existed (-Xptxas -v).
+template <int G, int HIST, int MINB, int THREADS, bool LOG>
 __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_constant__ StepParams p)
 {
     constexpr int EPW = 32 / G;                 // envs per warp
@@ -392,6 +394,26 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
 
             warp_stats(wb + STA * 16, lane, leader, goal_reached, done, colliding, oob, timeout, all_goals, r.ret, r.steps);
             do_reset = done && p.auto_reset;
+            if (LOG) {
+                // episode log: the terminal row -- the previous frame and the newest one completed with this step's pose,
+                // rudder, nearest remaining goal and sticky lidar, i.e. what the frame block below writes without a reset --
+                // and the episode's numbers, before the reset replaces them
+                const unsigned lm = __ballot_sync(kFull, leader && done);
+                if (lm) {
+                    const unsigned slot = log_reserve(p, lane, lm);
+                    if (leader && done && slot < (unsigned)p.log_cap) {
+                        float4 *row = p.log_rows + (size_t)slot * p.log_row4 + (p.log_row4 - OBS4);
+                        if (HIST == 2) { row[0] = lds4(EA(0)); row[1] = lds4(EA(1)); row[2] = lds4(EA(2)); row[3] = lds4(EA(3)); }
+                        const float4 f1 = lds4(EA(OBS4 - 3));
+                        row[OBS4 - 4] = make_float4(r.x, r.y, lds1(EA(OBS4 - 4) + 8), r.th);
+                        row[OBS4 - 3] = make_float4(gx, gy, f1.z, f1.w);
+                        row[OBS4 - 2] = lds4(EA(OBS4 - 2));
+                        row[OBS4 - 1] = lds4(EA(OBS4 - 1));
+                        log_meta(p, slot, k, e, r.steps, r.ret, end_bits(colliding, all_goals, oob, timeout, goal_reached), r.scen,
+                                 __float_as_int(lds1(EA(GOL + 2) + 12)));
+                    }
+                }
+            }
             int ep_g = 0;
             if (G > 1) {                        // read by every lane while the warp is converged, before the leader stores the next one
                 ep_g = __float_as_int(lds1(EA(GOL + 2) + 12)) + 1;
@@ -762,6 +784,24 @@ __global__ void __launch_bounds__(256) history_rows_kernel(const float4 *frames,
     __stcs(o + 4, cur);
 }
 
+// Episode log on the frames-only path of shipsim_step_host, where the step kernel runs in its one-frame mode and puts the
+// terminal frame into the second half of a record's row: the first half, the env's previous frame, comes from the chunk's
+// frames (prev0 = the frames before the chunk's first step).  One thread per record slot; only the records of call
+// `call` whose step lies in this chunk are touched.
+__global__ void __launch_bounds__(256) log_prev_frames_kernel(const float4 *frames, const float4 *prev0, int N, int k0, int kc, int call,
+                                                              float4 *rows, const int4 *meta, const int *count, int cap)
+{
+    const int n = min(*count, cap);
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const int4 m0 = meta[2 * (size_t)i], m1 = meta[2 * (size_t)i + 1];
+        if (m1.w != call || m0.x < k0 || m0.x >= k0 + kc) continue;
+        const int kk = m0.x - k0, e = m0.y;
+        const float4 *src = kk > 0 ? frames + ((size_t)(kk - 1) * N + e) * 4 : prev0 + (size_t)e * 4;
+#pragma unroll
+        for (int q = 0; q < 4; ++q) rows[(size_t)i * 8 + q] = src[q];
+    }
+}
+
 // stats slots -> out[kStatLen]; one warp per statistic column
 __global__ void stats_reduce_kernel(double *slots, double *out, int clear)
 {
@@ -779,6 +819,13 @@ __global__ void stats_reduce_kernel(double *slots, double *out, int clear)
 // ------------------------------------------------------------------------------------------------------------
 // launch wrappers (called from the C ABI)
 // ------------------------------------------------------------------------------------------------------------
+template <int G, int HIST, int MB, int T>
+static void launch_gh(const StepParams &p, int blocks, cudaStream_t stream)
+{
+    if (p.log_count) step_kernel<G, HIST, MB, T, true><<<blocks, T, 0, stream>>>(p);
+    else step_kernel<G, HIST, MB, T, false><<<blocks, T, 0, stream>>>(p);
+}
+
 template <int G>
 static cudaError_t launch_g(const StepParams &p, cudaStream_t stream, LaunchShape *shape)
 {
@@ -790,8 +837,8 @@ static cudaError_t launch_g(const StepParams &p, cudaStream_t stream, LaunchShap
         if (blocks >= 148 * 8) {
             threads = SHIPSIM_BIG_THREADS;
             blocks = (p.N + threads - 1) / threads;
-            if (p.history == 2) step_kernel<G, 2, SHIPSIM_BIG_MIN_BLOCKS, SHIPSIM_BIG_THREADS><<<blocks, threads, 0, stream>>>(p);
-            else step_kernel<G, 1, SHIPSIM_BIG_MIN_BLOCKS, SHIPSIM_BIG_THREADS><<<blocks, threads, 0, stream>>>(p);
+            if (p.history == 2) launch_gh<G, 2, SHIPSIM_BIG_MIN_BLOCKS, SHIPSIM_BIG_THREADS>(p, blocks, stream);
+            else launch_gh<G, 1, SHIPSIM_BIG_MIN_BLOCKS, SHIPSIM_BIG_THREADS>(p, blocks, stream);
             launched = true;
         }
     }
@@ -801,8 +848,8 @@ static cudaError_t launch_g(const StepParams &p, cudaStream_t stream, LaunchShap
         constexpr int T = SHIPSIM_SMALL_THREADS, MB = SHIPSIM_MIN_BLOCKS * kThreads / SHIPSIM_SMALL_THREADS;
         threads = T;
         blocks = (p.N + T / G - 1) / (T / G);
-        if (p.history == 2) step_kernel<G, 2, MB, T><<<blocks, T, 0, stream>>>(p);
-        else step_kernel<G, 1, MB, T><<<blocks, T, 0, stream>>>(p);
+        if (p.history == 2) launch_gh<G, 2, MB, T>(p, blocks, stream);
+        else launch_gh<G, 1, MB, T>(p, blocks, stream);
     }
     if (shape) { shape->lanes_per_env = G; shape->threads = threads; shape->blocks = blocks; shape->window = 1; }
     return cudaGetLastError();
@@ -873,6 +920,13 @@ cudaError_t launch_build_grid(const double *hull_xy, const int *hull_n, int n_sc
 cudaError_t launch_build_spawn_rows(const StepParams &p, float4 *rows, cudaStream_t stream)
 {
     build_spawn_rows_kernel<<<(p.n_scen + 127) / 128, 128, 0, stream>>>(p, rows);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_log_prev_frames(const StepParams &p, const float4 *frames, const float4 *prev0, int k0, int kc, cudaStream_t stream)
+{
+    const int blocks = p.log_cap < 1184 * 256 ? (p.log_cap + 255) / 256 : 1184;
+    log_prev_frames_kernel<<<blocks, 256, 0, stream>>>(frames, prev0, p.N, k0, kc, p.log_call, p.log_rows, p.log_meta, p.log_count, p.log_cap);
     return cudaGetLastError();
 }
 

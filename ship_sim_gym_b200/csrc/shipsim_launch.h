@@ -36,6 +36,8 @@ cudaError_t launch_gae(const float *rew, const float *val, const unsigned char *
 cudaError_t launch_mlp_policy(const float *obs, int n, const float *w1, const float *b1, const float *w2, const float *b2, const float *w3,
                               const float *b3, const float *noise, float *out, long long *actions, cudaStream_t stream);
 cudaError_t launch_render(const StepParams &p, int e, int img_w, int img_h, uint8_t *rgb, cudaStream_t stream);
+// episode log, frames-only host path: the previous frame of the records of chunk [k0, k0 + kc) of call p.log_call
+cudaError_t launch_log_prev_frames(const StepParams &p, const float4 *frames, const float4 *prev0, int k0, int kc, cudaStream_t stream);
 cudaError_t launch_stats_reduce(double *slots, double *out, int clear, cudaStream_t stream);
 
 }  // namespace shipsim

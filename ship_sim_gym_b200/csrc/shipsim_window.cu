@@ -53,7 +53,9 @@ constexpr int kWinThreads = SHIPSIM_WIN_THREADS;      // one-warp CTAs: a latenc
 #define SHIPSIM_WIN_BOUNDS __launch_bounds__(kWinThreads, 512 / SHIPSIM_WIN_THREADS)
 #endif
 
-template <int T, int HIST>
+// LOG: write the episode log (shipsim_episode_log_bind).  The log-free kernel is a separate instantiation: its registers
+// and spills are those of the kernel before the log existed (-Xptxas -v; this kernel sits at the 128-register wall).
+template <int T, int HIST, bool LOG>
 __global__ void SHIPSIM_WIN_BOUNDS window_kernel(const __grid_constant__ StepParams p)
 {
     constexpr int E = 32 / T;                   // envs per warp
@@ -596,6 +598,25 @@ SHIPSIM_UNROLL(SHIPSIM_SCAN_UNROLL)
             if (p.reward) p.reward[row] = reward;
             if (p.done) p.done[row] = done ? 1 : 0;
         }
+        if (LOG) {
+            // episode log: the lane of the window's first done step writes the terminal row -- frame slots t and t + 1,
+            // complete since the sticky-lidar scan, not yet overwritten by the reset below -- and the episode's numbers
+            // (r is still the finished episode's state)
+            const bool mine = do_reset && t == ncommit - 1;
+            const unsigned lm = __ballot_sync(kFull, mine);
+            if (lm) {
+                const unsigned slot = log_reserve(p, lane, lm);
+                if (mine && slot < (unsigned)p.log_cap) {
+                    float4 *row = p.log_rows + (size_t)slot * p.log_row4 + (p.log_row4 - OBS4);
+                    const float4 *fp = myfr - (HIST - 1) * FS4;
+#pragma unroll
+                    for (int h = 0; h < HIST; ++h)
+#pragma unroll
+                        for (int i = 0; i < 4; ++i) row[4 * h + i] = fp[h * FS4 + i];
+                    log_meta(p, slot, k0 + t, e, steps_t, my_ret, end_bits(colliding, all_goals, oob, timeout, goal_reached), r.scen, r.episode);
+                }
+            }
+        }
         __syncwarp();                           // rows and frames have been read: the carry may move
 
         if (ncommit > 0) {
@@ -643,8 +664,13 @@ static cudaError_t launch_t(const StepParams &p, cudaStream_t stream, LaunchShap
     const int envs_per_cta = (kWinThreads / 32) * (32 / T);
     const int blocks = (p.N + envs_per_cta - 1) / envs_per_cta;
     if (shape) { shape->lanes_per_env = T; shape->threads = kWinThreads; shape->blocks = blocks; shape->window = T; }
-    if (p.history == 2) window_kernel<T, 2><<<blocks, kWinThreads, 0, stream>>>(p);
-    else window_kernel<T, 1><<<blocks, kWinThreads, 0, stream>>>(p);
+    if (p.log_count) {
+        if (p.history == 2) window_kernel<T, 2, true><<<blocks, kWinThreads, 0, stream>>>(p);
+        else window_kernel<T, 1, true><<<blocks, kWinThreads, 0, stream>>>(p);
+    } else {
+        if (p.history == 2) window_kernel<T, 2, false><<<blocks, kWinThreads, 0, stream>>>(p);
+        else window_kernel<T, 1, false><<<blocks, kWinThreads, 0, stream>>>(p);
+    }
     return cudaGetLastError();
 }
 

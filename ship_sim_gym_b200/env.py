@@ -71,6 +71,40 @@ def _dtype_code(t):
     raise TypeError("actions must be int32, int64 or uint8, got %s" % t.dtype)
 
 
+def episode_dict(meta, rows, env_id_offset=0):
+    """Episode-log records -> the dict `BatchedShipEnv.episodes()` returns, sorted by (call, k, env).
+
+    meta: int32 [n, 8] (columns _abi.EP_*), rows: float32 [n, D] terminal observations.  Pure torch, any device.
+    `truncated` = the episode ended on the step cap alone (SHIPSIM_END_TIMEOUT; a goal taken on that step does not change
+    it), `terminated` = everything else: collision, out of bounds or all goals taken."""
+    meta = meta.to(torch.int32).contiguous()
+    order = torch.arange(meta.shape[0], device=meta.device)
+    for col in (_abi.EP_ENV, _abi.EP_K, _abi.EP_CALL):          # least significant key first, stable sorts
+        order = order[torch.sort(meta[order, col], stable=True).indices]
+    m = meta[order]
+    end = m[:, _abi.EP_END]
+    reasons = end & (_abi.END_COLLISION | _abi.END_ALL_GOALS | _abi.END_OOB | _abi.END_TIMEOUT)
+    truncated = reasons == _abi.END_TIMEOUT
+    col = lambda c: m[:, c].long()      # noqa: E731
+    return {
+        "env": col(_abi.EP_ENV), "global_env": col(_abi.EP_ENV) + int(env_id_offset), "k": col(_abi.EP_K), "call": col(_abi.EP_CALL),
+        "length": col(_abi.EP_LENGTH), "return": m[:, _abi.EP_RETURN].contiguous().view(torch.float32),
+        "terminated": ~truncated, "truncated": truncated, "collision": (end & _abi.END_COLLISION) != 0,
+        "oob": (end & _abi.END_OOB) != 0, "all_goals": (end & _abi.END_ALL_GOALS) != 0, "goal": (end & _abi.END_GOAL) != 0,
+        "scenario": col(_abi.EP_SCENARIO), "episode": col(_abi.EP_EPISODE), "terminal_obs": rows[order],
+    }
+
+
+def long_history_terminal_rows(prev_rows, rows, k, env, frame):
+    """HISTORY_SIZE > 2: the kernel logs the terminal FRAME; the terminal row is the env's row before the done step
+    (`rows[k - 1]`, or `prev_rows` -- the rows before the call -- for k = 0) moved on by one frame, then that frame, i.e.
+    the H - 1 frames before the done step with -1 beyond the env's previous reset, as step() / rollout() build rows.
+    prev_rows [N, H*F], rows [K, N, H*F], k / env [n] int64, frame [n, F] -> [n, H*F]."""
+    F = frame.shape[1]
+    before = torch.where((k > 0)[:, None], rows[(k - 1).clamp(min=0), env], prev_rows[env])
+    return torch.cat([before[:, F:], frame], dim=1)
+
+
 class BatchedShipEnv(object):
     """`num_envs` independent ShipEnvs on one GPU.
 
@@ -160,6 +194,8 @@ class BatchedShipEnv(object):
         self.total_steps = 0
         self._state_bound = True
         self.graph_safe = True                 # False: kernel parameters change between launches (no CUDA-graph replay)
+        self._calls = 0                        # shipsim_step / shipsim_step_host calls (mirrors the handle's SHIPSIM_EP_CALL)
+        self._eplog = None                     # episode log: (rows, meta, count, capacity)
         if fresh_maps:
             self.fresh_maps(True)
 
@@ -327,6 +363,7 @@ class BatchedShipEnv(object):
                 fresh = torch.full_like(shifted, -1.0)
                 fresh[:, -_abi.FRAME:] = frame
                 shifted = torch.where(done[:, None], fresh, shifted)
+            self._log_long_terminal(self._hist, shifted[None])
             self._hist = shifted
             obs = shifted.clone()
         return obs, rew, done, {}
@@ -349,7 +386,10 @@ class BatchedShipEnv(object):
             a = None
         if self.history > 2:
             frames, rew, done = self._launch(a, K, None)          # the kernel runs in its one-frame mode
-            return self._long_history_rows(frames, done), rew, done
+            before = self._hist
+            rows = self._long_history_rows(frames, done)
+            self._log_long_terminal(before, rows)
+            return rows, rew, done
         return self._launch(a, K, out)
 
     def _long_history_rows(self, frames, done):
@@ -386,6 +426,7 @@ class BatchedShipEnv(object):
                                  torch.cuda.current_stream(self.device).cuda_stream)
         if rc:
             _abi.check(rc)
+        self._calls += 1
         self.total_steps += K * self.num_envs
         return obs, rew, done
 
@@ -411,6 +452,7 @@ class BatchedShipEnv(object):
         ptr = lambda x: None if x is None else x.ctypes.data    # noqa: E731
         with torch.cuda.device(self.device):
             _abi.check(self.L.shipsim_step_host(self._h, a.ctypes.data, K, ptr(obs), ptr(rew), ptr(done), self._stream()))
+        self._calls += 1
         self.total_steps += K * self.num_envs
         return obs, rew, done
 
@@ -433,6 +475,7 @@ class BatchedShipEnv(object):
             assert ((a >= 0) & (a <= 2)).all(), "%r invalid" % (actions,)
         with torch.cuda.device(self.device):
             _abi.check(self.L.shipsim_step_host(self._h, a.ctypes.data, 1, obs.ctypes.data, rew.ctypes.data, done.ctypes.data, self._stream()))
+        self._calls += 1
         self.total_steps += self.num_envs
         return obs[0], rew[0], done[0].view(np.bool_)
 
@@ -447,6 +490,61 @@ class BatchedShipEnv(object):
         a, b = C.c_int64(), C.c_int64()
         _abi.check(self.L.shipsim_host_traffic(self._h, C.byref(a), C.byref(b)))
         return a.value, b.value
+
+    # ------------------------------------------------------------------------------------------ episode log
+    def enable_episode_log(self, capacity=None, pinned=False):
+        """Record every finished episode (shipsim_episode_log_bind): its terminal observation -- the row an auto_reset=False
+        batch would have returned for the done step, which the auto-reset replaces by the reset row -- why it ended, its
+        return and length.  Read the records with episodes().  `capacity` = records kept between two episodes() calls
+        (default num_envs: one K = 1 step); 0 turns the log off.  `pinned`: rows and metadata in page-locked host memory
+        (written over PCIe by the kernel: a numpy caller reads them after step_np's own wait, with no copy).  Needs
+        auto_reset."""
+        capacity = self.num_envs if capacity is None else int(capacity)
+        self.params_epoch += 1                 # (the buffers' addresses travel in the kernel parameters: captured graphs go stale)
+        if capacity == 0:
+            _abi.check(self.L.shipsim_episode_log_bind(self._h, None, None, 0, None))
+            self._eplog = None
+            return
+        if pinned and self.history > 2:
+            raise ValueError("pinned episode logs need HISTORY_SIZE <= 2 (longer terminal rows are assembled on the device)")
+        where = dict(pin_memory=True) if pinned else dict(device=self.device)
+        rows = torch.zeros(capacity, self._obs_dim_kernel, dtype=torch.float32, **where)
+        meta = torch.zeros(capacity, _abi.EPISODE_META, dtype=torch.int32, **where)
+        count = torch.zeros(1, dtype=torch.int32, device=self.device)
+        with torch.cuda.device(self.device):
+            _abi.check(self.L.shipsim_episode_log_bind(self._h, rows.data_ptr(), meta.data_ptr(), capacity, count.data_ptr()))
+        self._eplog = (rows, meta, count, capacity)
+        if self.history > 2:
+            self._ep_term = torch.full((capacity, self.states_history), -1.0, dtype=torch.float32, device=self.device)
+
+    def _log_long_terminal(self, prev_rows, rows):
+        """HISTORY_SIZE > 2: complete the terminal rows of the records the last launch appended (no host sync)."""
+        if self._eplog is None:
+            return
+        _, meta, count, cap = self._eplog
+        K, N = rows.shape[0], self.num_envs
+        new = (torch.arange(cap, device=self.device) < count) & (meta[:, _abi.EP_CALL] == self._calls - 1)
+        k = meta[:, _abi.EP_K].long().clamp(0, K - 1)
+        env = meta[:, _abi.EP_ENV].long().clamp(0, N - 1)
+        term = long_history_terminal_rows(prev_rows, rows, k, env, self._eplog[0])
+        self._ep_term = torch.where(new[:, None], term, self._ep_term)
+
+    def episodes(self, clear=True):
+        """The records of the episodes that finished since the log was last cleared, as a dict of device tensors sorted by
+        (call, k, env): env, global_env (+ env_id_offset: shard logs concatenate), k (step within the call), call (sequence
+        number of the step call), length, return, terminated, truncated (step cap alone), collision, oob, all_goals, goal,
+        scenario, episode (of the finished episode) and terminal_obs.  `clear` empties the log.  Raises ShipsimError when
+        more episodes finished than the log could hold."""
+        if self._eplog is None:
+            raise _abi.ShipsimError("no episode log: call enable_episode_log() first")
+        rows, meta, count, cap = self._eplog
+        n = int(count.item())                  # (waits for the stream: the records of every launch so far are in place)
+        if clear:
+            count.zero_()
+        if n > cap:
+            raise _abi.ShipsimError("episode log overflow: %d episodes finished, capacity %d: %d records lost" % (n, cap, n - cap))
+        r = self._ep_term[:n] if self.history > 2 else rows[:n].to(self.device)
+        return episode_dict(meta[:n].to(self.device), r, self.cfg.env_id_offset)
 
     # ------------------------------------------------------------------------------------------ stats / state
     def stats_tensor(self, clear=False, out=None):

@@ -41,9 +41,13 @@ class RolloutCollector(object):
     leaves one fused multiply-add per step for the GAE recurrence.  Per step: 7 torch kernels + the env kernel -- or, for
     the reference's own shape (32 -> 64 -> 64 -> 3 | 1), ONE launch of the library's policy kernel (both trunks, heads and
     the Gumbel-max sample: `shipsim_mlp_policy_forward`) + the env kernel.
-    Any other policy module (`forward(obs) -> (logits, value)`) takes the generic per-step path."""
+    Any other policy module (`forward(obs) -> (logits, value)`) takes the generic per-step path.
 
-    def __init__(self, env, policy, T=128, gamma=0.99, lam=0.95, use_graph=True, use_kernel=True):
+    episode_log=True: the env's episode log (BatchedShipEnv.enable_episode_log, room for T * N records: every env-step
+    could end an episode) is emptied at the start of every rollout, inside the graph; episodes() returns the rollout's
+    finished episodes with `t` = the rollout step -- what a PPO loop logs as ep_reward_mean / ep_len_mean."""
+
+    def __init__(self, env, policy, T=128, gamma=0.99, lam=0.95, use_graph=True, use_kernel=True, episode_log=False):
         assert isinstance(env, BatchedShipEnv) and env.history <= 2
         self.env, self.policy, self.T, self.gamma, self.lam = env, policy, int(T), gamma, lam
         N, D, dev = env.num_envs, env.states_history, env.device
@@ -75,6 +79,10 @@ class RolloutCollector(object):
         self._coef = torch.empty(T, N, **f32)
         self._delta = torch.empty(T, N, **f32)
         env.validate_actions = False                            # the range check would need a host sync per step
+        self.episode_log = bool(episode_log)
+        self._call0 = 0                                         # the env's step-call number of the rollout's first launch
+        if self.episode_log:
+            env.enable_episode_log(self.T * N)
         self.obs[0].copy_(env.reset())
         self._seen_reset_epoch = env.reset_epoch
 
@@ -121,6 +129,10 @@ class RolloutCollector(object):
     @torch.no_grad()
     def _collect(self):
         env, T = self.env, self.T
+        if self.episode_log:
+            env._eplog[2].zero_()
+            # (a replayed graph repeats the call numbers of its capture: this value is the capture's, like the records')
+            self._call0 = env._calls
         # categorical sampling by Gumbel-max (no host sync, graph-capturable): the noise of the whole rollout at once
         self._noise.uniform_().clamp_(1e-10, 1.0).log_().neg_().log_().neg_()
         if self._fused:
@@ -171,6 +183,15 @@ class RolloutCollector(object):
             torch.addcmul(self._delta[t], self._coef[t], self.adv[t + 1], out=self.adv[t])
         torch.add(self.adv, self.values[:T], out=self.returns)
 
+    def episodes(self):
+        """The episodes that finished during the last rollout (BatchedShipEnv.episodes), plus `t` = the rollout step at
+        which each ended (0 .. T-1)."""
+        if not self.episode_log:
+            raise RuntimeError("RolloutCollector(episode_log=True) keeps the episode log")
+        ep = self.env.episodes(clear=False)
+        ep["t"] = ep["call"] - self._call0
+        return ep
+
     def collect(self):
         """One rollout; the buffers (obs, actions, logp, values, rewards, dones, adv, returns) hold the result.
         The captured graph freezes the kernel parameters (StepParams travels by value: episode cap, scenario-bank
@@ -195,14 +216,17 @@ class RolloutCollector(object):
                     self._collect()                             # warm-up outside capture (cuBLAS handles, allocator)
                     self.obs[0].copy_(self.obs[self.T])
                 torch.cuda.current_stream(self.env.device).wait_stream(s)
+                call0 = self._call0
                 self._graph = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(self._graph):
                     self._collect()
                     self.obs[0].copy_(self.obs[self.T])         # next rollout continues where this one ended
                 # the capture pass enqueued nothing: only the warm-up rollout ran
                 self.env.total_steps = steps_before + self.T * self.env.num_envs
+                self._graph_call0, self._call0 = self._call0, call0
                 return self
             self._graph.replay()
+            self._call0 = self._graph_call0
             self.env.total_steps += self.T * self.env.num_envs
             return self
         self.obs[0].copy_(self.obs[self.T])
