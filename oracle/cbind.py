@@ -148,7 +148,8 @@ class OracleEnv(object):
 
     def __init__(self, n_envs, bank, W=600.0, H=600.0, speed=10.0, history=2, max_steps=1000, n_beams=10,
                  lidar_spread_deg=90.0, lidar_distance=100.0, seed=0, env_id_offset=0, auto_reset=False,
-                 n_threads=1, pick_base=0, pick_count=0):
+                 n_threads=1, pick_base=0, pick_count=0, ship_w=2.0, ship_h=3.0, mass=5.0, thrust=100.0,
+                 goal_radius=5.0, step_penalty=-0.01, spawn_y=25.0):
         self.L = lib()
         self.n = int(n_envs)
         self.n_threads = n_threads
@@ -157,8 +158,8 @@ class OracleEnv(object):
         self.bank_goals = np.ascontiguousarray(bank["goals"], dtype=np.float64)
         S, _, maxv, _ = self.hull_xy.shape
         self.cfg = _Config(W=W, H=H, dt=0.1 * speed, space_damping=0.4, lidar_spread_deg=lidar_spread_deg,
-                           lidar_distance=lidar_distance, ship_w=2.0, ship_h=3.0, mass=5.0, thrust=100.0,
-                           goal_radius=5.0, step_penalty=-0.01, spawn_y=25.0, seed=seed, env_id_offset=env_id_offset,
+                           lidar_distance=lidar_distance, ship_w=ship_w, ship_h=ship_h, mass=mass, thrust=thrust,
+                           goal_radius=goal_radius, step_penalty=step_penalty, spawn_y=spawn_y, seed=seed, env_id_offset=env_id_offset,
                            max_steps=max_steps, history=history, n_beams=n_beams, auto_reset=int(auto_reset),
                            n_scenarios=S, maxv=maxv, pick_base=int(pick_base), pick_count=int(pick_count))
         self.frame = 6 + n_beams

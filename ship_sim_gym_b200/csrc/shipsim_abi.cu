@@ -274,6 +274,10 @@ static int derive_params(shipsim_handle *h)
         const double mid = start + delta * (kBeams - 1) * 0.5, half = std::fabs(delta) * (kBeams - 1) * 0.5;
         p.fan_cx = (float)std::cos(mid); p.fan_cy = (float)std::sin(mid);
         p.fan_cos = (float)std::cos(half); p.fan_sin = (float)std::sin(half);
+        // A fan of half-width >= 180 degrees covers every direction: the bound of plane_at_pose,
+        // cos(max(0, angle - half)), is then 1.  cos/sin(half) would wrap around and bound it too low (dropping planes
+        // that rays hit), so the cull is switched off: with fan_cos = -1 the bound is 1 (or more) for every plane.
+        if (half >= 3.14159265358979323846) { p.fan_cos = -1.f; p.fan_sin = 0.f; }
     }
     // reach grid: kGridN x kGridN cells over the bounds plus a pad (the ray origin of a live env lies within
     // [0, W + ship extent]); the border cells are unbounded
@@ -296,6 +300,15 @@ extern "C" int shipsim_create(const shipsim_config *cfg, int device, shipsim_t *
     if (!(cfg->dt > 0.f) || !(cfg->bounds_w > 0.f) || !(cfg->bounds_h > 0.f) || !(cfg->lidar_distance > 0.f) || cfg->max_steps < 1
         || cfg->max_steps >= (1 << 22))
         return fail(SHIPSIM_ERR_ARG, "dt, bounds, lidar_distance must be positive and 1 <= max_steps < 2^22");
+    // the ship and goal knobs: a zero mass would give a zero moment and infinite accelerations, a zero scale no hull
+    if (!(cfg->mass > 0.f) || !std::isfinite(cfg->mass) || !(cfg->ship_w > 0.f) || !std::isfinite(cfg->ship_w)
+        || !(cfg->ship_h > 0.f) || !std::isfinite(cfg->ship_h))
+        return fail(SHIPSIM_ERR_ARG, "mass, ship_w and ship_h must be positive and finite");
+    if (!(cfg->goal_radius >= 0.f) || !std::isfinite(cfg->goal_radius))
+        return fail(SHIPSIM_ERR_ARG, "goal_radius must be >= 0 and finite");
+    if (!std::isfinite(cfg->thrust) || !std::isfinite(cfg->lidar_spread_deg) || !std::isfinite(cfg->spawn_y)
+        || !std::isfinite(cfg->step_penalty))
+        return fail(SHIPSIM_ERR_ARG, "thrust, lidar_spread_deg, spawn_y and step_penalty must be finite");
     {
         const int g = cfg->lanes_per_env;
         if (g != 0 && g != 1 && g != 2 && g != 4 && g != 8 && g != 16 && g != 32)

@@ -28,8 +28,25 @@ STRICT_FRAC = 0.99
 M_SAT, M_GOAL, M_OOB, M_TIE, M_RAY0 = 0, 1, 2, 3, 4
 
 
-def random_states(rng, n, W, H, n_scen, bank_goals, max_steps=1000, near=None):
-    """Injected-state distribution of SURVEY.md §8(d)."""
+SHIP_TEMPLATE = np.array([[0.0, 0.0], [0.0, 10.0], [5.0, 15.0], [10.0, 10.0], [10.0, 0.0]])   # models.py:6
+
+
+def ship_hull(ship_w=2.0, ship_h=3.0):
+    """The ship's hull in the body frame: SHIP_TEMPLATE scaled by (ship_w, ship_h) (game.py:275)."""
+    return SHIP_TEMPLATE * np.array([ship_w, ship_h])
+
+
+SHIP_HULL = ship_hull()     # the default ship
+
+
+def _hull_rmax(hull):
+    return float(np.sqrt((hull ** 2).sum(1)).max())
+
+
+def random_states(rng, n, W, H, n_scen, bank_goals, max_steps=1000, near=None, hull=SHIP_HULL):
+    """Injected-state distribution of SURVEY.md §8(d).  With `near`, every other ship is put within a box around a bank
+    vertex whose half width (60 for the default hull) grows with the size of `hull` (the body-frame hull)."""
+    spread = 60.0 * _hull_rmax(hull) / _hull_rmax(SHIP_HULL)
     pose = np.zeros((n, 6))
     pose[:, 0] = rng.uniform(0, W, n)
     pose[:, 1] = rng.uniform(0, H, n)
@@ -51,24 +68,21 @@ def random_states(rng, n, W, H, n_scen, bank_goals, max_steps=1000, near=None):
             s = ints[e, 3]
             b = rng.randint(0, 2)
             v = hull_xy[s, b, rng.randint(0, hull_n[s, b])]
-            pose[e, 0:2] = v + rng.uniform(-60, 60, 2)
+            pose[e, 0:2] = v + rng.uniform(-spread, spread, 2)
     return pose, ints, lidar, goals, ret
 
 
-SHIP_HULL = np.array([[0.0, 0.0], [0.0, 30.0], [10.0, 45.0], [20.0, 30.0], [20.0, 0.0]])     # models.py:6 scaled by (2, 3), game.py:275
-
-
-def lidar_origin_offset(theta):
+def lidar_origin_offset(theta, hull=SHIP_HULL):
     """(hx, hy): half extents of the rotated hull's AABB -- LiDAR.query's origin relative to the body (models.py:51-53)."""
     c, s = np.cos(theta), np.sin(theta)
-    wx = SHIP_HULL[:, 0][None] * c[:, None] - SHIP_HULL[:, 1][None] * s[:, None]
-    wy = SHIP_HULL[:, 0][None] * s[:, None] + SHIP_HULL[:, 1][None] * c[:, None]
+    wx = hull[:, 0][None] * c[:, None] - hull[:, 1][None] * s[:, None]
+    wy = hull[:, 0][None] * s[:, None] + hull[:, 1][None] * c[:, None]
     return 0.5 * (wx.max(1) - wx.min(1)), 0.5 * (wy.max(1) - wy.min(1))
 
 
-def goal_shell_states(rng, n, W, H, n_scen, deltas=(-1e-2, -5e-3, -2e-3, 2e-3, 5e-3, 1e-2)):
+def goal_shell_states(rng, n, W, H, n_scen, deltas=(-1e-2, -5e-3, -2e-3, 2e-3, 5e-3, 1e-2), hull=SHIP_HULL, radius=5.0):
     """Adversarial set "goal at distance r +- eps" (SURVEY.md section 8d): the ship at rest (so the step leaves the pose
-    where it is), goal k of every env placed at distance 5 + delta from the hull -- off an edge or off a vertex."""
+    where it is), goal k of every env placed at distance `radius` + delta from `hull` -- off an edge or off a vertex."""
     pose = np.zeros((n, 6))
     pose[:, 0] = rng.uniform(100, W - 100, n)
     pose[:, 1] = rng.uniform(100, H - 100, n)
@@ -86,36 +100,36 @@ def goal_shell_states(rng, n, W, H, n_scen, deltas=(-1e-2, -5e-3, -2e-3, 2e-3, 5
     c, s = np.cos(pose[:, 2]), np.sin(pose[:, 2])
     for e in range(n):
         j = rng.randint(0, 5)
-        a, b = SHIP_HULL[j - 1], SHIP_HULL[j]
+        a, b = hull[j - 1], hull[j]
         if rng.rand() < 0.5:                           # off the edge a -> b (outward normal of a CCW... the template is CW here)
             t = rng.uniform(0.05, 0.95)
             q = a + t * (b - a)
             ed = (b - a) / np.linalg.norm(b - a)
             nrm = np.array([-ed[1], ed[0]])
-            cen = SHIP_HULL.mean(0)
+            cen = hull.mean(0)
             if np.dot(nrm, q - cen) < 0:
                 nrm = -nrm
         else:                                          # off the vertex b, along the bisector of its outward normals
             q = b
-            nrm = (b - SHIP_HULL.mean(0))
+            nrm = (b - hull.mean(0))
             nrm = nrm / np.linalg.norm(nrm)
             # keep the direction inside the vertex' normal cone: the bisector of the two edge normals
             e0 = (b - a) / np.linalg.norm(b - a)
-            nxt = SHIP_HULL[(j + 1) % 5]
+            nxt = hull[(j + 1) % 5]
             e1 = (nxt - b) / np.linalg.norm(nxt - b)
             n0, n1 = np.array([-e0[1], e0[0]]), np.array([-e1[1], e1[0]])
-            cen = SHIP_HULL.mean(0)
+            cen = hull.mean(0)
             if np.dot(n0, b - cen) < 0:
                 n0, n1 = -n0, -n1
             nrm = (n0 + n1) / np.linalg.norm(n0 + n1)
-        loc = q + nrm * (5.0 + delta[e])
+        loc = q + nrm * (radius + delta[e])
         k = rng.randint(0, 5)
         goals[e, k, 0] = pose[e, 0] + loc[0] * c[e] - loc[1] * s[e]
         goals[e, k, 1] = pose[e, 1] + loc[0] * s[e] + loc[1] * c[e]
     return pose, ints, lidar, goals.reshape(n, 10), np.zeros(n), delta
 
 
-def origin_inside_bank_states(rng, n, hull_xy, hull_n, n_scen):
+def origin_inside_bank_states(rng, n, hull_xy, hull_n, n_scen, hull=SHIP_HULL):
     """Adversarial set "ray origin inside a bank" (App. B Q11): the lidar origin (body origin + half the rotated hull's
     AABB) sits strictly inside one of the env's banks, so every ray reports the full length for that bank."""
     pose = np.zeros((n, 6))
@@ -123,7 +137,7 @@ def origin_inside_bank_states(rng, n, hull_xy, hull_n, n_scen):
     ints = np.zeros((n, 5), dtype=np.int32)
     ints[:, 1] = 31
     ints[:, 3] = rng.randint(0, n_scen, n)
-    hx, hy = lidar_origin_offset(pose[:, 2])
+    hx, hy = lidar_origin_offset(pose[:, 2], hull)
     which = np.zeros(n, dtype=np.int64)
     for e in range(n):
         s = ints[e, 3]
@@ -136,6 +150,62 @@ def origin_inside_bank_states(rng, n, hull_xy, hull_n, n_scen):
         pose[e, 0], pose[e, 1] = pt[0] - hx[e], pt[1] - hy[e]
     lidar = np.where(rng.rand(n, 10) < 0.5, -1.0, rng.uniform(0, 100, (n, 10)))
     return pose, ints, lidar, which
+
+
+# Reach grid of derive_params (shipsim_abi.cu): GRID_N x GRID_N cells over [-GRID_PAD, W + GRID_PAD] x [-GRID_PAD, H + GRID_PAD],
+# looked up at the lidar origin as floor((o + GRID_PAD) * inv_cell) in fp32 and clamped, so the border cells are unbounded.
+GRID_N = 32
+GRID_PAD = 32.0
+
+
+def grid_boundaries(W, H):
+    """Cell boundaries of the reach grid along x and y, float64: -GRID_PAD + i * cell for i = 0 .. GRID_N."""
+    i = np.arange(GRID_N + 1)
+    return -GRID_PAD + i * ((W + 2 * GRID_PAD) / GRID_N), -GRID_PAD + i * ((H + 2 * GRID_PAD) / GRID_N)
+
+
+def grid_cell(o, extent):
+    """The kernel's cell index of lidar-origin coordinates `o` along an axis of length `extent`, in fp32 arithmetic."""
+    inv = np.float32(GRID_N / (extent + 2.0 * GRID_PAD))
+    t = (np.asarray(o, dtype=np.float32) + np.float32(GRID_PAD)) * inv
+    return np.clip(np.floor(t).astype(np.int64), 0, GRID_N - 1)
+
+
+def lidar_origin(pose, hull=SHIP_HULL):
+    hx, hy = lidar_origin_offset(pose[:, 2], hull)
+    return pose[:, 0] + hx, pose[:, 1] + hy
+
+
+GRID_ULPS = (-2, -1, 0, 1, 2)
+
+
+def grid_boundary_states(rng, n, W, H, n_scen, bank_goals, hull=SHIP_HULL, max_steps=1000):
+    """Adversarial set "lidar origin on a reach-grid cell boundary": the origin (body + half the rotated hull's AABB) lies
+    on a boundary, or 1 or 2 fp32 ulps to either side of it, along x, y or both; every boundary is used, the outer ones
+    (the edges of the unbounded border cells) included, and one env in eight has its origin beyond the pad.  Half the
+    ships point straight up, where the offset to the origin is exact in fp32.  Returns random_states' tuple and
+    `target` [n, 2]: the intended ulp offset per axis (a value outside GRID_ULPS = that axis is free)."""
+    pose, ints, lidar, goals, ret = random_states(rng, n, W, H, n_scen, bank_goals, max_steps=max_steps, hull=hull)
+    pose[:, 2] = np.where(rng.rand(n) < 0.5, 0.0, pose[:, 2].astype(np.float32).astype(np.float64))
+    off = lidar_origin_offset(pose[:, 2], hull)
+    bnd = grid_boundaries(W, H)
+    ext = (W, H)
+    target = np.full((n, 2), 99, dtype=np.int64)
+    mode = rng.randint(0, 8, n)                        # 0-2: x, 3-5: y, 6: both, 7: beyond the pad
+    for e in range(n):
+        axes = (0,) if mode[e] < 3 else ((1,) if mode[e] < 6 else ((0, 1) if mode[e] == 6 else ()))
+        for a in axes:
+            k = GRID_ULPS[rng.randint(0, len(GRID_ULPS))]
+            t = np.float32(bnd[a][rng.randint(0, GRID_N + 1)])
+            for _ in range(abs(k)):
+                t = np.nextafter(t, np.float32(np.inf if k > 0 else -np.inf))
+            pose[e, a] = float(t) - off[a][e]
+            target[e, a] = k
+        if mode[e] == 7:
+            a = rng.randint(0, 2)
+            o = -GRID_PAD - rng.uniform(0.5, 40.0) if rng.rand() < 0.5 else ext[a] + GRID_PAD + rng.uniform(0.5, 40.0)
+            pose[e, a] = o - off[a][e]
+    return (pose, ints, lidar, goals, ret), target
 
 
 def f32_inputs(pose, ints, lidar, goals, ret):

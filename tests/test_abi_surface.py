@@ -75,6 +75,16 @@ def test_argument_errors_do_not_need_a_gpu():
     cfg = _abi.default_config()
     cfg.struct_size = 4
     assert lib.shipsim_create(C.byref(cfg), 0, C.byref(h)) == -1
+    # the ship and goal knobs are checked before any device is looked for
+    nan, inf = float("nan"), float("inf")
+    for field, bad in [("mass", 0.0), ("mass", -5.0), ("mass", nan), ("mass", inf), ("ship_w", 0.0), ("ship_w", -2.0),
+                       ("ship_h", 0.0), ("ship_h", nan), ("ship_w", inf), ("goal_radius", -0.5), ("goal_radius", nan),
+                       ("thrust", inf), ("thrust", nan), ("lidar_spread_deg", inf), ("lidar_spread_deg", nan),
+                       ("spawn_y", nan), ("spawn_y", -inf), ("step_penalty", nan)]:
+        cfg = _abi.default_config()
+        setattr(cfg, field, bad)
+        assert lib.shipsim_create(C.byref(cfg), 0, C.byref(h)) == -1, (field, bad)
+        assert field.split("_")[0].encode() in lib.shipsim_last_error(), (field, lib.shipsim_last_error())
     assert lib.shipsim_step(None, None, 0, 1, None, None, None, None) == -1
     assert lib.shipsim_destroy(None) == 0
 

@@ -6,12 +6,18 @@
    segment-vs-convex-polygon (cpPolyShapeSegmentQuery) against Cyrus-Beck clipping, polygon-vs-polygon contact against
    exhaustive edge intersection / containment, point-to-polygon distance against the edge-by-edge minimum.
 The oracle is test infrastructure; nothing here touches the CUDA path."""
+import os
+import re
+
 import numpy as np
 import pytest
 
 import oracle
+import parity
 from oracle import cbind
 from ship_sim_gym_b200 import ScenarioBank
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _env(speed, W=600.0, H=600.0, n=1, seed=0, **kw):
@@ -201,3 +207,153 @@ def test_scenario_picks_are_uniform_and_independent_of_neighbours():
     b = np.array([cbind.pick_scenario(12345 + (1 << 32), g, 3, 1 << 20) for g in range(64)])
     c = np.array([cbind.pick_scenario(12345, g + (1 << 32), 3, 1 << 20) for g in range(64)])
     assert (a != b).mean() > 0.95 and (a != c).mean() > 0.95
+
+
+# ---------------------------------------------------------------------------------------------- the other knobs
+# Appendix D holds the default ship only; the same closed forms hold for every mass, thrust and scale, and they pin the
+# knob-dependent paths of the oracle before the GPU tests use it as the reference for those knobs.
+def _fan_moment(mass, hull):
+    """Moment about the body origin of a uniform polygon, summed over the triangles (0, v_i, v_i+1): each triangle's
+    moment about its centroid, m (a^2 + b^2 + c^2) / 36, moved to the origin by the parallel-axis term m |centroid|^2."""
+    v = np.asarray(hull, dtype=np.float64)
+    w = np.roll(v, -1, axis=0)
+    area = 0.5 * (v[:, 0] * w[:, 1] - v[:, 1] * w[:, 0])
+    rho = mass / area.sum()
+    sides = (v ** 2).sum(1) + (w ** 2).sum(1) + ((w - v) ** 2).sum(1)
+    cen = (v + w) / 3.0
+    m = rho * area
+    return float((m * sides / 36.0 + m * (cen ** 2).sum(1)).sum())
+
+
+@pytest.mark.parametrize("ship_w,ship_h,want", [(2.0, 3.0, 3087.5), (4.0, 5.0, 28112.5 / 3), (0.5, 0.5, None), (1.0, 7.0, None)])
+def test_ship_moment_of_scaled_template(ship_w, ship_h, want):
+    env = _env(10, ship_w=ship_w, ship_h=ship_h, mass=5.0)
+    hull = env.ship_hull()
+    tpl = parity.ship_hull(ship_w, ship_h)
+    assert sorted(map(tuple, hull)) == sorted(map(tuple, tpl))         # the scaled template is its own convex hull
+    assert env.moment == pytest.approx(_fan_moment(5.0, hull), rel=1e-12)
+    if want is not None:
+        assert env.moment == pytest.approx(want, rel=1e-12)
+    env2 = _env(10, ship_w=ship_w, ship_h=ship_h, mass=12.5)
+    assert env2.moment == pytest.approx(env.moment * 2.5, rel=1e-12)   # linear in the mass
+
+
+@pytest.mark.parametrize("mass,thrust", [(5.0, 100.0), (1.5, 400.0), (50.0, 20.0), (0.25, 3.0)])
+@pytest.mark.parametrize("speed", [1, 10])
+def test_straight_thrust_follows_mass_and_thrust(mass, thrust, speed):
+    W = 4000.0
+    env = _env(speed, W, W, mass=mass, thrust=thrust)
+    K = 5
+    out = env.step(np.zeros((K, 1), dtype=np.int32))
+    obs = out["obs"][:, 0, 16:]
+    dt, damp = 0.1 * speed, 0.4 ** (0.1 * speed)
+    v, y, ys = 0.0, 25.0, []
+    for _ in range(K):
+        y += v * dt                                                 # position first (cpBodyUpdatePosition), then velocity
+        v = v * damp + (thrust / mass) * dt
+        ys.append(y)
+    assert np.allclose(obs[:, 1], ys, rtol=1e-12, atol=1e-9)
+    assert np.all(obs[:, 0] == W / 2) and np.all(obs[:, 3] == 0.0)
+    assert env.pose[0, 4] == pytest.approx(v, rel=1e-12) and env.pose[0, 3] == 0.0
+
+
+@pytest.mark.parametrize("ship_w,ship_h,mass,thrust", [(2.0, 3.0, 5.0, 100.0), (4.0, 5.0, 5.0, 100.0), (0.5, 0.5, 1.5, 400.0),
+                                                       (2.0, 3.0, 50.0, 20.0)])
+def test_rudder_then_thrust_turns_by_torque_over_moment(ship_w, ship_h, mass, thrust):
+    env = _env(10, 4000.0, 4000.0, ship_w=ship_w, ship_h=ship_h, mass=mass, thrust=thrust)
+    out = env.step(np.array([[1], [0], [0], [0], [0]], dtype=np.int32))
+    obs = out["obs"][:, 0, 16:]
+    moment = _fan_moment(mass, parity.ship_hull(ship_w, ship_h))
+    dt, damp = 1.0, 0.4
+    w, a, angles = 0.0, 0.0, [0.0]
+    for _ in range(4):
+        a += w * dt
+        w = w * damp + (5.0 * thrust / moment) * dt                 # torque = -rudder * F at rudder -5
+        angles.append(a)
+    assert np.allclose(obs[:, 3], angles, rtol=1e-10, atol=1e-12)
+    assert env.pose[0, 5] == pytest.approx(w, rel=1e-10)
+
+
+@pytest.mark.parametrize("W,H,spawn_y", [(900.0, 400.0, 25.0), (400.0, 1000.0, 25.0), (900.0, 400.0, 300.0), (1000.0, 1000.0, 300.0)])
+def test_reset_observation_follows_bounds_and_spawn(W, H, spawn_y):
+    bank = ScenarioBank.generate(4, (W, H), seed=1).as_dict()
+    env = oracle.OracleEnv(3, bank, W=W, H=H, spawn_y=spawn_y)
+    obs = env.reset(scen=[0, 1, 2])
+    for e in range(3):
+        g = bank["goals"][e]
+        k = np.argmin(np.hypot(g[:, 0] - W / 2, g[:, 1] - spawn_y))
+        want = [-1.0] * 16 + [W / 2, spawn_y, 0.0, 0.0, g[k, 0], g[k, 1]] + [-1.0] * 10
+        assert list(obs[e]) == want
+
+
+@pytest.mark.parametrize("penalty", [-0.01, -0.37, 0.0, 0.25])
+def test_uneventful_step_returns_the_step_penalty(penalty):
+    env = _env(10, step_penalty=penalty)
+    out = env.step(np.array([[1], [2], [1]], dtype=np.int32))      # rudder only: the hull stays at the spawn pose
+    assert np.all(out["reward"] == penalty) and not out["done"].any() and not out["flags"].any()
+    assert env.ep_return[0] == pytest.approx(3 * penalty, abs=1e-15)
+
+
+@pytest.mark.parametrize("radius", [0.5, 5.0, 40.0])
+@pytest.mark.parametrize("ship", [(2.0, 3.0), (4.0, 5.0)])
+def test_goal_taken_exactly_within_the_radius(radius, ship):
+    W = H = 1000.0
+    n = 600
+    hull = parity.ship_hull(*ship)
+    bank = ScenarioBank.generate(8, (W, H), seed=2).as_dict()
+    rng = np.random.RandomState(3)
+    pose, ints, lidar, goals, ret, delta = parity.goal_shell_states(rng, n, W, H, 8, hull=hull, radius=radius)
+    env = oracle.OracleEnv(n, bank, W=W, H=H, goal_radius=radius, ship_w=ship[0], ship_h=ship[1], n_threads=4)
+    parity.load_oracle_state(env, pose, ints, lidar, goals, ret)
+    out = env.step(rng.randint(1, 3, n).astype(np.int32))           # rudder actions: the ship at rest stays put
+    taken = (out["flags"] & oracle.FLAG_GOAL) != 0
+    assert np.array_equal(taken, delta < 0)
+    assert np.all(out["reward"][taken] == 1.0)
+    assert np.allclose(out["margins"][:, parity.M_GOAL], np.abs(delta), rtol=0, atol=1e-9)
+
+
+# ---------------------------------------------------------------------------------------------- reach-grid boundaries
+def _source_constant(path, pattern):
+    with open(os.path.join(ROOT, "ship_sim_gym_b200", "csrc", path)) as f:
+        return float(re.search(pattern, f.read()).group(1))
+
+
+@pytest.mark.parametrize("W,H", [(600.0, 600.0), (900.0, 400.0), (400.0, 1000.0), (4000.0, 4000.0)])
+@pytest.mark.parametrize("ship", [(2.0, 3.0), (4.0, 5.0)])
+def test_grid_boundary_states_straddle_the_cell_boundaries(W, H, ship):
+    """The generator must put lidar origins within the stated ulps of the kernel's reach-grid boundaries: checked
+    against the grid constants of the CUDA source, so that a change of the grid makes this fail instead of leaving the
+    GPU tests that use the generator testing nothing in particular."""
+    assert parity.GRID_N == _source_constant("shipsim_device.cuh", r"constexpr int kGridN = (\d+);")
+    assert parity.GRID_PAD == _source_constant("shipsim_abi.cu", r"const double pad = ([0-9.]+);")
+    hull = parity.ship_hull(*ship)
+    rng = np.random.RandomState(0)
+    n = 6000
+    st, target = parity.grid_boundary_states(rng, n, W, H, 16, np.zeros((16, 5, 2)), hull=hull)
+    pose = parity.f32_inputs(*st)[0]
+    ox, oy = parity.lidar_origin(pose, hull)
+    bnd = parity.grid_boundaries(W, H)
+    beyond = np.zeros(n, dtype=bool)
+    for a, (o, b, ext) in enumerate(((ox, bnd[0], W), (oy, bnd[1], H))):
+        beyond |= (o < -parity.GRID_PAD) | (o > ext + parity.GRID_PAD)
+        on = np.isin(target[:, a], parity.GRID_ULPS)
+        i = np.abs(o[on, None] - b[None]).argmin(1)
+        # the intended origin: the fp32 boundary moved by k ulps; the body coordinate that puts the origin there is
+        # rounded to fp32, which may move it by half an ulp of that coordinate
+        want = b[i].astype(np.float32)
+        for k in (1, 2):
+            for sgn in (1, -1):
+                m = target[on, a] * sgn >= k
+                want[m] = np.nextafter(want[m], np.float32(sgn * np.inf))
+        slack = 0.5 * np.abs(np.spacing(pose[on, a].astype(np.float32))).astype(np.float64)
+        assert np.all(np.abs(o[on] - want.astype(np.float64)) <= slack * (1 + 1e-9))
+        assert set(np.unique(target[on, a])) == set(parity.GRID_ULPS)
+        assert set(np.unique(i)) == set(range(parity.GRID_N + 1))      # every boundary, the outer ones included
+        # at the inner boundaries the kernel's fp32 cell lookup lands on both sides
+        o32 = np.float32(o[on])
+        cell = parity.grid_cell(o32, ext)
+        inner = (i > 0) & (i < parity.GRID_N)
+        assert np.all((cell[inner] == i[inner]) | (cell[inner] == i[inner] - 1))
+        assert (cell[inner] == i[inner]).sum() > 100 and (cell[inner] == i[inner] - 1).sum() > 100
+        assert np.isin(cell, [0, parity.GRID_N - 1]).sum() > 20                # the unbounded border cells
+    assert 0.08 < beyond.mean() < 0.2
