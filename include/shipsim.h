@@ -31,7 +31,8 @@ extern "C" {
 
 #define SHIPSIM_ABI_VERSION 4
 #define SHIPSIM_N_GOALS 5        /* game.py:17  N_GOALS */
-#define SHIPSIM_N_BEAMS 10       /* models.py:29 LiDAR(n_beams=10): the only beam count the reference ever uses */
+#define SHIPSIM_N_BEAMS 10       /* models.py:29 LiDAR(n_beams=10): the only beam count the reference ever uses; the default */
+#define SHIPSIM_MAX_BEAMS 32     /* widest lidar fan (lidar_beams in [1, SHIPSIM_MAX_BEAMS])                               */
 #define SHIPSIM_FRAME 16         /* ship_env.py:43 n_states = 2+1+1+2+n_beams */
 #define SHIPSIM_STATE_PLANES 8   /* float4 planes per env, see shipsim_state_bytes() */
 #define SHIPSIM_MAX_HULL 32      /* max convex-hull vertices per river bank */
@@ -103,7 +104,10 @@ typedef struct shipsim_config {
                                     builds longer histories from the frames                           */
     int32_t auto_reset;          /* 1: a done env is reset inside the step and its obs replaced by the reset
                                     obs (the SubprocVecEnv worker behind train/stable_baselines/ppo.py:123) */
-    int32_t lidar_beams;         /* must be SHIPSIM_N_BEAMS                                          */
+    int32_t lidar_beams;         /* rays of the fan, 1..32 (LidarConfig.N_BEAMS config.py:9 when honoured; default
+                                    SHIPSIM_N_BEAMS).  An observation frame is 6 + lidar_beams floats.  10 runs the tuned
+                                    kernels; any other count the wide serial-in-time kernel: steps_in_flight must then be
+                                    0 or 1 (SHIPSIM_ERR_UNSUPPORTED otherwise)                       */
     float lidar_spread_deg;      /* models.py:29 (90); LidarConfig.ANGULAR_SPREAD config.py:11 when honoured */
     float lidar_distance;        /* models.py:29 (100)                                               */
     float ship_w, ship_h;        /* game.py:275 (2, 3): scale of models.py:6 SHIP_TEMPLATE           */
@@ -180,6 +184,8 @@ int shipsim_set_max_steps(shipsim_t *h, int32_t max_steps);
  *   0: x, y, angle, vx          1: vy, w, episode_return, bits{rudder/5+2 | alive<<3 | step_count<<8}
  *   2: lidar[0..3]              3: lidar[4..7]            4: lidar[8], lidar[9], bits(scenario), bits(episode)
  *   5: goal0.xy, goal1.xy       6: goal2.xy, goal3.xy     7: goal4.xy, 0, 0
+ * (readings past a fan of fewer than 10 beams are unused), then for lidar_beams > 10 ceil((lidar_beams - 10) / 4) more
+ * planes: 8 + q holds lidar[10 + 4q .. 13 + 4q].
  * dev_stats: shipsim_stats_bytes() bytes of scratch for the episode statistics (zeroed by bind). */
 size_t shipsim_state_bytes(const shipsim_t *h);
 size_t shipsim_stats_bytes(const shipsim_t *h);
@@ -188,21 +194,22 @@ int shipsim_bind_state(shipsim_t *h, void *dev_state, void *dev_stats, void *str
 /* Replaces ShipEnv.reset (ship_env.py:171-184) / ShipGame.reset (game.py:260-277).
  * dev_mask: uint8[num_envs], non-zero = reset that env (NULL = all).  dev_scenario: int32[num_envs] scenario
  * ids to use (NULL = Philox(seed, global env id, episode)).  first != 0 restarts the episode counter at 0.
- * dev_obs (optional): float[num_envs][16*history] receives the reset observation of the envs that were reset. */
+ * dev_obs (optional): float[num_envs][(6 + lidar_beams) * history] receives the reset observation of the envs that were
+ * reset: [-1 x (6 + lidar_beams) | x, y, 0, 0, gx, gy, -1 x lidar_beams] for history 2. */
 int shipsim_reset(shipsim_t *h, const uint8_t *dev_mask, const int32_t *dev_scenario, int first, float *dev_obs,
                   void *stream);
 
 /* Replaces ShipEnv.step (ship_env.py:136-156) for all envs, K consecutive steps in ONE launch.
  * dev_actions: [K][num_envs] of `action_dtype`, values in {0,1,2} (Discrete(3), ship_env.py:19; anything else
  * is treated like the decoder's no-op, game.py:152-153 -- range checking is the host layer's AssertionError).
- * Outputs, each [K][num_envs] leading: dev_obs float[..][16*history], dev_reward float, dev_done uint8.
- * Any output pointer may be NULL to skip it. */
+ * Outputs, each [K][num_envs] leading: dev_obs float[..][(6 + lidar_beams) * history] (16-byte aligned for 10 beams, 4-byte
+ * otherwise: the rows are dense), dev_reward float, dev_done uint8.  Any output pointer may be NULL to skip it. */
 int shipsim_step(shipsim_t *h, const void *dev_actions, int action_dtype, int32_t K, float *dev_obs,
                  float *dev_reward, uint8_t *dev_done, void *stream);
 
 /* Episode log.  With auto_reset a done env's observation is replaced by the reset observation; with a log bound, the
  * step kernels first append one record per finished episode: dev_meta[i][SHIPSIM_EPISODE_META] (SHIPSIM_EP_*) and
- * dev_rows[i][16 * history] = exactly the row an auto_reset = 0 launch writes for that env at that step (terminal
+ * dev_rows[i][(6 + lidar_beams) * history] = exactly the row an auto_reset = 0 launch writes for that env at that step (terminal
  * observation; history = the config's 1 or 2).  Slots are reserved with an atomic add on *dev_count (int32, the records
  * appended so far); a record whose slot is >= capacity is not written, but the count keeps counting, so a caller sees
  * the loss.  The caller owns the three buffers (device memory; dev_rows and dev_meta may also be page-locked host
@@ -219,18 +226,20 @@ int shipsim_episode_log_bind(shipsim_t *h, float *dev_rows, int32_t *dev_meta, i
  * call: up to 64 KB of rows with page-locked buffers -- no copies, the kernel works on the caller's (mapped) memory; small
  * calls -- plain copies on `stream`; large ones with HISTORY_SIZE = 2 -- frames compacted on the device (~22 bytes per
  * env-step over PCIe) and expanded into the rows by `host_threads` host threads, optionally with a share of the envs as
- * complete rows by DMA (INTEGRATION.md).  The results are identical bit for bit in every case. */
+ * complete rows by DMA (INTEGRATION.md); the compacted format is that of 10-beam frames, so other fans use the first two
+ * regimes at every size.  host_obs[K][num_envs][(6 + lidar_beams) * history].  The results are identical bit for bit in
+ * every case. */
 int shipsim_step_host(shipsim_t *h, const int32_t *host_actions, int32_t K, float *host_obs, float *host_reward,
                       uint8_t *host_done, void *stream);
 
 /* The host half of shipsim_step_host, exposed for callers that move frames themselves (and for the CPU tests): build
- * HISTORY_SIZE = 2 observation rows (ship_env.py:112-113) from frames.  host_frames holds the frame of the state before
+ * HISTORY_SIZE = 2 observation rows (ship_env.py:112-113) from 10-beam (16-float) frames.  host_frames holds the frame of the state before
  * the first step for every env (num_envs x 16 floats) followed by one 16-float frame per row, rows ordered [step][env];
  * host_obs[row] = [host_frames[row] | host_frames[row + num_envs]], except that where host_cut[row] != 0 (may be NULL)
  * the first half is 16 x -1: the observation ShipEnv.reset returns (ship_env.py:180-184).  Pure host code, no device. */
 int shipsim_assemble_history(float *host_obs, const float *host_frames, const uint8_t *host_cut, int64_t n_rows, int64_t num_envs);
 
-/* The host half of the compacted wire format shipsim_step_host uses for HISTORY_SIZE = 2 (exposed for callers that move
+/* The host half of the compacted wire format shipsim_step_host uses for HISTORY_SIZE = 2 and 10-beam frames (exposed for callers that move
  * the data themselves, and for the CPU tests).  Per env-step a 16-byte record {bits(x), bits(y), bits(angle), word} with
  * word = (rudder / 5 + 2) | reward code << 3 (0 = step penalty, 1 = +1, 2 = -1) | done << 5 | change mask << 8, where bit j
  * of the mask says that slot 4 + j of the frame (gx, gy, lidar 0..9; ship_env.py:108-110) differs from the env's previous
@@ -268,7 +277,7 @@ int shipsim_stats_read(shipsim_t *h, double *dev_out, int clear, void *stream);
 
 /* State injection / extraction for parity tests and checkpointing (SURVEY.md §5: the env has no save/restore in
  * the reference).  Host arrays, row-major: pose[n][6] = x y angle vx vy w; ints[n][5] = rudder, alive_mask,
- * step_count, scenario, episode; lidar[n][10]; goals[n][5][2]; ep_return[n].  Synchronous. */
+ * step_count, scenario, episode; lidar[n][lidar_beams]; goals[n][5][2]; ep_return[n].  Synchronous. */
 int shipsim_set_state(shipsim_t *h, const float *host_pose, const int32_t *host_ints, const float *host_lidar,
                       const float *host_goals, const float *host_ep_return);
 int shipsim_get_state(shipsim_t *h, float *host_pose, int32_t *host_ints, float *host_lidar, float *host_goals,

@@ -13,7 +13,8 @@ LIB_PATH = os.environ.get("SHIPSIM_LIB") or os.path.join(HERE, "libshipsim.so") 
 ACTION_I32, ACTION_I64, ACTION_U8, ACTION_RANDOM = 0, 1, 2, 3
 STATS_LEN = 16
 STAT_NAMES = ("episodes", "return_sum", "length_sum", "goal_steps", "collision", "oob", "timeout", "all_goals", "steps")
-N_GOALS, N_BEAMS, FRAME, STATE_PLANES, MAX_HULL = 5, 10, 16, 8, 32
+N_GOALS, N_BEAMS, FRAME, STATE_PLANES, MAX_HULL = 5, 10, 16, 8, 32       # (N_BEAMS, FRAME: the default 10-beam fan)
+MAX_BEAMS = 32                  # lidar_beams in [1, MAX_BEAMS]; a frame is 6 + lidar_beams floats
 # episode log (shipsim_episode_log_bind): columns of a record's metadata, and the SHIPSIM_END_* bits
 EPISODE_META = 8
 EP_K, EP_ENV, EP_LENGTH, EP_RETURN, EP_END, EP_SCENARIO, EP_EPISODE, EP_CALL = range(8)

@@ -10,7 +10,7 @@ is constructed (`snapshot()`), so later mutation of the class does not reach int
 class LidarConfig(object):
     """config.py:8-11.  The reference never reads it -- LiDAR is built with its constructor defaults
     (10 beams / 90 degrees / 100 units, models.py:29,149-150).  BatchedShipEnv honours it only when asked
-    (`honour_lidar_config=True`); N_BEAMS must stay 10 (the observation is 6 + 10 values per frame)."""
+    (`honour_lidar_config=True`); N_BEAMS may then be 1 to 32 (a frame is 6 + N_BEAMS values)."""
     N_BEAMS = 10
     DISTANCE = 100
     ANGULAR_SPREAD = 180

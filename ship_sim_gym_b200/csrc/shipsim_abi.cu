@@ -269,9 +269,13 @@ static int derive_params(shipsim_handle *h)
     const double deg = 3.14159265358979323846 / 180.0;
     const double delta = ((double)c.lidar_spread_deg / c.lidar_beams) * deg;
     const double start = (90.0 - (double)c.lidar_spread_deg / 2.0) * deg;
+    const int nb = c.lidar_beams;
+    p.n_beams = nb;
     for (int i = 0; i < kBeams; ++i) { p.ray_c[i] = (float)std::cos(start + delta * i); p.ray_s[i] = (float)std::sin(start + delta * i); }
+    for (int i = 0; i < kMaxBeams; ++i) { p.ray_cw[i] = (float)std::cos(start + delta * i); p.ray_sw[i] = (float)std::sin(start + delta * i); }
     {
-        const double mid = start + delta * (kBeams - 1) * 0.5, half = std::fabs(delta) * (kBeams - 1) * 0.5;
+        // the fan-reach cull: the fan's axis and half opening (a single ray: half width 0)
+        const double mid = start + delta * (nb - 1) * 0.5, half = std::fabs(delta) * (nb - 1) * 0.5;
         p.fan_cx = (float)std::cos(mid); p.fan_cy = (float)std::sin(mid);
         p.fan_cos = (float)std::cos(half); p.fan_sin = (float)std::sin(half);
         // A fan of half-width >= 180 degrees covers every direction: the bound of plane_at_pose,
@@ -296,7 +300,7 @@ extern "C" int shipsim_create(const shipsim_config *cfg, int device, shipsim_t *
     if (cfg->history < 1) return fail(SHIPSIM_ERR_ARG, "history_size must be greater than zero");   // ship_env.py:46-47
     if (cfg->host_threads < 0) return fail(SHIPSIM_ERR_ARG, "host_threads must be >= 0");
     if (cfg->history > 2) return fail(SHIPSIM_ERR_UNSUPPORTED, "history > 2 is assembled by the host layer from 1-frame observations");
-    if (cfg->lidar_beams != SHIPSIM_N_BEAMS) return fail(SHIPSIM_ERR_UNSUPPORTED, "lidar_beams must be 10");
+    if (cfg->lidar_beams < 1 || cfg->lidar_beams > kMaxBeams) return fail(SHIPSIM_ERR_ARG, "lidar_beams must be in [1, 32]");
     if (!(cfg->dt > 0.f) || !(cfg->bounds_w > 0.f) || !(cfg->bounds_h > 0.f) || !(cfg->lidar_distance > 0.f) || cfg->max_steps < 1
         || cfg->max_steps >= (1 << 22))
         return fail(SHIPSIM_ERR_ARG, "dt, bounds, lidar_distance must be positive and 1 <= max_steps < 2^22");
@@ -316,6 +320,8 @@ extern "C" int shipsim_create(const shipsim_config *cfg, int device, shipsim_t *
         const int w = cfg->steps_in_flight;
         if (w != 0 && w != 1 && w != 4 && w != 8 && w != 16 && w != 32)
             return fail(SHIPSIM_ERR_ARG, "steps_in_flight must be 0 (auto), 1 (off), 4, 8, 16 or 32");
+        if (w > 1 && cfg->lidar_beams != SHIPSIM_N_BEAMS)
+            return fail(SHIPSIM_ERR_UNSUPPORTED, "steps_in_flight > 1 (the time-parallel kernel) needs lidar_beams = 10");
     }
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(SHIPSIM_ERR_CUDA, "no CUDA device: libshipsim has no CPU fallback");
@@ -347,7 +353,9 @@ extern "C" int shipsim_create(const shipsim_config *cfg, int device, shipsim_t *
         // 128 registers per SM x 148 SMs = 2,368 warps of 32 / T envs); beyond 32,768 envs the serial-in-time kernel
         // is faster.  An explicit lanes_per_env asks for the serial-in-time kernel.
         const int n = cfg->num_envs;
-        h->window = (cfg->lanes_per_env || n > SHIPSIM_WINDOW_AUTO_MAX_ENVS) ? 1 : (n <= 2368 ? 32 : (n <= 4736 ? 16 : 8));
+        // Fans other than 10 beams have no time-parallel kernel: the serial-in-time one runs them at every size.
+        h->window = (cfg->lanes_per_env || n > SHIPSIM_WINDOW_AUTO_MAX_ENVS || cfg->lidar_beams != SHIPSIM_N_BEAMS)
+                        ? 1 : (n <= 2368 ? 32 : (n <= 4736 ? 16 : 8));
     }
     *out = h;
     return SHIPSIM_OK;
@@ -676,7 +684,10 @@ extern "C" int shipsim_set_max_steps(shipsim_t *h, int32_t max_steps)
     return SHIPSIM_OK;
 }
 
-extern "C" size_t shipsim_state_bytes(const shipsim_t *h) { return h ? (size_t)h->cfg.num_envs * kPlanes * sizeof(float4) : 0; }
+static int state_planes(const shipsim_t *h) { return kPlanes + extra_lidar_planes(h->cfg.lidar_beams); }
+static int frame_floats(const shipsim_t *h) { return 6 + h->cfg.lidar_beams; }      // ShipEnv.n_states (ship_env.py:43)
+
+extern "C" size_t shipsim_state_bytes(const shipsim_t *h) { return h ? (size_t)h->cfg.num_envs * state_planes(h) * sizeof(float4) : 0; }
 extern "C" size_t shipsim_stats_bytes(const shipsim_t *) { return (size_t)kStatSlots * kStatLen * sizeof(double); }
 
 extern "C" int shipsim_bind_state(shipsim_t *h, void *dev_state, void *dev_stats, void *stream)
@@ -738,7 +749,7 @@ extern "C" int shipsim_episode_log_bind(shipsim_t *h, float *dev_rows, int32_t *
     p.log_meta = (int4 *)device_alias(dev_meta);
     p.log_count = (int *)dev_count;
     p.log_cap = capacity;
-    p.log_row4 = 4 * h->cfg.history;
+    p.log_row4 = 4 * h->cfg.history;         // (the wide kernel's rows are dense: (6 + lidar_beams) * history floats)
     return SHIPSIM_OK;
 }
 
@@ -750,7 +761,9 @@ static int step_impl(shipsim_t *h, const void *dev_actions, int action_dtype, in
     if (K < 1) return fail(SHIPSIM_ERR_ARG, "K must be >= 1");
     if (action_dtype < 0 || action_dtype > 3) return fail(SHIPSIM_ERR_ARG, "bad action_dtype");
     if (action_dtype != SHIPSIM_ACTION_RANDOM && !dev_actions) return fail(SHIPSIM_ERR_ARG, "dev_actions is NULL");
-    if ((uintptr_t)dev_obs & 15) return fail(SHIPSIM_ERR_ARG, "dev_obs must be 16-byte aligned");
+    // (the tuned 10-beam kernel stores rows as float4; the wide kernel's rows are dense floats)
+    if ((uintptr_t)dev_obs & (h->cfg.lidar_beams == SHIPSIM_N_BEAMS ? 15 : 3))
+        return fail(SHIPSIM_ERR_ARG, h->cfg.lidar_beams == SHIPSIM_N_BEAMS ? "dev_obs must be 16-byte aligned" : "dev_obs must be 4-byte aligned");
     DeviceGuard g(h->device);
     {
         const int rcf = fresh_tick(h, K, (cudaStream_t)stream);
@@ -801,7 +814,8 @@ extern "C" int shipsim_step_host(shipsim_t *h, const int32_t *host_actions, int3
     // Tiny calls with page-locked buffers (the gym facade: one env, one step): no copies at all -- the kernel reads the
     // actions from the caller's memory and writes rows, rewards and done flags straight into it (mapped pinned memory;
     // a few hundred bytes over PCIe), one launch and one wait.
-    if (n * kFrame * h->cfg.history * sizeof(float) <= ((size_t)1 << 16) && host_obs && host_reward && host_done) {
+    const size_t F = (size_t)frame_floats(h);                       // floats per frame
+    if (n * F * h->cfg.history * sizeof(float) <= ((size_t)1 << 16) && host_obs && host_reward && host_done) {
         auto mapped = [&](const void *ptr, void **dev) {
             cudaPointerAttributes attr{};
             const bool ok = cudaPointerGetAttributes(&attr, ptr) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer;
@@ -826,19 +840,20 @@ extern "C" int shipsim_step_host(shipsim_t *h, const int32_t *host_actions, int3
             const int rc2 = step_impl(h, da, SHIPSIM_ACTION_I32, K, (float *)dobs, (float *)dr, (uint8_t *)dd, stream, h->cfg.history);
             if (rc2) return rc2;
             h->last_h2d = (int64_t)(n * sizeof(int32_t));
-            h->last_d2h = (int64_t)(n * (kFrame * h->cfg.history * sizeof(float) + 5));
+            h->last_d2h = (int64_t)(n * (F * h->cfg.history * sizeof(float) + 5));
             CU(cudaStreamSynchronize((cudaStream_t)stream));
             return SHIPSIM_OK;
         }
     }
-    const bool frames_only = h->cfg.history == 2 && host_obs != nullptr && !small;
+    // (the compacted wire format is that of 16-float frames: other fans take the plain copies)
+    const bool frames_only = h->cfg.history == 2 && host_obs != nullptr && !small && h->cfg.lidar_beams == SHIPSIM_N_BEAMS;
     int nd = 0;                                                      // envs [0, nd) by DMA (frames_only)
     bool adaptive = false;
     if (K > h->stage_K) {
         cudaFree(h->d_act); cudaFree(h->d_obs); cudaFree(h->d_rew); cudaFree(h->d_done);
         h->d_act = nullptr; h->d_obs = nullptr; h->d_rew = nullptr; h->d_done = nullptr; h->stage_K = 0;
         CU(cudaMalloc(&h->d_act, n * sizeof(int32_t)));
-        CU(cudaMalloc(&h->d_obs, n * kFrame * h->cfg.history * sizeof(float)));
+        CU(cudaMalloc(&h->d_obs, n * F * h->cfg.history * sizeof(float)));
         CU(cudaMalloc(&h->d_rew, n * sizeof(float)));
         CU(cudaMalloc(&h->d_done, n));
         h->stage_K = K;
@@ -938,7 +953,7 @@ extern "C" int shipsim_step_host(shipsim_t *h, const int32_t *host_actions, int3
     h->last_d2h = 0;
     // The rollout is cut into chunks of steps: while chunk i+1 is being computed on the caller's stream, the results
     // of chunk i travel to the host on the copy stream and chunk i-1 is being expanded by the host threads.
-    const size_t row_full = (size_t)kFrame * h->cfg.history;        // floats per complete row; chunk regions of d_obs are sized for it
+    const size_t row_full = F * h->cfg.history;                     // floats per complete row; chunk regions of d_obs are sized for it
     float *d_var = h->d_var;
     if (const char *ev = std::getenv("SHIPSIM_HOST_VAR_DENSITY")) h->var_density = atof(ev);      // (test hook: 0 forces the fetch-the-rest path)
     size_t spec[shipsim_handle::kMaxChunks] = {};                    // floats of each chunk's value stream copied down unasked
@@ -1204,9 +1219,13 @@ extern "C" int shipsim_set_state(shipsim_t *h, const float *pose, const int32_t 
     if (rc) return rc;
     if (!pose || !ints || !lidar || !goals || !ep_return) return fail(SHIPSIM_ERR_ARG, "NULL argument");
     const size_t N = (size_t)h->cfg.num_envs;
-    std::vector<float4> st(N * kPlanes);
+    const int nb = h->cfg.lidar_beams, planes = state_planes(h);
+    std::vector<float4> st(N * planes);
     for (size_t e = 0; e < N; ++e) {
-        const float *q = pose + e * 6, *l = lidar + e * 10, *gl = goals + e * 10;
+        // lidar[e][lidar_beams]; readings past the fan (planes 2-4 of a fan of fewer than 10 beams) hold -1
+        float l[kBeams + 4 * ((kMaxBeams - kBeams) / 4 + 1)];
+        for (int j = 0; j < (int)(sizeof(l) / sizeof(l[0])); ++j) l[j] = j < nb ? lidar[e * nb + j] : -1.f;
+        const float *q = pose + e * 6, *gl = goals + e * 10;
         const int32_t *in = ints + e * 5;
         if (in[0] % 5 != 0 || in[0] < -10 || in[0] > 10) return fail(SHIPSIM_ERR_ARG, "rudder must be in {-10,-5,0,5,10}");
         if (in[3] < 0 || in[3] >= h->p.n_scen) return fail(SHIPSIM_ERR_ARG, "scenario id out of range");
@@ -1221,6 +1240,10 @@ extern "C" int shipsim_set_state(shipsim_t *h, const float *pose, const int32_t 
         st[5 * N + e] = make_float4(gl[0], gl[1], gl[2], gl[3]);
         st[6 * N + e] = make_float4(gl[4], gl[5], gl[6], gl[7]);
         st[7 * N + e] = make_float4(gl[8], gl[9], 0.f, 0.f);
+        for (int pl = kPlanes; pl < planes; ++pl) {
+            const float *x = l + kBeams + 4 * (pl - kPlanes);
+            st[pl * N + e] = make_float4(x[0], x[1], x[2], x[3]);
+        }
     }
     DeviceGuard g(h->device);
     CU(cudaDeviceSynchronize());
@@ -1233,7 +1256,8 @@ extern "C" int shipsim_get_state(shipsim_t *h, float *pose, int32_t *ints, float
     const int rc = ready(h);
     if (rc) return rc;
     const size_t N = (size_t)h->cfg.num_envs;
-    std::vector<float4> st(N * kPlanes);
+    const int nb = h->cfg.lidar_beams, planes = state_planes(h);
+    std::vector<float4> st(N * planes);
     DeviceGuard g(h->device);
     CU(cudaDeviceSynchronize());
     CU(cudaMemcpy(st.data(), h->p.state, st.size() * sizeof(float4), cudaMemcpyDeviceToHost));
@@ -1245,7 +1269,15 @@ extern "C" int shipsim_get_state(shipsim_t *h, float *pose, int32_t *ints, float
         if (pose) { float *q = pose + e * 6; q[0] = a.x; q[1] = a.y; q[2] = a.z; q[3] = a.w; q[4] = b.x; q[5] = b.y; }
         if (ep_return) ep_return[e] = b.z;
         if (ints) { int32_t *in = ints + e * 5; in[0] = ((bits & 7) - 2) * 5; in[1] = (bits >> 3) & 31; in[2] = bits >> 8; in[3] = scen; in[4] = ep; }
-        if (lidar) { float *l = lidar + e * 10; l[0] = l0.x; l[1] = l0.y; l[2] = l0.z; l[3] = l0.w; l[4] = l1.x; l[5] = l1.y; l[6] = l1.z; l[7] = l1.w; l[8] = l2.x; l[9] = l2.y; }
+        if (lidar) {
+            float l[kBeams + 4 * ((kMaxBeams - kBeams) / 4 + 1)] = {l0.x, l0.y, l0.z, l0.w, l1.x, l1.y, l1.z, l1.w, l2.x, l2.y};
+            for (int pl = kPlanes; pl < planes; ++pl) {
+                const float4 x = st[pl * N + e];
+                float *d = l + kBeams + 4 * (pl - kPlanes);
+                d[0] = x.x; d[1] = x.y; d[2] = x.z; d[3] = x.w;
+            }
+            std::memcpy(lidar + e * nb, l, nb * sizeof(float));
+        }
         if (goals) { float *gl = goals + e * 10; gl[0] = g0.x; gl[1] = g0.y; gl[2] = g0.z; gl[3] = g0.w; gl[4] = g1.x; gl[5] = g1.y; gl[6] = g1.z; gl[7] = g1.w; gl[8] = g2.x; gl[9] = g2.y; }
     }
     return SHIPSIM_OK;

@@ -18,7 +18,8 @@
 namespace shipsim {
 
 constexpr int kGoals = 5;
-constexpr int kBeams = 10;
+constexpr int kBeams = 10;         // the reference's fan: the tuned kernels' compile-time beam count
+constexpr int kMaxBeams = 32;      // widest fan (one warp lane per ray)
 constexpr int kFrame = 16;
 constexpr int kPlanes = 8;
 constexpr int kShipVerts = 5;
@@ -106,7 +107,14 @@ struct StepParams {
     int log_cap, log_row4;                           // log_row4 = float4 per record row (4 * the config's history)
     int log_k0;                                      // added to the step index (the chunk offset of shipsim_step_host)
     int log_call;                                    // sequence number of the step call
+    // lidar fans other than the reference's 10 beams (the wide step kernel; appended so that the fields above keep their
+    // parameter offsets in the tuned kernels)
+    int n_beams;                                     // 1 .. kMaxBeams
+    float ray_cw[kMaxBeams], ray_sw[kMaxBeams];      // the whole fan's ray table (entries past n_beams: unused)
 };
+
+// State planes [kPlanes, kPlanes + extra_lidar_planes(n)) hold lidar[10 .. n-1], four readings per plane.
+__host__ __device__ __forceinline__ int extra_lidar_planes(int n_beams) { return n_beams > kBeams ? (n_beams - kBeams + 3) / 4 : 0; }
 
 // SHIPSIM_END_* (include/shipsim.h)
 constexpr int kEndCollision = 1, kEndAllGoals = 2, kEndOob = 4, kEndTimeout = 8, kEndGoal = 16;

@@ -307,4 +307,35 @@ static __device__ __noinline__ void ray_query_serial(const StepParams &p, const 
     }
 }
 
+// The same query for a fan of p.n_beams rays (the wide step kernel), ray by ray: the planes are evaluated again for
+// every ray (the same arithmetic on the same inputs, so every ray sees exactly the values the loop above would), which
+// keeps no per-ray array -- 32 of them would live in local memory.  Per ray: the first bank (list order) that is hit or
+// holds the origin decides; within a bank the last accepted plane wins.
+static __device__ __noinline__ void ray_query_serial_wide(const StepParams &p, const float4 *row, float *lid)
+{
+    const float L = p.lidar_len;
+    const float4 h = row[0], a = row[1], b4 = row[2];
+    const float c = h.x, s = h.y;
+    const int scen = __float_as_int(b4.x);
+    const unsigned masks[2] = {__float_as_uint(b4.y), __float_as_uint(b4.z)};
+    const unsigned flags = __float_as_uint(b4.w);
+    const EdgeD *E = p.edges_d + (size_t)scen * (2 * kMaxHull);
+    for (int j = 0; j < p.n_beams; ++j) {
+        float dirx, diry;
+        ray_dir(c, s, p.ray_cw[j], p.ray_sw[j], dirx, diry);
+        for (int b = 0; b < 2; ++b) {
+            bool out = false, hit = false;
+            float v = 0.f;
+            for (unsigned m = masks[b]; m; m &= m - 1u) {
+                const PlaneEval pe = eval_plane(E + b * kMaxHull + (__ffs(m) - 1), a.x, a.y, a.z, a.w);
+                out = out || (pe.d > 0.f);
+                float val;
+                if (ray_vs_plane(pe.d, pe.ta, __fmul_rn(-L, pe.nx), __fmul_rn(-L, pe.ny), pe.len, dirx, diry, L, val)) { v = val; hit = true; }
+            }
+            if (((flags >> b) & 1u) && !out) { lid[j] = L; break; }
+            if (hit) { lid[j] = v; break; }
+        }
+    }
+}
+
 }  // namespace shipsim

@@ -14,6 +14,8 @@
 #include "shipsim_geom.cuh"
 #include "shipsim_launch.h"
 
+#include <atomic>
+
 #ifndef SHIPSIM_MIN_BLOCKS
 #define SHIPSIM_MIN_BLOCKS 4
 #endif
@@ -54,15 +56,49 @@ constexpr float kDeadGoal = 3.0e19f;        // coordinate of a goal that has bee
 // in their registers.)
 // LOG: write the episode log (shipsim_episode_log_bind).  The log-free kernel is a separate instantiation: its registers
 // and spills are those of the kernel before the log existed (-Xptxas -v).
-template <int G, int HIST, int MINB, int THREADS, bool LOG>
+// NB: lidar capacity.  kBeams (10) is the tuned kernel of the reference's fan, with the beam count a compile-time constant;
+// kMaxBeams (32) is the wide kernel: a 32-reading frame slot, p.n_beams (1..32) rays at run time, and its shared memory
+// allocated dynamically (StepLayout::BYTES; the G = 1 blocks exceed the 48 KB of a static allocation).  Everything else --
+// physics, goals, SAT, reward / done, reset, statistics, episode log -- is this one body of code for both.
+template <int G, int HIST, int NB, int THREADS>
+struct StepLayout {
+    static constexpr bool WIDE = NB != kBeams;
+    static constexpr int EPW = 32 / G;                      // envs per warp
+    static constexpr int FR4 = WIDE ? 10 : 4;               // float4 per frame slot: 6 + NB floats, rounded up
+    static constexpr int OBS4 = FR4 * HIST;                 // float4 per tile row
+    static constexpr int RAW = OBS4 + kScr4 + 3;
+    static constexpr int EB4 = (RAW + (G > 1 ? 2 * kMaxCand : 0)) | 1;
+    static constexpr int WX4 = EPW * EB4;
+    static constexpr int RAYN = WIDE ? kMaxBeams : kBeams;  // ray table entries
+    static constexpr int WB4 = WX4 + 4 + RAYN / 2;
+    static constexpr int BYTES = THREADS / 32 * WB4 * 16;
+};
+
+template <int G, int HIST, int NB, int THREADS>
+__device__ __forceinline__ float4 *step_smem()
+{
+    if constexpr (NB == kBeams) {
+        __shared__ float4 smem[StepLayout<G, HIST, NB, THREADS>::BYTES / 16];
+        return smem;
+    } else {
+        extern __shared__ float4 smem_dyn[];
+        return smem_dyn;
+    }
+}
+
+template <int G, int HIST, int MINB, int THREADS, bool LOG, int NB>
 __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_constant__ StepParams p)
 {
+    using LY = StepLayout<G, HIST, NB, THREADS>;
+    constexpr bool WIDE = LY::WIDE;
     constexpr int EPW = 32 / G;                 // envs per warp
-    constexpr int OBS4 = 4 * HIST;              // float4 per obs row
+    constexpr int FR4 = LY::FR4;                // float4 per frame slot
+    constexpr int OBS4 = LY::OBS4;              // float4 per tile row
+    constexpr int NF = OBS4 - FR4;              // float4 index of the newest frame inside the tile row
     // ray pass: two passes (six envs) per loop trip in the 128-register build (grids that do not fill the machine are
     // latency bound: +4 % on the hard map at 65,536 envs); the 96-register build has no room for it (-1 % at 1M envs)
     constexpr int kRayPassUnroll = MINB * THREADS <= 512 ? 2 : 1;       // (512 threads per SM = the 128-register builds)
-    constexpr int CF = 16 * (HIST - 1);         // float offset of the newest frame inside the tile row
+    constexpr int CF = 4 * NF;                  // float offset of the newest frame inside the tile row
     constexpr int NW = THREADS / 32;
     // env block: [0, OBS4) tile row = [older frame | newest frame] (lidar slots = the sticky readings);
     // [SCR, SCR + kScr4) plane row; [GOL, GOL + 3) goals (taken goals hold kDeadGoal)
@@ -70,16 +106,19 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
     // [RAW, RAW + 2 * kMaxCand): raw candidate-plane records (cp.async targets) -- only with G > 1 (few envs per CTA),
     // where they are requested at the top of the iteration; with G = 1 that would cost 16 KB, so they land in the plane
     // row itself once the ray pass has finished with it
-    constexpr int RAW = GOL + 3;
-    constexpr int EB4 = (RAW + (G > 1 ? 2 * kMaxCand : 0)) | 1;
-    // warp block: the env blocks, then 2 float4 of ray-pass list, 2 of statistics, 5 of ray directions (cos[10], sin[10])
-    constexpr int WX4 = EPW * EB4;
+    constexpr int RAW = LY::RAW;
+    constexpr int EB4 = LY::EB4;
+    // warp block: the env blocks, then 2 float4 of ray-pass list, 2 of statistics, RAYN / 2 of ray directions
+    // (cos[RAYN], sin[RAYN])
+    constexpr int WX4 = LY::WX4;
+    constexpr int RAYN = LY::RAYN;
     constexpr int SRC = WX4, STA = WX4 + 2, RAY = WX4 + 4;
-    constexpr int WB4 = WX4 + 9;
+    constexpr int WB4 = LY::WB4;
     // the last float4 of an env block exists only to make the stride odd: it is the landing slot of fetch_cell_async
     constexpr int CEL = EB4 - 1;
     static_assert(CEL >= RAW + (G > 1 ? 2 * kMaxCand : 0), "the cell slot must not overlap the block's contents");
-    __shared__ float4 smem[NW * WB4];
+    float4 *const smem = step_smem<G, HIST, NB, THREADS>();
+    const int nb = WIDE ? p.n_beams : kBeams;  // rays of the fan
 
     // Everything a lane needs to find its data -- lane, warp, shared-memory offsets, output indices -- follows from ONE
     // value, the env index e, by a mask, a shift or a multiply-add; e itself is laundered (a shuffle from the own lane:
@@ -107,9 +146,9 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
 #define WA(env, i) (wb + (unsigned)(env) * (EB4 * 16u) + 16u * (unsigned)(i))
     const float L = p.lidar_len;
 
-    if (lane < kBeams) {                                            // ray direction table (body frame), one per warp
-        sts1(wb + RAY * 16 + 4 * lane, p.ray_c[lane]);
-        sts1(wb + RAY * 16 + 40 + 4 * lane, p.ray_s[lane]);
+    if (lane < RAYN) {                                              // ray direction table (body frame), one per warp
+        sts1(wb + RAY * 16 + 4 * lane, WIDE ? p.ray_cw[lane] : p.ray_c[lane]);
+        sts1(wb + RAY * 16 + 4 * RAYN + 4 * lane, WIDE ? p.ray_sw[lane] : p.ray_s[lane]);
     }
     if (lane < 8) sts1(wb + STA * 16 + 4 * lane, 0.f);
     if (!valid && gl == 0) sts4(EA(SCR), make_float4(1.f, 0.f, 0.f, 0.f));      // idle groups: a defined heading for the shadow lanes
@@ -131,10 +170,14 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
             // the only things that touch them)
             sts4(EA(GOL + 2), make_float4(g[4].x, g[4].y, __int_as_float(r.alive), __int_as_float(r.episode)));
             // newest frame of the resident tile = frame of the current state
-            sts4(EA(OBS4 - 4), make_float4(r.x, r.y, (float)r.rudder, r.th));
-            sts4(EA(OBS4 - 3), make_float4(gx, gy, l0.x, l0.y));
-            sts4(EA(OBS4 - 2), make_float4(l0.z, l0.w, l1.x, l1.y));
-            sts4(EA(OBS4 - 1), make_float4(l1.z, l1.w, l2.x, l2.y));
+            sts4(EA(NF), make_float4(r.x, r.y, (float)r.rudder, r.th));
+            sts4(EA(NF + 1), make_float4(gx, gy, l0.x, l0.y));
+            sts4(EA(NF + 2), make_float4(l0.z, l0.w, l1.x, l1.y));
+            sts4(EA(NF + 3), make_float4(l1.z, l1.w, l2.x, l2.y));
+            if (WIDE) {                         // lidar[10 ..] from the appended state planes: float4 q of them = tile float4 NF + 4 + q
+                const int nx = extra_lidar_planes(nb);
+                for (int q = 0; q < nx; ++q) sts4(EA(NF + 4 + q), p.state[(size_t)(kPlanes + q) * p.N + (valid ? e : p.N - 1)]);
+            }
         }
     }
     float c, s, hx, hy;
@@ -160,12 +203,19 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
             // previous frame <- newest frame of the last step / reset (SURVEY.md App. A note N2); lidar stays in place
             if (SHIPSIM_TMA_STORE && k > 0) bulk_store_wait_read();      // last step's row has left the tile: it may be rewritten
             if (HIST == 2 && gl == 0) {
-                const float4 f0 = lds4(EA(4)), f1 = lds4(EA(5)), f2 = lds4(EA(6)), f3 = lds4(EA(7));
-                sts4(EA(0), f0); sts4(EA(1), f1); sts4(EA(2), f2); sts4(EA(3), f3);
+                if (!WIDE) {
+                    const float4 f0 = lds4(EA(4)), f1 = lds4(EA(5)), f2 = lds4(EA(6)), f3 = lds4(EA(7));
+                    sts4(EA(0), f0); sts4(EA(1), f1); sts4(EA(2), f2); sts4(EA(3), f3);
+                } else {                        // the float4 that hold the 6 + n values of a frame
+                    const int f4 = (6 + nb + 3) >> 2;
+#pragma unroll
+                    for (int i = 0; i < FR4; ++i) if (i < f4) sts4(EA(i), lds4(EA(FR4 + i)));
+                }
             }
 
             // ---- LiDAR.query (models.py:39-76) at the PRE-integration pose (game.py:193 precedes :194): the plane
-            // rows hold that pose's planes.  Up to three needy envs per pass, lanes 0-9 / 10-19 / 20-29 = their rays.
+            // rows hold that pose's planes.  Up to three needy envs per pass, lanes 0-9 / 10-19 / 20-29 = their rays
+            // (the wide kernel: 32 / n envs per pass, lanes [n * slot, n * slot + n) = the rays of slot `slot`).
             const float4 h0 = lds4(EA(SCR));    // header of the pose the step starts from: its trig, and what its lidar needs
             const int hz_own = __float_as_int(h0.z);
             const bool big = leader && (hz_own & kHdrBig);
@@ -174,18 +224,20 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
             if (HIST == 2) __syncwarp();        // the frame copy has read the old readings before any lane overwrites them
             if (big) {                          // (rare: generic pointers are good enough)
                 float4 *blk = smem + ((e / EPW) & (NW - 1)) * WB4 + grp * EB4;
-                ray_query_serial(p, blk + SCR, reinterpret_cast<float *>(blk) + CF + 6);
+                if (WIDE) ray_query_serial_wide(p, blk + SCR, reinterpret_cast<float *>(blk) + CF + 6);
+                else ray_query_serial(p, blk + SCR, reinterpret_cast<float *>(blk) + CF + 6);
             }
             if (need) {
                 // needy envs, compacted: entry q of the warp's list = the env slot of the q-th needy env
                 if (wants) sts_u8(wb + SRC * 16 + __popc(need & ((1u << lane) - 1u)), (unsigned)grp);
                 __syncwarp();
                 const int cnt = __popc(need);
-                const int rslot = lane / kBeams, rj = lane - rslot * kBeams;    // env slot 0..2 of the pass (lanes 30, 31 idle), ray
-                const float ray_c = lds1(wb + RAY * 16 + 4 * rj), ray_s = lds1(wb + RAY * 16 + 40 + 4 * rj);     // (lanes of a ray: broadcast)
+                const int rslot = lane / nb, rj = lane - rslot * nb;        // env slot 0..2 of the pass (lanes 30, 31 idle), ray
+                const int rpp = WIDE ? 32 / nb : 3;                         // envs per pass
+                const float ray_c = lds1(wb + RAY * 16 + 4 * rj), ray_s = lds1(wb + RAY * 16 + 4 * RAYN + 4 * rj);     // (lanes of a ray: broadcast)
 #pragma unroll kRayPassUnroll
-                for (int q = rslot; q < cnt; q += 3) {          // lanes 30, 31 (rslot 3) only keep the others company
-                    if (rslot < 3) {
+                for (int q = rslot; q < cnt; q += rpp) {        // lanes 30, 31 (rslot 3) only keep the others company
+                    if (rslot < rpp) {
                         const unsigned ra = WA(lds_u8(wb + SRC * 16 + q), 0);      // the env's block
                         const float4 hdr = lds4(ra + SCR * 16);
                         float dirx, diry;
@@ -215,7 +267,7 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
             // ---- ShipGame.handle_discrete_action (game.py:140-153); Ship.move_forward / rotate (models.py:129-146)
             // The rudder angle lives in the tile, as the third value of the newest frame (exact: a small integer in fp32).
             float dvx = 0.f, dvy = 0.f, dw = 0.f;
-            const unsigned rud_slot = EA(OBS4 - 4) + 8;
+            const unsigned rud_slot = EA(NF) + 8;
             const float rud = lds1(rud_slot);
             if (G > 1) __syncwarp();            // every lane has the old angle before the leader stores the new one
             if (a == 0) {                       // thrust along the heading the step starts from
@@ -402,13 +454,24 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
                 if (lm) {
                     const unsigned slot = log_reserve(p, lane, lm);
                     if (leader && done && slot < (unsigned)p.log_cap) {
-                        float4 *row = p.log_rows + (size_t)slot * p.log_row4 + (p.log_row4 - OBS4);
-                        if (HIST == 2) { row[0] = lds4(EA(0)); row[1] = lds4(EA(1)); row[2] = lds4(EA(2)); row[3] = lds4(EA(3)); }
-                        const float4 f1 = lds4(EA(OBS4 - 3));
-                        row[OBS4 - 4] = make_float4(r.x, r.y, lds1(EA(OBS4 - 4) + 8), r.th);
-                        row[OBS4 - 3] = make_float4(gx, gy, f1.z, f1.w);
-                        row[OBS4 - 2] = lds4(EA(OBS4 - 2));
-                        row[OBS4 - 1] = lds4(EA(OBS4 - 1));
+                        if (!WIDE) {
+                            float4 *row = p.log_rows + (size_t)slot * p.log_row4 + (p.log_row4 - OBS4);
+                            if (HIST == 2) { row[0] = lds4(EA(0)); row[1] = lds4(EA(1)); row[2] = lds4(EA(2)); row[3] = lds4(EA(3)); }
+                            const float4 f1 = lds4(EA(OBS4 - 3));
+                            row[OBS4 - 4] = make_float4(r.x, r.y, lds1(EA(OBS4 - 4) + 8), r.th);
+                            row[OBS4 - 3] = make_float4(gx, gy, f1.z, f1.w);
+                            row[OBS4 - 2] = lds4(EA(OBS4 - 2));
+                            row[OBS4 - 1] = lds4(EA(OBS4 - 1));
+                        } else {                // dense rows of (6 + n) * HIST floats
+                            const int F = 6 + nb;
+                            float *row = reinterpret_cast<float *>(p.log_rows) + (size_t)slot * (F * HIST);
+                            if (HIST == 2) {
+                                for (int i = 0; i < F; ++i) row[i] = lds1(EA(0) + 4 * i);
+                                row += F;
+                            }
+                            row[0] = r.x; row[1] = r.y; row[2] = lds1(EA(NF) + 8); row[3] = r.th; row[4] = gx; row[5] = gy;
+                            for (int i = 6; i < F; ++i) row[i] = lds1(EA(NF) + 4 * i);
+                        }
                         log_meta(p, slot, k, e, r.steps, r.ret, end_bits(colliding, all_goals, oob, timeout, goal_reached), r.scen,
                                  __float_as_int(lds1(EA(GOL + 2) + 12)));
                     }
@@ -453,15 +516,18 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
             // slots are already there) BEFORE the pose moves on, so that no copy of this step's pose has to be kept.
             if (do_reset) {                                     // ship_env.py:180-184: [-1 x 16 | reset frame], vals = -1
                 const float4 neg = make_float4(-1.f, -1.f, -1.f, -1.f);
-                if (HIST == 2) { sts4(EA(0), neg); sts4(EA(1), neg); sts4(EA(2), neg); sts4(EA(3), neg); }
-                sts4(EA(OBS4 - 4), make_float4(r.x, r.y, 0.f, r.th));       // rudder 0 (models.py:108)
-                sts4(EA(OBS4 - 3), make_float4(gx, gy, -1.f, -1.f));
-                sts4(EA(OBS4 - 2), neg);
-                sts4(EA(OBS4 - 1), neg);
+                if (HIST == 2) {
+#pragma unroll
+                    for (int i = 0; i < FR4; ++i) sts4(EA(i), neg);
+                }
+                sts4(EA(NF), make_float4(r.x, r.y, 0.f, r.th));             // rudder 0 (models.py:108)
+                sts4(EA(NF + 1), make_float4(gx, gy, -1.f, -1.f));
+#pragma unroll
+                for (int i = 2; i < FR4; ++i) sts4(EA(NF + i), neg);
             } else {                            // the rudder slot already holds this step's angle
-                sts2(EA(OBS4 - 4), make_float2(r.x, r.y));
-                sts1(EA(OBS4 - 4) + 12, r.th);
-                sts2(EA(OBS4 - 3), make_float2(gx, gy));
+                sts2(EA(NF), make_float2(r.x, r.y));
+                sts1(EA(NF) + 12, r.th);
+                sts2(EA(NF + 1), make_float2(gx, gy));
             }
         }
         // ---- cpSpaceStep of the NEXT step, positions first (cpBodyUpdatePosition).  Done before this step's copy-out
@@ -479,6 +545,28 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
             // fully coalesced 128-bit streaming stores.
             if (SHIPSIM_TMA_STORE) fence_proxy_async();     // this lane's writes to the tiles (its own frame, other envs' rays)
             __syncwarp();
+            if (WIDE) {
+                // Rows of R = (6 + n) * HIST floats are dense in global memory and in general not 16-byte aligned, so the
+                // warp's EPW rows go out as one run of 32-bit streaming stores, lane l taking floats l, l + 32, ... of
+                // it.  (row, col) of a lane's float moves on by 32 floats per round: 32 / R rows and 32 % R columns.
+                // A store is real iff it lies before the end of this step's rows (as below).
+                if (p.obs) {
+                    const int F = 6 + nb, R = F * HIST;
+                    const int drow = 32 / R, dcol = 32 - drow * R;
+                    int row = lane / R, col = lane - row * R;
+                    float *o = reinterpret_cast<float *>(p.obs) + ((size_t)k * p.N + (e - grp)) * R + lane;
+                    const float *o_end = reinterpret_cast<const float *>(p.obs) + (size_t)(k + 1) * p.N * R;
+#pragma unroll 1
+                    for (int i = lane; i < EPW * R; i += 32) {
+                        // tile float of row column col: the older frame's F values, then the newest frame's
+                        const int tc = col < F ? col : col + (4 * FR4 - F);
+                        if (o < o_end) __stcs(o, lds1(WA(row, 0) + 4u * (unsigned)tc));
+                        o += 32;
+                        row += drow; col += dcol;
+                        if (col >= R) { col -= R; ++row; }
+                    }
+                }
+            } else {
 #if SHIPSIM_TMA_STORE
             if (p.obs && leader) bulk_store(p.obs + ((size_t)k * p.N + e) * OBS4, EA(0), OBS4 * 16);
 #else
@@ -495,6 +583,7 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
                     if (o + i * 32 < o_end) __stcs(o + i * 32, lds4(cp_src + i * (32 / OBS4) * (EB4 * 16)));
             }
 #endif
+            }
             if (leader) {
                 const size_t row = (size_t)k * p.N + e;
                 if (p.reward) p.reward[row] = reward;
@@ -506,11 +595,15 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
     // the loop leaves the pose of the last step in r (no integration after it)
     if (SHIPSIM_TMA_STORE) bulk_store_wait_read();
     if (leader) {
-        const float4 l1 = lds4(EA(OBS4 - 3)), l2 = lds4(EA(OBS4 - 2)), l3 = lds4(EA(OBS4 - 1));
+        const float4 l1 = lds4(EA(NF + 1)), l2 = lds4(EA(NF + 2)), l3 = lds4(EA(NF + 3));
         r.episode = __float_as_int(lds1(EA(GOL + 2) + 12));
         r.alive = __float_as_int(lds1(EA(GOL + 2) + 8));
-        r.rudder = (int)lds1(EA(OBS4 - 4) + 8);
+        r.rudder = (int)lds1(EA(NF) + 8);
         store_env(p, e, r, make_float4(l1.z, l1.w, l2.x, l2.y), make_float4(l2.z, l2.w, l3.x, l3.y), l3.z, l3.w);
+        if (WIDE) {
+            const int nx = extra_lidar_planes(nb);
+            for (int q = 0; q < nx; ++q) p.state[(size_t)(kPlanes + q) * p.N + e] = lds4(EA(NF + 4 + q));
+        }
     }
 
     // episode statistics: one red.add per non-zero value per warp into a slot row
@@ -647,8 +740,22 @@ __global__ void __launch_bounds__(256) reset_kernel(const __grid_constant__ Step
     g0 = __ldg(rec + 2); g1 = __ldg(rec + 3); g2 = __ldg(rec + 4);
     const float4 neg4 = make_float4(-1.f, -1.f, -1.f, -1.f);      // models.py:36: LiDAR.vals start at -1
     store_env(p, e, r, neg4, neg4, -1.f, -1.f);
+    for (int q = 0; q < extra_lidar_planes(p.n_beams); ++q) p.state[(size_t)(kPlanes + q) * p.N + e] = neg4;
     store_goals(p, e, g0, g1, g2);
-    if (obs) {
+    if (obs && p.n_beams != kBeams) {           // rows of (6 + n) * history floats: [-1 x (6 + n) | x, y, 0, 0, gx, gy, -1 x n]
+        float gx, gy;
+        float2 g[kGoals];
+        unpack_goals(g0, g1, g2, g);
+        closest_goal(g, r.alive, r.x, r.y, gx, gy);
+        const int F = 6 + p.n_beams;
+        float *o = reinterpret_cast<float *>(obs) + (size_t)e * F * p.history;
+        if (p.history == 2) {
+            for (int i = 0; i < F; ++i) o[i] = -1.f;
+            o += F;
+        }
+        o[0] = r.x; o[1] = r.y; o[2] = 0.f; o[3] = 0.f; o[4] = gx; o[5] = gy;
+        for (int i = 6; i < F; ++i) o[i] = -1.f;
+    } else if (obs) {
         float gx, gy;
         float2 g[kGoals];
         unpack_goals(g0, g1, g2, g);
@@ -819,26 +926,48 @@ __global__ void stats_reduce_kernel(double *slots, double *out, int clear)
 // ------------------------------------------------------------------------------------------------------------
 // launch wrappers (called from the C ABI)
 // ------------------------------------------------------------------------------------------------------------
-template <int G, int HIST, int MB, int T>
-static void launch_gh(const StepParams &p, int blocks, cudaStream_t stream)
+template <int G, int HIST, int MB, int T, int NB>
+static cudaError_t launch_gh(const StepParams &p, int blocks, cudaStream_t stream)
 {
-    if (p.log_count) step_kernel<G, HIST, MB, T, true><<<blocks, T, 0, stream>>>(p);
-    else step_kernel<G, HIST, MB, T, false><<<blocks, T, 0, stream>>>(p);
+    if constexpr (NB == kBeams) {
+        if (p.log_count) step_kernel<G, HIST, MB, T, true, NB><<<blocks, T, 0, stream>>>(p);
+        else step_kernel<G, HIST, MB, T, false, NB><<<blocks, T, 0, stream>>>(p);
+    } else {
+        // the wide kernel's shared memory is dynamic: up to 68 KB per CTA (G = 1, 128 threads, HISTORY_SIZE 2), beyond the
+        // 48 KB a launch gets without asking -- the opt-in is made once per instantiation and device
+        constexpr int bytes = StepLayout<G, HIST, NB, T>::BYTES;
+        void (*kern)(StepParams) = p.log_count ? step_kernel<G, HIST, MB, T, true, NB> : step_kernel<G, HIST, MB, T, false, NB>;
+        if (bytes > 48 * 1024) {
+            static std::atomic<unsigned long long> opted[2] = {};
+            int dev = 0;
+            cudaError_t err = cudaGetDevice(&dev);
+            if (err != cudaSuccess) return err;
+            const unsigned long long bit = 1ull << (dev & 63);
+            if (!(opted[p.log_count ? 1 : 0].load() & bit)) {
+                err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+                if (err != cudaSuccess) return err;
+                opted[p.log_count ? 1 : 0].fetch_or(bit);
+            }
+        }
+        kern<<<blocks, T, bytes, stream>>>(p);
+    }
+    return cudaSuccess;
 }
 
-template <int G>
+template <int G, int NB>
 static cudaError_t launch_g(const StepParams &p, cudaStream_t stream, LaunchShape *shape)
 {
     const int envs_per_cta = kThreads / G;
     int blocks = (p.N + envs_per_cta - 1) / envs_per_cta;
     int threads = kThreads;
     bool launched = false;
+    cudaError_t err = cudaSuccess;
     if constexpr (G == 1) {
         if (blocks >= 148 * 8) {
             threads = SHIPSIM_BIG_THREADS;
             blocks = (p.N + threads - 1) / threads;
-            if (p.history == 2) launch_gh<G, 2, SHIPSIM_BIG_MIN_BLOCKS, SHIPSIM_BIG_THREADS>(p, blocks, stream);
-            else launch_gh<G, 1, SHIPSIM_BIG_MIN_BLOCKS, SHIPSIM_BIG_THREADS>(p, blocks, stream);
+            if (p.history == 2) err = launch_gh<G, 2, SHIPSIM_BIG_MIN_BLOCKS, SHIPSIM_BIG_THREADS, NB>(p, blocks, stream);
+            else err = launch_gh<G, 1, SHIPSIM_BIG_MIN_BLOCKS, SHIPSIM_BIG_THREADS, NB>(p, blocks, stream);
             launched = true;
         }
     }
@@ -848,24 +977,33 @@ static cudaError_t launch_g(const StepParams &p, cudaStream_t stream, LaunchShap
         constexpr int T = SHIPSIM_SMALL_THREADS, MB = SHIPSIM_MIN_BLOCKS * kThreads / SHIPSIM_SMALL_THREADS;
         threads = T;
         blocks = (p.N + T / G - 1) / (T / G);
-        if (p.history == 2) launch_gh<G, 2, MB, T>(p, blocks, stream);
-        else launch_gh<G, 1, MB, T>(p, blocks, stream);
+        if (p.history == 2) err = launch_gh<G, 2, MB, T, NB>(p, blocks, stream);
+        else err = launch_gh<G, 1, MB, T, NB>(p, blocks, stream);
     }
     if (shape) { shape->lanes_per_env = G; shape->threads = threads; shape->blocks = blocks; shape->window = 1; }
-    return cudaGetLastError();
+    return err != cudaSuccess ? err : cudaGetLastError();
 }
 
-cudaError_t launch_step(const StepParams &p, int lanes_per_env, cudaStream_t stream, LaunchShape *shape)
+template <int NB>
+static cudaError_t launch_step_nb(const StepParams &p, int lanes_per_env, cudaStream_t stream, LaunchShape *shape)
 {
     switch (lanes_per_env) {
-        case 1: return launch_g<1>(p, stream, shape);
-        case 2: return launch_g<2>(p, stream, shape);
-        case 4: return launch_g<4>(p, stream, shape);
-        case 8: return launch_g<8>(p, stream, shape);
-        case 16: return launch_g<16>(p, stream, shape);
-        case 32: return launch_g<32>(p, stream, shape);
+        case 1: return launch_g<1, NB>(p, stream, shape);
+        case 2: return launch_g<2, NB>(p, stream, shape);
+        case 4: return launch_g<4, NB>(p, stream, shape);
+        case 8: return launch_g<8, NB>(p, stream, shape);
+        case 16: return launch_g<16, NB>(p, stream, shape);
+        case 32: return launch_g<32, NB>(p, stream, shape);
         default: return cudaErrorInvalidValue;
     }
+}
+
+// the reference's 10-beam fan runs the tuned kernels; every other beam count (1..32) the wide ones
+cudaError_t launch_step(const StepParams &p, int lanes_per_env, cudaStream_t stream, LaunchShape *shape)
+{
+    if (p.n_beams == kBeams) return launch_step_nb<kBeams>(p, lanes_per_env, stream, shape);
+    if (p.n_beams < 1 || p.n_beams > kMaxBeams) return cudaErrorInvalidValue;
+    return launch_step_nb<kMaxBeams>(p, lanes_per_env, stream, shape);
 }
 
 cudaError_t launch_reset(const StepParams &p, const uint8_t *mask, const int *scenario, int first, float4 *obs,

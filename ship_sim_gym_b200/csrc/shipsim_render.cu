@@ -20,7 +20,16 @@ __global__ void __launch_bounds__(256) render_kernel(const __grid_constant__ Ste
     EnvRegs r;
     float4 l0, l1, l2, g0, g1, g2;
     load_env(p, e, r, l0, l1, l2, g0, g1, g2);
-    const float lid[kBeams] = {l0.x, l0.y, l0.z, l0.w, l1.x, l1.y, l1.z, l1.w, l2.x, l2.y};
+    // lidar[0..9] in state planes 2-4, lidar[10..] in the appended planes (shipsim_state_bytes)
+    auto reading = [&](int j) {
+        if (j >= kBeams) {
+            const float4 v = p.state[(size_t)(kPlanes + (j - kBeams) / 4) * p.N + e];
+            const int c = (j - kBeams) & 3;
+            return c == 0 ? v.x : (c == 1 ? v.y : (c == 2 ? v.z : v.w));
+        }
+        const float lid[kBeams] = {l0.x, l0.y, l0.z, l0.w, l1.x, l1.y, l1.z, l1.w, l2.x, l2.y};
+        return lid[j];
+    };
     float2 g[kGoals];
     unpack_goals(g0, g1, g2, g);
 
@@ -64,10 +73,11 @@ __global__ void __launch_bounds__(256) render_kernel(const __grid_constant__ Ste
             minx = fminf(minx, hx); maxx = fmaxf(maxx, hx); miny = fminf(miny, hy); maxy = fmaxf(maxy, hy);
         }
         const float ox = r.x + 0.5f * (maxx - minx), oy = r.y + 0.5f * (maxy - miny);
-        for (int j = 0; j < kBeams; ++j) {
-            const float dirx = c * p.ray_c[j] - s * p.ray_s[j], diry = s * p.ray_c[j] + c * p.ray_s[j];
-            const bool hit = lid[j] >= 0.f && lid[j] < p.lidar_len;
-            const float len = hit ? lid[j] : p.lidar_len;
+        for (int j = 0; j < p.n_beams; ++j) {             // one marker per ray of the fan
+            const float dirx = c * p.ray_cw[j] - s * p.ray_sw[j], diry = s * p.ray_cw[j] + c * p.ray_sw[j];
+            const float v = reading(j);
+            const bool hit = v >= 0.f && v < p.lidar_len;
+            const float len = hit ? v : p.lidar_len;
             const float dx = wx - (ox + len * dirx), dy = wy - (oy + len * diry);
             if (dx * dx + dy * dy <= 100.f) col = hit ? make_uchar3(255, 0, 0) : make_uchar3(0, 255, 0);
         }

@@ -108,8 +108,10 @@ def long_history_terminal_rows(prev_rows, rows, k, env, frame):
 class BatchedShipEnv(object):
     """`num_envs` independent ShipEnvs on one GPU.
 
-    step(actions) -> (obs [N,16*H] f32, reward [N] f32, done [N] bool, info {})      one env-step per call
-    rollout(actions [K,N] | None, K) -> (obs [K,N,16*H], reward [K,N], done [K,N])   K steps in ONE launch
+    step(actions) -> (obs [N,F*H] f32, reward [N] f32, done [N] bool, info {})      one env-step per call
+    rollout(actions [K,N] | None, K) -> (obs [K,N,F*H], reward [K,N], done [K,N])   K steps in ONE launch
+    F = n_states = 6 + n_beams floats per frame: 16 with the reference's 10-beam lidar; with `honour_lidar_config=True`
+    LidarConfig.N_BEAMS (1..32) sets the fan.
     With auto_reset (default, the SubprocVecEnv worker semantics behind train/stable_baselines/ppo.py:123) a
     done env is reset inside the kernel and the obs returned for that step is the reset obs.
     """
@@ -122,8 +124,7 @@ class BatchedShipEnv(object):
                  env_id_offset=0, lanes_per_env=0, validate_actions=True, scenario_source="host", steps_in_flight=0,
                  host_threads=0, fresh_maps=False):
         self.knobs = snapshot(game_config, env_config, honour_lidar_config)
-        if self.knobs["lidar"]["N_BEAMS"] != _abi.N_BEAMS:
-            raise NotImplementedError("N_BEAMS must be 10")
+        self.n_beams = self.knobs["lidar"]["N_BEAMS"]         # 1..32 (shipsim_create checks the range)
         self.num_envs = int(num_envs)
         self.device = torch.device("cuda") if device is None else torch.device(device)
         if self.device.type != "cuda":
@@ -134,7 +135,7 @@ class BatchedShipEnv(object):
         self._needs_reset = True
         self.action_space = Discrete(3)                        # ship_env.py:19
         self.history = self.knobs["history"]
-        self.n_states = 2 + 1 + 1 + 2 + _abi.N_BEAMS           # ship_env.py:43
+        self.n_states = 2 + 1 + 1 + 2 + self.n_beams           # ship_env.py:43: floats per frame
         self.states_history = self.n_states * self.history     # ship_env.py:44
         self.observation_space = Box(0, max(self.knobs["W"], self.knobs["H"]), (self.states_history,), np.uint8)
         self.bounds = (self.knobs["W"], self.knobs["H"])
@@ -156,6 +157,7 @@ class BatchedShipEnv(object):
         cfg.auto_reset = int(self.auto_reset)
         cfg.lidar_spread_deg = self.knobs["lidar"]["ANGULAR_SPREAD"]
         cfg.lidar_distance = self.knobs["lidar"]["DISTANCE"]
+        cfg.lidar_beams = self.n_beams
         cfg.lanes_per_env = int(lanes_per_env)
         cfg.steps_in_flight = int(steps_in_flight)     # 0 auto, 1 serial-in-time kernel, 4/8/16/32 time-parallel window
         if not host_threads:
@@ -170,7 +172,7 @@ class BatchedShipEnv(object):
         self.params_epoch = 0                  # bumped whenever kernel parameters change (captured CUDA graphs go stale)
         self._h = C.c_void_p()
         _abi.check(self.L.shipsim_create(C.byref(cfg), self.device.index, C.byref(self._h)))
-        self._obs_dim_kernel = _abi.FRAME * cfg.history
+        self._obs_dim_kernel = self.n_states * cfg.history
 
         self._n_generated = 0
         if scenario_source not in ("host", "device"):
@@ -186,7 +188,8 @@ class BatchedShipEnv(object):
 
         with torch.cuda.device(self.device):
             nbytes = self.L.shipsim_state_bytes(self._h)
-            self.state = torch.zeros(nbytes // 4, dtype=torch.float32, device=self.device).view(_abi.STATE_PLANES, self.num_envs, 4)
+            # planes [0, 8) as for every fan, then ceil((n - 10) / 4) planes of lidar[10 ..] for fans of more than 10 beams
+            self.state = torch.zeros(nbytes // 4, dtype=torch.float32, device=self.device).view(nbytes // (16 * self.num_envs), self.num_envs, 4)
             self._stats_slots = torch.zeros(self.L.shipsim_stats_bytes(self._h) // 8, dtype=torch.float64, device=self.device)
             self._stats_out = torch.zeros(_abi.STATS_LEN, dtype=torch.float64, device=self.device)
             _abi.check(self.L.shipsim_bind_state(self._h, self.state.data_ptr(), self._stats_slots.data_ptr(), self._stream()))
@@ -329,11 +332,11 @@ class BatchedShipEnv(object):
             frame = obs
             if self._hist is None or mask is None:
                 self._hist = torch.full((N, self.states_history), -1.0, dtype=torch.float32, device=self.device)
-                self._hist[:, -_abi.FRAME:] = frame
+                self._hist[:, -self.n_states:] = frame
             else:
                 mb = m.bool()
                 fresh = torch.full_like(self._hist, -1.0)
-                fresh[:, -_abi.FRAME:] = frame
+                fresh[:, -self.n_states:] = frame
                 self._hist = torch.where(mb[:, None], fresh, self._hist)
             return self._hist.clone()
         return obs
@@ -358,10 +361,10 @@ class BatchedShipEnv(object):
         obs, rew, done = obs[0], rew[0], done[0].bool()
         if self.history > 2:
             frame = obs
-            shifted = torch.cat([self._hist[:, _abi.FRAME:], frame], dim=1)
+            shifted = torch.cat([self._hist[:, self.n_states:], frame], dim=1)
             if self.auto_reset:
                 fresh = torch.full_like(shifted, -1.0)
-                fresh[:, -_abi.FRAME:] = frame
+                fresh[:, -self.n_states:] = frame
                 shifted = torch.where(done[:, None], fresh, shifted)
             self._log_long_terminal(self._hist, shifted[None])
             self._hist = shifted
@@ -396,7 +399,7 @@ class BatchedShipEnv(object):
         """HISTORY_SIZE > 2 (SURVEY App. A, N2): rows [frame t-H+1 | ... | frame t] put together from the K frames of a
         rollout and the running history, with -1 for everything older than an env's latest reset (under auto-reset the
         frame of a done step IS the reset frame: ship_env.py:180-184)."""
-        K, N, H, F = frames.shape[0], self.num_envs, self.history, _abi.FRAME
+        K, N, H, F = frames.shape[0], self.num_envs, self.history, self.n_states
         prev = self._hist.view(N, H, F).permute(1, 0, 2)          # [H][N][F], oldest first
         allf = torch.cat([prev, frames], dim=0)                   # frame of step k sits at index H + k
         rows = allf.unfold(0, H, 1)[1:].permute(0, 1, 3, 2)       # [K][N][H][F]: rows[k] = frames k-H+1 .. k
@@ -458,7 +461,7 @@ class BatchedShipEnv(object):
 
     def step_np(self, actions):
         """One env-step for a caller on the CPU (the gym facade, the vector-env adapters): numpy int actions [N] in,
-        (obs [N, 16 * history] float32, reward [N] float32, done [N] bool) out -- ONE call into shipsim_step_host with
+        (obs [N, n_states * history] float32, reward [N] float32, done [N] bool) out -- ONE call into shipsim_step_host with
         page-locked buffers kept on the env; no torch ops, one stream wait.  The returned arrays are the env's buffers:
         valid until the next call (copy them to keep them)."""
         if self.history > 2:
@@ -564,11 +567,11 @@ class BatchedShipEnv(object):
 
     def get_state(self):
         """dict of numpy arrays: pose [N,6] (x y angle vx vy w), ints [N,5] (rudder, alive_mask, step_count,
-        scenario, episode), lidar [N,10], goals [N,5,2], ep_return [N]."""
+        scenario, episode), lidar [N,n_beams], goals [N,5,2], ep_return [N]."""
         N = self.num_envs
         pose = np.zeros((N, 6), dtype=np.float32)
         ints = np.zeros((N, 5), dtype=np.int32)
-        lidar = np.zeros((N, 10), dtype=np.float32)
+        lidar = np.zeros((N, self.n_beams), dtype=np.float32)
         goals = np.zeros((N, 5, 2), dtype=np.float32)
         ret = np.zeros(N, dtype=np.float32)
         with torch.cuda.device(self.device):
@@ -580,7 +583,7 @@ class BatchedShipEnv(object):
         N = self.num_envs
         pose = np.ascontiguousarray(pose, dtype=np.float32).reshape(N, 6)
         ints = np.ascontiguousarray(ints, dtype=np.int32).reshape(N, 5)
-        lidar = np.ascontiguousarray(lidar, dtype=np.float32).reshape(N, 10)
+        lidar = np.ascontiguousarray(lidar, dtype=np.float32).reshape(N, self.n_beams)
         goals = np.ascontiguousarray(goals, dtype=np.float32).reshape(N, 10)
         ret = np.ascontiguousarray(ep_return, dtype=np.float32).reshape(N)
         with torch.cuda.device(self.device):
