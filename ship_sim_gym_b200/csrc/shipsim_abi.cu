@@ -1,7 +1,7 @@
 // shipsim_abi.cu -- the C ABI of libshipsim.so (include/shipsim.h): handle management, scenario packing,
 // parameter derivation and kernel launches.  Host-side C++; no torch types anywhere.
 #include "../../include/shipsim.h"
-#include "shipsim_device.cuh"
+#include "shipsim_geom.cuh"
 #include "shipsim_launch.h"
 #include "shipsim_host.h"
 
@@ -10,6 +10,7 @@
 #include <cmath>
 #include <condition_variable>
 #include <functional>
+#include <memory>
 #include <mutex>
 #include <thread>
 #include <cstdio>
@@ -17,12 +18,13 @@
 #include <chrono>
 #include <cstring>
 #include <string>
+#include <utility>
 #include <vector>
 
 using namespace shipsim;
 
 // Small persistent worker pool for the host half of shipsim_step_host (assembling observation histories from frames
-// while later chunks are still crossing PCIe).  run(n, fn) calls fn(i) for i in [0, n) on the workers + the caller.
+// while later chunks are still crossing PCIe): fn(i) for i in [0, n) runs on the workers + the caller.
 class HostPool {
 public:
     explicit HostPool(int n_threads)
@@ -35,7 +37,6 @@ public:
         cv_.notify_all();
         for (auto &t : workers_) t.join();
     }
-    void run(int n, const std::function<void(int)> &fn) { start(n, fn); finish(); }
     // start(): the workers begin on fn(0..n-1) and the caller carries on; finish(): the caller joins in and waits for all
     void start(int n, const std::function<void(int)> &fn)
     {
@@ -80,45 +81,136 @@ private:
     bool quit_ = false;
 };
 
+namespace {
+// ---- owned CUDA resources ----------------------------------------------------------------------------------------
+// Move-only owner of one CUDA handle, released with Release when the owner dies or takes another handle.  size_ is the
+// element count of an allocation (Buffer).
+template <class H, cudaError_t (*Release)(H)>
+class Owned {
+public:
+    Owned() = default;
+    Owned(Owned &&o) noexcept : h_(std::exchange(o.h_, H{})), size_(std::exchange(o.size_, 0)) {}
+    Owned &operator=(Owned &&o) noexcept { if (this != &o) { reset(); std::swap(h_, o.h_); std::swap(size_, o.size_); } return *this; }
+    ~Owned() { reset(); }
+    void reset() { if (h_) Release(std::exchange(h_, H{})); size_ = 0; }
+    H *out() { reset(); return &h_; }                 // where the call that creates the next handle writes it
+    operator H() const { return h_; }
+
+protected:
+    H h_{};
+    size_t size_ = 0;
+};
+using Stream = Owned<cudaStream_t, cudaStreamDestroy>;
+using Event = Owned<cudaEvent_t, cudaEventDestroy>;
+
+// Buffer of T that grows on demand: ensure(count) frees the old allocation, then allocates the new one; if that fails,
+// the capacity is 0 and the CUDA error is returned.
+template <class T, cudaError_t (*Alloc)(void **, size_t), cudaError_t (*Release)(void *)>
+struct Buffer : Owned<void *, Release> {
+    cudaError_t ensure(size_t count)
+    {
+        if (count <= this->size_) return cudaSuccess;
+        const cudaError_t e = Alloc(this->out(), count * sizeof(T));
+        if (e == cudaSuccess) this->size_ = count;
+        return e;
+    }
+    operator T *() const { return static_cast<T *>(this->h_); }
+};
+template <class T> using DeviceBuf = Buffer<T, cudaMalloc, cudaFree>;
+template <class T> using PinnedBuf = Buffer<T, cudaMallocHost, cudaFreeHost>;
+
+// One scenario bank on the device, in the layout the kernels read it with.
+struct Bank {
+    DeviceBuf<float4> rec;                   // [n_scen][stride4] packed scenario records
+    DeviceBuf<EdgeD> edges;                  // [n_scen][2][kMaxHull] two-float planes
+    DeviceBuf<uint4> grid;                   // [n_scen][kGridN * kGridN] reach grid
+    DeviceBuf<float4> spawn;                 // [n_scen][kScr4] plane rows at the spawn pose
+    int n_scen = 0, maxv = 0, stride4 = 0, hull_max = 0;
+    bool generated = false;                  // by shipsim_generate_scenarios: fresh maps may regenerate it in place
+
+    cudaError_t alloc(int n, int edge_stride)
+    {
+        n_scen = n; maxv = edge_stride; stride4 = kBankHeader4 + 2 * edge_stride;
+        cudaError_t e = rec.ensure((size_t)n * stride4);
+        if (e == cudaSuccess) e = edges.ensure((size_t)n * 2 * kMaxHull);
+        if (e == cudaSuccess) e = grid.ensure((size_t)n * kGridN * kGridN);
+        if (e == cudaSuccess) e = spawn.ensure((size_t)n * kScr4);
+        return e;
+    }
+};
+
+// Raw output of the device scenario generator: double hull vertices ([n][2][kMaxHull][2]), hull sizes and goals.
+struct Generated {
+    DeviceBuf<double> xy, goals;
+    DeviceBuf<int> n;
+    int count = 0;
+};
+
+constexpr int kMaxChunks = 64;               // shipsim_step_host cuts a call into at most this many chunks of steps
+
+// The share of a frames-only shipsim_step_host call that goes home as complete rows by DMA: envs [0, envs).  The host
+// threads expand the others.
+struct DmaSplit {
+    int envs = -1;                           // -1: not chosen yet
+    int for_n = 0, for_k = 0;
+    int step = 0, dir = 1;                   // the split climbs towards the shorter call: step size and direction
+    double last_t = 0.0;                     // seconds per env-step of the previous call
+
+    int choose(int N, int K, int threads)
+    {
+        if (envs < 0 || for_n != N || for_k != K) {
+            // First guess.  With a core per ~4 GB/s of rows the host threads alone are the faster engine, and DMA
+            // writes landing next to their streaming stores slow both (B200 box, 16 cores: 6.4 ms per 4,096 x 1,000
+            // call with the host threads alone, 8-10 ms with any share by DMA; profiles/r02_e2e_sweep.log); with few
+            // cores per GPU the copy engine has to carry most of it.
+            envs = threads >= 8 ? 0 : (int)((double)N * 50.0 / (50.0 + 9.0 * threads));
+            for_n = N; for_k = K; step = std::max(32, N / 8 / 32 * 32); dir = 1; last_t = 0.0;
+        }
+        return envs;
+    }
+    // Keep going while the time per env-step improves, turn round (with half the step) when it gets worse, stay when it
+    // no longer changes.  `nd` is the split this call ran with, `t` its seconds per env-step.
+    void update(int N, int nd, double t)
+    {
+        if (last_t > 0.0 && t > last_t * 1.015) {
+            dir = -dir;
+            step = std::max(32, step / 2 / 32 * 32);
+        }
+        if (last_t == 0.0 || t < last_t * 0.985 || t > last_t * 1.015) envs = std::max(0, std::min(N, nd + dir * step));
+        last_t = t;
+    }
+};
+
+}  // namespace
+
 struct shipsim_handle {
     shipsim_config cfg;
     int device = 0;
     StepParams p;
-    float4 *d_bank = nullptr;
-    EdgeD *d_edges = nullptr;
-    uint4 *d_grid = nullptr;
-    float4 *d_spawn = nullptr;
-    double *d_gen_xy = nullptr, *d_gen_goals = nullptr;   // raw output of the device scenario generator (for read-back)
-    int *d_gen_n = nullptr;
-    int gen_count = 0;
-    float ship_reach = 0.f;                  // bound on the distance of any hull point from the lidar origin
+    Bank bank;                               // the bank the kernels read
+    Generated gen;                           // the last shipsim_generate_scenarios (for read-back)
+    struct { double cw, ch, margin, reach; } grid_geom;   // of the reach grid's cells (derive_params, launch_build_grid)
     int lanes = 1;
     int window = 1;                          // steps of one env speculated together (1 = the serial-in-time kernel)
     // staging for shipsim_step_host (allocated on first use, sized for the largest K seen)
-    int32_t *d_act = nullptr; float *d_obs = nullptr; float *d_rew = nullptr; uint8_t *d_done = nullptr;
-    int stage_K = 0;
-    cudaStream_t copy_stream = nullptr;      // shipsim_step_host: results of chunk i go home while chunk i+1 is computed
-    static constexpr int kMaxChunks = 64;
-    cudaEvent_t chunk_done[kMaxChunks] = {}, copy_done[kMaxChunks] = {}, trace0 = nullptr, trace_mid[kMaxChunks] = {};
-    float4 *d_frame0 = nullptr;
+    DeviceBuf<int32_t> d_act; DeviceBuf<float> d_obs; DeviceBuf<float> d_rew; DeviceBuf<uint8_t> d_done;
+    Stream copy_stream;                      // shipsim_step_host: results of chunk i go home while chunk i+1 is computed
+    Event chunk_done[kMaxChunks], copy_done[kMaxChunks];
+    int chunk_events = -1;                   // -1: not created yet; else whether they time (for a trace)
+    Event trace0, trace_mid[kMaxChunks];     // created by the first call that asks for a trace
+    DeviceBuf<float4> d_frame0;
     // compacted wire format of the host path (compact_frames_kernel / expand_delta_rows)
-    uint4 *d_rec = nullptr;                  // [K][N] records
-    unsigned *d_off = nullptr, *d_count = nullptr;   // [K][N/32] value offsets; one counter per chunk
-    uint32_t *h_rec = nullptr, *h_off = nullptr, *h_count = nullptr;     // pinned mirrors
-    float *h_var = nullptr, *d_var = nullptr;   // the changed values (a dense stream per chunk), host mirror and device buffer
+    DeviceBuf<uint4> d_rec;                  // [K][N] records
+    DeviceBuf<unsigned> d_off, d_count;      // [K][N/32] value offsets; one counter per chunk
+    PinnedBuf<uint32_t> h_rec, h_off, h_count;   // pinned mirrors
+    PinnedBuf<float> h_var;                  // the changed values (a dense stream per chunk), host mirror ...
+    DeviceBuf<float> d_var;                  // ... and device buffer
     double var_density = 2.0;                // floats per env-step the speculative D2H copy of a chunk's values is sized for
-    cudaStream_t aux_stream = nullptr;       // actions of chunks 1.. go up here; the (rare) rest of a chunk's values comes down
-    cudaEvent_t act_up = nullptr;
-    float *h_cur = nullptr;                  // one frame per env: the decoder's running state
-    size_t rec_cap = 0, var_cap = 0, cur_cap = 0;
-    int var_per_step = 0;                    // capacity of the value stream, floats per env-step
-    // the envs [0, dma_envs) go home as complete rows by DMA, the others compacted + expanded by the host threads
-    float *d_rows = nullptr;                 // [K][dma_envs][32]
-    size_t rows_cap = 0;
-    int dma_envs = -1;                       // -1: not chosen yet
-    int dma_for_n = 0, dma_for_k = 0;
-    int dma_step = 0, dma_dir = 1;           // the split climbs towards the shorter call: step size and direction
-    double dma_last_t = 0.0;                 // seconds per env-step of the previous call
+    Stream aux_stream;                       // actions of chunks 1.. go up here; the (rare) rest of a chunk's values comes down
+    Event act_up;
+    PinnedBuf<float> h_cur;                  // one frame per env: the decoder's running state
+    DeviceBuf<float> d_rows;                 // [K][dma envs][32]: the complete rows that go home by DMA
+    DmaSplit dma;
     // fresh-maps mode (shipsim_fresh_maps): the device-generated bank is regenerated a quarter at a time behind the envs
     struct {
         bool on = false, pending = false;
@@ -129,16 +221,17 @@ struct shipsim_handle {
         long long steps = 0;                 // env-steps (per env) since the period began
         int max_steps = 0;                   // the longest episode cap seen: a period lasts at least that many steps
         int generation[4] = {0, 0, 0, 0};    // how many times each quarter has been regenerated
-        cudaStream_t stream = nullptr;
-        cudaEvent_t period_begin = nullptr, gen_done = nullptr;
+        Stream stream;
+        Event period_begin, gen_done;
     } fresh;
     const void *zc_host[4] = {nullptr, nullptr, nullptr, nullptr};     // the last tiny call's buffers and their device aliases
     void *zc_dev[4] = {nullptr, nullptr, nullptr, nullptr};
-    HostPool *pool = nullptr;
+    std::unique_ptr<HostPool> pool;
     int64_t last_h2d = 0, last_d2h = 0;      // bytes the last shipsim_step_host moved over PCIe
     int64_t launches = 0;
     int32_t calls = 0;                       // shipsim_step / shipsim_step_host calls so far (SHIPSIM_EP_CALL)
     LaunchShape shape{1, kThreads, 0, 1};
+    __attribute__((visibility("hidden"))) ~shipsim_handle() = default;     // (not one of the library's exported symbols)
 };
 
 static thread_local std::string g_err;
@@ -154,6 +247,12 @@ static int fail(int code, const std::string &msg)
         cudaError_t _e = (expr);                                                                      \
         if (_e != cudaSuccess)                                                                        \
             return fail(SHIPSIM_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e));       \
+    } while (0)
+// the same for a shipsim status: a failure is passed on
+#define TRY(expr)                                                                                     \
+    do {                                                                                              \
+        const int _rc = (expr);                                                                       \
+        if (_rc != SHIPSIM_OK) return _rc;                                                            \
     } while (0)
 
 struct DeviceGuard {
@@ -262,7 +361,6 @@ static int derive_params(shipsim_handle *h)
     double rmax = 0;
     for (auto &v : hull) rmax = std::max(rmax, std::sqrt(v.x * v.x + v.y * v.y));
     p.goal_cull_r2 = (float)((rmax + c.goal_radius) * (rmax + c.goal_radius) * 1.0001);
-    h->ship_reach = (float)(2.0 * rmax);
     p.acc_dt = (float)((double)c.thrust / c.mass * c.dt);
     p.ang_dt = (float)((double)c.thrust / moment * c.dt);
     // lidar fan (models.py:48-49,62)
@@ -289,6 +387,14 @@ static int derive_params(shipsim_handle *h)
     p.gridp.x0 = (float)(-pad); p.gridp.y0 = (float)(-pad);
     p.gridp.inv_cx = (float)(kGridN / (c.bounds_w + 2.0 * pad));
     p.gridp.inv_cy = (float)(kGridN / (c.bounds_h + 2.0 * pad));
+    // The grid is built in double: cell size, touch margin and the reach of a cell's masks.  The cell is looked up at the
+    // LIDAR ORIGIN, and its masks also decide "bank not near => no ship-vs-bank test": the reach must cover the hull as
+    // seen from that origin (every hull point lies within 2 * max |hull vertex|, taken in fp32).
+    auto &gg = h->grid_geom;
+    gg.cw = ((double)c.bounds_w + 2.0 * pad) / kGridN;
+    gg.ch = ((double)c.bounds_h + 2.0 * pad) / kGridN;
+    gg.margin = 0.05 + 1e-4 * std::max((double)c.bounds_w, (double)c.bounds_h);
+    gg.reach = std::max({(double)c.lidar_distance, (double)(float)(2.0 * rmax), std::sqrt(gg.cw * gg.cw + gg.ch * gg.ch)}) + gg.margin;
     return SHIPSIM_OK;
 }
 
@@ -365,27 +471,43 @@ extern "C" int shipsim_destroy(shipsim_t *h)
 {
     if (!h) return SHIPSIM_OK;
     DeviceGuard g(h->device);
-    if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
-    for (auto &ev : h->chunk_done) if (ev) cudaEventDestroy(ev);
-    for (auto &ev : h->copy_done) if (ev) cudaEventDestroy(ev);
-    if (h->trace0) cudaEventDestroy(h->trace0);
-    for (auto &ev : h->trace_mid) if (ev) cudaEventDestroy(ev);
-    if (h->fresh.stream) cudaStreamDestroy(h->fresh.stream);
-    if (h->fresh.period_begin) cudaEventDestroy(h->fresh.period_begin);
-    if (h->fresh.gen_done) cudaEventDestroy(h->fresh.gen_done);
-    if (h->h_rec) cudaFreeHost(h->h_rec);
-    if (h->h_off) cudaFreeHost(h->h_off);
-    if (h->h_count) cudaFreeHost(h->h_count);
-    if (h->h_var) cudaFreeHost(h->h_var);
-    if (h->h_cur) cudaFreeHost(h->h_cur);
-    cudaFree(h->d_rec); cudaFree(h->d_off); cudaFree(h->d_count); cudaFree(h->d_rows); cudaFree(h->d_var);
-    if (h->aux_stream) cudaStreamDestroy(h->aux_stream);
-    if (h->act_up) cudaEventDestroy(h->act_up);
-    cudaFree(h->d_frame0);
-    delete h->pool;
-    cudaFree(h->d_bank); cudaFree(h->d_edges); cudaFree(h->d_grid); cudaFree(h->d_spawn); cudaFree(h->d_act);
-    cudaFree(h->d_gen_xy); cudaFree(h->d_gen_goals); cudaFree(h->d_gen_n); cudaFree(h->d_obs); cudaFree(h->d_rew); cudaFree(h->d_done);
-    delete h;
+    delete h;                                // (the owners release the handle's resources on its device)
+    return SHIPSIM_OK;
+}
+
+// The reach grid (one thread per cell, in double) and the plane rows at the spawn pose (what an env that is reset inside
+// the kernel starts from) of the scenarios [s0, s0 + n) of bank b, from their double hull vertices: hull_stride per hull,
+// hull_xy and hull_n start at scenario s0.
+static cudaError_t build_reach_tables(const shipsim_t *h, const Bank &b, size_t s0, int n, const double *hull_xy, const int *hull_n,
+                                      int hull_stride, cudaStream_t s)
+{
+    const auto &gg = h->grid_geom;
+    uint4 *grid = b.grid + s0 * kGridN * kGridN;
+    const cudaError_t e = launch_build_grid(hull_xy, hull_n, n, hull_stride, (double)h->p.gridp.x0, (double)h->p.gridp.y0, gg.cw, gg.ch,
+                                            gg.reach, gg.margin, grid, s);
+    if (e != cudaSuccess) return e;
+    StepParams q = h->p;
+    q.bank = b.rec + s0 * b.stride4; q.edges_d = b.edges + s0 * 2 * kMaxHull; q.grid = grid; q.n_scen = n;
+    q.maxv = b.maxv; q.scen_stride4 = b.stride4; q.hull_max = b.hull_max;
+    return launch_build_spawn_rows(q, b.spawn + s0 * kScr4, s);
+}
+
+// Make `b` the bank the kernels read; the device is idle, so no launch still reads the old one.  A new bank leaves
+// fresh-maps mode, and live envs may hold scenario ids of an old, larger bank: those are folded into range.
+static int install(shipsim_t *h, Bank &&b, cudaStream_t s)
+{
+    const int old_n = h->p.n_scen;
+    h->bank = std::move(b);
+    const Bank &nb = h->bank;
+    StepParams &p = h->p;
+    p.bank = nb.rec; p.edges_d = nb.edges; p.grid = nb.grid; p.spawn_rows = nb.spawn;
+    p.n_scen = nb.n_scen; p.maxv = nb.maxv; p.scen_stride4 = nb.stride4; p.hull_max = nb.hull_max;
+    h->fresh.on = false; h->fresh.pending = false; p.pick_base = 0; p.pick_count = 0;
+    if (p.state && nb.n_scen < old_n) {
+        CU(launch_clamp_scenarios(p.state, h->cfg.num_envs, nb.n_scen, s));
+        CU(cudaStreamSynchronize(s));
+        h->launches++;
+    }
     return SHIPSIM_OK;
 }
 
@@ -443,56 +565,21 @@ extern "C" int shipsim_load_scenarios(shipsim_t *h, const double *hull_xy, const
     }
     if (n_scen >= (1 << 28)) return fail(SHIPSIM_ERR_ARG, "too many scenarios");
     DeviceGuard g(h->device);
-    float4 *d = nullptr;
-    EdgeD *de = nullptr;
-    uint4 *dg = nullptr;
-    float4 *dsp = nullptr;
-    double *dxy = nullptr;
-    int *dn = nullptr;
-    const size_t grid_cells = (size_t)n_scen * kGridN * kGridN;
-    auto cleanup = [&]() { cudaFree(d); cudaFree(de); cudaFree(dg); cudaFree(dsp); cudaFree(dxy); cudaFree(dn); };
-    cudaError_t e = cudaMalloc(&d, host.size() * sizeof(float4));
-    if (e == cudaSuccess) e = cudaMalloc(&de, edges.size() * sizeof(EdgeD));
-    if (e == cudaSuccess) e = cudaMalloc(&dg, grid_cells * sizeof(uint4));
-    if (e == cudaSuccess) e = cudaMalloc(&dsp, (size_t)n_scen * (1 + 2 * 4) * sizeof(float4)   /* kScr4, shipsim_geom.cuh */);
-    if (e == cudaSuccess) e = cudaMalloc(&dxy, rxy.size() * sizeof(double));
-    if (e == cudaSuccess) e = cudaMalloc(&dn, (size_t)n_scen * 2 * sizeof(int));
-    if (e == cudaSuccess) e = cudaMemcpy(d, host.data(), host.size() * sizeof(float4), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemcpy(de, edges.data(), edges.size() * sizeof(EdgeD), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemcpy(dxy, rxy.data(), rxy.size() * sizeof(double), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemcpy(dn, hull_n, (size_t)n_scen * 2 * sizeof(int), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) {
-        // reach grid, built on the device in double (one thread per cell)
-        const double pad = -(double)h->p.gridp.x0;
-        const double cw = ((double)h->cfg.bounds_w + 2.0 * pad) / kGridN, ch = ((double)h->cfg.bounds_h + 2.0 * pad) / kGridN;
-        const double margin = 0.05 + 1e-4 * std::max((double)h->cfg.bounds_w, (double)h->cfg.bounds_h);
-        // the cell is looked up at the LIDAR ORIGIN, and its masks also decide "bank not near => no ship-vs-bank test":
-        // the reach must cover the hull as seen from that origin (every hull point lies within 2 * max |hull vertex|)
-        const double reach = std::max({(double)h->cfg.lidar_distance, (double)h->ship_reach, std::sqrt(cw * cw + ch * ch)}) + margin;
-        e = launch_build_grid(dxy, dn, n_scen, dev_maxv, (double)h->p.gridp.x0, (double)h->p.gridp.y0, cw, ch, reach, margin, dg, 0);
-    }
-    if (e == cudaSuccess) {
-        // plane phase at the spawn pose of every scenario (what an env that is reset inside the kernel starts from)
-        StepParams q = h->p;
-        q.bank = d; q.edges_d = de; q.grid = dg; q.n_scen = n_scen; q.maxv = dev_maxv; q.scen_stride4 = stride4; q.hull_max = dev_maxv;
-        e = launch_build_spawn_rows(q, dsp, 0);
-    }
-    if (e == cudaSuccess) e = cudaDeviceSynchronize();           // also: no launch may still be reading the old bank
-    if (e != cudaSuccess) { cleanup(); return fail(SHIPSIM_ERR_CUDA, cudaGetErrorString(e)); }
-    cudaFree(dxy); cudaFree(dn);
-    cudaFree(h->d_bank); cudaFree(h->d_edges); cudaFree(h->d_grid); cudaFree(h->d_spawn);
-    h->d_bank = d; h->d_edges = de; h->d_grid = dg; h->d_spawn = dsp;
-    h->p.bank = d; h->p.edges_d = de; h->p.grid = dg; h->p.spawn_rows = dsp;
-    const int old_n = h->p.n_scen;
-    h->p.n_scen = n_scen; h->p.maxv = dev_maxv; h->p.scen_stride4 = stride4; h->p.hull_max = dev_maxv;
-    h->fresh.on = false; h->fresh.pending = false; h->p.pick_base = 0; h->p.pick_count = 0;     // (a host bank cannot be regenerated)
+    Bank b;
+    DeviceBuf<double> dxy;
+    DeviceBuf<int> dn;
+    CU(b.alloc(n_scen, dev_maxv));
+    CU(dxy.ensure(rxy.size()));
+    CU(dn.ensure((size_t)n_scen * 2));
+    CU(cudaMemcpy(b.rec, host.data(), host.size() * sizeof(float4), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(b.edges, edges.data(), edges.size() * sizeof(EdgeD), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(dxy, rxy.data(), rxy.size() * sizeof(double), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(dn, hull_n, (size_t)n_scen * 2 * sizeof(int), cudaMemcpyHostToDevice));
+    b.hull_max = dev_maxv;
+    CU(build_reach_tables(h, b, 0, n_scen, dxy, dn, dev_maxv, 0));
+    CU(cudaDeviceSynchronize());                                 // also: no launch may still be reading the old bank
     h->launches += 2;
-    if (h->p.state && n_scen < old_n) {      // live envs may hold ids of the old, larger bank
-        CU(launch_clamp_scenarios(h->p.state, h->cfg.num_envs, n_scen, 0));
-        CU(cudaDeviceSynchronize());
-        h->launches++;
-    }
-    return SHIPSIM_OK;
+    return install(h, std::move(b), 0);
 }
 
 // ---- scenario generation on the device (SURVEY.md §8 f2) ------------------------------------------------------
@@ -504,73 +591,40 @@ extern "C" int shipsim_generate_scenarios(shipsim_t *h, int32_t n_scen, uint64_t
     if (!(width_frac > 0.f) || !(width_frac <= 1.f)) return fail(SHIPSIM_ERR_ARG, "width_frac must be in (0, 1]");
     DeviceGuard g(h->device);
     cudaStream_t s = (cudaStream_t)stream;
-    const int maxv = kMaxHull, stride4 = kBankHeader4 + 2 * maxv;
-    float4 *d = nullptr, *dsp = nullptr;
-    EdgeD *de = nullptr;
-    uint4 *dg = nullptr;
-    double *dxy = nullptr, *dgo = nullptr;
-    int *dn = nullptr, *dmax = nullptr;
-    auto cleanup = [&]() { cudaFree(d); cudaFree(de); cudaFree(dg); cudaFree(dsp); cudaFree(dxy); cudaFree(dgo); cudaFree(dn); cudaFree(dmax); };
-    cudaError_t e = cudaMalloc(&d, (size_t)n_scen * stride4 * sizeof(float4));
-    if (e == cudaSuccess) e = cudaMalloc(&de, (size_t)n_scen * 2 * kMaxHull * sizeof(EdgeD));
-    if (e == cudaSuccess) e = cudaMalloc(&dg, (size_t)n_scen * kGridN * kGridN * sizeof(uint4));
-    if (e == cudaSuccess) e = cudaMalloc(&dsp, (size_t)n_scen * (1 + 2 * 4) * sizeof(float4)   /* kScr4, shipsim_geom.cuh */);
-    if (e == cudaSuccess) e = cudaMalloc(&dxy, (size_t)n_scen * 2 * kMaxHull * 2 * sizeof(double));
-    if (e == cudaSuccess) e = cudaMalloc(&dgo, (size_t)n_scen * 10 * sizeof(double));
-    if (e == cudaSuccess) e = cudaMalloc(&dn, (size_t)n_scen * 2 * sizeof(int));
-    if (e == cudaSuccess) e = cudaMalloc(&dmax, sizeof(int));
-    if (e == cudaSuccess) e = cudaMemsetAsync(d, 0, (size_t)n_scen * stride4 * sizeof(float4), s);
-    if (e == cudaSuccess) e = cudaMemsetAsync(de, 0, (size_t)n_scen * 2 * kMaxHull * sizeof(EdgeD), s);
-    if (e == cudaSuccess) e = launch_gen_scenarios(seed, n_scen, h->cfg.bounds_w, h->cfg.bounds_h, map_N, width_frac, dxy, dn, dgo, s);
-    if (e == cudaSuccess) e = launch_max_hull(dn, n_scen * 2, dmax, s);
-    if (e == cudaSuccess) e = launch_pack_bank(dxy, dn, dgo, n_scen, maxv, stride4, d, de, s);
-    if (e == cudaSuccess) {
-        const double pad = -(double)h->p.gridp.x0;
-        const double cw = ((double)h->cfg.bounds_w + 2.0 * pad) / kGridN, ch = ((double)h->cfg.bounds_h + 2.0 * pad) / kGridN;
-        const double margin = 0.05 + 1e-4 * std::max((double)h->cfg.bounds_w, (double)h->cfg.bounds_h);
-        // the cell is looked up at the LIDAR ORIGIN, and its masks also decide "bank not near => no ship-vs-bank test":
-        // the reach must cover the hull as seen from that origin (every hull point lies within 2 * max |hull vertex|)
-        const double reach = std::max({(double)h->cfg.lidar_distance, (double)h->ship_reach, std::sqrt(cw * cw + ch * ch)}) + margin;
-        e = launch_build_grid(dxy, dn, n_scen, kMaxHull, (double)h->p.gridp.x0, (double)h->p.gridp.y0, cw, ch, reach, margin, dg, s);
-    }
-    int hull_max = 0;
-    if (e == cudaSuccess) e = cudaMemcpyAsync(&hull_max, dmax, sizeof(int), cudaMemcpyDeviceToHost, s);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(s);          // 4-byte read-back: the SAT pass lane layout depends on it
-    if (e == cudaSuccess) {
-        StepParams q = h->p;
-        q.bank = d; q.edges_d = de; q.grid = dg; q.n_scen = n_scen; q.maxv = maxv; q.scen_stride4 = stride4; q.hull_max = hull_max;
-        e = launch_build_spawn_rows(q, dsp, s);
-    }
-    if (e == cudaSuccess) e = cudaDeviceSynchronize();            // no launch may still be reading the old bank
-    if (e != cudaSuccess) { cleanup(); return fail(SHIPSIM_ERR_CUDA, cudaGetErrorString(e)); }
-    cudaFree(dmax);
-    cudaFree(h->d_bank); cudaFree(h->d_edges); cudaFree(h->d_grid); cudaFree(h->d_spawn);
-    cudaFree(h->d_gen_xy); cudaFree(h->d_gen_goals); cudaFree(h->d_gen_n);
-    h->d_bank = d; h->d_edges = de; h->d_grid = dg; h->d_spawn = dsp;
-    h->d_gen_xy = dxy; h->d_gen_goals = dgo; h->d_gen_n = dn; h->gen_count = n_scen;
-    h->fresh.on = false; h->fresh.pending = false; h->fresh.map_N = map_N; h->fresh.width_frac = width_frac; h->fresh.seed = seed;
-    h->p.pick_base = 0; h->p.pick_count = 0;
-    h->p.bank = d; h->p.edges_d = de; h->p.grid = dg; h->p.spawn_rows = dsp;
-    const int old_n = h->p.n_scen;
-    h->p.n_scen = n_scen; h->p.maxv = maxv; h->p.scen_stride4 = stride4; h->p.hull_max = hull_max;
+    Bank b;
+    Generated gen;
+    DeviceBuf<int> dmax;
+    CU(b.alloc(n_scen, kMaxHull));
+    CU(gen.xy.ensure((size_t)n_scen * 2 * kMaxHull * 2));
+    CU(gen.goals.ensure((size_t)n_scen * 10));
+    CU(gen.n.ensure((size_t)n_scen * 2));
+    CU(dmax.ensure(1));
+    CU(cudaMemsetAsync(b.rec, 0, (size_t)n_scen * b.stride4 * sizeof(float4), s));
+    CU(cudaMemsetAsync(b.edges, 0, (size_t)n_scen * 2 * kMaxHull * sizeof(EdgeD), s));
+    CU(launch_gen_scenarios(seed, n_scen, h->cfg.bounds_w, h->cfg.bounds_h, map_N, width_frac, gen.xy, gen.n, gen.goals, s));
+    CU(launch_max_hull(gen.n, n_scen * 2, dmax, s));
+    CU(launch_pack_bank(gen.xy, gen.n, gen.goals, n_scen, b.maxv, b.stride4, b.rec, b.edges, s));
+    CU(cudaMemcpyAsync(&b.hull_max, dmax, sizeof(int), cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));                                // 4-byte read-back: the SAT pass lane layout depends on it
+    CU(build_reach_tables(h, b, 0, n_scen, gen.xy, gen.n, kMaxHull, s));
+    CU(cudaDeviceSynchronize());                                 // no launch may still be reading the old bank
     h->launches += 5;
-    if (h->p.state && n_scen < old_n) {
-        CU(launch_clamp_scenarios(h->p.state, h->cfg.num_envs, n_scen, s));
-        CU(cudaStreamSynchronize(s));
-        h->launches++;
-    }
-    return SHIPSIM_OK;
+    b.generated = true;
+    gen.count = n_scen;
+    h->gen = std::move(gen);
+    h->fresh.map_N = map_N; h->fresh.width_frac = width_frac; h->fresh.seed = seed;
+    return install(h, std::move(b), s);
 }
 
 extern "C" int shipsim_read_scenarios(shipsim_t *h, double *host_hull_xy, int32_t *host_hull_n, double *host_goals)
 {
     if (!h || !host_hull_xy || !host_hull_n || !host_goals) return fail(SHIPSIM_ERR_ARG, "NULL argument");
-    if (!h->d_gen_xy) return fail(SHIPSIM_ERR_STATE, "no device-generated bank: call shipsim_generate_scenarios first");
+    if (!h->gen.count) return fail(SHIPSIM_ERR_STATE, "no device-generated bank: call shipsim_generate_scenarios first");
     DeviceGuard g(h->device);
-    const size_t S = (size_t)h->gen_count;
-    CU(cudaMemcpy(host_hull_xy, h->d_gen_xy, S * 2 * kMaxHull * 2 * sizeof(double), cudaMemcpyDeviceToHost));
-    CU(cudaMemcpy(host_hull_n, h->d_gen_n, S * 2 * sizeof(int), cudaMemcpyDeviceToHost));
-    CU(cudaMemcpy(host_goals, h->d_gen_goals, S * 10 * sizeof(double), cudaMemcpyDeviceToHost));
+    const size_t S = (size_t)h->gen.count;
+    CU(cudaMemcpy(host_hull_xy, h->gen.xy, S * 2 * kMaxHull * 2 * sizeof(double), cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(host_hull_n, h->gen.n, S * 2 * sizeof(int), cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(host_goals, h->gen.goals, S * 10 * sizeof(double), cudaMemcpyDeviceToHost));
     return SHIPSIM_OK;
 }
 
@@ -583,27 +637,19 @@ static uint64_t fresh_seed(uint64_t seed, int period) { return seed + 0x9E3779B9
 
 static int fresh_regenerate(shipsim_t *h, int slice, uint64_t seed)
 {
-    const int q = h->gen_count / 4;
-    const int maxv = kMaxHull, stride4 = kBankHeader4 + 2 * maxv;
+    const Bank &b = h->bank;
+    const int q = b.n_scen / 4;
     const size_t s0 = (size_t)slice * q;
     cudaStream_t gs = h->fresh.stream;
-    double *dxy = h->d_gen_xy + s0 * 2 * kMaxHull * 2, *dgo = h->d_gen_goals + s0 * 10;
-    int *dn = h->d_gen_n + s0 * 2;
-    float4 *d = h->d_bank + s0 * stride4, *dsp = h->d_spawn + s0 * (1 + 2 * 4);
-    EdgeD *de = h->d_edges + s0 * 2 * kMaxHull;
-    uint4 *dg = h->d_grid + s0 * kGridN * kGridN;
-    CU(cudaMemsetAsync(d, 0, (size_t)q * stride4 * sizeof(float4), gs));
+    double *dxy = h->gen.xy + s0 * 2 * kMaxHull * 2, *dgo = h->gen.goals + s0 * 10;
+    int *dn = h->gen.n + s0 * 2;
+    float4 *d = b.rec + s0 * b.stride4;
+    EdgeD *de = b.edges + s0 * 2 * kMaxHull;
+    CU(cudaMemsetAsync(d, 0, (size_t)q * b.stride4 * sizeof(float4), gs));
     CU(cudaMemsetAsync(de, 0, (size_t)q * 2 * kMaxHull * sizeof(EdgeD), gs));
     CU(launch_gen_scenarios(seed, q, h->cfg.bounds_w, h->cfg.bounds_h, h->fresh.map_N, h->fresh.width_frac, dxy, dn, dgo, gs));
-    CU(launch_pack_bank(dxy, dn, dgo, q, maxv, stride4, d, de, gs));
-    const double pad = -(double)h->p.gridp.x0;
-    const double cw = ((double)h->cfg.bounds_w + 2.0 * pad) / kGridN, ch = ((double)h->cfg.bounds_h + 2.0 * pad) / kGridN;
-    const double margin = 0.05 + 1e-4 * std::max((double)h->cfg.bounds_w, (double)h->cfg.bounds_h);
-    const double reach = std::max({(double)h->cfg.lidar_distance, (double)h->ship_reach, std::sqrt(cw * cw + ch * ch)}) + margin;
-    CU(launch_build_grid(dxy, dn, q, kMaxHull, (double)h->p.gridp.x0, (double)h->p.gridp.y0, cw, ch, reach, margin, dg, gs));
-    StepParams sp = h->p;
-    sp.bank = d; sp.edges_d = de; sp.grid = dg; sp.n_scen = q;
-    CU(launch_build_spawn_rows(sp, dsp, gs));
+    CU(launch_pack_bank(dxy, dn, dgo, q, b.maxv, b.stride4, d, de, gs));
+    CU(build_reach_tables(h, b, s0, q, dxy, dn, kMaxHull, gs));
     h->launches += 4;
     return SHIPSIM_OK;
 }
@@ -617,7 +663,7 @@ static int fresh_tick(shipsim_t *h, int K, cudaStream_t s)
     if (f.steps >= f.max_steps) {
         f.period++;
         f.steps = 0;
-        const int q = h->gen_count / 4, slice = f.period % 4;
+        const int q = h->bank.n_scen / 4, slice = f.period % 4;
         if (f.pending) {                                 // this period's slice was regenerated while the last one ran
             CU(cudaStreamWaitEvent(s, f.gen_done, 0));
             f.pending = false;
@@ -627,8 +673,7 @@ static int fresh_tick(shipsim_t *h, int K, cudaStream_t s)
             const int nxt = (f.period + 1) % 4;
             CU(cudaEventRecord(f.period_begin, s));      // every launch that could still read it precedes this point
             CU(cudaStreamWaitEvent(f.stream, f.period_begin, 0));
-            const int rc = fresh_regenerate(h, nxt, fresh_seed(f.seed, f.period + 1));
-            if (rc) return rc;
+            TRY(fresh_regenerate(h, nxt, fresh_seed(f.seed, f.period + 1)));
             CU(cudaEventRecord(f.gen_done, f.stream));
             f.generation[nxt]++;
             f.pending = true;
@@ -649,21 +694,22 @@ extern "C" int shipsim_fresh_maps(shipsim_t *h, int32_t enable)
         h->p.pick_base = 0; h->p.pick_count = 0;
         return SHIPSIM_OK;
     }
-    if (!h->d_gen_xy || h->p.bank != h->d_bank || h->gen_count != h->p.n_scen)
-        return fail(SHIPSIM_ERR_STATE, "fresh maps need a device-generated bank: call shipsim_generate_scenarios first");
-    const int q = h->gen_count / 4;
-    if (h->gen_count % 4 != 0 || q < 1 || (q & (q - 1)) != 0)
+    Bank &b = h->bank;
+    if (!b.generated) return fail(SHIPSIM_ERR_STATE, "fresh maps need a device-generated bank: call shipsim_generate_scenarios first");
+    const int q = b.n_scen / 4;
+    if (b.n_scen % 4 != 0 || q < 1 || (q & (q - 1)) != 0)
         return fail(SHIPSIM_ERR_ARG, "fresh maps need a bank of 4 * 2^k scenarios");
     if (!h->cfg.auto_reset) return fail(SHIPSIM_ERR_STATE, "fresh maps need auto_reset (an env that is never reset would outlive its map)");
-    if (!f.stream) {
-        CU(cudaStreamCreateWithFlags(&f.stream, cudaStreamNonBlocking));
-        CU(cudaEventCreateWithFlags(&f.period_begin, cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&f.gen_done, cudaEventDisableTiming));
+    if (!f.stream || !f.period_begin || !f.gen_done) {
+        CU(cudaStreamCreateWithFlags(f.stream.out(), cudaStreamNonBlocking));
+        CU(cudaEventCreateWithFlags(f.period_begin.out(), cudaEventDisableTiming));
+        CU(cudaEventCreateWithFlags(f.gen_done.out(), cudaEventDisableTiming));
     }
     f.on = true; f.pending = false; f.period = 0; f.steps = 0; f.max_steps = h->cfg.max_steps;
     for (int &gen : f.generation) gen = 0;
     h->p.pick_base = 0; h->p.pick_count = q;
-    h->p.hull_max = std::max(h->p.hull_max, std::min(kMaxHull, f.map_N + 2));   // regenerated hulls: at most map_N + 2 vertices
+    b.hull_max = std::max(b.hull_max, std::min(kMaxHull, f.map_N + 2));       // regenerated hulls: at most map_N + 2 vertices
+    h->p.hull_max = b.hull_max;
     return SHIPSIM_OK;
 }
 
@@ -711,12 +757,26 @@ static int ready(const shipsim_t *h)
 
 extern "C" int shipsim_reset(shipsim_t *h, const uint8_t *dev_mask, const int32_t *dev_scenario, int first, float *dev_obs, void *stream)
 {
-    const int rc = ready(h);
-    if (rc) return rc;
+    TRY(ready(h));
     DeviceGuard g(h->device);
     CU(launch_reset(h->p, dev_mask, dev_scenario, first, (float4 *)dev_obs, (cudaStream_t)stream));
     h->launches++;
     return SHIPSIM_OK;
+}
+
+// What the runtime knows of a pointer: its memory type and, for page-locked host memory that is mapped, its device alias.
+// Memory the runtime does not know reads as unregistered; the error of that query is cleared, so no later call sees it.
+struct PtrInfo {
+    cudaMemoryType type;
+    void *alias;
+};
+static PtrInfo pointer_info(const void *ptr)
+{
+    cudaPointerAttributes attr{};
+    const bool ok = cudaPointerGetAttributes(&attr, ptr) == cudaSuccess;
+    cudaGetLastError();
+    if (!ok) return {cudaMemoryTypeUnregistered, nullptr};
+    return {attr.type, attr.type == cudaMemoryTypeHost ? attr.devicePointer : nullptr};
 }
 
 extern "C" int shipsim_episode_log_bind(shipsim_t *h, float *dev_rows, int32_t *dev_meta, int32_t capacity, int32_t *dev_count)
@@ -732,21 +792,12 @@ extern "C" int shipsim_episode_log_bind(shipsim_t *h, float *dev_rows, int32_t *
     if (((uintptr_t)dev_rows & 15) || ((uintptr_t)dev_meta & 15) || ((uintptr_t)dev_count & 3))
         return fail(SHIPSIM_ERR_ARG, "dev_rows / dev_meta must be 16-byte aligned");
     DeviceGuard g(h->device);
+    if (pointer_info(dev_count).type != cudaMemoryTypeDevice)
+        return fail(SHIPSIM_ERR_ARG, "dev_count must be device memory (it is the target of device atomics)");
     // rows and metadata may sit in page-locked host memory (written over PCIe): the kernels need its device alias
-    auto device_alias = [](void *ptr) {
-        cudaPointerAttributes attr{};
-        const bool host = cudaPointerGetAttributes(&attr, ptr) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer;
-        cudaGetLastError();
-        return host ? attr.devicePointer : ptr;
-    };
-    {
-        cudaPointerAttributes attr{};
-        const bool dev = cudaPointerGetAttributes(&attr, dev_count) == cudaSuccess && attr.type == cudaMemoryTypeDevice;
-        cudaGetLastError();
-        if (!dev) return fail(SHIPSIM_ERR_ARG, "dev_count must be device memory (it is the target of device atomics)");
-    }
-    p.log_rows = (float4 *)device_alias(dev_rows);
-    p.log_meta = (int4 *)device_alias(dev_meta);
+    const PtrInfo rows = pointer_info(dev_rows), meta = pointer_info(dev_meta);
+    p.log_rows = (float4 *)(rows.alias ? rows.alias : dev_rows);
+    p.log_meta = (int4 *)(meta.alias ? meta.alias : dev_meta);
     p.log_count = (int *)dev_count;
     p.log_cap = capacity;
     p.log_row4 = 4 * h->cfg.history;         // (the wide kernel's rows are dense: (6 + lidar_beams) * history floats)
@@ -756,8 +807,7 @@ extern "C" int shipsim_episode_log_bind(shipsim_t *h, float *dev_rows, int32_t *
 static int step_impl(shipsim_t *h, const void *dev_actions, int action_dtype, int32_t K, float *dev_obs, float *dev_reward,
                      uint8_t *dev_done, void *stream, int history)
 {
-    const int rc = ready(h);
-    if (rc) return rc;
+    TRY(ready(h));
     if (K < 1) return fail(SHIPSIM_ERR_ARG, "K must be >= 1");
     if (action_dtype < 0 || action_dtype > 3) return fail(SHIPSIM_ERR_ARG, "bad action_dtype");
     if (action_dtype != SHIPSIM_ACTION_RANDOM && !dev_actions) return fail(SHIPSIM_ERR_ARG, "dev_actions is NULL");
@@ -765,10 +815,7 @@ static int step_impl(shipsim_t *h, const void *dev_actions, int action_dtype, in
     if ((uintptr_t)dev_obs & (h->cfg.lidar_beams == SHIPSIM_N_BEAMS ? 15 : 3))
         return fail(SHIPSIM_ERR_ARG, h->cfg.lidar_beams == SHIPSIM_N_BEAMS ? "dev_obs must be 16-byte aligned" : "dev_obs must be 4-byte aligned");
     DeviceGuard g(h->device);
-    {
-        const int rcf = fresh_tick(h, K, (cudaStream_t)stream);
-        if (rcf) return rcf;
-    }
+    TRY(fresh_tick(h, K, (cudaStream_t)stream));
     StepParams p = h->p;
     p.actions = dev_actions; p.action_dtype = action_dtype; p.K = K;
     p.obs = (float4 *)dev_obs; p.reward = dev_reward; p.done = dev_done;
@@ -788,199 +835,223 @@ extern "C" int shipsim_step(shipsim_t *h, const void *dev_actions, int action_dt
     return step_impl(h, dev_actions, action_dtype, K, dev_obs, dev_reward, dev_done, stream, h ? h->p.history : 1);
 }
 
-extern "C" int shipsim_step_host(shipsim_t *h, const int32_t *host_actions, int32_t K, float *host_obs, float *host_reward,
-                                 uint8_t *host_done, void *stream)
+// ---- shipsim_step_host ------------------------------------------------------------------------------------------------
+// With HISTORY_SIZE = 2 an observation is [frame of the previous step | frame of this step] (ship_env.py:112-113): half
+// of every row repeats the row before it, and between consecutive frames of an env little changes besides the pose.
+// Three regimes, by size:
+//  * zero copy: tiny calls with page-locked buffers (the gym facade: one env, one step) -- the kernel reads the actions
+//    from the caller's memory and writes rows, rewards and done flags straight into it (mapped pinned memory), one
+//    launch and one wait;
+//  * plain copies of complete rows.  Small calls are latency bound: everything goes through the caller's stream;
+//  * frames only: the kernel runs in its one-frame mode, and the caller's rows are produced by two engines at once,
+//    because either alone is the bottleneck (PCIe at ~55 GB/s for 128-byte rows; the host cores' stores for the
+//    expansion).  Envs [0, nd): complete rows are put together on the device (history_rows_kernel) and DMA-ed straight
+//    into the caller's buffer (when it is page-locked).  Envs [nd, N): a kernel turns the frames into 16-byte records + a
+//    stream of changed values (~20 bytes per env-step instead of 64 + 5) and host threads rebuild the rows -- reset
+//    observations included.  nd follows the measured balance of the two (DmaSplit).
+// The last two cut the rollout into chunks of steps: while chunk i+1 is being computed on the caller's stream, the
+// results of chunk i travel to the host on the copy stream (and chunk i-1 is being expanded by the host threads).
+
+// Room in the value stream for all 12 variable slots of every env-step (measured need on the default map: 0.9), so that
+// it cannot overflow; untouched pages of the mapping cost nothing.
+constexpr int kVarPerStep = 12;
+
+// One chunked shipsim_step_host call
+struct HostCall {
+    const int32_t *actions;
+    float *obs, *reward;                     // (any output may be NULL: it is then not copied back)
+    uint8_t *done;
+    cudaStream_t s;                          // the caller's stream
+    int K;
+    size_t N, n, row_full;                   // envs, env-steps, floats per complete row
+    bool small, trace;
+    int n_chunks = 1, kbeg[kMaxChunks + 1] = {};   // chunk c holds the steps [kbeg[c], kbeg[c + 1])
+    bool adaptive = false;                   // frames only: the DMA split nd is DmaSplit's choice
+    int nd = 0;
+
+    int kc(int ci) const { return kbeg[ci + 1] - kbeg[ci]; }
+    size_t off(int ci) const { return (size_t)kbeg[ci] * N; }     // the chunk's first env-step
+};
+
+// Chunk ci of a chunked call: its actions go up (the first chunk's ahead of its kernel, the rest on the aux stream while
+// it runs) and its steps are launched on the caller's stream with `hist` frames per row.
+static int step_chunk(shipsim_t *h, const HostCall &c, int ci, int hist)
 {
-    const int rc = ready(h);
-    if (rc) return rc;
-    if (K < 1 || !host_actions) return fail(SHIPSIM_ERR_ARG, "K must be >= 1 and host_actions non-NULL");
-    DeviceGuard g(h->device);
-    h->p.log_call = h->calls++;
+    if (ci == 0) {
+        CU(cudaMemcpyAsync(h->d_act, c.actions, (size_t)c.kc(0) * c.N * sizeof(int32_t), cudaMemcpyHostToDevice, c.s));
+        if (c.n_chunks > 1) {
+            CU(cudaEventRecord(h->act_up, c.s));                 // (orders the copy behind whatever the caller's stream did before)
+            CU(cudaStreamWaitEvent(h->aux_stream, h->act_up, 0));
+            CU(cudaMemcpyAsync(h->d_act + c.off(1), c.actions + c.off(1), (c.n - c.off(1)) * sizeof(int32_t), cudaMemcpyHostToDevice,
+                               h->aux_stream));
+            CU(cudaEventRecord(h->act_up, h->aux_stream));
+        }
+    } else if (ci == 1) CU(cudaStreamWaitEvent(c.s, h->act_up, 0));
+    h->p.log_k0 = c.kbeg[ci];                                    // episode-log records carry the step index within the call
+    const size_t off = c.off(ci);
+    const int rc = step_impl(h, h->d_act + off, SHIPSIM_ACTION_I32, c.kc(ci), h->d_obs + off * c.row_full, h->d_rew + off, h->d_done + off,
+                             c.s, hist);
     h->p.log_k0 = 0;
-    const size_t N = (size_t)h->cfg.num_envs;
-    const size_t n = N * K;
-    // With HISTORY_SIZE = 2 an observation is [frame of the previous step | frame of this step] (ship_env.py:112-113):
-    // half of every row repeats the row before it, and between consecutive frames of an env little changes besides the
-    // pose.  The kernel runs in its one-frame mode.  The caller's rows are then produced by two engines at once, because
-    // either alone is the bottleneck (PCIe at ~55 GB/s for 128-byte rows; the host cores' stores for the expansion):
-    //  * envs [0, nd): complete rows are put together on the device (history_rows_kernel) and DMA-ed straight into the
-    //    caller's buffer (when it is page-locked);
-    //  * envs [nd, N): a kernel turns the frames into 16-byte records + a stream of changed values (~20 bytes per
-    //    env-step instead of 64 + 5) and host threads rebuild the rows -- reset observations included;
-    // chunk by chunk, while later chunks are still being computed.  nd follows the measured balance of the two.
-    // (Small calls -- a gym-style caller stepping a handful of envs one step at a time -- are latency bound: for them the
-    // kernel writes complete rows and everything, copies included, goes through the caller's stream with one wait.)
-    const bool small = n < ((size_t)1 << 16);
-    // Tiny calls with page-locked buffers (the gym facade: one env, one step): no copies at all -- the kernel reads the
-    // actions from the caller's memory and writes rows, rewards and done flags straight into it (mapped pinned memory;
-    // a few hundred bytes over PCIe), one launch and one wait.
-    const size_t F = (size_t)frame_floats(h);                       // floats per frame
-    if (n * F * h->cfg.history * sizeof(float) <= ((size_t)1 << 16) && host_obs && host_reward && host_done) {
-        auto mapped = [&](const void *ptr, void **dev) {
-            cudaPointerAttributes attr{};
-            const bool ok = cudaPointerGetAttributes(&attr, ptr) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer;
-            cudaGetLastError();
-            if (ok) *dev = attr.devicePointer;
-            return ok;
-        };
-        void *da = nullptr, *dobs = nullptr, *dr = nullptr, *dd = nullptr;
-        bool all = false;
-        if (h->zc_host[0] == host_actions && h->zc_host[1] == host_obs && h->zc_host[2] == host_reward && h->zc_host[3] == host_done) {
-            da = h->zc_dev[0]; dobs = h->zc_dev[1]; dr = h->zc_dev[2]; dd = h->zc_dev[3];
-            all = da != nullptr;
-        } else if (mapped(host_actions, &da) && mapped(host_obs, &dobs) && mapped(host_reward, &dr) && mapped(host_done, &dd)) {
-            h->zc_host[0] = host_actions; h->zc_host[1] = host_obs; h->zc_host[2] = host_reward; h->zc_host[3] = host_done;
-            h->zc_dev[0] = da; h->zc_dev[1] = dobs; h->zc_dev[2] = dr; h->zc_dev[3] = dd;
-            all = true;
-        } else {
-            h->zc_host[0] = host_actions; h->zc_host[1] = host_obs; h->zc_host[2] = host_reward; h->zc_host[3] = host_done;
-            h->zc_dev[0] = h->zc_dev[1] = h->zc_dev[2] = h->zc_dev[3] = nullptr;                 // (remembered as not mapped)
+    return rc;
+}
+
+static int step_plain_copies(shipsim_t *h, const HostCall &c)
+{
+    for (int ci = 0; ci < c.n_chunks; ++ci) {
+        const size_t off = c.off(ci), rows = (size_t)c.kc(ci) * c.N;
+        TRY(step_chunk(h, c, ci, h->cfg.history));
+        if (c.trace) CU(cudaEventRecord(h->trace_mid[ci], c.s));
+        cudaStream_t cs = c.s;                                  // small: one stream, no event hops
+        if (!c.small) {
+            cs = h->copy_stream;
+            CU(cudaEventRecord(h->chunk_done[ci], c.s));
+            CU(cudaStreamWaitEvent(h->copy_stream, h->chunk_done[ci], 0));
         }
-        if (all) {
-            const int rc2 = step_impl(h, da, SHIPSIM_ACTION_I32, K, (float *)dobs, (float *)dr, (uint8_t *)dd, stream, h->cfg.history);
-            if (rc2) return rc2;
-            h->last_h2d = (int64_t)(n * sizeof(int32_t));
-            h->last_d2h = (int64_t)(n * (F * h->cfg.history * sizeof(float) + 5));
-            CU(cudaStreamSynchronize((cudaStream_t)stream));
-            return SHIPSIM_OK;
+        h->last_d2h += (int64_t)rows * ((c.reward ? 4 : 0) + (c.done ? 1 : 0));
+        if (c.obs) {
+            h->last_d2h += (int64_t)(rows * c.row_full * sizeof(float));
+            CU(cudaMemcpyAsync(c.obs + off * c.row_full, h->d_obs + off * c.row_full, rows * c.row_full * sizeof(float), cudaMemcpyDeviceToHost, cs));
         }
+        if (c.reward) CU(cudaMemcpyAsync(c.reward + off, h->d_rew + off, rows * sizeof(float), cudaMemcpyDeviceToHost, cs));
+        if (c.done) CU(cudaMemcpyAsync(c.done + off, h->d_done + off, rows, cudaMemcpyDeviceToHost, cs));
+        if (!c.small) CU(cudaEventRecord(h->copy_done[ci], h->copy_stream));
     }
-    // (the compacted wire format is that of 16-float frames: other fans take the plain copies)
-    const bool frames_only = h->cfg.history == 2 && host_obs != nullptr && !small && h->cfg.lidar_beams == SHIPSIM_N_BEAMS;
-    int nd = 0;                                                      // envs [0, nd) by DMA (frames_only)
-    bool adaptive = false;
-    if (K > h->stage_K) {
-        cudaFree(h->d_act); cudaFree(h->d_obs); cudaFree(h->d_rew); cudaFree(h->d_done);
-        h->d_act = nullptr; h->d_obs = nullptr; h->d_rew = nullptr; h->d_done = nullptr; h->stage_K = 0;
-        CU(cudaMalloc(&h->d_act, n * sizeof(int32_t)));
-        CU(cudaMalloc(&h->d_obs, n * F * h->cfg.history * sizeof(float)));
-        CU(cudaMalloc(&h->d_rew, n * sizeof(float)));
-        CU(cudaMalloc(&h->d_done, n));
-        h->stage_K = K;
+    return SHIPSIM_OK;
+}
+
+// The buffers of the compacted wire format, the host threads, and the first frame of every env; then how many envs
+// travel as complete rows.
+static int frames_setup(shipsim_t *h, HostCall &c)
+{
+    const size_t N = c.N, n = c.n, nblk = (N + 31) / 32;
+    CU(h->d_rec.ensure(n));
+    CU(h->d_off.ensure((size_t)c.K * nblk));
+    CU(h->d_count.ensure(kMaxChunks));
+    CU(h->h_rec.ensure(n * 4));
+    CU(h->h_off.ensure((size_t)c.K * nblk));
+    CU(h->h_count.ensure(kMaxChunks));
+    CU(h->h_var.ensure(n * kVarPerStep));
+    CU(h->d_var.ensure(n * kVarPerStep));
+    CU(h->h_cur.ensure(N * kFrame));
+    CU(h->d_frame0.ensure(N * kFrame / 4));
+    if (!h->pool) {
+        int nt = std::max(1, std::min(16, (int)std::thread::hardware_concurrency()));
+        if (h->cfg.host_threads > 0) nt = std::min(h->cfg.host_threads, 256);
+        if (const char *ev = std::getenv("SHIPSIM_HOST_THREADS")) nt = std::max(1, atoi(ev));
+        h->pool = std::make_unique<HostPool>(nt - 1);
     }
-    cudaStream_t s = (cudaStream_t)stream;
-    if (!h->copy_stream) {
-        CU(cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
-        const unsigned evf = std::getenv("SHIPSIM_HOST_TRACE") ? cudaEventDefault : cudaEventDisableTiming;
-        for (auto &ev : h->chunk_done) CU(cudaEventCreateWithFlags(&ev, evf));
-        for (auto &ev : h->copy_done) CU(cudaEventCreateWithFlags(&ev, evf));
-        CU(cudaEventCreateWithFlags(&h->trace0, evf));
-        CU(cudaStreamCreateWithFlags(&h->aux_stream, cudaStreamNonBlocking));
-        CU(cudaEventCreateWithFlags(&h->act_up, cudaEventDisableTiming));
-        if (std::getenv("SHIPSIM_HOST_TRACE")) for (auto &ev : h->trace_mid) CU(cudaEventCreate(&ev));
+    CU(launch_frame(h->p, h->d_frame0, c.s));
+    CU(cudaMemsetAsync(h->d_count, 0, kMaxChunks * sizeof(unsigned), c.s));
+    h->launches++;
+    const char *fixed = std::getenv("SHIPSIM_HOST_DMA_ENVS");
+    int nd;
+    if (pointer_info(c.obs).type != cudaMemoryTypeHost) nd = 0;
+    else if (fixed) nd = std::max(0, std::min(atoi(fixed), (int)N));
+    else if (n < ((size_t)1 << 18)) nd = 0;                         // (small calls are latency bound either way)
+    else {
+        c.adaptive = true;
+        nd = h->dma.choose((int)N, c.K, h->pool->size());
     }
-    int n_chunks = small ? 1 : (K >= 64 ? 16 : (K >= 8 ? 8 : 1));
-    if (const char *ev = std::getenv("SHIPSIM_HOST_CHUNKS")) n_chunks = std::max(1, std::min({atoi(ev), (int)shipsim_handle::kMaxChunks, (int)K}));
-    int kbeg[shipsim_handle::kMaxChunks + 1];
-    for (int c = 0; c <= n_chunks; ++c) kbeg[c] = (int)((int64_t)K * c / n_chunks);
-    const size_t nblk = (N + 31) / 32;
-    for (int c = 0; c < n_chunks; ++c)
-        if (kbeg[c + 1] <= kbeg[c]) return fail(SHIPSIM_ERR_ARG, "internal: empty chunk");
-    if (frames_only) {
-        // Value stream: room for all 12 variable slots of every env-step (measured need on the default map: 0.9), so
-        // that it cannot overflow; untouched pages of the mapping cost nothing.
-        h->var_per_step = 12;
-        if (n > h->rec_cap) {
-            cudaFree(h->d_rec); cudaFree(h->d_off); cudaFree(h->d_count);
-            if (h->h_rec) cudaFreeHost(h->h_rec);
-            if (h->h_off) cudaFreeHost(h->h_off);
-            if (h->h_count) cudaFreeHost(h->h_count);
-            if (h->h_var) cudaFreeHost(h->h_var);
-            cudaFree(h->d_var); h->d_var = nullptr;
-            h->d_rec = nullptr; h->d_off = nullptr; h->d_count = nullptr; h->h_rec = nullptr; h->h_off = nullptr; h->h_count = nullptr;
-            h->h_var = nullptr; h->rec_cap = 0;
-            CU(cudaMalloc(&h->d_rec, n * sizeof(uint4)));
-            CU(cudaMalloc(&h->d_off, (size_t)K * nblk * sizeof(unsigned)));
-            CU(cudaMalloc(&h->d_count, shipsim_handle::kMaxChunks * sizeof(unsigned)));
-            CU(cudaHostAlloc(&h->h_rec, n * sizeof(uint4), cudaHostAllocDefault));
-            CU(cudaHostAlloc(&h->h_off, (size_t)K * nblk * sizeof(unsigned), cudaHostAllocDefault));
-            CU(cudaHostAlloc(&h->h_count, shipsim_handle::kMaxChunks * sizeof(unsigned), cudaHostAllocDefault));
-            CU(cudaHostAlloc(&h->h_var, n * h->var_per_step * sizeof(float), cudaHostAllocDefault));
-            CU(cudaMalloc(&h->d_var, n * h->var_per_step * sizeof(float)));
-            h->rec_cap = n;
+    c.nd = nd >= (int)N ? (int)N : (nd / 32) * 32;
+    CU(h->d_rows.ensure((size_t)c.nd * c.K * 2 * kFrame));
+    return SHIPSIM_OK;
+}
+
+// The stream work of a frames-only call, chunk by chunk: step kernel, compaction and/or complete rows, and the copies home.
+// `issued` counts the chunks whose copies (and copy_done event) are in the copy stream; spec[c] = floats of chunk c's
+// value stream copied down unasked.
+static int issue_frames(shipsim_t *h, const HostCall &c, size_t *spec, std::atomic<int> &issued)
+{
+    const size_t N = c.N, nblk = (N + 31) / 32, row_full = c.row_full;
+    const int nd = c.nd;
+    const bool expand = nd < (int)N;
+    cudaStream_t s = c.s;
+    const float4 *prev_frames = h->d_frame0;                     // the frames the next chunk's first step is compared with
+    for (int ci = 0; ci < c.n_chunks; ++ci) {
+        const int k0 = c.kbeg[ci], kc = c.kc(ci);
+        const size_t off = c.off(ci);
+        const float4 *frames = (const float4 *)(h->d_obs + off * row_full);
+        TRY(step_chunk(h, c, ci, 1));
+        if (h->p.log_count) {                                    // the one-frame kernel logged the terminal frame only
+            CU(launch_log_prev_frames(h->p, frames, prev_frames, k0, kc, s));
+            h->launches++;
         }
-        if (N > h->cur_cap) {
-            if (h->h_cur) cudaFreeHost(h->h_cur);
-            h->h_cur = nullptr; h->cur_cap = 0;
-            CU(cudaHostAlloc(&h->h_cur, N * kFrame * sizeof(float), cudaHostAllocDefault));
-            h->cur_cap = N;
+        if (c.trace) CU(cudaEventRecord(h->trace_mid[ci], s));
+        if (expand) {
+            CU(launch_compact_frames(frames, prev_frames, h->d_rew + off, h->d_done + off, (int)N, nd, kc, h->cfg.step_penalty, h->d_rec + off,
+                                     h->d_off + (size_t)k0 * nblk, h->d_var + off * kVarPerStep,
+                                     (unsigned)std::min<size_t>((size_t)kc * N * kVarPerStep, 0xffffffffu), h->d_count + ci, s));
+            h->launches++;
         }
-        if (!h->d_frame0) CU(cudaMalloc(&h->d_frame0, N * kFrame * sizeof(float)));
-        if (!h->pool) {
-            int nt = std::max(1, std::min(16, (int)std::thread::hardware_concurrency()));
-            if (h->cfg.host_threads > 0) nt = std::min(h->cfg.host_threads, 256);
-            if (const char *ev = std::getenv("SHIPSIM_HOST_THREADS")) nt = std::max(1, atoi(ev));
-            h->pool = new HostPool(nt - 1);
+        if (nd > 0) {
+            CU(launch_history_rows(frames, prev_frames, h->d_done + off, (int)N, nd, kc, h->cfg.auto_reset != 0,
+                                   (float4 *)(h->d_rows + (size_t)k0 * nd * row_full), s));
+            h->launches++;
         }
-        CU(launch_frame(h->p, h->d_frame0, s));
-        CU(cudaMemsetAsync(h->d_count, 0, shipsim_handle::kMaxChunks * sizeof(unsigned), s));
-        h->launches++;
-        // how many envs travel as complete rows
-        cudaPointerAttributes attr{};
-        const bool pinned = cudaPointerGetAttributes(&attr, host_obs) == cudaSuccess && attr.type == cudaMemoryTypeHost;
-        cudaGetLastError();
-        const char *fixed = std::getenv("SHIPSIM_HOST_DMA_ENVS");
-        if (!pinned) nd = 0;
-        else if (fixed) nd = std::max(0, std::min(atoi(fixed), (int)N));
-        else if (n < ((size_t)1 << 18)) nd = 0;                       // (small calls are latency bound either way)
-        else {
-            adaptive = true;
-            if (h->dma_envs < 0 || h->dma_for_n != (int)N || h->dma_for_k != K) {
-                // First guess.  With a core per ~4 GB/s of rows the host threads alone are the faster engine, and DMA
-                // writes landing next to their streaming stores slow both (B200 box, 16 cores: 6.4 ms per 4,096 x 1,000
-                // call with the host threads alone, 8-10 ms with any share by DMA; profiles/r02_e2e_sweep.log); with few
-                // cores per GPU the copy engine has to carry most of it.
-                const int thr = h->pool->size();
-                h->dma_envs = thr >= 8 ? 0 : (int)((double)N * 50.0 / (50.0 + 9.0 * thr));
-                h->dma_for_n = (int)N; h->dma_for_k = K;
-                h->dma_step = std::max(32, (int)(N / 8) / 32 * 32);
-                h->dma_dir = 1;
-                h->dma_last_t = 0.0;
+        prev_frames = frames + ((size_t)(kc - 1) * N) * 4;
+        CU(cudaEventRecord(h->chunk_done[ci], s));
+        CU(cudaStreamWaitEvent(h->copy_stream, h->chunk_done[ci], 0));
+        if (expand) {
+            if (ci == 0) {
+                CU(cudaMemcpyAsync(h->h_cur, h->d_frame0, N * kFrame * sizeof(float), cudaMemcpyDeviceToHost, h->copy_stream));
+                h->last_d2h += (int64_t)(N * kFrame * sizeof(float));
             }
-            nd = h->dma_envs;
+            if (nd == 0) CU(cudaMemcpyAsync(h->h_rec + off * 4, h->d_rec + off, (size_t)kc * N * sizeof(uint4), cudaMemcpyDeviceToHost, h->copy_stream));
+            else CU(cudaMemcpy2DAsync(h->h_rec + (off + nd) * 4, N * sizeof(uint4), h->d_rec + off + nd, N * sizeof(uint4), (N - nd) * sizeof(uint4),
+                                      kc, cudaMemcpyDeviceToHost, h->copy_stream));
+            CU(cudaMemcpyAsync(h->h_off + (size_t)k0 * nblk, h->d_off + (size_t)k0 * nblk, (size_t)kc * nblk * sizeof(unsigned),
+                               cudaMemcpyDeviceToHost, h->copy_stream));
+            CU(cudaMemcpyAsync(h->h_count + ci, h->d_count + ci, sizeof(unsigned), cudaMemcpyDeviceToHost, h->copy_stream));
+            // the values: how many there are is only known on the device, so a size that has been enough so far goes
+            // down unasked (a host thread fetches the rest in the rare case that it was not)
+            spec[ci] = std::min((size_t)kc * N * kVarPerStep, (size_t)((double)kc * (N - nd) * h->var_density) + 1024);
+            CU(cudaMemcpyAsync(h->h_var + off * kVarPerStep, h->d_var + off * kVarPerStep, spec[ci] * sizeof(float), cudaMemcpyDeviceToHost,
+                               h->copy_stream));
+            h->last_d2h += (int64_t)kc * (N - nd) * sizeof(uint4) + (int64_t)kc * nblk * sizeof(unsigned) + sizeof(unsigned)
+                           + (int64_t)spec[ci] * sizeof(float);
         }
-        nd = nd >= (int)N ? (int)N : (nd / 32) * 32;
-        if ((size_t)nd * K > h->rows_cap) {
-            cudaFree(h->d_rows);
-            h->d_rows = nullptr; h->rows_cap = 0;
-            CU(cudaMalloc(&h->d_rows, (size_t)nd * K * 2 * kFrame * sizeof(float)));
-            h->rows_cap = (size_t)nd * K;
+        CU(cudaEventRecord(h->copy_done[ci], h->copy_stream));          // what the host threads wait for
+        issued.store(ci + 1, std::memory_order_release);
+        if (nd > 0) {
+            const size_t w = (size_t)nd * row_full * sizeof(float);
+            CU(cudaMemcpy2DAsync(c.obs + off * row_full, N * row_full * sizeof(float), h->d_rows + (size_t)k0 * nd * row_full, w, w, kc,
+                                 cudaMemcpyDeviceToHost, h->copy_stream));
+            if (c.reward) CU(cudaMemcpy2DAsync(c.reward + off, N * sizeof(float), h->d_rew + off, N * sizeof(float), nd * sizeof(float), kc,
+                                               cudaMemcpyDeviceToHost, h->copy_stream));
+            if (c.done) CU(cudaMemcpy2DAsync(c.done + off, N, h->d_done + off, N, nd, kc, cudaMemcpyDeviceToHost, h->copy_stream));
+            h->last_d2h += (int64_t)kc * nd * (row_full * sizeof(float) + (c.reward ? 4 : 0) + (c.done ? 1 : 0));
         }
     }
-    const bool trace = std::getenv("SHIPSIM_HOST_TRACE") != nullptr;
-    if (trace) CU(cudaEventRecord(h->trace0, s));
-    h->last_h2d = (int64_t)(n * sizeof(int32_t));                   // (the actions go up chunk by chunk, ahead of the chunk's kernel)
-    h->last_d2h = 0;
-    // The rollout is cut into chunks of steps: while chunk i+1 is being computed on the caller's stream, the results
-    // of chunk i travel to the host on the copy stream and chunk i-1 is being expanded by the host threads.
-    const size_t row_full = F * h->cfg.history;                     // floats per complete row; chunk regions of d_obs are sized for it
-    float *d_var = h->d_var;
-    if (const char *ev = std::getenv("SHIPSIM_HOST_VAR_DENSITY")) h->var_density = atof(ev);      // (test hook: 0 forces the fetch-the-rest path)
-    size_t spec[shipsim_handle::kMaxChunks] = {};                    // floats of each chunk's value stream copied down unasked
+    return SHIPSIM_OK;
+}
+
+static int step_frames_only(shipsim_t *h, const HostCall &c)
+{
+    const size_t N = c.N, nblk = (N + 31) / 32;
+    const int nd = c.nd;
+    size_t spec[kMaxChunks] = {};
     // Every host thread owns a contiguous range of env blocks for the whole call (the running frames of its envs stay in its
     // cache) and walks the chunks as their records arrive: no barrier between chunks.  Whoever finds the next chunk missing
     // polls its event.  The threads are started BEFORE the stream work is issued (launching 16 chunks of kernels and copies
     // takes the calling thread ~1 ms, a fifth of the call), and the calling thread joins them when it is done.
-    const bool expand = frames_only && nd < (int)N;
-    const bool cut = h->cfg.auto_reset != 0;
+    const bool expand = nd < (int)N;
     const size_t blk0 = (size_t)nd / 32;
     const int jobs = expand ? (int)std::min<size_t>(nblk - blk0, (size_t)h->pool->size()) : 0;
-    std::atomic<int> ready{0};                                       // chunks whose records are in host memory
-    std::atomic<int> issued{0};                                      // chunks whose copies (and event) are in the copy stream
+    std::atomic<int> ready{0};                                   // chunks whose records are in host memory
+    std::atomic<int> issued{0};                                  // chunks whose copies (and event) are in the copy stream
     std::atomic<int> bad{0};
     std::mutex poll, fix;
-    bool fixed[shipsim_handle::kMaxChunks] = {};
+    bool fixed[kMaxChunks] = {};
     std::atomic<long long> extra_d2h{0};
-    const int dev = h->device;
     const std::function<void(int)> worker = [&](int j) {
-        cudaSetDevice(dev);
+        cudaSetDevice(h->device);
         const size_t b0 = blk0 + (nblk - blk0) * (size_t)j / jobs, b1 = blk0 + (nblk - blk0) * (size_t)(j + 1) / jobs;
-        for (int c = 0; c < n_chunks; ++c) {
-            while (ready.load(std::memory_order_acquire) <= c) {
+        for (int ci = 0; ci < c.n_chunks; ++ci) {
+            while (ready.load(std::memory_order_acquire) <= ci) {
                 if (bad.load(std::memory_order_relaxed)) return;
                 if (poll.try_lock()) {
                     const int r = ready.load(std::memory_order_relaxed);
-                    if (r <= c && r < issued.load(std::memory_order_acquire)) {      // (an event not yet recorded by this call reads as complete)
+                    if (r <= ci && r < issued.load(std::memory_order_acquire)) {     // (an event not yet recorded by this call reads as complete)
                         const cudaError_t q = cudaEventQuery(h->copy_done[r]);
                         if (q == cudaSuccess) ready.store(r + 1, std::memory_order_release);
                         else if (q != cudaErrorNotReady) bad.store((int)q);
@@ -991,159 +1062,116 @@ extern "C" int shipsim_step_host(shipsim_t *h, const int32_t *host_actions, int3
                 __builtin_ia32_pause();
 #endif
             }
-            const int k0 = kbeg[c], kc = kbeg[c + 1] - kbeg[c];
-            const size_t off = (size_t)k0 * N;
-            if (h->h_count[c] > spec[c]) {                       // the speculative copy fell short: one thread fetches the rest
+            const size_t off = c.off(ci);
+            if (h->h_count[ci] > spec[ci]) {                     // the speculative copy fell short: one thread fetches the rest
                 std::lock_guard<std::mutex> lk(fix);
-                if (!fixed[c]) {
-                    const size_t at = off * h->var_per_step + spec[c];
-                    cudaError_t q = cudaMemcpyAsync(h->h_var + at, d_var + at, (h->h_count[c] - spec[c]) * sizeof(float), cudaMemcpyDeviceToHost,
+                if (!fixed[ci]) {
+                    const size_t at = off * kVarPerStep + spec[ci];
+                    cudaError_t q = cudaMemcpyAsync(h->h_var + at, h->d_var + at, (h->h_count[ci] - spec[ci]) * sizeof(float), cudaMemcpyDeviceToHost,
                                                     h->aux_stream);
                     if (q == cudaSuccess) q = cudaStreamSynchronize(h->aux_stream);
                     if (q != cudaSuccess) { bad.store((int)q); return; }
-                    extra_d2h.fetch_add((long long)(h->h_count[c] - spec[c]) * (long long)sizeof(float));
-                    fixed[c] = true;
+                    extra_d2h.fetch_add((long long)(h->h_count[ci] - spec[ci]) * (long long)sizeof(float));
+                    fixed[ci] = true;
                 }
             }
-            expand_delta_rows(host_obs + off * row_full, host_reward ? host_reward + off : nullptr, host_done ? host_done + off : nullptr,
-                              h->h_rec + off * 4, h->h_off + (size_t)k0 * nblk, h->h_var + off * h->var_per_step, h->h_cur, kc, N, b0, b1,
-                              h->cfg.step_penalty, cut, 2);
+            expand_delta_rows(c.obs + off * c.row_full, c.reward ? c.reward + off : nullptr, c.done ? c.done + off : nullptr, h->h_rec + off * 4,
+                              h->h_off + (size_t)c.kbeg[ci] * nblk, h->h_var + off * kVarPerStep, h->h_cur, c.kc(ci), N, b0, b1,
+                              h->cfg.step_penalty, h->cfg.auto_reset != 0, 2);
         }
     };
+    if (expand) h->pool->start(jobs, worker);
+    const int rc_issue = issue_frames(h, c, spec, issued);
+    if (!expand) return rc_issue;
+    if (rc_issue) bad.store(-1);
+    h->pool->finish();
+    if (rc_issue) return rc_issue;
+    if (bad.load()) return fail(SHIPSIM_ERR_CUDA, std::string("copy stream: ") + cudaGetErrorString((cudaError_t)bad.load()));
+    h->last_d2h += extra_d2h.load();
+    double dens = 0.0;
+    for (int ci = 0; ci < c.n_chunks; ++ci) dens = std::max(dens, (double)h->h_count[ci] / ((double)c.kc(ci) * (double)(N - nd)));
+    h->var_density = std::max(0.9 * h->var_density, std::min(12.0, 1.25 * dens + 0.25));       // follows the need up at once, down slowly
+    return SHIPSIM_OK;
+}
+
+extern "C" int shipsim_step_host(shipsim_t *h, const int32_t *host_actions, int32_t K, float *host_obs, float *host_reward,
+                                 uint8_t *host_done, void *stream)
+{
+    TRY(ready(h));
+    if (K < 1 || !host_actions) return fail(SHIPSIM_ERR_ARG, "K must be >= 1 and host_actions non-NULL");
+    DeviceGuard g(h->device);
+    h->p.log_call = h->calls++;
+    h->p.log_k0 = 0;
+    const size_t N = (size_t)h->cfg.num_envs, n = N * K, row_full = (size_t)frame_floats(h) * h->cfg.history;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (n * row_full * sizeof(float) <= ((size_t)1 << 16) && host_obs && host_reward && host_done) {
+        // zero copy, when all four buffers are mapped page-locked memory (the aliases of the last call's are remembered)
+        const void *host[4] = {host_actions, host_obs, host_reward, host_done};
+        if (!std::equal(host, host + 4, h->zc_host)) {
+            std::copy(host, host + 4, h->zc_host);
+            for (int i = 0; i < 4; ++i)
+                if (!(h->zc_dev[i] = pointer_info(host[i]).alias)) { std::fill(h->zc_dev, h->zc_dev + 4, nullptr); break; }
+        }
+        if (h->zc_dev[0]) {
+            void *const *dev = h->zc_dev;
+            TRY(step_impl(h, dev[0], SHIPSIM_ACTION_I32, K, (float *)dev[1], (float *)dev[2], (uint8_t *)dev[3], s, h->cfg.history));
+            h->last_h2d = (int64_t)(n * sizeof(int32_t));
+            h->last_d2h = (int64_t)(n * (row_full * sizeof(float) + 5));
+            CU(cudaStreamSynchronize(s));
+            return SHIPSIM_OK;
+        }
+    }
+    // the chunked regimes: staging buffers, the copy and aux streams and the per-chunk events.  A trace reads the times
+    // of the chunk events, so they are created with timing while calls ask for a trace (without, which is cheaper, else).
+    const bool small = n < ((size_t)1 << 16), trace = std::getenv("SHIPSIM_HOST_TRACE") != nullptr;
+    CU(h->d_act.ensure(n));
+    CU(h->d_obs.ensure(n * row_full));
+    CU(h->d_rew.ensure(n));
+    CU(h->d_done.ensure(n));
+    if (!h->act_up) {                                               // (the last of the three to be created)
+        CU(cudaStreamCreateWithFlags(h->copy_stream.out(), cudaStreamNonBlocking));
+        CU(cudaStreamCreateWithFlags(h->aux_stream.out(), cudaStreamNonBlocking));
+        CU(cudaEventCreateWithFlags(h->act_up.out(), cudaEventDisableTiming));
+    }
+    if (h->chunk_events != (int)trace) {
+        for (auto &ev : h->chunk_done) CU(cudaEventCreateWithFlags(ev.out(), trace ? cudaEventDefault : cudaEventDisableTiming));
+        for (auto &ev : h->copy_done) CU(cudaEventCreateWithFlags(ev.out(), trace ? cudaEventDefault : cudaEventDisableTiming));
+        h->chunk_events = (int)trace;
+    }
+    if (trace && !h->trace0) {                                      // (trace0 is created last)
+        for (auto &ev : h->trace_mid) CU(cudaEventCreate(ev.out()));
+        CU(cudaEventCreate(h->trace0.out()));
+    }
+    HostCall c{host_actions, host_obs, host_reward, host_done, s, K, N, n, row_full, small, trace};
+    c.n_chunks = small ? 1 : (K >= 64 ? 16 : (K >= 8 ? 8 : 1));
+    if (const char *ev = std::getenv("SHIPSIM_HOST_CHUNKS")) c.n_chunks = std::max(1, std::min({atoi(ev), kMaxChunks, (int)K}));
+    for (int ci = 0; ci <= c.n_chunks; ++ci) c.kbeg[ci] = (int)((int64_t)K * ci / c.n_chunks);
+    for (int ci = 0; ci < c.n_chunks; ++ci)
+        if (c.kc(ci) <= 0) return fail(SHIPSIM_ERR_ARG, "internal: empty chunk");
+    // (the compacted wire format is that of 16-float frames: other fans take the plain copies)
+    const bool frames_only = h->cfg.history == 2 && host_obs != nullptr && !small && h->cfg.lidar_beams == SHIPSIM_N_BEAMS;
+    if (frames_only) TRY(frames_setup(h, c));
+    if (trace) CU(cudaEventRecord(h->trace0, s));
+    h->last_h2d = (int64_t)(n * sizeof(int32_t));                // (the actions go up chunk by chunk, ahead of the chunk's kernel)
+    h->last_d2h = 0;
+    if (const char *ev = std::getenv("SHIPSIM_HOST_VAR_DENSITY")) h->var_density = atof(ev);      // (test hook: 0 forces the fetch-the-rest path)
     using clk = std::chrono::steady_clock;
     const auto t_begin = clk::now();
-    if (expand) h->pool->start(jobs, worker);
-    const int rc_issue = [&]() -> int {
-        const float4 *prev_frames = h->d_frame0;                        // the frames the next chunk's first step is compared with
-        for (int c = 0; c < n_chunks; ++c) {
-            const int k0 = kbeg[c], kc = kbeg[c + 1] - kbeg[c];
-            if (kc <= 0) continue;
-            const size_t off = (size_t)k0 * N;
-            const int hist_c = frames_only ? 1 : h->cfg.history;
-            float *d_chunk = h->d_obs + off * row_full;
-            if (c == 0) {
-                // the first chunk's actions go up ahead of its kernel; the rest follows on another stream while it runs
-                CU(cudaMemcpyAsync(h->d_act, host_actions, (size_t)kc * N * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-                if (n_chunks > 1) {
-                    CU(cudaEventRecord(h->act_up, s));                   // (orders the copy behind whatever the caller's stream did before)
-                    CU(cudaStreamWaitEvent(h->aux_stream, h->act_up, 0));
-                    CU(cudaMemcpyAsync(h->d_act + (size_t)kc * N, host_actions + (size_t)kc * N, (n - (size_t)kc * N) * sizeof(int32_t),
-                                       cudaMemcpyHostToDevice, h->aux_stream));
-                    CU(cudaEventRecord(h->act_up, h->aux_stream));
-                }
-            } else if (c == 1) CU(cudaStreamWaitEvent(s, h->act_up, 0));
-            h->p.log_k0 = k0;                                       // episode-log records carry the step index within the call
-            const int rc2 = step_impl(h, h->d_act + off, SHIPSIM_ACTION_I32, kc, d_chunk, h->d_rew + off, h->d_done + off, stream, hist_c);
-            h->p.log_k0 = 0;
-            if (rc2) return rc2;
-            if (frames_only && h->p.log_count && h->cfg.history == 2) {     // the one-frame kernel logged the terminal frame only
-                CU(launch_log_prev_frames(h->p, (const float4 *)d_chunk, prev_frames, k0, kc, s));
-                h->launches++;
-            }
-            if (trace) CU(cudaEventRecord(h->trace_mid[c], s));
-            if (frames_only) {
-                if (nd < (int)N) {
-                    CU(launch_compact_frames((const float4 *)d_chunk, prev_frames, h->d_rew + off, h->d_done + off, (int)N, nd, kc, h->cfg.step_penalty,
-                                             h->d_rec + off, h->d_off + (size_t)k0 * nblk, d_var + off * h->var_per_step,
-                                             (unsigned)std::min<size_t>((size_t)kc * N * h->var_per_step, 0xffffffffu), h->d_count + c, s));
-                    h->launches++;
-                }
-                if (nd > 0) {
-                    CU(launch_history_rows((const float4 *)d_chunk, prev_frames, h->d_done + off, (int)N, nd, kc, h->cfg.auto_reset != 0,
-                                           (float4 *)(h->d_rows + (size_t)k0 * nd * row_full), s));
-                    h->launches++;
-                }
-                prev_frames = (const float4 *)d_chunk + ((size_t)(kc - 1) * N) * 4;
-            }
-            cudaStream_t cs = h->copy_stream;
-            if (small) cs = s;                                      // one stream, no event hops
-            else {
-                CU(cudaEventRecord(h->chunk_done[c], s));
-                CU(cudaStreamWaitEvent(h->copy_stream, h->chunk_done[c], 0));
-            }
-            if (frames_only) {
-                if (nd < (int)N) {
-                    if (c == 0) {
-                        CU(cudaMemcpyAsync(h->h_cur, h->d_frame0, N * kFrame * sizeof(float), cudaMemcpyDeviceToHost, h->copy_stream));
-                        h->last_d2h += (int64_t)(N * kFrame * sizeof(float));
-                    }
-                    if (nd == 0) CU(cudaMemcpyAsync(h->h_rec + off * 4, h->d_rec + off, (size_t)kc * N * sizeof(uint4), cudaMemcpyDeviceToHost, h->copy_stream));
-                    else CU(cudaMemcpy2DAsync(h->h_rec + (off + nd) * 4, N * sizeof(uint4), h->d_rec + off + nd, N * sizeof(uint4), (N - nd) * sizeof(uint4),
-                                              kc, cudaMemcpyDeviceToHost, h->copy_stream));
-                    CU(cudaMemcpyAsync(h->h_off + (size_t)k0 * nblk, h->d_off + (size_t)k0 * nblk, (size_t)kc * nblk * sizeof(unsigned),
-                                       cudaMemcpyDeviceToHost, h->copy_stream));
-                    CU(cudaMemcpyAsync(h->h_count + c, h->d_count + c, sizeof(unsigned), cudaMemcpyDeviceToHost, h->copy_stream));
-                    // the values: how many there are is only known on the device, so a size that has been enough so far goes
-                    // down unasked (a host thread fetches the rest in the rare case that it was not)
-                    spec[c] = std::min((size_t)kc * N * h->var_per_step, (size_t)((double)kc * (N - nd) * h->var_density) + 1024);
-                    CU(cudaMemcpyAsync(h->h_var + off * h->var_per_step, d_var + off * h->var_per_step, spec[c] * sizeof(float),
-                                       cudaMemcpyDeviceToHost, h->copy_stream));
-                    h->last_d2h += (int64_t)kc * (N - nd) * sizeof(uint4) + (int64_t)kc * nblk * sizeof(unsigned) + sizeof(unsigned)
-                                   + (int64_t)spec[c] * sizeof(float);
-                }
-                CU(cudaEventRecord(h->copy_done[c], h->copy_stream));       // what the host threads wait for
-                issued.store(c + 1, std::memory_order_release);
-                if (nd > 0) {
-                    const size_t w = (size_t)nd * row_full * sizeof(float);
-                    CU(cudaMemcpy2DAsync(host_obs + off * row_full, N * row_full * sizeof(float), h->d_rows + (size_t)k0 * nd * row_full, w, w, kc,
-                                         cudaMemcpyDeviceToHost, h->copy_stream));
-                    if (host_reward) CU(cudaMemcpy2DAsync(host_reward + off, N * sizeof(float), h->d_rew + off, N * sizeof(float), nd * sizeof(float), kc,
-                                                          cudaMemcpyDeviceToHost, h->copy_stream));
-                    if (host_done) CU(cudaMemcpy2DAsync(host_done + off, N, h->d_done + off, N, nd, kc, cudaMemcpyDeviceToHost, h->copy_stream));
-                    h->last_d2h += (int64_t)kc * nd * (row_full * sizeof(float) + (host_reward ? 4 : 0) + (host_done ? 1 : 0));
-                }
-                continue;
-            } else {
-                h->last_d2h += (int64_t)kc * N * ((host_reward ? 4 : 0) + (host_done ? 1 : 0));
-                if (host_obs) {
-                    h->last_d2h += (int64_t)kc * N * row_full * sizeof(float);
-                    CU(cudaMemcpyAsync(host_obs + off * row_full, d_chunk, (size_t)kc * N * row_full * sizeof(float), cudaMemcpyDeviceToHost, cs));
-                }
-                if (host_reward) CU(cudaMemcpyAsync(host_reward + off, h->d_rew + off, (size_t)kc * N * sizeof(float), cudaMemcpyDeviceToHost, cs));
-                if (host_done) CU(cudaMemcpyAsync(host_done + off, h->d_done + off, (size_t)kc * N, cudaMemcpyDeviceToHost, cs));
-            }
-            if (!small) CU(cudaEventRecord(h->copy_done[c], h->copy_stream));
-        }
-        return SHIPSIM_OK;
-    }();
-    if (expand) {
-        if (rc_issue) bad.store(-1);
-        h->pool->finish();
-    }
-    if (rc_issue) return rc_issue;
-    if (expand) {
-        if (bad.load()) return fail(SHIPSIM_ERR_CUDA, std::string("copy stream: ") + cudaGetErrorString((cudaError_t)bad.load()));
-        h->last_d2h += extra_d2h.load();
-        double dens = 0.0;
-        for (int c = 0; c < n_chunks; ++c) dens = std::max(dens, (double)h->h_count[c] / ((double)(kbeg[c + 1] - kbeg[c]) * (double)(N - nd)));
-        h->var_density = std::max(0.9 * h->var_density, std::min(12.0, 1.25 * dens + 0.25));       // follows the need up at once, down slowly
-    }
+    TRY(frames_only ? step_frames_only(h, c) : step_plain_copies(h, c));
     if (!small) CU(cudaStreamSynchronize(h->copy_stream));
     CU(cudaStreamSynchronize(s));
     if (trace && !small) {
         std::fprintf(stderr, "step_host trace (ms since the call's first stream op): host done %.2f\n",
                      std::chrono::duration<double, std::milli>(clk::now() - t_begin).count());
-        for (int c = 0; c < n_chunks; ++c) {
-            float a = 0.f, b = 0.f;
-            cudaEventElapsedTime(&a, h->trace0, h->chunk_done[c]);
-            cudaEventElapsedTime(&b, h->trace0, h->copy_done[c]);
-            float m = 0.f;
-            cudaEventElapsedTime(&m, h->trace0, h->trace_mid[c]);
-            std::fprintf(stderr, "  chunk %2d: step kernel done %.2f  compaction done %.2f  records home %.2f\n", c, m, a, b);
+        for (int ci = 0; ci < c.n_chunks; ++ci) {
+            float a = 0.f, b = 0.f, m = 0.f;
+            cudaEventElapsedTime(&a, h->trace0, h->chunk_done[ci]);
+            cudaEventElapsedTime(&b, h->trace0, h->copy_done[ci]);
+            cudaEventElapsedTime(&m, h->trace0, h->trace_mid[ci]);
+            std::fprintf(stderr, "  chunk %2d: step kernel done %.2f  compaction done %.2f  records home %.2f\n", ci, m, a, b);
         }
     }
-    if (adaptive) {
-        // The split for the next call climbs towards the shorter call: keep going while the time per env-step improves, turn
-        // round (with half the step) when it gets worse, stay when it no longer changes.
-        const double t = std::chrono::duration<double>(clk::now() - t_begin).count() / (double)n;
-        if (h->dma_last_t > 0.0 && t > h->dma_last_t * 1.015) {
-            h->dma_dir = -h->dma_dir;
-            h->dma_step = std::max(32, h->dma_step / 2 / 32 * 32);
-        }
-        if (h->dma_last_t == 0.0 || t < h->dma_last_t * 0.985 || t > h->dma_last_t * 1.015)
-            h->dma_envs = std::max(0, std::min((int)N, nd + h->dma_dir * h->dma_step));
-        h->dma_last_t = t;
-    }
+    if (c.adaptive) h->dma.update((int)N, c.nd, std::chrono::duration<double>(clk::now() - t_begin).count() / (double)n);
     return SHIPSIM_OK;
 }
 
@@ -1203,8 +1231,7 @@ extern "C" int shipsim_assemble_history(float *host_obs, const float *host_frame
 
 extern "C" int shipsim_stats_read(shipsim_t *h, double *dev_out, int clear, void *stream)
 {
-    const int rc = ready(h);
-    if (rc) return rc;
+    TRY(ready(h));
     if (!dev_out) return fail(SHIPSIM_ERR_ARG, "dev_out is NULL");
     DeviceGuard g(h->device);
     CU(launch_stats_reduce(h->p.stats, dev_out, clear, (cudaStream_t)stream));
@@ -1212,38 +1239,33 @@ extern "C" int shipsim_stats_read(shipsim_t *h, double *dev_out, int clear, void
     return SHIPSIM_OK;
 }
 
+// An env's state as the floats of its planes (plane-major, 4 per plane): pose [0, 6), episode return 6, packed rudder /
+// alive / steps 7, lidar[0, 10) from 8, scenario 18 and episode 19 (int bits), goals [20, 30), 0 at 30 and 31, then
+// lidar[10 ..) from 32.  Readings past the fan hold -1.
+constexpr int kStateFloats = 4 * (kPlanes + (kMaxBeams - kBeams + 3) / 4);
+static int lidar_slot(int j) { return j < kBeams ? 8 + j : 4 * kPlanes + j - kBeams; }
+
 extern "C" int shipsim_set_state(shipsim_t *h, const float *pose, const int32_t *ints, const float *lidar, const float *goals,
                                  const float *ep_return)
 {
-    const int rc = ready(h);
-    if (rc) return rc;
+    TRY(ready(h));
     if (!pose || !ints || !lidar || !goals || !ep_return) return fail(SHIPSIM_ERR_ARG, "NULL argument");
     const size_t N = (size_t)h->cfg.num_envs;
     const int nb = h->cfg.lidar_beams, planes = state_planes(h);
     std::vector<float4> st(N * planes);
     for (size_t e = 0; e < N; ++e) {
-        // lidar[e][lidar_beams]; readings past the fan (planes 2-4 of a fan of fewer than 10 beams) hold -1
-        float l[kBeams + 4 * ((kMaxBeams - kBeams) / 4 + 1)];
-        for (int j = 0; j < (int)(sizeof(l) / sizeof(l[0])); ++j) l[j] = j < nb ? lidar[e * nb + j] : -1.f;
-        const float *q = pose + e * 6, *gl = goals + e * 10;
         const int32_t *in = ints + e * 5;
         if (in[0] % 5 != 0 || in[0] < -10 || in[0] > 10) return fail(SHIPSIM_ERR_ARG, "rudder must be in {-10,-5,0,5,10}");
         if (in[3] < 0 || in[3] >= h->p.n_scen) return fail(SHIPSIM_ERR_ARG, "scenario id out of range");
         const int bits = ((in[0] / 5 + 2) & 7) | ((in[1] & 31) << 3) | (in[2] << 8);
-        float fb, fs, fe;
-        std::memcpy(&fb, &bits, 4); std::memcpy(&fs, &in[3], 4); std::memcpy(&fe, &in[4], 4);
-        st[0 * N + e] = make_float4(q[0], q[1], q[2], q[3]);
-        st[1 * N + e] = make_float4(q[4], q[5], ep_return[e], fb);
-        st[2 * N + e] = make_float4(l[0], l[1], l[2], l[3]);
-        st[3 * N + e] = make_float4(l[4], l[5], l[6], l[7]);
-        st[4 * N + e] = make_float4(l[8], l[9], fs, fe);
-        st[5 * N + e] = make_float4(gl[0], gl[1], gl[2], gl[3]);
-        st[6 * N + e] = make_float4(gl[4], gl[5], gl[6], gl[7]);
-        st[7 * N + e] = make_float4(gl[8], gl[9], 0.f, 0.f);
-        for (int pl = kPlanes; pl < planes; ++pl) {
-            const float *x = l + kBeams + 4 * (pl - kPlanes);
-            st[pl * N + e] = make_float4(x[0], x[1], x[2], x[3]);
-        }
+        float f[kStateFloats] = {};
+        std::copy(pose + e * 6, pose + e * 6 + 6, f);
+        f[6] = ep_return[e];
+        std::memcpy(f + 7, &bits, 4);
+        std::memcpy(f + 18, in + 3, 8);
+        std::copy(goals + e * 10, goals + e * 10 + 10, f + 20);
+        for (int j = 0; j < kBeams + 4 * (planes - kPlanes); ++j) f[lidar_slot(j)] = j < nb ? lidar[e * nb + j] : -1.f;
+        for (int pl = 0; pl < planes; ++pl) std::memcpy(&st[pl * N + e], f + 4 * pl, sizeof(float4));
     }
     DeviceGuard g(h->device);
     CU(cudaDeviceSynchronize());
@@ -1253,8 +1275,7 @@ extern "C" int shipsim_set_state(shipsim_t *h, const float *pose, const int32_t 
 
 extern "C" int shipsim_get_state(shipsim_t *h, float *pose, int32_t *ints, float *lidar, float *goals, float *ep_return)
 {
-    const int rc = ready(h);
-    if (rc) return rc;
+    TRY(ready(h));
     const size_t N = (size_t)h->cfg.num_envs;
     const int nb = h->cfg.lidar_beams, planes = state_planes(h);
     std::vector<float4> st(N * planes);
@@ -1262,31 +1283,26 @@ extern "C" int shipsim_get_state(shipsim_t *h, float *pose, int32_t *ints, float
     CU(cudaDeviceSynchronize());
     CU(cudaMemcpy(st.data(), h->p.state, st.size() * sizeof(float4), cudaMemcpyDeviceToHost));
     for (size_t e = 0; e < N; ++e) {
-        const float4 a = st[0 * N + e], b = st[1 * N + e], l0 = st[2 * N + e], l1 = st[3 * N + e], l2 = st[4 * N + e];
-        const float4 g0 = st[5 * N + e], g1 = st[6 * N + e], g2 = st[7 * N + e];
-        int bits, scen, ep;
-        std::memcpy(&bits, &b.w, 4); std::memcpy(&scen, &l2.z, 4); std::memcpy(&ep, &l2.w, 4);
-        if (pose) { float *q = pose + e * 6; q[0] = a.x; q[1] = a.y; q[2] = a.z; q[3] = a.w; q[4] = b.x; q[5] = b.y; }
-        if (ep_return) ep_return[e] = b.z;
-        if (ints) { int32_t *in = ints + e * 5; in[0] = ((bits & 7) - 2) * 5; in[1] = (bits >> 3) & 31; in[2] = bits >> 8; in[3] = scen; in[4] = ep; }
-        if (lidar) {
-            float l[kBeams + 4 * ((kMaxBeams - kBeams) / 4 + 1)] = {l0.x, l0.y, l0.z, l0.w, l1.x, l1.y, l1.z, l1.w, l2.x, l2.y};
-            for (int pl = kPlanes; pl < planes; ++pl) {
-                const float4 x = st[pl * N + e];
-                float *d = l + kBeams + 4 * (pl - kPlanes);
-                d[0] = x.x; d[1] = x.y; d[2] = x.z; d[3] = x.w;
-            }
-            std::memcpy(lidar + e * nb, l, nb * sizeof(float));
+        float f[kStateFloats];
+        for (int pl = 0; pl < planes; ++pl) std::memcpy(f + 4 * pl, &st[pl * N + e], sizeof(float4));
+        int bits;
+        std::memcpy(&bits, f + 7, 4);
+        if (pose) std::copy(f, f + 6, pose + e * 6);
+        if (ep_return) ep_return[e] = f[6];
+        if (ints) {
+            int32_t *in = ints + e * 5;
+            in[0] = ((bits & 7) - 2) * 5; in[1] = (bits >> 3) & 31; in[2] = bits >> 8;
+            std::memcpy(in + 3, f + 18, 8);
         }
-        if (goals) { float *gl = goals + e * 10; gl[0] = g0.x; gl[1] = g0.y; gl[2] = g0.z; gl[3] = g0.w; gl[4] = g1.x; gl[5] = g1.y; gl[6] = g1.z; gl[7] = g1.w; gl[8] = g2.x; gl[9] = g2.y; }
+        if (lidar) for (int j = 0; j < nb; ++j) lidar[e * nb + j] = f[lidar_slot(j)];
+        if (goals) std::copy(f + 20, f + 30, goals + e * 10);
     }
     return SHIPSIM_OK;
 }
 
 extern "C" int shipsim_render(shipsim_t *h, int32_t env_index, int32_t width, int32_t height, uint8_t *dev_rgb, void *stream)
 {
-    const int rc = ready(h);
-    if (rc) return rc;
+    TRY(ready(h));
     if (env_index < 0 || env_index >= h->cfg.num_envs) return fail(SHIPSIM_ERR_ARG, "env_index out of range");
     if (width < 1 || height < 1 || !dev_rgb) return fail(SHIPSIM_ERR_ARG, "bad image size / NULL buffer");
     DeviceGuard g(h->device);
