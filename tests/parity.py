@@ -214,12 +214,20 @@ def f32_inputs(pose, ints, lidar, goals, ret):
             goals.astype(np.float32).astype(np.float64), ret.astype(np.float32).astype(np.float64))
 
 
-def load_oracle_state(orc, pose, ints, lidar, goals, ret):
+def concat_states(parts):
+    """Injected states (pose, ints, lidar, goals, ret) of several generators -> one state of all their envs, in order."""
+    st = [np.concatenate([np.asarray(p[j]).reshape(len(p[0]), -1) for p in parts]) for j in range(5)]
+    st[4] = st[4].reshape(-1)
+    return tuple(st)
+
+
+def load_oracle_state(orc, pose, ints, lidar, goals, ret, n_beams=10):
+    """Inject a state into the oracle, as env.set_state does into the kernel; lidar [n, n_beams]."""
     n = orc.n
     orc.pose[:] = pose
     orc.ints[:] = ints
     orc.lidar[:] = -1.0
-    orc.lidar[:, :10] = lidar
+    orc.lidar[:, :n_beams] = lidar
     orc.goals[:] = goals.reshape(n, 5, 2)
     orc.ep_return[:] = ret
     # history deque: older frames are unknowable for an injected state; newest frame = current pre-step frame
@@ -237,19 +245,21 @@ def load_oracle_state(orc, pose, ints, lidar, goals, ret):
     has = alive.any(1)
     fr[:, 4] = np.where(has, g[np.arange(n), k, 0], -1.0)
     fr[:, 5] = np.where(has, g[np.arange(n), k, 1], -1.0)
-    fr[:, 6:16] = lidar
+    fr[:, 6:6 + n_beams] = lidar
     orc.hist[:, -F:] = fr
 
 
 def compare_steps(ref, got_obs, got_rew, got_done, margin_thr=1e-3, rel_tol=REL_TOL, label="", scale=600.0,
-                  stop_at_done=False):
+                  stop_at_done=False, n_beams=10):
     """ref: oracle dict of [K,N,...]; got_*: numpy [K,N,...] from the kernel.  An env is compared up to (not
     including) the first step at which any margin drops below `margin_thr` (after a grazing decision the two
-    trajectories may legitimately diverge).  Returns a report dict; raises AssertionError on mismatch."""
+    trajectories may legitimately diverge).  Returns a report dict; raises AssertionError on mismatch.  Frames of
+    6 + n_beams floats; rows of one or two frames."""
     K, N = ref["reward"].shape
     mg = ref["margins"]
     F = got_obs.shape[-1]
-    nb = 10
+    nb = n_beams
+    Fr = 6 + nb                 # floats per frame
     graze = (mg[:, :, :4].min(-1) < margin_thr) | (mg[:, :, M_RAY0:M_RAY0 + nb].min(-1) < margin_thr)
     # valid[k, e]: no grazing at any step <= k
     valid = np.cumsum(graze, axis=0) == 0
@@ -278,11 +288,11 @@ def compare_steps(ref, got_obs, got_rew, got_done, margin_thr=1e-3, rel_tol=REL_
     cond_run = np.maximum.accumulate(cond, axis=0)          # sticky readings keep the cond of the step that wrote them
     lid_tol_scale = np.ones_like(tol)
     lid_abs = np.zeros_like(tol)
-    new0 = F - 16 + 6
+    new0 = F - Fr + 6
     lid_tol_scale[:, :, new0:new0 + nb] = cond_run
     lid_abs[:, :, new0:new0 + nb] = POSE_ABS * scale
-    lid_abs[:, :, F - 16:F - 14] = POSE_ABS * scale          # x, y: sums of O(scale) fp32 terms (cancellation near 0)
-    if F == 32:
+    lid_abs[:, :, F - Fr:F - Fr + 2] = POSE_ABS * scale      # x, y: sums of O(scale) fp32 terms (cancellation near 0)
+    if F == 2 * Fr:
         lid_abs[:, :, 0:2] = POSE_ABS * scale
         prev = np.concatenate([np.ones_like(cond_run[:1]), cond_run[:-1]], axis=0)
         lid_tol_scale[:, :, 6:6 + nb] = prev
@@ -309,5 +319,5 @@ def compare_steps(ref, got_obs, got_rew, got_done, margin_thr=1e-3, rel_tol=REL_
     return dict(compared=n_cmp, total=K * N, eligible=eligible, excluded_frac=1.0 - n_cmp / float(max(1, eligible)),
                 grazing_frac=n_graze / float(max(1, n_cmp + n_graze)), strict_frac=strict_frac,
                 max_rel_err=float((err / np.maximum(1.0, np.abs(ref["obs"])) / lid_tol_scale)[valid].max()) if n_cmp else 0.0,
-                max_pose_rel_err=float((np.maximum(0.0, err - lid_abs) / np.maximum(1.0, np.abs(ref["obs"])))[:, :, F - 16:F - 12][valid].max()) if n_cmp else 0.0,
+                max_pose_rel_err=float((np.maximum(0.0, err - lid_abs) / np.maximum(1.0, np.abs(ref["obs"])))[:, :, F - Fr:F - Fr + 4][valid].max()) if n_cmp else 0.0,
                 frame=F)

@@ -10,16 +10,7 @@ import pytest
 
 import oracle
 import parity
-import parity_beams
-from helpers import pack_bank
-from ship_sim_gym_b200 import ScenarioBank
-
-
-def _bank(n=16, seed=5):
-    d = ScenarioBank.generate(n, (600, 600), seed=seed).as_dict()
-    d["hull_xy"] = d["hull_xy"].astype(np.float32).astype(np.float64)
-    d["goals"] = d["goals"].astype(np.float32).astype(np.float64)
-    return d
+from helpers import fp32_bank, pack_bank
 
 
 @pytest.mark.parametrize("spread", [90.0, 180.0, -120.0])
@@ -27,7 +18,7 @@ def test_twenty_beams_contain_the_ten_beam_fan(spread):
     """Ray 2i of a 20-beam fan has the angle of ray i of the 10-beam fan (delta halves, the start stays): over 32
     auto-reset steps from near-bank states its readings equal the 10-beam run's, and nothing else changes."""
     n, K = 512, 32
-    bank = _bank()
+    bank = fp32_bank(16, 600, 600, seed=5)
     rng = np.random.RandomState(1)
     pose, ints, lidar, goals, ret = parity.f32_inputs(*parity.random_states(rng, n, 600, 600, 16, bank["goals"],
                                                                             near=(bank["hull_xy"], bank["hull_n"])))
@@ -38,7 +29,7 @@ def test_twenty_beams_contain_the_ten_beam_fan(spread):
     for nb, li in ((10, lidar), (20, lidar20)):
         orc = oracle.OracleEnv(n, bank, n_beams=nb, lidar_spread_deg=spread, auto_reset=True, seed=3)
         orc.reset()
-        parity_beams.load_oracle_state(orc, pose, ints, li, goals, ret, n_beams=nb)
+        parity.load_oracle_state(orc, pose, ints, li, goals, ret, n_beams=nb)
         out[nb] = (orc.step(acts), orc.pose.copy(), orc.ints.copy())
     (r10, p10, i10), (r20, p20, i20) = out[10], out[20]
     o10, o20 = r10["obs"].reshape(K, n, 2, 16), r20["obs"].reshape(K, n, 2, 26)
@@ -65,7 +56,7 @@ def test_single_ray_against_a_hand_computed_hit():
     x, y = 300.0, 200.0
     pose = np.array([[x, y, 0.0, 0.0, 0.0, 0.0]])
     ints = np.array([[0, 31, 0, 0, 0]], dtype=np.int32)
-    parity_beams.load_oracle_state(orc, pose, ints, np.array([[-1.0]]), goals.reshape(1, 10), np.zeros(1), n_beams=1)
+    parity.load_oracle_state(orc, pose, ints, np.array([[-1.0]]), goals.reshape(1, 10), np.zeros(1), n_beams=1)
     hx, hy = parity.lidar_origin_offset(np.zeros(1))
     ang = np.radians(90.0 - spread / 2.0)
     expect = (260.0 - (y + hy[0])) / np.sin(ang)
@@ -79,7 +70,7 @@ def test_single_ray_against_a_hand_computed_hit():
 @pytest.mark.parametrize("nb", [1, 7, 32])
 def test_reset_observation_layout(nb):
     """ShipEnv.reset for n beams: [-1 x (6 + n) | x, y, 0, 0, gx, gy, -1 x n] (ship_env.py:180-184)."""
-    bank = _bank(4)
+    bank = fp32_bank(4, 600, 600, seed=5)
     orc = oracle.OracleEnv(3, bank, n_beams=nb)
     obs = orc.reset()
     assert obs.shape == (3, 2 * (6 + nb))

@@ -8,13 +8,9 @@ pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
 
 import oracle  # noqa: E402
+from helpers import fp32_bank  # noqa: E402
 import parity  # noqa: E402
-
-
-def _bank(n=16, seed=4):
-    from ship_sim_gym_b200 import ScenarioBank
-    b = ScenarioBank.generate(n, (600, 600), seed=seed)
-    return ScenarioBank(b.hull_xy.astype(np.float32), b.hull_n, b.goals.astype(np.float32), b.bounds)
+from ship_sim_gym_b200 import ScenarioBank  # noqa: E402
 
 
 def test_vec_env_protocol_and_auto_reset_obs():
@@ -22,7 +18,7 @@ def test_vec_env_protocol_and_auto_reset_obs():
     reset obs; reward / done are those of the terminal step.  Checked against the oracle with auto-reset."""
     from ship_sim_gym_b200.adapters import ShipVecEnv
     n, T = 256, 60
-    bank = _bank()
+    bank = ScenarioBank(bounds=(600, 600), **fp32_bank(16, 600, 600, seed=4))
     venv = ShipVecEnv(n, bank=bank, seed=9)
     orc = oracle.OracleEnv(n, bank.as_dict(), auto_reset=True, seed=9)
     assert venv.num_envs == n and venv.action_space.n == 3 and venv.observation_space.shape == (32,)
@@ -53,7 +49,7 @@ def test_vec_env_protocol_and_auto_reset_obs():
 def test_vector_env_protocol_reset_at():
     from ship_sim_gym_b200.adapters import ShipVectorEnv
     n = 8
-    env = ShipVectorEnv(n, bank=_bank(), seed=2)
+    env = ShipVectorEnv(n, bank=ScenarioBank(bounds=(600, 600), **fp32_bank(16, 600, 600, seed=4)), seed=2)
     obs = env.vector_reset()
     assert len(obs) == n and obs[0].shape == (32,) and (obs[0][:16] == -1).all()
     done_seen = False
@@ -80,7 +76,7 @@ def test_random_agent_script_shape():
 
     class GC(GameConfig):
         SPEED = 30              # big steps so that episodes end quickly
-    env = ShipEnv(GC, EnvConfig, bank=_bank(), seed=0)
+    env = ShipEnv(GC, EnvConfig, bank=ScenarioBank(bounds=(600, 600), **fp32_bank(16, 600, 600, seed=4)), seed=0)
     env.seed(0)
     env.reset()
     episodes = 0
@@ -102,7 +98,7 @@ def test_policy_rollout_graph_replay_matches_eager():
     from ship_sim_gym_b200 import BatchedShipEnv
     from ship_sim_gym_b200.rollout import MlpPolicy, RolloutCollector
     n, T = 2048, 16
-    bank = _bank(32)
+    bank = ScenarioBank(bounds=(600, 600), **fp32_bank(32, 600, 600, seed=4))
     torch.manual_seed(0)
     policy = MlpPolicy().cuda()
     out = []
@@ -139,7 +135,7 @@ def test_policy_kernel_matches_the_torch_module(n):
     policy = MlpPolicy().cuda()
     for lin in (policy.pi[4], policy.vf[4]):                      # livelier heads than the default init
         lin.weight.data.mul_(4.0)
-    env = BatchedShipEnv(n, bank=_bank(8), seed=1)
+    env = BatchedShipEnv(n, bank=ScenarioBank(bounds=(600, 600), **fp32_bank(8, 600, 600, seed=4)), seed=1)
     col = RolloutCollector(env, policy, T=2, use_graph=False)
     assert col._kernel
     obs = torch.rand(n, 32, device="cuda") * 600.0
@@ -191,7 +187,7 @@ def test_curriculum_driver_on_a_live_batch():
     time-out statistics follow it."""
     from ship_sim_gym_b200 import BatchedShipEnv, Curriculum, CurriculumDriver
     n = 1024
-    env = BatchedShipEnv(n, bank=_bank(), seed=0)
+    env = BatchedShipEnv(n, bank=ScenarioBank(bounds=(600, 600), **fp32_bank(16, 600, 600, seed=4)), seed=0)
     cur = Curriculum([5, 12], [-10.0], repeat_condition=0)            # any mean return > -10 passes
     drv = CurriculumDriver(env, cur, knob="max_steps", min_episodes=n)
     env.reset()

@@ -8,29 +8,26 @@ pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
 
 import oracle  # noqa: E402
+from helpers import fp32_bank, knobs, make_env, make_oracle  # noqa: E402
 import parity  # noqa: E402
-from test_gpu_parity import _bank, _make_pair  # noqa: E402
 
 
 @pytest.mark.parametrize("lanes,window", [(1, 1), (8, 1), (0, 16)])
 def test_goal_at_radius_plus_minus_eps(lanes, window):
     """collide_goal (game.py:243-257) fires iff distance(goal centre, ship polygon) <= 5: goals placed 2e-3 ... 1e-2
     inside and outside that shell, off edges and off vertices, must be classified exactly as the oracle does."""
-    from ship_sim_gym_b200 import BatchedShipEnv, ScenarioBank
     W = H = 600
     n = 4096 + 7
-    bank = _bank(8, W, H, seed=2)
+    bank = fp32_bank(8, W, H, seed=2)
     rng = np.random.RandomState(17)
     pose, ints, lidar, goals, ret, delta = parity.goal_shell_states(rng, n, W, H, 8)
     st = parity.f32_inputs(pose, ints, lidar, goals, ret)
     if window > 1:          # the time-parallel kernel needs a rollout of at least one window
-        sb = ScenarioBank(bank["hull_xy"], bank["hull_n"], bank["goals"], (W, H))
-        env = BatchedShipEnv(n, bank=sb, auto_reset=False, seed=0, steps_in_flight=window)
-        orc = oracle.OracleEnv(n, bank, W=W, H=H, auto_reset=False, seed=0)
-        K = window
+        env = make_env(knobs(), n, bank, auto_reset=False, steps_in_flight=window)
     else:
-        env, orc = _make_pair(n, bank, W, H, 10, 2, auto_reset=False, lanes=lanes)
-        K = 1
+        env = make_env(knobs(), n, bank, auto_reset=False, lanes_per_env=lanes)
+    orc = make_oracle(knobs(), n, bank)
+    K = window
     env.reset()
     orc.reset()
     env.set_state(*st)
@@ -56,12 +53,12 @@ def test_ray_origin_inside_a_bank(lanes):
     LiDAR.query stores the full ray length for every beam (App. B Q11, App. C4)."""
     W = H = 600
     n = 4096 - 3
-    bank = _bank(32, W, H, seed=4)
+    bank = fp32_bank(32, W, H, seed=4)
     rng = np.random.RandomState(23)
     pose, ints, lidar, which = parity.origin_inside_bank_states(rng, n, bank["hull_xy"], bank["hull_n"], 32)
     goals = bank["goals"][ints[:, 3]].reshape(n, 10)
     st = parity.f32_inputs(pose, ints, lidar, goals, np.zeros(n))
-    env, orc = _make_pair(n, bank, W, H, 10, 2, auto_reset=False, lanes=lanes)
+    env, orc = make_env(knobs(), n, bank, auto_reset=False, lanes_per_env=lanes), make_oracle(knobs(), n, bank)
     env.reset()
     orc.reset()
     env.set_state(*st)

@@ -3,9 +3,6 @@
 The wide kernel is the tuned kernel's code with a 32-reading frame slot and the beam count read at run time, so besides
 the float64 oracle it is held to the tuned kernel itself: lidar feeds nothing back into the dynamics, so for the same
 seed, actions and map every non-lidar output must equal the 10-beam run's bit for bit."""
-import functools
-import os
-
 import numpy as np
 import pytest
 
@@ -13,47 +10,11 @@ pytestmark = pytest.mark.gpu
 
 torch = pytest.importorskip("torch")
 
-import oracle  # noqa: E402
+from helpers import ORACLE_THREADS, assert_same, config_classes, fp32_bank, knobs, make_env, make_oracle, run  # noqa: E402
 import parity  # noqa: E402
-import parity_beams  # noqa: E402
-from test_gpu_parity import _bank  # noqa: E402
-from test_gpu_window import _assert_same, _run as _wrun  # noqa: E402
 
-N_THREADS = max(1, min(16, os.cpu_count() or 1))
 BEAMS = [1, 3, 7, 11, 16, 20, 32]                   # 32, 10, 4, 2, 2, 1 and 1 envs per ray pass
 SPREADS = [90.0, 180.0, 360.0, -120.0]
-
-
-def _cfgs(nb, spread=90.0, hist=2, max_steps=1000):
-    from ship_sim_gym_b200.config import EnvConfig, LidarConfig
-
-    class LC(LidarConfig):
-        N_BEAMS = nb
-        DISTANCE = 100
-        ANGULAR_SPREAD = spread
-
-    class EC(EnvConfig):
-        HISTORY_SIZE = hist
-        MAX_STEPS = max_steps
-        LIDAR_CONFIG = LC
-    return EC
-
-
-def make_env(n, bank, nb, spread=90.0, hist=2, max_steps=1000, **kw):
-    from ship_sim_gym_b200 import BatchedShipEnv, ScenarioBank
-    b = bank if isinstance(bank, ScenarioBank) else ScenarioBank(bank["hull_xy"], bank["hull_n"], bank["goals"], (600.0, 600.0))
-    env = BatchedShipEnv(n, None, _cfgs(nb, spread, hist, max_steps), bank=b, honour_lidar_config=True, **kw)
-    assert env.n_beams == nb and env.cfg.lidar_beams == nb and env.n_states == 6 + nb
-    return env
-
-
-def make_oracle(n, bank, nb, spread=90.0, hist=2, **kw):
-    return oracle.OracleEnv(n, bank, n_beams=nb, lidar_spread_deg=spread, history=hist, n_threads=N_THREADS, **kw)
-
-
-@functools.lru_cache(maxsize=None)
-def bank_of(seed, map_N=10, wf=0.5):
-    return _bank(64, 600, 600, seed=seed, map_N=map_N, wf=wf)
 
 
 def widen(lidar, nb, rng):
@@ -67,7 +28,7 @@ def widen(lidar, nb, rng):
 
 def injected(nb, n, seed):
     """Random states, ships near a bank vertex and lidar origins inside a bank, with nb injected readings each."""
-    bank = bank_of(3)
+    bank = fp32_bank(64, 600, 600, seed=3)
     rng = np.random.RandomState(seed)
     q = n // 3
     near = (bank["hull_xy"], bank["hull_n"])
@@ -76,9 +37,7 @@ def injected(nb, n, seed):
     m = n - 2 * q
     p, i, li, _ = parity.origin_inside_bank_states(rng, m, bank["hull_xy"], bank["hull_n"], 64)
     parts.append((p, i, li, bank["goals"][i[:, 3]].reshape(m, 10), np.zeros(m)))
-    st = [np.concatenate([np.asarray(pp[j]).reshape(len(pp[0]), -1) for pp in parts]) for j in range(5)]
-    st[4] = st[4].reshape(-1)
-    pose, ints, lidar, goals, ret = parity.f32_inputs(*st)
+    pose, ints, lidar, goals, ret = parity.f32_inputs(*parity.concat_states(parts))
     return bank, (pose, ints, widen(lidar, nb, rng), goals, ret), rng.randint(0, 3, n).astype(np.int32)
 
 
@@ -89,16 +48,17 @@ def injected(nb, n, seed):
 def test_wide_single_step_against_oracle(nb, spread, lanes):
     n = 4096 - 5
     bank, st, acts = injected(nb, n, 7 + nb)
-    orc = make_oracle(n, bank, nb, spread)
-    parity_beams.load_oracle_state(orc, *st, n_beams=nb)
+    k = knobs(n_beams=nb, spread=spread)
+    orc = make_oracle(k, n, bank, n_threads=ORACLE_THREADS)
+    parity.load_oracle_state(orc, *st, n_beams=nb)
     ref = orc.step(acts[None])
-    env = make_env(n, bank, nb, spread, auto_reset=False, lanes_per_env=lanes)
+    env = make_env(k, n, bank, auto_reset=False, lanes_per_env=lanes)
     env.reset()
     env.set_state(*st)
     o, r, d, _ = env.step(torch.tensor(acts, device=env.device))
     assert o.shape == (n, 2 * (6 + nb))
     o, r, d = o.cpu().numpy()[None], r.cpu().numpy()[None], d.cpu().numpy()[None]
-    rep = parity_beams.compare_steps(ref, o, r, d, label="nb=%d spread=%g" % (nb, spread), n_beams=nb)
+    rep = parity.compare_steps(ref, o, r, d, label="nb=%d spread=%g" % (nb, spread), n_beams=nb)
     assert rep["excluded_frac"] < 0.01 and rep["max_pose_rel_err"] < 2 * parity.REL_TOL, rep
     lid = o[0, :, -nb:]
     assert (lid[n - n // 3:] == 100.0).mean() > 0.5        # origins inside a bank: full-length readings
@@ -119,17 +79,18 @@ STAT_KEYS = ("episodes", "collision", "oob", "timeout", "all_goals", "length_sum
 def test_wide_rollout_against_oracle(nb, spread):
     n, K = 2048 + 3, 32
     hist = 1 if nb in (3, 20) else 2
-    bank = bank_of(7)
+    bank = fp32_bank(64, 600, 600, seed=7)
+    k = knobs(n_beams=nb, spread=spread, hist=hist)
     acts = np.random.RandomState(21).choice([0, 0, 1, 2], size=(K, n)).astype(np.int32)
-    orc = make_oracle(n, bank, nb, spread, hist=hist, auto_reset=True, seed=11)
+    orc = make_oracle(k, n, bank, auto_reset=True, seed=11, n_threads=ORACLE_THREADS)
     orc.reset()
     ref = orc.step(acts)
     so = orc.stats_dict()
-    env = make_env(n, bank, nb, spread, hist=hist, auto_reset=True, seed=11, steps_in_flight=1)
+    env = make_env(k, n, bank, auto_reset=True, seed=11, steps_in_flight=1)
     env.reset()
     obs, rew, done = [t.cpu().numpy() for t in env.rollout(torch.tensor(acts, device=env.device))]
     assert obs.shape == (K, n, hist * (6 + nb))
-    rep = parity_beams.compare_steps(ref, obs, rew, done, margin_thr=parity.MARGIN_THR, label="nb=%d" % nb, n_beams=nb)
+    rep = parity.compare_steps(ref, obs, rew, done, margin_thr=parity.MARGIN_THR, label="nb=%d" % nb, n_beams=nb)
     assert rep["grazing_frac"] < parity.MAX_EXCLUDED and rep["excluded_frac"] < parity.MAX_EXCLUDED_CUMULATIVE, rep
     assert rep["max_pose_rel_err"] < 2 * parity.REL_TOL
     s = env.stats()
@@ -140,16 +101,6 @@ def test_wide_rollout_against_oracle(nb, spread):
 
 
 # ---------------------------------------------------------------------------------------------- physics untouched
-def _run(env, acts, K, st=None):
-    env.reset()
-    if st is not None:
-        env.set_state(*st)
-    s0 = env.stats_tensor().clone()
-    out = [t.cpu().numpy() for t in env.rollout(acts, K=K)]
-    torch.cuda.synchronize()
-    return out, env.get_state(), (env.stats_tensor() - s0).cpu().numpy(), env.launch_info()
-
-
 def _non_lidar(obs, nb, hist):
     F = 6 + nb
     return obs.reshape(obs.shape[0], obs.shape[1], hist, F)[..., :6]
@@ -158,36 +109,38 @@ def _non_lidar(obs, nb, hist):
 @pytest.mark.parametrize("hist", [1, 2])
 def test_physics_bit_identical_to_the_ten_beam_kernel(hist):
     n, K = 3000, 40
-    bank = bank_of(5)
+    bank = fp32_bank(64, 600, 600, seed=5)
     rng = np.random.RandomState(2)
     pose, ints, lidar, goals, ret = parity.f32_inputs(*parity.random_states(rng, n, 600, 600, 64, bank["goals"], near=(bank["hull_xy"], bank["hull_n"])))
     acts = torch.tensor(rng.choice([0, 0, 1, 2], size=(K, n)).astype(np.int32), device="cuda")
-    (o10, r10, d10), s10, t10, _ = _run(make_env(n, bank, 10, hist=hist, seed=9, lanes_per_env=4, max_steps=60), acts, K,
-                                         (pose, ints, lidar, goals, ret))
+    (o10, r10, d10), s10, t10, _ = run(make_env(knobs(hist=hist, max_steps=60), n, bank, seed=9, lanes_per_env=4), acts, K,
+                                        (pose, ints, lidar, goals, ret))
     for nb in BEAMS:
-        (o, r, d), s, t, info = _run(make_env(n, bank, nb, hist=hist, seed=9, lanes_per_env=4, max_steps=60), acts, K,
-                                     (pose, ints, widen(lidar, nb, rng), goals, ret))
+        (o, r, d), s, t, info = run(make_env(knobs(n_beams=nb, hist=hist, max_steps=60), n, bank, seed=9, lanes_per_env=4), acts, K,
+                                    (pose, ints, widen(lidar, nb, rng), goals, ret))
         assert info["steps_in_flight"] == 1
         assert np.array_equal(_non_lidar(o, nb, hist), _non_lidar(o10, 10, hist)), nb
         assert np.array_equal(r, r10) and np.array_equal(d, d10), nb
         for key in ("pose", "ints", "goals", "ep_return"):
             assert np.array_equal(s[key], s10[key]), (nb, key)
-        assert np.array_equal(np.delete(t, 1), np.delete(t10, 1)), nb      # counts and lengths
-        assert t[1] == pytest.approx(t10[1], rel=1e-9)                      # return sum (cross-CTA atomics: any order)
+        counts = [key for key in t if key != "return_sum"]
+        assert [t[key] for key in counts] == [t10[key] for key in counts], nb           # counts and lengths
+        assert t["return_sum"] == pytest.approx(t10["return_sum"], rel=1e-9)           # cross-CTA atomics: any order
     assert d10.sum() > n // 4
 
 
 @pytest.mark.parametrize("spread", [90.0, 180.0])
 def test_twenty_beam_even_slots_match_the_tuned_kernel(spread):
     n, K = 4096, 32
-    bank = bank_of(9)
+    bank = fp32_bank(64, 600, 600, seed=9)
     rng = np.random.RandomState(4)
     pose, ints, lidar, goals, ret = parity.f32_inputs(*parity.random_states(rng, n, 600, 600, 64, bank["goals"], near=(bank["hull_xy"], bank["hull_n"])))
     l20 = np.full((n, 20), -1.0)
     l20[:, 0::2] = lidar
     acts = torch.tensor(rng.choice([0, 0, 1, 2], size=(K, n)).astype(np.int32), device="cuda")
-    (o10, _, _), _, _, _ = _run(make_env(n, bank, 10, spread, seed=3, steps_in_flight=1), acts, K, (pose, ints, lidar, goals, ret))
-    (o20, _, _), _, _, _ = _run(make_env(n, bank, 20, spread, seed=3, steps_in_flight=1), acts, K, (pose, ints, l20, goals, ret))
+    (o10, _, _), _, _, _ = run(make_env(knobs(spread=spread), n, bank, seed=3, steps_in_flight=1), acts, K, (pose, ints, lidar, goals, ret))
+    (o20, _, _), _, _, _ = run(make_env(knobs(n_beams=20, spread=spread), n, bank, seed=3, steps_in_flight=1), acts, K,
+                               (pose, ints, l20, goals, ret))
     a = o10.reshape(K, n, 2, 16)[..., 6:].astype(np.float64)
     b = o20.reshape(K, n, 2, 26)[..., 6::2].astype(np.float64)
     # the two fans' rays agree to an ulp of the angle: within the lidar tolerance at the worst conditioning seen
@@ -201,18 +154,19 @@ def test_twenty_beam_even_slots_match_the_tuned_kernel(spread):
 @pytest.mark.parametrize("nb", [7, 32])
 def test_lanes_launches_and_sharding_are_invisible(nb):
     n, K = 1500, 36
-    bank = bank_of(11)
+    bank = fp32_bank(64, 600, 600, seed=11)
+    k = knobs(n_beams=nb, max_steps=40)
     rng = np.random.RandomState(8)
     pose, ints, lidar, goals, ret = parity.f32_inputs(*parity.random_states(rng, n, 600, 600, 64, bank["goals"], near=(bank["hull_xy"], bank["hull_n"])))
     st = (pose, ints, widen(lidar, nb, rng), goals, ret)
     acts = torch.tensor(rng.choice([0, 0, 1, 2], size=(K, n)).astype(np.int32), device="cuda")
-    ref = _wrun(make_env(n, bank, nb, seed=6, lanes_per_env=1, max_steps=40), acts, K, st)
+    ref = run(make_env(k, n, bank, seed=6, lanes_per_env=1), acts, K, st)
     for g in (2, 4, 8, 16, 32):
-        got = _wrun(make_env(n, bank, nb, seed=6, lanes_per_env=g, max_steps=40), acts, K, st)
+        got = run(make_env(k, n, bank, seed=6, lanes_per_env=g), acts, K, st)
         assert got[3]["lanes_per_env"] == g
-        _assert_same(got, ref, "nb=%d lanes=%d" % (nb, g))
+        assert_same(got, ref, "nb=%d lanes=%d" % (nb, g))
     # K launches of one step = one launch of K steps
-    env = make_env(n, bank, nb, seed=6, lanes_per_env=8, max_steps=40)
+    env = make_env(k, n, bank, seed=6, lanes_per_env=8)
     env.reset()
     env.set_state(*st)
     rows = [[t.cpu().numpy() for t in env.rollout(acts[k:k + 1])] for k in range(K)]
@@ -222,8 +176,8 @@ def test_lanes_launches_and_sharding_are_invisible(nb):
     h = n // 2
     parts = []
     for lo, hi in ((0, h), (h, n)):
-        e = make_env(hi - lo, bank, nb, seed=6, lanes_per_env=2, max_steps=40, env_id_offset=lo)
-        parts.append(_wrun(e, acts[:, lo:hi].contiguous(), K, tuple(np.asarray(x)[lo:hi] for x in st)))
+        e = make_env(k, hi - lo, bank, seed=6, lanes_per_env=2, env_id_offset=lo)
+        parts.append(run(e, acts[:, lo:hi].contiguous(), K, tuple(np.asarray(x)[lo:hi] for x in st)))
     for j in range(3):
         assert np.array_equal(np.concatenate([p[0][j] for p in parts], axis=1), ref[0][j])
     assert ref[0][2].sum() > 0
@@ -232,45 +186,46 @@ def test_lanes_launches_and_sharding_are_invisible(nb):
 def test_full_size_build_against_small_build_and_oracle():
     """262,144 envs at one lane each: the 128-thread G = 1 build with its 68 KB of dynamic shared memory."""
     nb, n, K = 32, 262144, 8
-    bank = bank_of(5)
-    big = make_env(n, bank, nb, seed=12, lanes_per_env=1)
-    small = make_env(n, bank, nb, seed=12, lanes_per_env=2)
-    a = _wrun(big, None, K)
-    b = _wrun(small, None, K)
+    bank = fp32_bank(64, 600, 600, seed=5)
+    k = knobs(n_beams=nb)
+    big = make_env(k, n, bank, seed=12, lanes_per_env=1)
+    small = make_env(k, n, bank, seed=12, lanes_per_env=2)
+    a = run(big, None, K)
+    b = run(small, None, K)
     assert a[3]["threads_per_cta"] == 128 and a[3]["lanes_per_env"] == 1
-    _assert_same(a, b, "full size")
+    assert_same(a, b, "full size")
     sub = 4096
-    orc = make_oracle(n, bank, nb, auto_reset=True, seed=12)
+    orc = make_oracle(k, n, bank, auto_reset=True, seed=12, n_threads=ORACLE_THREADS)
     orc.reset()
     ref = orc.step(None, K=K)
-    rep = parity_beams.compare_steps({k: v[:, :sub] for k, v in ref.items()}, a[0][0][:, :sub], a[0][1][:, :sub], a[0][2][:, :sub],
+    rep = parity.compare_steps({key: v[:, :sub] for key, v in ref.items()}, a[0][0][:, :sub], a[0][1][:, :sub], a[0][2][:, :sub],
                                margin_thr=parity.MARGIN_THR, label="full size", n_beams=nb)
     assert rep["excluded_frac"] < parity.MAX_EXCLUDED_CUMULATIVE, rep
 
 
 def test_auto_selection_runs_the_serial_kernel():
-    env = make_env(4096, bank_of(1), 16)
+    env = make_env(knobs(n_beams=16), 4096, fp32_bank(64, 600, 600, seed=1))
     env.reset()
     env.rollout(None, K=64)
     torch.cuda.synchronize()
     assert env.launch_info()["steps_in_flight"] == 1
-    from ship_sim_gym_b200 import BatchedShipEnv
     with pytest.raises(NotImplementedError, match="steps_in_flight"):
-        BatchedShipEnv(64, None, _cfgs(16), honour_lidar_config=True, steps_in_flight=8, n_scenarios=4)
+        make_env(knobs(n_beams=16), 64, None, steps_in_flight=8, n_scenarios=4)
 
 
 # ---------------------------------------------------------------------------------------------- surfaces
 @pytest.mark.parametrize("hist", [1, 2])
 def test_episode_log_rows_equal_no_reset_rows(hist):
     nb, n, K = 32, 700, 64
-    bank = bank_of(13)
+    bank = fp32_bank(64, 600, 600, seed=13)
     rng = np.random.RandomState(3)
     pose, ints, lidar, goals, ret = parity.f32_inputs(*parity.random_states(rng, n, 600, 600, 64, bank["goals"], max_steps=200,
                                                                             near=(bank["hull_xy"], bank["hull_n"])))
     st = (pose, ints, widen(lidar, nb, rng), goals, ret)
     acts = torch.tensor(rng.choice([0, 0, 1, 2], size=(K, n)).astype(np.int32), device="cuda")
-    ref = make_env(n, bank, nb, hist=hist, max_steps=200, auto_reset=False, seed=5, lanes_per_env=4)
-    got = make_env(n, bank, nb, hist=hist, max_steps=200, auto_reset=True, seed=5, lanes_per_env=4)
+    k = knobs(n_beams=nb, hist=hist, max_steps=200)
+    ref = make_env(k, n, bank, auto_reset=False, seed=5, lanes_per_env=4)
+    got = make_env(k, n, bank, auto_reset=True, seed=5, lanes_per_env=4)
     got.enable_episode_log(K * n)
     outs = []
     for e in (ref, got):
@@ -294,8 +249,8 @@ def test_episode_log_rows_equal_no_reset_rows(hist):
 @pytest.mark.parametrize("n,K", [(8, 1), (5000, 40)])
 def test_step_host_equals_device_rollout(n, K):
     nb = 20
-    bank = bank_of(2)
-    envs = [make_env(n, bank, nb, seed=1, max_steps=50) for _ in range(2)]
+    bank = fp32_bank(64, 600, 600, seed=2)
+    envs = [make_env(knobs(n_beams=nb, max_steps=50), n, bank, seed=1) for _ in range(2)]
     for e in envs:
         e.reset()
     rng = np.random.RandomState(4)
@@ -312,17 +267,18 @@ def test_step_host_equals_device_rollout(n, K):
 
 def test_history_three_against_oracle():
     nb, n, K = 16, 1024, 24
-    bank = bank_of(7)
+    bank = fp32_bank(64, 600, 600, seed=7)
+    k = knobs(n_beams=nb, hist=3, max_steps=30)
     acts = np.random.RandomState(5).choice([0, 0, 1, 2], size=(K, n)).astype(np.int32)
-    orc = make_oracle(n, bank, nb, hist=3, auto_reset=True, seed=2, max_steps=30)
+    orc = make_oracle(k, n, bank, auto_reset=True, seed=2, n_threads=ORACLE_THREADS)
     orc.reset()
     ref = orc.step(acts)
-    env = make_env(n, bank, nb, hist=3, auto_reset=True, seed=2, max_steps=30)
+    env = make_env(k, n, bank, auto_reset=True, seed=2)
     env.reset()
     obs, rew, done = [t.cpu().numpy() for t in env.rollout(torch.tensor(acts, device=env.device))]
     assert obs.shape == (K, n, 3 * 22)
     # compare_steps knows the 1- and 2-frame layouts: hold the newest two frames to it, the oldest to the one before
-    rep = parity_beams.compare_steps(dict(ref, obs=ref["obs"][..., 22:]), obs[..., 22:], rew, done, margin_thr=parity.MARGIN_THR,
+    rep = parity.compare_steps(dict(ref, obs=ref["obs"][..., 22:]), obs[..., 22:], rew, done, margin_thr=parity.MARGIN_THR,
                                label="hist3", n_beams=nb)
     assert rep["excluded_frac"] < parity.MAX_EXCLUDED_CUMULATIVE, rep
     assert np.array_equal(obs[1:, :, :22], np.where(done[1:, :, None].astype(bool), -1.0, obs[:-1, :, 22:44]).astype(np.float32))
@@ -331,7 +287,7 @@ def test_history_three_against_oracle():
 
 def test_state_round_trip_and_render():
     nb, n = 32, 64
-    env = make_env(n, bank_of(1), nb, seed=1)
+    env = make_env(knobs(n_beams=nb), n, fp32_bank(64, 600, 600, seed=1), seed=1)
     env.reset()
     env.rollout(None, K=20)
     s = env.get_state()
@@ -363,7 +319,8 @@ def test_state_round_trip_and_render():
 def test_vec_env_episode_info_at_32_beams():
     from ship_sim_gym_b200.adapters import ShipVecEnv
     n = 128
-    vec = ShipVecEnv(n, episode_info=True, seed=8, n_scenarios=32, env_config=_cfgs(32, max_steps=30), honour_lidar_config=True)
+    vec = ShipVecEnv(n, episode_info=True, seed=8, n_scenarios=32, env_config=config_classes(knobs(n_beams=32, max_steps=30))[1],
+                     honour_lidar_config=True)
     obs = vec.reset()
     assert obs.shape == (n, 76)
     rng = np.random.RandomState(1)
@@ -388,7 +345,7 @@ def test_rollout_collector_graph_replay_matches_eager_at_76_inputs():
     policy = MlpPolicy(obs_dim=76).cuda()
     out = []
     for use_graph in (False, True):
-        env = make_env(n, bank_of(1), 32, seed=1)
+        env = make_env(knobs(n_beams=32), n, fp32_bank(64, 600, 600, seed=1), seed=1)
         col = RolloutCollector(env, policy, T=T, use_graph=use_graph)
         assert not col._kernel
         col.collect()
@@ -409,24 +366,23 @@ def test_rollout_collector_graph_replay_matches_eager_at_76_inputs():
 
 
 def test_fresh_maps_against_oracle_at_32_beams():
-    from ship_sim_gym_b200 import BatchedShipEnv
     nb, n, K, S = 32, 2048, 32, 64
-    env = BatchedShipEnv(n, None, _cfgs(nb), honour_lidar_config=True, n_scenarios=S, seed=11, scenario_source="device",
-                         auto_reset=True, fresh_maps=True)
+    k = knobs(n_beams=nb)
+    env = make_env(k, n, None, n_scenarios=S, seed=11, scenario_source="device", auto_reset=True, fresh_maps=True)
     bank = env.read_scenarios()
     bd = dict(hull_xy=bank.hull_xy, hull_n=bank.hull_n, goals=bank.goals.astype(np.float32).astype(np.float64))
-    orc = make_oracle(n, bd, nb, auto_reset=True, seed=11, pick_base=0, pick_count=S // 4)
+    orc = make_oracle(k, n, bd, auto_reset=True, seed=11, pick_base=0, pick_count=S // 4, n_threads=ORACLE_THREADS)
     env.reset()
     orc.reset()
     rng = np.random.RandomState(3)
     pose, ints, lidar, goals, ret = parity.f32_inputs(*parity.random_states(rng, n, 600, 600, S, bd["goals"], near=(bd["hull_xy"], bd["hull_n"])))
     st = (pose, ints, widen(lidar, nb, rng), goals, ret)
     env.set_state(*st)
-    parity_beams.load_oracle_state(orc, *st, n_beams=nb)
+    parity.load_oracle_state(orc, *st, n_beams=nb)
     acts = rng.randint(0, 3, (K, n)).astype(np.int32)
     obs, rew, done = [t.cpu().numpy() for t in env.rollout(torch.tensor(acts, device=env.device))]
     ref = orc.step(acts)
-    rep = parity_beams.compare_steps(ref, obs, rew, done, margin_thr=parity.MARGIN_THR, label="fresh maps", n_beams=nb)
+    rep = parity.compare_steps(ref, obs, rew, done, margin_thr=parity.MARGIN_THR, label="fresh maps", n_beams=nb)
     assert done.sum() > n // 4
     assert rep["grazing_frac"] < parity.MAX_EXCLUDED and rep["excluded_frac"] < parity.MAX_EXCLUDED_CUMULATIVE, rep
     env.close()
@@ -434,7 +390,7 @@ def test_fresh_maps_against_oracle_at_32_beams():
 
 def test_reset_observation_layout_on_the_device():
     for nb in (1, 7, 32):
-        env = make_env(5, bank_of(1), nb, seed=1)
+        env = make_env(knobs(n_beams=nb), 5, fp32_bank(64, 600, 600, seed=1), seed=1)
         obs = env.reset().cpu().numpy()
         F = 6 + nb
         assert obs.shape == (5, 2 * F)

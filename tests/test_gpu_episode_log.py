@@ -12,15 +12,8 @@ pytestmark = pytest.mark.gpu
 
 torch = pytest.importorskip("torch")
 
+from helpers import config_classes, fp32_bank, knobs, make_env  # noqa: E402
 import parity  # noqa: E402
-from test_gpu_parity import _bank, _cfg  # noqa: E402
-
-
-def _env(n, bank, W=600, H=600, hist=2, max_steps=1000, auto_reset=True, seed=0, **kw):
-    from ship_sim_gym_b200 import BatchedShipEnv, ScenarioBank
-    GC, EC = _cfg(W, H, 10, hist, max_steps)
-    sb = ScenarioBank(bank["hull_xy"], bank["hull_n"], bank["goals"], (W, H))
-    return BatchedShipEnv(n, GC, EC, bank=sb, auto_reset=auto_reset, seed=seed, **kw)
 
 
 def _np(ep):
@@ -53,13 +46,14 @@ KERNELS = [dict(steps_in_flight=1, lanes_per_env=1), dict(steps_in_flight=1, lan
 def test_terminal_rows_equal_no_reset_rows(kern, hist):
     W = H = 600
     n, K, max_steps = 700, 64, 200
-    bank = _bank(48, W, H, seed=13)
+    bank = fp32_bank(48, W, H, seed=13)
     rng = np.random.RandomState(3)
     st = parity.f32_inputs(*parity.random_states(rng, n, W, H, 48, bank["goals"], max_steps=max_steps,
                                                  near=(bank["hull_xy"], bank["hull_n"])))
     acts = torch.tensor(rng.choice([0, 0, 1, 2], size=(K, n)).astype(np.int32), device="cuda")
-    ref = _env(n, bank, hist=hist, max_steps=max_steps, auto_reset=False, seed=5, **kern)
-    got = _env(n, bank, hist=hist, max_steps=max_steps, auto_reset=True, seed=5, **kern)
+    k = knobs(hist=hist, max_steps=max_steps)
+    ref = make_env(k, n, bank, auto_reset=False, seed=5, **kern)
+    got = make_env(k, n, bank, auto_reset=True, seed=5, **kern)
     got.enable_episode_log(K * n)
     outs = []
     for e in (ref, got):
@@ -93,8 +87,7 @@ def test_terminal_rows_equal_no_reset_rows(kern, hist):
 
 
 def _run_full(n, K, log, **kw):
-    bank = _bank(64, 600, 600, seed=5)
-    env = _env(n, bank, seed=17, **kw)
+    env = make_env(knobs(), n, fp32_bank(64, 600, 600, seed=5), seed=17, **kw)
     if log:
         env.enable_episode_log(n * K // 4)
     env.reset()
@@ -136,10 +129,10 @@ def test_full_size_both_kernels_and_log_changes_nothing():
 @pytest.mark.parametrize("regime", ["k1_zero_copy", "small_copies", "large_compacted", "dma_share"])
 def test_step_host_records_equal_device_rollout(regime, monkeypatch):
     n, K = {"k1_zero_copy": (256, 1), "small_copies": (1024, 8), "large_compacted": (4096, 64), "dma_share": (4096, 64)}[regime]
-    bank = _bank(64, 600, 600, seed=5)
+    bank = fp32_bank(64, 600, 600, seed=5)
     rng = np.random.RandomState(7)
     acts = rng.randint(0, 3, (K, n)).astype(np.int32)
-    dev, host = _env(n, bank, seed=9, max_steps=40), _env(n, bank, seed=9, max_steps=40)
+    dev, host = make_env(knobs(max_steps=40), n, bank, seed=9), make_env(knobs(max_steps=40), n, bank, seed=9)
     for e in (dev, host):
         e.enable_episode_log(n * (K + 30))
         e.reset()
@@ -170,10 +163,11 @@ def test_step_host_records_equal_device_rollout(regime, monkeypatch):
 @pytest.mark.parametrize("hist", [3, 4])
 def test_long_histories_terminal_obs(hist):
     n, K = 600, 40
-    bank = _bank(48, 600, 600, seed=13)
+    bank = fp32_bank(48, 600, 600, seed=13)
     rng = np.random.RandomState(11)
-    ref = _env(n, bank, hist=hist, max_steps=25, auto_reset=False, seed=2)
-    got = _env(n, bank, hist=hist, max_steps=25, auto_reset=True, seed=2)
+    k = knobs(hist=hist, max_steps=25)
+    ref = make_env(k, n, bank, auto_reset=False, seed=2)
+    got = make_env(k, n, bank, auto_reset=True, seed=2)
     got.enable_episode_log(n * K)
     for e in (ref, got):
         e.reset()
@@ -232,7 +226,7 @@ def test_shards_concatenate_to_the_whole_batch():
 
 def test_binding_needs_auto_reset():
     from ship_sim_gym_b200 import _abi
-    env = _env(64, _bank(8, 600, 600), auto_reset=False)
+    env = make_env(knobs(), 64, fp32_bank(8, 600, 600), auto_reset=False)
     rows = torch.zeros(64, 32, device="cuda")
     meta = torch.zeros(64, 8, dtype=torch.int32, device="cuda")
     cnt = torch.zeros(1, dtype=torch.int32, device="cuda")
@@ -245,7 +239,7 @@ def test_binding_needs_auto_reset():
 def test_overflow_writes_nothing_past_capacity_and_counts_on():
     from ship_sim_gym_b200 import _abi
     n, K, cap = 512, 100, 37
-    env = _env(n, _bank(16, 600, 600), max_steps=20)
+    env = make_env(knobs(max_steps=20), n, fp32_bank(16, 600, 600))
     rows = torch.full((cap + 5, 32), 7.0, device="cuda")
     meta = torch.full((cap + 5, 8), 7, dtype=torch.int32, device="cuda")
     cnt = torch.zeros(1, dtype=torch.int32, device="cuda")
@@ -266,9 +260,10 @@ def test_vec_env_episode_info():
     from ship_sim_gym_b200 import BatchedShipEnv
     from ship_sim_gym_b200.adapters import ShipVecEnv
     n, steps = 256, 120
-    vec = ShipVecEnv(n, episode_info=True, seed=8, n_scenarios=32, env_config=_cfg(hist=2, max_steps=50)[1])
-    plain = ShipVecEnv(n, seed=8, n_scenarios=32, env_config=_cfg(hist=2, max_steps=50)[1])
-    ref = BatchedShipEnv(n, seed=8, n_scenarios=32, auto_reset=False, env_config=_cfg(hist=2, max_steps=50)[1])
+    _, EC = config_classes(knobs(max_steps=50))
+    vec = ShipVecEnv(n, episode_info=True, seed=8, n_scenarios=32, env_config=EC)
+    plain = ShipVecEnv(n, seed=8, n_scenarios=32, env_config=EC)
+    ref = BatchedShipEnv(n, seed=8, n_scenarios=32, auto_reset=False, env_config=EC)
     vec.reset(), plain.reset(), ref.reset()
     rng = np.random.RandomState(1)
     acc = np.zeros(n, dtype=np.float32)
@@ -302,7 +297,7 @@ def test_rollout_collector_episode_log(use_graph):
     from ship_sim_gym_b200.rollout import MlpPolicy, RolloutCollector
     torch.manual_seed(0)
     n, T = 1024, 64
-    env = BatchedShipEnv(n, seed=3, n_scenarios=64, env_config=_cfg(hist=2, max_steps=30)[1])
+    env = BatchedShipEnv(n, seed=3, n_scenarios=64, env_config=config_classes(knobs(max_steps=30))[1])
     col = RolloutCollector(env, MlpPolicy().cuda(), T=T, use_graph=use_graph, episode_log=True)
     ret = torch.zeros(n, dtype=torch.float32, device="cuda")
     length = torch.zeros(n, dtype=torch.int64, device="cuda")

@@ -7,10 +7,6 @@ reach grid; the grid builder, the spawn-row builder and the host path's reward t
 tests run at the reference defaults only, where a knob read from the wrong field, or a constant that silently assumes
 the default, cannot show.  Every case here also checks that it is sensitive to its knob: the oracle run again with
 the knobs set back to the defaults must disagree with the kernel on a stated share of the compared env-steps."""
-import functools
-import os
-import re
-
 import numpy as np
 import pytest
 
@@ -19,17 +15,9 @@ pytestmark = pytest.mark.gpu
 torch = pytest.importorskip("torch")
 
 import oracle  # noqa: E402
-from helpers import ROOT, pack_bank  # noqa: E402
+from helpers import ORACLE_THREADS, assert_same, case_knobs, fp32_bank, knobs, make_env, make_oracle  # noqa: E402
+from helpers import pack_bank, run, source_constant  # noqa: E402
 import parity  # noqa: E402
-from test_gpu_parity import _bank  # noqa: E402
-from test_gpu_window import _assert_same, _run  # noqa: E402
-
-N_THREADS = max(1, min(16, os.cpu_count() or 1))      # oracle threads
-
-DEFAULTS = dict(W=600.0, H=600.0, speed=10, max_steps=1000, spread=90.0, lidar=100.0, ship_w=2.0, ship_h=3.0, mass=5.0,
-                thrust=100.0, goal_radius=5.0, step_penalty=-0.01, spawn_y=25.0, map_N=10, wf=0.5)
-# knobs the Python layer does not expose: set on shipsim_config itself
-RAW_KNOBS = ("ship_w", "ship_h", "mass", "thrust", "goal_radius", "step_penalty", "spawn_y")
 
 # guard: (which run, share) -- the share of compared env-steps ("step": envs of the single injected step, post-step
 # velocities included; "roll": env-steps of the 32-step auto-reset rollout) on which the kernel must DISAGREE with the
@@ -64,73 +52,9 @@ CASES = [
 IDS = [c["name"] for c in CASES]
 
 
-def knobs(case):
-    k = dict(DEFAULTS)
-    k.update({f: v for f, v in case.items() if f in DEFAULTS})
-    return k
-
-
-def make_env(k, n, bank, auto_reset, seed=0, env_id_offset=0, **kw):
-    """BatchedShipEnv at the knobs `k`: bounds, speed, cap and lidar through the config classes, the rest set on the
-    shipsim_config that env.py takes from _abi.default_config()."""
-    from ship_sim_gym_b200 import BatchedShipEnv, ScenarioBank, _abi
-    from ship_sim_gym_b200.config import EnvConfig, GameConfig, LidarConfig
-
-    class LC(LidarConfig):
-        DISTANCE = k["lidar"]
-        ANGULAR_SPREAD = k["spread"]
-
-    class EC(EnvConfig):
-        HISTORY_SIZE = 2
-        MAX_STEPS = k["max_steps"]
-        LIDAR_CONFIG = LC
-
-    class GC(GameConfig):
-        BOUNDS = (k["W"], k["H"])
-        SPEED = k["speed"]
-
-    default_config = _abi.default_config
-
-    def config():
-        cfg = default_config()
-        for f in RAW_KNOBS:
-            setattr(cfg, f, k[f])
-        return cfg
-    _abi.default_config = config
-    try:
-        env = BatchedShipEnv(n, GC, EC, bank=ScenarioBank(bank["hull_xy"], bank["hull_n"], bank["goals"], (k["W"], k["H"])),
-                             auto_reset=auto_reset, seed=seed, env_id_offset=env_id_offset, honour_lidar_config=True, **kw)
-    finally:
-        _abi.default_config = default_config
-    for f in RAW_KNOBS:
-        assert getattr(env.cfg, f) == float(np.float32(k[f])), f
-    assert (env.cfg.bounds_w, env.cfg.bounds_h, env.cfg.max_steps) == (k["W"], k["H"], k["max_steps"])
-    assert (env.cfg.lidar_spread_deg, env.cfg.lidar_distance) == (k["spread"], k["lidar"])
-    return env
-
-
-def make_oracle(k, n, bank, auto_reset, seed=0, env_id_offset=0):
-    """The float64 oracle at the knobs `k` (fp32-rounded, as the kernel holds them)."""
-    f32 = {f: float(np.float32(k[f])) for f in RAW_KNOBS}
-    return oracle.OracleEnv(n, bank, W=k["W"], H=k["H"], speed=k["speed"], history=2, max_steps=k["max_steps"],
-                            lidar_spread_deg=k["spread"], lidar_distance=k["lidar"], seed=seed, env_id_offset=env_id_offset,
-                            auto_reset=auto_reset, n_threads=N_THREADS, **f32)
-
-
-@functools.lru_cache(maxsize=None)
-def _bank_for(W, H, seed, map_N, wf):
-    return _bank(64, W, H, seed=seed, map_N=map_N, wf=wf)
-
-
-def bank_for(k, seed):
-    return _bank_for(k["W"], k["H"], seed, k["map_N"], k["wf"])
-
-
 def default_knobs_of(k):
     """The knobs set back to the defaults, on the case's map."""
-    d = dict(DEFAULTS)
-    d["map_N"], d["wf"] = k["map_N"], k["wf"]
-    return d
+    return knobs(map_N=k["map_N"], wf=k["wf"])
 
 
 # ---------------------------------------------------------------------------------------------- inputs
@@ -155,9 +79,7 @@ def injected_states(case, k, bank, n, seed):
         parts.append((p, i, li, g, r))
     else:
         parts.append(parity.random_states(rng, m, W, H, 64, bank["goals"], max_steps=k["max_steps"], near=near, hull=hull))
-    st = [np.concatenate([np.asarray(p[j]).reshape(len(p[0]), -1) for p in parts]) for j in range(5)]
-    st[4] = st[4].reshape(-1)
-    return parity.f32_inputs(*st), rng.randint(0, 3, n).astype(np.int32)
+    return parity.f32_inputs(*parity.concat_states(parts)), rng.randint(0, 3, n).astype(np.int32)
 
 
 def _disagree(ref, obs, rew, done):
@@ -181,24 +103,24 @@ def oracle_runs():
 
 
 def _single_step_ref(case):
-    k = knobs(case)
-    bank = bank_for(k, 3)
+    k = case_knobs(case)
+    bank = fp32_bank(64, k["W"], k["H"], seed=3, map_N=k["map_N"], wf=k["wf"])
     st, acts = injected_states(case, k, bank, N_STEP, 7)
     out = {}
     for which, kk in (("case", k), ("default", default_knobs_of(k))):
-        orc = make_oracle(kk, N_STEP, bank, auto_reset=False)
+        orc = make_oracle(kk, N_STEP, bank, auto_reset=False, n_threads=ORACLE_THREADS)
         parity.load_oracle_state(orc, *st)
         out[which] = (orc.step(acts[None]), orc.pose.copy(), orc.ints.copy(), orc.lidar[:, :10].copy())
     return bank, st, acts, out
 
 
 def _rollout_ref(case):
-    k = knobs(case)
-    bank = bank_for(k, 7)
+    k = case_knobs(case)
+    bank = fp32_bank(64, k["W"], k["H"], seed=7, map_N=k["map_N"], wf=k["wf"])
     acts = np.random.RandomState(21).choice([0, 0, 1, 2], size=(K_ROLL, N_ROLL)).astype(np.int32)
     out = {}
     for which, kk in (("case", k), ("default", default_knobs_of(k))):
-        orc = make_oracle(kk, N_ROLL, bank, auto_reset=True, seed=11)
+        orc = make_oracle(kk, N_ROLL, bank, auto_reset=True, seed=11, n_threads=ORACLE_THREADS)
         orc.reset()
         out[which] = (orc.step(acts), orc.stats_dict())
     return bank, acts, out
@@ -208,7 +130,7 @@ def _rollout_ref(case):
 @pytest.mark.parametrize("case", CASES, ids=IDS)
 @pytest.mark.parametrize("lanes", [1, 32])
 def test_knob_single_step_against_oracle(case, lanes, oracle_runs):
-    k = knobs(case)
+    k = case_knobs(case)
     bank, st, acts, out = oracle_runs("step", case)
     ref, pose, ints, lidar = out["case"]
     env = make_env(k, N_STEP, bank, auto_reset=False, lanes_per_env=lanes, steps_in_flight=1)
@@ -250,7 +172,7 @@ STAT_KEYS = ("episodes", "collision", "oob", "timeout", "all_goals", "length_sum
 @pytest.mark.parametrize("case", CASES, ids=IDS)
 @pytest.mark.parametrize("variant", ["serial", "T8", "T32"])
 def test_knob_rollout_against_oracle(case, variant, oracle_runs):
-    k = knobs(case)
+    k = case_knobs(case)
     bank, acts, out = oracle_runs("roll", case)
     ref, so = out["case"]
     kw = dict(lanes_per_env=1, steps_in_flight=1) if variant == "serial" else dict(steps_in_flight=int(variant[1:]))
@@ -276,17 +198,17 @@ def test_knob_rollout_against_oracle(case, variant, oracle_runs):
 @pytest.mark.parametrize("case", CASES, ids=IDS)
 @pytest.mark.parametrize("T", [4, 32])
 def test_knob_window_is_bit_identical_to_serial(case, T):
-    k = knobs(case)
+    k = case_knobs(case)
     n, K = 1000 + 3, 37
-    bank = bank_for(k, 13)
+    bank = fp32_bank(64, k["W"], k["H"], seed=13, map_N=k["map_N"], wf=k["wf"])
     rng = np.random.RandomState(3)
     acts = torch.tensor(rng.choice([0, 0, 1, 2], size=(K, n)).astype(np.int32), device="cuda")
     st = parity.f32_inputs(*parity.random_states(rng, n, k["W"], k["H"], 64, bank["goals"], max_steps=k["max_steps"],
                                                  near=(bank["hull_xy"], bank["hull_n"]), hull=parity.ship_hull(k["ship_w"], k["ship_h"])))
-    ref = _run(make_env(k, n, bank, auto_reset=True, seed=5, lanes_per_env=1, steps_in_flight=1), acts, K, st)
-    got = _run(make_env(k, n, bank, auto_reset=True, seed=5, steps_in_flight=T), acts, K, st)
+    ref = run(make_env(k, n, bank, auto_reset=True, seed=5, lanes_per_env=1, steps_in_flight=1), acts, K, st)
+    got = run(make_env(k, n, bank, auto_reset=True, seed=5, steps_in_flight=T), acts, K, st)
     assert ref[3]["steps_in_flight"] == 1 and got[3]["steps_in_flight"] == T
-    _assert_same(got, ref, "%s T=%d" % (case["name"], T))
+    assert_same(got, ref, "%s T=%d" % (case["name"], T))
     assert ref[0][2].sum() > 0
 
 
@@ -299,8 +221,8 @@ HOST_CASES = [c for c in CASES if c["name"] in ("wide", "penalty", "cap1", "spaw
 def test_knob_host_path_matches_rollout(case, n, K):
     """shipsim_step_host rebuilds the rows and rewards from compacted frames with a reward-code table built from the
     step penalty: bit-identical to the device-resident rollout at these knobs."""
-    k = knobs(case)
-    bank = bank_for(k, 2)
+    k = case_knobs(case)
+    bank = fp32_bank(64, k["W"], k["H"], seed=2, map_N=k["map_N"], wf=k["wf"])
     rng = np.random.RandomState(4)
     envs = [make_env(k, n, bank, auto_reset=True, seed=1) for _ in range(2)]
     for e in envs:
@@ -325,11 +247,6 @@ def test_knob_host_path_matches_rollout(case, n, K):
 def _regular(cx, cy, r, m, phase=0.0):
     a = phase + np.linspace(0, 2 * np.pi, m, endpoint=False)
     return np.stack([cx + r * np.cos(a), cy + r * np.sin(a)], 1)
-
-
-def _source_int(path, pattern):
-    with open(os.path.join(ROOT, "ship_sim_gym_b200", "csrc", path)) as f:
-        return int(re.search(pattern, f.read()).group(1))
 
 
 def _fan_reach_planes(hull, origin, k):
@@ -375,25 +292,25 @@ def test_spawn_row_geometry(kind, spawn_y):
     """Episodes of three steps, so that every env is reset inside the kernel every few steps and each episode's first
     step runs from the spawn row built by build_spawn_rows_kernel: the lidar origin inside a bank, more planes facing
     the fan than a scratch row holds (the big-row path), and an edge at the lidar's reach."""
-    k = dict(DEFAULTS, max_steps=3, spawn_y=spawn_y)
+    k = knobs(max_steps=3, spawn_y=spawn_y)
     bank = _spawn_bank(kind, spawn_y)
     n, K = 515, 24
     if kind == "big_row":
-        n_cand = _source_int("shipsim_geom.cuh", r"constexpr int kMaxCand = (\d+);")
+        n_cand = source_constant("shipsim_geom.cuh", r"constexpr int kMaxCand = (\d+);")
         assert _fan_reach_planes(bank["hull_xy"][0, 0, :bank["hull_n"][0, 0]], _spawn_origin(spawn_y), k).sum() > n_cand
     acts = np.random.RandomState(1).randint(0, 3, (K, n)).astype(np.int32)
-    orc = make_oracle(k, n, bank, auto_reset=True, seed=4)
+    orc = make_oracle(k, n, bank, auto_reset=True, seed=4, n_threads=ORACLE_THREADS)
     orc.reset()
     ref = orc.step(acts)
     runs = {}
     for name, kw in (("lanes1", dict(lanes_per_env=1, steps_in_flight=1)), ("lanes8", dict(lanes_per_env=8, steps_in_flight=1)),
                      ("T4", dict(steps_in_flight=4)), ("T32", dict(steps_in_flight=32))):
-        runs[name] = _run(make_env(k, n, bank, auto_reset=True, seed=4, **kw), torch.tensor(acts, device="cuda"), K)
+        runs[name] = run(make_env(k, n, bank, auto_reset=True, seed=4, **kw), torch.tensor(acts, device="cuda"), K)
         (obs, rew, done), _, _, _ = runs[name]
         rep = parity.compare_steps(ref, obs, rew, done, margin_thr=parity.MARGIN_THR, label="%s %s" % (kind, name))
         assert rep["grazing_frac"] < parity.MAX_EXCLUDED and rep["excluded_frac"] < parity.MAX_EXCLUDED_CUMULATIVE, rep
     for name in ("T4", "T32"):
-        _assert_same(runs[name], runs["lanes1"], "%s %s" % (kind, name))
+        assert_same(runs[name], runs["lanes1"], "%s %s" % (kind, name))
     first = np.concatenate([np.ones((1, n), dtype=bool), ref["done"][:-1].astype(bool)])     # steps that begin at the spawn
     lid = ref["obs"][:, :, 22:32]
     if kind == "inside":
@@ -410,10 +327,10 @@ def test_64_bit_seed_and_env_ids():
     """A seed and global env ids above 2^32: the random agent's actions and the scenario picks are keyed by all 64
     bits; truncating either anywhere between Python, ctypes and the kernels changes the episodes."""
     seed, off = 2 ** 63 + 12345, 2 ** 32 + 7
-    k = dict(DEFAULTS, max_steps=5)
-    bank = _bank(64, 600.0, 600.0, seed=9)
+    k = knobs(max_steps=5)
+    bank = fp32_bank(64, 600.0, 600.0, seed=9)
     n, K = 2048, 24
-    orc = make_oracle(k, n, bank, auto_reset=True, seed=seed, env_id_offset=off)
+    orc = make_oracle(k, n, bank, auto_reset=True, seed=seed, env_id_offset=off, n_threads=ORACLE_THREADS)
     orc.reset()
     ref = orc.step(None, K=K)
     for kw in (dict(lanes_per_env=1, steps_in_flight=1), dict(steps_in_flight=8)):
@@ -429,7 +346,7 @@ def test_64_bit_seed_and_env_ids():
         env.close()
     # the keys matter: 32-bit truncations pick other scenarios
     for s, o in ((seed & 0xFFFFFFFF, off), (seed, off & 0xFFFFFFFF)):
-        t = make_oracle(k, n, bank, auto_reset=True, seed=s, env_id_offset=o)
+        t = make_oracle(k, n, bank, auto_reset=True, seed=s, env_id_offset=o, n_threads=ORACLE_THREADS)
         t.reset()
         t.step(None, K=K)
         assert (t.ints[:, 3] != orc.ints[:, 3]).mean() > 0.9

@@ -8,38 +8,8 @@ torch = pytest.importorskip("torch")
 
 import oracle  # noqa: E402
 from oracle import cbind  # noqa: E402
-from helpers import load_trajectories, pack_bank  # noqa: E402
+from helpers import case_knobs, fp32_bank, knobs, load_trajectories, make_env, make_oracle, pack_bank  # noqa: E402
 import parity  # noqa: E402
-
-
-def _cfg(W=600, H=600, speed=10, hist=2, max_steps=1000, spread=None):
-    from ship_sim_gym_b200.config import EnvConfig, GameConfig, LidarConfig
-
-    class GC(GameConfig):
-        BOUNDS = (W, H)
-        SPEED = speed
-
-    class LC(LidarConfig):
-        ANGULAR_SPREAD = 180 if spread is None else spread
-
-    class EC(EnvConfig):
-        HISTORY_SIZE = hist
-        MAX_STEPS = max_steps
-        LIDAR_CONFIG = LC
-
-    return GC, EC
-
-
-def _make_pair(n, bank, W=600, H=600, speed=10, hist=2, max_steps=1000, auto_reset=False, seed=0, spread=None,
-               env_id_offset=0, lanes=0):
-    from ship_sim_gym_b200 import BatchedShipEnv, ScenarioBank
-    GC, EC = _cfg(W, H, speed, hist, max_steps, spread)
-    sb = ScenarioBank(bank["hull_xy"], bank["hull_n"], bank["goals"], (W, H))
-    env = BatchedShipEnv(n, GC, EC, bank=sb, auto_reset=auto_reset, seed=seed, honour_lidar_config=spread is not None,
-                         env_id_offset=env_id_offset, lanes_per_env=lanes)
-    orc = oracle.OracleEnv(n, bank, W=W, H=H, speed=speed, history=hist, max_steps=max_steps, auto_reset=auto_reset,
-                           seed=seed, lidar_spread_deg=90.0 if spread is None else float(spread), env_id_offset=env_id_offset)
-    return env, orc
 
 
 def _np(*ts):
@@ -61,7 +31,8 @@ def test_golden_trajectories(lanes):
             continue          # assembled by the host layer: covered by test_long_history
         h0, h1 = cbind.convex_hull(ep["raw0"]), cbind.convex_hull(ep["raw1"])
         bank = pack_bank([(h0, h1)], [ep["goals"]])
-        env, orc = _make_pair(1, bank, W, H, speed, int(hist), int(max_steps), lanes=lanes)
+        k = knobs(W=W, H=H, speed=speed, hist=int(hist), max_steps=int(max_steps))
+        env, orc = make_env(k, 1, bank, auto_reset=False, lanes_per_env=lanes), make_oracle(k, 1, bank)
         obs0 = env.reset(scenario=[0])
         orc.reset(scen=[0])
         tol0 = parity.REL_TOL * np.maximum(1, np.abs(ep["obs"][0]))
@@ -83,7 +54,7 @@ def test_long_history_host_layer():
     ep = [e for e in EPS if e["cfg"][3] == 3][0]
     W, H, speed, hist, max_steps = ep["cfg"][:5]
     bank = pack_bank([(cbind.convex_hull(ep["raw0"]), cbind.convex_hull(ep["raw1"]))], [ep["goals"]])
-    env, _ = _make_pair(1, bank, W, H, speed, 3, int(max_steps))
+    env = make_env(knobs(W=W, H=H, speed=speed, hist=3, max_steps=int(max_steps)), 1, bank, auto_reset=False)
     obs0 = env.reset(scenario=[0])
     assert obs0.shape == (1, 48)
     np.testing.assert_allclose(obs0[0].cpu().numpy(), ep["obs"][0], rtol=1e-4, atol=1e-4)
@@ -94,16 +65,6 @@ def test_long_history_host_layer():
 
 
 # ---------------------------------------------------------------------------------------------- injected states
-def _bank(n, W, H, seed=0, map_N=10, wf=0.5):
-    """Scenario bank rounded to fp32: the map is part of the injected state, so the oracle and the kernel (which
-    stores hull vertices and goals as fp32) must start from IDENTICAL geometry."""
-    from ship_sim_gym_b200 import ScenarioBank
-    d = ScenarioBank.generate(n, (W, H), seed=seed, map_N=map_N, width_frac=wf).as_dict()
-    d["hull_xy"] = d["hull_xy"].astype(np.float32).astype(np.float64)
-    d["goals"] = d["goals"].astype(np.float32).astype(np.float64)
-    return d
-
-
 CASES = [
     dict(name="default", W=600, H=600, speed=10),
     dict(name="random_py", W=600, H=600, speed=1),
@@ -119,8 +80,9 @@ CASES = [
 def test_injected_single_step(case, adversarial, lanes):
     W, H = case["W"], case["H"]
     n = 8192 - 5          # not a multiple of the warp / CTA size: exercises the ragged tail
-    bank = _bank(64, W, H, seed=3, map_N=case.get("map_N", 10), wf=case.get("wf", 0.5))
-    env, orc = _make_pair(n, bank, W, H, case["speed"], case.get("hist", 2), spread=case.get("spread"), lanes=lanes)
+    k = case_knobs(case)
+    bank = fp32_bank(64, W, H, seed=3, map_N=k["map_N"], wf=k["wf"])
+    env, orc = make_env(k, n, bank, auto_reset=False, lanes_per_env=lanes), make_oracle(k, n, bank)
     env.reset()
     rng = np.random.RandomState(7 + adversarial)
     st = parity.f32_inputs(*parity.random_states(rng, n, W, H, 64, bank["goals"],
@@ -153,8 +115,10 @@ def test_injected_single_step(case, adversarial, lanes):
 def test_32_step_transitions(case, auto_reset, lanes):
     W, H = case["W"], case["H"]
     n, K = 4096 + 3, 32
-    bank = _bank(64, W, H, seed=5, map_N=case.get("map_N", 10), wf=case.get("wf", 0.5))
-    env, orc = _make_pair(n, bank, W, H, case["speed"], 2, auto_reset=auto_reset, seed=11, spread=case.get("spread"), lanes=lanes)
+    k = case_knobs(case)
+    bank = fp32_bank(64, W, H, seed=5, map_N=k["map_N"], wf=k["wf"])
+    env = make_env(k, n, bank, auto_reset=auto_reset, seed=11, lanes_per_env=lanes)
+    orc = make_oracle(k, n, bank, auto_reset=auto_reset, seed=11)
     env.reset()
     orc.reset()
     rng = np.random.RandomState(21)
@@ -205,8 +169,8 @@ def test_k_fusion_and_sharding_invariance():
 def test_random_agent_matches_oracle_philox():
     """ACTION_RANDOM (in-kernel Philox actions, the train/random.py agent) == oracle with the same counter RNG."""
     n, K = 2048, 24
-    bank = _bank(32, 600, 600, seed=9)
-    env, orc = _make_pair(n, bank, auto_reset=True, seed=123)
+    bank = fp32_bank(32, 600, 600, seed=9)
+    env, orc = make_env(knobs(), n, bank, auto_reset=True, seed=123), make_oracle(knobs(), n, bank, auto_reset=True, seed=123)
     env.reset()
     orc.reset()
     obs, rew, done = _np(*env.rollout(None, K=K))
@@ -280,7 +244,8 @@ def test_many_candidate_planes_serial_path(lanes):
     goals = np.array([[300, 100], [300, 200], [300, 300], [300, 400], [300, 500]], dtype=np.float64)
     bank = pack_bank([(h0, h1)], [goals])
     bank["hull_xy"] = bank["hull_xy"].astype(np.float32).astype(np.float64)
-    env, orc = _make_pair(n, bank, W, H, 10, 2, auto_reset=True, seed=3, lanes=lanes)
+    env = make_env(knobs(), n, bank, auto_reset=True, seed=3, lanes_per_env=lanes)
+    orc = make_oracle(knobs(), n, bank, auto_reset=True, seed=3)
     env.reset()
     orc.reset()
     rng = np.random.RandomState(5)

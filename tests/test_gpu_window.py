@@ -10,41 +10,8 @@ pytestmark = pytest.mark.gpu
 
 torch = pytest.importorskip("torch")
 
-import oracle  # noqa: E402
-from helpers import pack_bank  # noqa: E402
+from helpers import assert_same, case_knobs, fp32_bank, knobs, make_env, make_oracle, pack_bank, run  # noqa: E402
 import parity  # noqa: E402
-from test_gpu_parity import _bank, _cfg  # noqa: E402
-
-
-def _env(n, bank, W=600, H=600, speed=10, hist=2, max_steps=1000, auto_reset=True, seed=0, spread=None, **kw):
-    from ship_sim_gym_b200 import BatchedShipEnv, ScenarioBank
-    GC, EC = _cfg(W, H, speed, hist, max_steps, spread)
-    sb = ScenarioBank(bank["hull_xy"], bank["hull_n"], bank["goals"], (W, H))
-    return BatchedShipEnv(n, GC, EC, bank=sb, auto_reset=auto_reset, seed=seed, honour_lidar_config=spread is not None, **kw)
-
-
-def _run(env, acts, K, state=None):
-    env.reset()
-    if state is not None:
-        env.set_state(*state)
-    out = env.rollout(acts, K=K)
-    torch.cuda.synchronize()
-    return [t.cpu().numpy() for t in out], env.get_state(), env.stats(), env.launch_info()
-
-
-def _assert_same(a, b, label):
-    (oa, ra, da), sa, ta, _ = a
-    (ob, rb, db), sb, tb, _ = b
-    assert np.array_equal(da, db), label + ": done"
-    assert np.array_equal(ra, rb), label + ": reward"
-    bad = np.argwhere(oa != ob)
-    assert bad.size == 0, "%s: obs differ at %d places, first (k, env, col) = %s: %r vs %r" % (
-        label, len(bad), bad[:1], oa[tuple(bad[0])] if len(bad) else None, ob[tuple(bad[0])] if len(bad) else None)
-    for k in ("pose", "ints", "lidar", "goals", "ep_return"):
-        assert np.array_equal(sa[k], sb[k]), "%s: final state %s" % (label, k)
-    for k in ("episodes", "length_sum", "goal_steps", "collision", "oob", "timeout", "all_goals"):
-        assert ta[k] == tb[k], "%s: stat %s %r vs %r" % (label, k, ta[k], tb[k])
-    assert ta["return_sum"] == pytest.approx(tb["return_sum"], rel=1e-5, abs=1e-2)
 
 
 CASES = [
@@ -65,17 +32,17 @@ def test_window_kernel_is_bit_identical_to_serial_kernel(case, T):
     W, H = case.get("W", 600), case.get("H", 600)
     n = case["n"]
     K = case["K"] or T
-    bank = _bank(48, W, H, seed=13, map_N=case.get("map_N", 10), wf=case.get("wf", 0.5))
-    kw = dict(W=W, H=H, speed=case.get("speed", 10), hist=case.get("hist", 2), max_steps=case.get("max_steps", 1000),
-              auto_reset=case.get("auto_reset", True), seed=5, spread=case.get("spread"))
+    k = case_knobs(case)
+    bank = fp32_bank(48, W, H, seed=13, map_N=k["map_N"], wf=k["wf"])
+    kw = dict(auto_reset=case.get("auto_reset", True), seed=5)
     rng = np.random.RandomState(3)
     acts = None if case.get("random_agent") else torch.tensor(rng.choice([0, 0, 1, 2], size=(K, n)).astype(np.int32), device="cuda")
     # start from scattered states (near the banks too) so that lidar hits, collisions and goals all occur early
     st = parity.f32_inputs(*parity.random_states(rng, n, W, H, 48, bank["goals"], near=(bank["hull_xy"], bank["hull_n"])))
-    ref = _run(_env(n, bank, lanes_per_env=1, steps_in_flight=1, **kw), acts, K, st)
-    got = _run(_env(n, bank, steps_in_flight=T, **kw), acts, K, st)
+    ref = run(make_env(k, n, bank, lanes_per_env=1, steps_in_flight=1, **kw), acts, K, st)
+    got = run(make_env(k, n, bank, steps_in_flight=T, **kw), acts, K, st)
     assert ref[3]["steps_in_flight"] == 1 and got[3]["steps_in_flight"] == T
-    _assert_same(got, ref, "%s T=%d" % (case["name"], T))
+    assert_same(got, ref, "%s T=%d" % (case["name"], T))
     (o, r, d), _, stats, _ = ref
     if case.get("auto_reset", True) and K >= 24:
         assert d.sum() > 0 and stats["episodes"] == float(d.sum())      # windows were cut
@@ -96,8 +63,8 @@ def test_window_kernel_consecutive_rollouts_and_serial_path():
     bank["hull_xy"] = bank["hull_xy"].astype(np.float32).astype(np.float64)
     rng = np.random.RandomState(9)
     st = parity.f32_inputs(*parity.random_states(rng, n, W, H, 1, bank["goals"], near=(bank["hull_xy"], bank["hull_n"])))
-    envs = [_env(n, bank, seed=2, lanes_per_env=4, steps_in_flight=1), _env(n, bank, seed=2, steps_in_flight=8),
-            _env(n, bank, seed=2, steps_in_flight=32)]
+    envs = [make_env(knobs(), n, bank, seed=2, **kw) for kw in (dict(lanes_per_env=4, steps_in_flight=1), dict(steps_in_flight=8),
+                                                                   dict(steps_in_flight=32))]
     for e in envs:
         e.reset()
         e.set_state(*st)
@@ -118,9 +85,9 @@ def test_window_kernel_consecutive_rollouts_and_serial_path():
 def test_window_kernel_against_oracle(T):
     W = H = 600
     n, K = 4096 + 3, 32
-    bank = _bank(64, W, H, seed=5)
-    env = _env(n, bank, auto_reset=True, seed=11, steps_in_flight=T)
-    orc = oracle.OracleEnv(n, bank, W=W, H=H, speed=10, history=2, max_steps=1000, auto_reset=True, seed=11, lidar_spread_deg=90.0)
+    bank = fp32_bank(64, W, H, seed=5)
+    env = make_env(knobs(), n, bank, auto_reset=True, seed=11, steps_in_flight=T)
+    orc = make_oracle(knobs(), n, bank, auto_reset=True, seed=11)
     env.reset()
     orc.reset()
     rng = np.random.RandomState(21)
@@ -138,8 +105,8 @@ def test_window_kernel_against_oracle(T):
 def test_auto_selection():
     """steps_in_flight = 0: small batches with K >= window take the window kernel, K = 1 stepping and explicit
     lanes_per_env the serial one."""
-    bank = _bank(8, 600, 600, seed=1)
-    e = _env(256, bank)
+    bank = fp32_bank(8, 600, 600, seed=1)
+    e = make_env(knobs(), 256, bank)
     e.reset()
     e.rollout(None, K=16)
     assert e.launch_info()["steps_in_flight"] == 1            # fewer steps than the window (32 for so few envs)
@@ -147,15 +114,15 @@ def test_auto_selection():
     assert e.launch_info()["steps_in_flight"] == 32
     e.step(torch.zeros(256, dtype=torch.int32, device="cuda"))
     assert e.launch_info()["steps_in_flight"] == 1
-    e2 = _env(256, bank, lanes_per_env=8)
+    e2 = make_env(knobs(), 256, bank, lanes_per_env=8)
     e2.reset()
     e2.rollout(None, K=40)
     assert e2.launch_info()["steps_in_flight"] == 1
     with pytest.raises(ValueError):
-        _env(16, bank, steps_in_flight=5)
+        make_env(knobs(), 16, bank, steps_in_flight=5)
     # the window is as long as still lets every warp be resident (include/shipsim.h: SHIPSIM_WINDOW_AUTO_MAX_ENVS)
     for n, want in ((2368, 32), (2369, 16), (4736, 16), (4737, 8), (32768, 8), (32769, 1)):
-        e3 = _env(n, bank)
+        e3 = make_env(knobs(), n, bank)
         e3.reset()
         e3.rollout(None, K=32)
         assert e3.launch_info()["steps_in_flight"] == want, (n, e3.launch_info())

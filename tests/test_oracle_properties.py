@@ -6,18 +6,14 @@
    segment-vs-convex-polygon (cpPolyShapeSegmentQuery) against Cyrus-Beck clipping, polygon-vs-polygon contact against
    exhaustive edge intersection / containment, point-to-polygon distance against the edge-by-edge minimum.
 The oracle is test infrastructure; nothing here touches the CUDA path."""
-import os
-import re
-
 import numpy as np
 import pytest
 
 import oracle
 import parity
+from helpers import source_constant
 from oracle import cbind
 from ship_sim_gym_b200 import ScenarioBank
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 def _env(speed, W=600.0, H=600.0, n=1, seed=0, **kw):
@@ -313,19 +309,14 @@ def test_goal_taken_exactly_within_the_radius(radius, ship):
 
 
 # ---------------------------------------------------------------------------------------------- reach-grid boundaries
-def _source_constant(path, pattern):
-    with open(os.path.join(ROOT, "ship_sim_gym_b200", "csrc", path)) as f:
-        return float(re.search(pattern, f.read()).group(1))
-
-
 @pytest.mark.parametrize("W,H", [(600.0, 600.0), (900.0, 400.0), (400.0, 1000.0), (4000.0, 4000.0)])
 @pytest.mark.parametrize("ship", [(2.0, 3.0), (4.0, 5.0)])
 def test_grid_boundary_states_straddle_the_cell_boundaries(W, H, ship):
     """The generator must put lidar origins within the stated ulps of the kernel's reach-grid boundaries: checked
     against the grid constants of the CUDA source, so that a change of the grid makes this fail instead of leaving the
     GPU tests that use the generator testing nothing in particular."""
-    assert parity.GRID_N == _source_constant("shipsim_device.cuh", r"constexpr int kGridN = (\d+);")
-    assert parity.GRID_PAD == _source_constant("shipsim_abi.cu", r"const double pad = ([0-9.]+);")
+    assert parity.GRID_N == source_constant("shipsim_device.cuh", r"constexpr int kGridN = (\d+);")
+    assert parity.GRID_PAD == source_constant("shipsim_abi.cu", r"const double pad = ([0-9.]+);")
     hull = parity.ship_hull(*ship)
     rng = np.random.RandomState(0)
     n = 6000
