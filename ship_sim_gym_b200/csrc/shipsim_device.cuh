@@ -307,6 +307,15 @@ __device__ __forceinline__ void unpack_goals(float4 g0, float4 g1, float4 g2, fl
     g[3] = make_float2(g1.z, g1.w); g[4] = make_float2(g2.x, g2.y);
 }
 
+// The goals of scenario `scen`: bank record float4 2..4 (what the state's goal planes g0..g2 hold), unpacked into g.
+// (The nearest-goal search is left to the caller: window_kernel issues more loads and the next pick in between.)
+__device__ __forceinline__ void scenario_goals(const StepParams &p, int scen, float4 &g0, float4 &g1, float4 &g2, float2 (&g)[kGoals])
+{
+    const float4 *rec = p.bank + (size_t)scen * p.scen_stride4;
+    g0 = __ldg(rec + 2); g1 = __ldg(rec + 3); g2 = __ldg(rec + 4);
+    unpack_goals(g0, g1, g2, g);
+}
+
 // Circle-vs-poly contact (CircleToPoly): distance(goal centre, ship polygon) <= goal radius, evaluated in the
 // body frame where the hull is constant.  cpPolyShapePointQuery semantics: inside => negative distance.
 __device__ __forceinline__ bool goal_culled(const StepParams &p, float qx, float qy)
@@ -405,19 +414,6 @@ __device__ __forceinline__ void cp_async16_s(unsigned smem_dst, const void *gmem
 __device__ __forceinline__ void cp_async16(void *smem_dst, const void *gmem_src) { cp_async16_s(smem_addr(smem_dst), gmem_src); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
-// Bulk asynchronous shared -> global copy by the TMA unit (UBLKCP): one instruction moves a contiguous run of shared
-// memory (multiple of 16 bytes, 16-byte aligned at both ends) -- an env's whole observation row -- instead of a loop of
-// 128-bit loads and stores.  Writes made with ordinary st.shared must be fenced into the async proxy first
-// (fence_proxy_async by the writers, then a warp / CTA sync); bulk_store_wait_read returns once the unit has READ the
-// source, i.e. the row may be overwritten.
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void bulk_store(void *gmem_dst, unsigned smem_src, unsigned bytes)
-{
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gmem_dst), "r"(smem_src), "r"(bytes) : "memory");
-    asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-}
-__device__ __forceinline__ void bulk_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-
 // Episode statistics of one step for a whole warp: counters by ballot + popc, the two sums (episode return and length of
 // the envs that finished) by visiting the few finished lanes.  Lane 0 adds the totals to the warp's eight accumulators
 // (shared-space address `stat`): plain shared-memory read-modify-write, no atomics (measured: the shared atomics cost 4 %
@@ -450,8 +446,5 @@ __device__ __forceinline__ float sqrt_approx(float x)
     asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
     return r;
 }
-
-// order-preserving float <-> int map for __reduce_min_sync
-__device__ __forceinline__ int f2ord(float f) { const int k = __float_as_int(f); return k ^ ((k >> 31) & 0x7fffffff); }
 
 }  // namespace shipsim

@@ -1,24 +1,24 @@
-// shipsim_geom.cuh -- geometry pieces shared by the step kernels (serial-in-time step_kernel and the time-parallel
-// window_kernel): action fetch, hull AABB, reach-grid lookup, two-float plane evaluation, ray-vs-plane test,
-// the plane phase and the serial ray query.  Both kernels call exactly these functions on the same inputs, which is
-// what makes their results bit-identical (tests/test_gpu_window.py).
+// shipsim_geom.cuh -- pieces shared by the step kernels (serial-in-time step_kernel and the time-parallel
+// window_kernel): action fetch, hull AABB, reach-grid lookup, two-float plane evaluation, ray-vs-plane test, the plane
+// phase with its candidate staging, the ray query against a plane row (cooperative and serial), and the stores of a
+// frame, of the state and of the statistics.  The lidar and plane work of both kernels runs through these functions on
+// the same inputs.  What each kernel still spells out itself -- the integration, the goal tests, reward / done and the
+// separating-axis passes (whose lane layouts differ) -- performs the same operations in the same order.  Together that
+// makes their results bit-identical (tests/test_gpu_window.py).
 #pragma once
 #include "shipsim_device.cuh"
 
-// how action words are loaded: read once, never again by this SM (streaming: they do not displace the reach-grid and plane records in L1)
-#ifndef SHIPSIM_ACT_LD
-#define SHIPSIM_ACT_LD __ldcs
-#endif
-
 namespace shipsim {
 
+// Action words are read once, never again by this SM: streaming loads (__ldcs), so that they do not displace the
+// reach-grid and plane records in L1.
 // actions[k][e]: `ap` walks down this env's column (stride = one row of the action tensor, in bytes)
 __device__ __forceinline__ int load_action(const StepParams &p, const char *ap, int k, long long gid)
 {
     switch (p.action_dtype) {
-        case 0: return SHIPSIM_ACT_LD(reinterpret_cast<const int *>(ap));
-        case 1: return (int)SHIPSIM_ACT_LD(reinterpret_cast<const long long *>(ap));
-        case 2: return (int)SHIPSIM_ACT_LD(reinterpret_cast<const unsigned char *>(ap));
+        case 0: return __ldcs(reinterpret_cast<const int *>(ap));
+        case 1: return (int)__ldcs(reinterpret_cast<const long long *>(ap));
+        case 2: return (int)__ldcs(reinterpret_cast<const unsigned char *>(ap));
         default: return random_action(p, gid, p.step0 + (unsigned)k);
     }
 }
@@ -27,9 +27,9 @@ __device__ __forceinline__ int load_action(const StepParams &p, const char *ap, 
 __device__ __forceinline__ int load_action_at(const StepParams &p, size_t idx, int k, long long gid)
 {
     switch (p.action_dtype) {
-        case 0: return SHIPSIM_ACT_LD(reinterpret_cast<const int *>(p.actions) + idx);
-        case 1: return (int)SHIPSIM_ACT_LD(reinterpret_cast<const long long *>(p.actions) + idx);
-        case 2: return (int)SHIPSIM_ACT_LD(reinterpret_cast<const unsigned char *>(p.actions) + idx);
+        case 0: return __ldcs(reinterpret_cast<const int *>(p.actions) + idx);
+        case 1: return (int)__ldcs(reinterpret_cast<const long long *>(p.actions) + idx);
+        case 2: return (int)__ldcs(reinterpret_cast<const unsigned char *>(p.actions) + idx);
         default: return random_action(p, gid, p.step0 + (unsigned)k);
     }
 }
@@ -177,18 +177,98 @@ __device__ __forceinline__ PlaneOut plane_at_pose(const StepParams &p, const flo
     return o;
 }
 
-// Where a plane row lives: the hot loops keep theirs in shared memory and name it by its 32-bit shared address (see
-// "shared memory by address" in shipsim_device.cuh); the scenario-upload kernel writes rows to global memory.
+// Where a row of float4 (a plane row, a frame, the statistics accumulators) lives.  step_kernel names its shared memory
+// by 32-bit shared address (RowSmem; see "shared memory by address" in shipsim_device.cuh); window_kernel by generic
+// pointers into its shared arrays, and the scenario-upload and frame kernels write rows to global memory (RowPtr).  The
+// pieces below are written once against either and compile to each kernel's own addressing.
 struct RowPtr {
     float4 *p;
     __device__ __forceinline__ void st(int i, float4 v) const { p[i] = v; }
     __device__ __forceinline__ float4 ld(int i) const { return p[i]; }
+    __device__ __forceinline__ float2 ld2(int i) const { return *reinterpret_cast<const float2 *>(p + i); }
+    __device__ __forceinline__ float ldf(int j) const { return reinterpret_cast<const float *>(p)[j]; }   // float j
+    __device__ __forceinline__ void cp_async(int i, const float4 *src) const { cp_async16(p + i, src); }
 };
 struct RowSmem {
     unsigned a;
     __device__ __forceinline__ void st(int i, float4 v) const { sts4(a + 16u * (unsigned)i, v); }
     __device__ __forceinline__ float4 ld(int i) const { return lds4(a + 16u * (unsigned)i); }
+    __device__ __forceinline__ float2 ld2(int i) const { return lds2(a + 16u * (unsigned)i); }
+    __device__ __forceinline__ float ldf(int j) const { return lds1(a + 4u * (unsigned)j); }
+    __device__ __forceinline__ void cp_async(int i, const float4 *src) const { cp_async16_s(a + 16u * (unsigned)i, src); }
 };
+
+// The observation frame of a state (ShipEnv.__add_states, ship_env.py:79-113): pose, rudder, nearest goal (gx, gy) and
+// lidar[0..9] as the state planes hold them (l0, l1, l2.xy).
+template <class ROW>
+__device__ __forceinline__ void store_frame(const ROW f, const EnvRegs &r, float gx, float gy, float4 l0, float4 l1, float4 l2)
+{
+    f.st(0, make_float4(r.x, r.y, (float)r.rudder, r.th));
+    f.st(1, make_float4(gx, gy, l0.x, l0.y));
+    f.st(2, make_float4(l0.z, l0.w, l1.x, l1.y));
+    f.st(3, make_float4(l1.z, l1.w, l2.x, l2.y));
+}
+
+// The env's state planes from r and the lidar readings of frame f (the newest: it holds the sticky readings).
+template <class ROW>
+__device__ __forceinline__ void store_env_frame(const StepParams &p, int e, const EnvRegs &r, const ROW f)
+{
+    const float4 l1 = f.ld(1), l2 = f.ld(2), l3 = f.ld(3);
+    store_env(p, e, r, make_float4(l1.z, l1.w, l2.x, l2.y), make_float4(l2.z, l2.w, l3.x, l3.y), l3.z, l3.w);
+}
+
+// The warp's eight statistics accumulators (warp_stats) -> the slot row of this CTA: one red.add per non-zero value.
+template <class ROW>
+__device__ __forceinline__ void flush_stats(const StepParams &p, int lane, const ROW stat)
+{
+    __syncwarp();
+    if (p.stats && lane < 8) {
+        const float v = stat.ldf(lane);
+        if (v != 0.f) atomicAdd(p.stats + (size_t)(blockIdx.x % kStatSlots) * kStatLen + lane, (double)v);
+    }
+}
+
+// Copies the raw records of a staged cell's candidate planes (cell.w: up to kMaxCand record indices, 0xff = none) into
+// raw[2i], raw[2i+1] (cp.async: they land while the caller does other work; plane_phase<..., STAGED> reads them).
+template <class ROW>
+__device__ __forceinline__ void stage_candidates(const StepParams &p, int scen, const uint4 cell, const ROW raw)
+{
+    const float4 *E4 = reinterpret_cast<const float4 *>(p.edges_d + (size_t)scen * (2 * kMaxHull));
+#pragma unroll
+    for (int n = 0; n < kMaxCand; ++n) {
+        const unsigned idx = (cell.w >> (8 * n)) & 0xffu;
+        if (idx != 0xffu) {
+            raw.cp_async(2 * n, E4 + 2 * idx);
+            raw.cp_async(2 * n + 1, E4 + 2 * idx + 1);
+        }
+    }
+}
+
+// One ray of the fan (body-frame direction rc, rs) against an env's plane row: cpPolyShapeSegmentQuery over the row's
+// planes, later accepted planes overwriting earlier ones; an origin inside a bank reads L (alpha = 0, `point` stays at
+// the ray end).  LiDAR.query: the first bank (list order) that reports a hit wins.  Returns the reading, < 0 for none.
+template <class ROW>
+__device__ __forceinline__ float ray_vs_row(const ROW row, float rc, float rs, float L)
+{
+    const float4 hdr = row.ld(0);
+    float dirx, diry;
+    ray_dir(hdr.x, hdr.y, rc, rs, dirx, diry);
+    const int hz = __float_as_int(hdr.z);
+    const int n = hz & 0xff;
+    float v0 = -1.f, v1 = -1.f;                     // hit distance per bank (< 0: none)
+#pragma unroll 1
+    for (int i = 0; i < n; ++i) {
+        const float4 e0 = row.ld(kRowPlane0 + 2 * i);
+        const float2 e1 = row.ld2(kRowPlane0 + 1 + 2 * i);
+        float val;
+        const bool ok = ray_vs_plane(e0.x, e0.y, e0.z, e0.w, e1.x, dirx, diry, L, val);
+        if (ok && e1.y == 0.f) v0 = val;
+        if (ok && e1.y != 0.f) v1 = val;
+    }
+    if (hz & kHdrIn0) v0 = L;
+    if (hz & kHdrIn1) v1 = L;
+    return v0 >= 0.f ? v0 : v1;
+}
 
 // Plane phase for one env at pose (x, y, c, s): fills the env's scratch row for the next lidar query and returns,
 // when WITH_SAT, bit b set <=> bank b is near and none of its candidate planes has the whole ship in front of it

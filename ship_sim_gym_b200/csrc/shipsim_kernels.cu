@@ -16,32 +16,15 @@
 
 #include <atomic>
 
-#ifndef SHIPSIM_MIN_BLOCKS
-#define SHIPSIM_MIN_BLOCKS 4
-#endif
+namespace shipsim {
+
 // Grids that fill the machine (one lane per env, >= 1,184 CTAs of 128 envs' worth): CTA size and CTAs per SM to aim
 // for.  Registers per thread follow from the pair: 128 x 5 -> 96, 64 x 9 -> 112, 128 x 4 / 64 x 8 -> 128.  Spills are
 // ruinous here (the L1 that would catch them is almost entirely carved out as shared memory), so the shape is chosen
 // as the most warps per SM that still compile without any.
-#ifndef SHIPSIM_SMALL_THREADS
-#define SHIPSIM_SMALL_THREADS 64
-#endif
-#ifndef SHIPSIM_BIG_THREADS
-#define SHIPSIM_BIG_THREADS 128
-#endif
-#ifndef SHIPSIM_BIG_MIN_BLOCKS
-#define SHIPSIM_BIG_MIN_BLOCKS 5
-#endif
-// SHIPSIM_TMA_STORE=1: observation rows leave the SM by TMA bulk copies (one cp.async.bulk.global.shared::cta per env
-// row, fence.proxy.async + bulk wait_group) instead of the loop of 128-bit shared loads + streaming stores.  Correct
-// (the whole GPU suite passes with it) but measured 15-17 % SLOWER (1M envs x 32 steps: 1.68 -> 1.98 ms; hard map 65,536
-// envs: 0.52 -> 0.61 ms; profiles/r02_tma_store_ab.log): a 128-byte row is too small a unit for the TMA engine -- 640
-// bulk operations per SM per step against 8 LDS + 8 STG per lane that issue in the shadow of other warps.  Off.
-#ifndef SHIPSIM_TMA_STORE
-#define SHIPSIM_TMA_STORE 0
-#endif
-
-namespace shipsim {
+constexpr int kBigThreads = 128, kBigMinBlocks = 5;
+// All other grids: CTA size, and CTAs of kThreads threads per SM to aim for (launch_g)
+constexpr int kSmallThreads = 64, kMinBlocks = 4;
 
 constexpr float kDeadGoal = 3.0e19f;        // coordinate of a goal that has been taken: its squared distance is +inf
 
@@ -169,11 +152,7 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
             // .z, .w: the goals-alive mask and the episode number live here, not in registers (a taken goal and a reset are
             // the only things that touch them)
             sts4(EA(GOL + 2), make_float4(g[4].x, g[4].y, __int_as_float(r.alive), __int_as_float(r.episode)));
-            // newest frame of the resident tile = frame of the current state
-            sts4(EA(NF), make_float4(r.x, r.y, (float)r.rudder, r.th));
-            sts4(EA(NF + 1), make_float4(gx, gy, l0.x, l0.y));
-            sts4(EA(NF + 2), make_float4(l0.z, l0.w, l1.x, l1.y));
-            sts4(EA(NF + 3), make_float4(l1.z, l1.w, l2.x, l2.y));
+            store_frame(RowSmem{EA(NF)}, r, gx, gy, l0, l1, l2);    // newest frame of the resident tile = frame of the current state
             if (WIDE) {                         // lidar[10 ..] from the appended state planes: float4 q of them = tile float4 NF + 4 + q
                 const int nx = extra_lidar_planes(nb);
                 for (int q = 0; q < nx; ++q) sts4(EA(NF + 4 + q), p.state[(size_t)(kPlanes + q) * p.N + (valid ? e : p.N - 1)]);
@@ -201,7 +180,6 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
             // the one value the 96-register build spilled -- and a spilled prefetch is a synchronous load)
             const int a = load_action_at(p, (size_t)k * p.N + min(e, p.N - 1), k, p.env_id_offset + e);   // (idle lanes read the last env's)
             // previous frame <- newest frame of the last step / reset (SURVEY.md App. A note N2); lidar stays in place
-            if (SHIPSIM_TMA_STORE && k > 0) bulk_store_wait_read();      // last step's row has left the tile: it may be rewritten
             if (HIST == 2 && gl == 0) {
                 if (!WIDE) {
                     const float4 f0 = lds4(EA(4)), f1 = lds4(EA(5)), f2 = lds4(EA(6)), f3 = lds4(EA(7));
@@ -239,27 +217,8 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
                 for (int q = rslot; q < cnt; q += rpp) {        // lanes 30, 31 (rslot 3) only keep the others company
                     if (rslot < rpp) {
                         const unsigned ra = WA(lds_u8(wb + SRC * 16 + q), 0);      // the env's block
-                        const float4 hdr = lds4(ra + SCR * 16);
-                        float dirx, diry;
-                        ray_dir(hdr.x, hdr.y, ray_c, ray_s, dirx, diry);
-                        const int hz = __float_as_int(hdr.z);
-                        const int n = hz & 0xff;
-                        float v0 = -1.f, v1 = -1.f;                     // hit distance per bank (< 0: none)
-#pragma unroll 1
-                        for (int i = 0; i < n; ++i) {   // cpPolyShapeSegmentQuery: later accepted edges overwrite earlier ones
-                            const float4 e0 = lds4(ra + (SCR + kRowPlane0 + 2 * i) * 16);
-                            const float2 e1 = lds2(ra + (SCR + kRowPlane0 + 1 + 2 * i) * 16);
-                            float val;
-                            const bool ok = ray_vs_plane(e0.x, e0.y, e0.z, e0.w, e1.x, dirx, diry, L, val);
-                            if (ok && e1.y == 0.f) v0 = val;
-                            if (ok && e1.y != 0.f) v1 = val;
-                        }
-                        if (hz & kHdrIn0) v0 = L;       // origin inside the bank: alpha = 0, `point` stays at the ray end
-                        if (hz & kHdrIn1) v1 = L;
-                        // LiDAR.query: the first bank (list order) that reports a hit wins; misses keep the old reading
-                        // (sticky vals, models.py:71)
-                        const float v = v0 >= 0.f ? v0 : v1;
-                        if (v >= 0.f) sts1(ra + 4 * (CF + 6 + rj), v);
+                        const float v = ray_vs_row(RowSmem{ra + SCR * 16}, ray_c, ray_s, L);
+                        if (v >= 0.f) sts1(ra + 4 * (CF + 6 + rj), v);          // misses keep the old reading (sticky vals, models.py:71)
                     }
                 }
             }
@@ -292,17 +251,8 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
         const uint4 cell = lds4u(EA(CEL));
         const bool near_any = leader && (cell.x | cell.y | (cell.z & 3u)) != 0u;
         const bool staged = near_any && ((cell.z >> 8) & 0xffu) <= (unsigned)kMaxCand;
-        if (staged) {
-            const float4 *E4 = reinterpret_cast<const float4 *>(p.edges_d + (size_t)r.scen * (2 * kMaxHull));
-#pragma unroll
-            for (int n = 0; n < kMaxCand; ++n) {
-                const unsigned idx = (cell.w >> (8 * n)) & 0xffu;
-                if (idx != 0xffu) {
-                    cp_async16_s(EA((G > 1 ? RAW : SCR + 1) + 2 * n), E4 + 2 * idx);
-                    cp_async16_s(EA((G > 1 ? RAW : SCR + 1) + 2 * n + 1), E4 + 2 * idx + 1);
-                }
-            }
-        }
+        const RowSmem raw{G > 1 ? EA(RAW) : EA(SCR + 1)};
+        if (staged) stage_candidates(p, r.scen, cell, raw);
         bool all_goals = false;
         if (live) {     // (while the candidate planes are in flight)
             // ---- goals (collide_goal, game.py:243-257) and the nearest remaining goal (closest_goal, game.py:333-349).
@@ -358,7 +308,7 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
         cp_async_wait_all();
         unsigned ask = 0u;
         if (leader) {
-            if (staged) ask = plane_phase<true, true>(p, r.x, r.y, hx, hy, c, s, r.scen, cell, RowSmem{EA(SCR)}, RowSmem{G > 1 ? EA(RAW) : EA(SCR + 1)});
+            if (staged) ask = plane_phase<true, true>(p, r.x, r.y, hx, hy, c, s, r.scen, cell, RowSmem{EA(SCR)}, raw);
             else if (near_any) ask = plane_phase<true, false>(p, r.x, r.y, hx, hy, c, s, r.scen, cell, RowSmem{EA(SCR)}, RowSmem{0u});
             else sts4(EA(SCR), make_float4(c, s, 0.f, 0.f));
         }
@@ -488,10 +438,9 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
                 c = 1.f; s = 0.f;
                 hx = 0.5f * (p.ship_aabb[2] - p.ship_aabb[0]); hy = 0.5f * (p.ship_aabb[3] - p.ship_aabb[1]);
                 {
-                    const float4 *rec = p.bank + (size_t)r.scen * p.scen_stride4;
+                    float4 rg0, rg1, rg2;
                     float2 gn[kGoals];
-                    const float4 rg0 = __ldg(rec + 2), rg1 = __ldg(rec + 3), rg2 = __ldg(rec + 4);
-                    unpack_goals(rg0, rg1, rg2, gn);
+                    scenario_goals(p, r.scen, rg0, rg1, rg2, gn);
                     closest_goal(gn, r.alive, r.x, r.y, gx, gy);
                     if (gl == 0) {
                         sts4(EA(GOL), rg0); sts4(EA(GOL + 1), rg1);
@@ -543,7 +492,6 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
         if (live) {
             // ---- outputs: obs rows of the warp's envs are contiguous in global memory, so the tile is copied out with
             // fully coalesced 128-bit streaming stores.
-            if (SHIPSIM_TMA_STORE) fence_proxy_async();     // this lane's writes to the tiles (its own frame, other envs' rays)
             __syncwarp();
             if (WIDE) {
                 // Rows of R = (6 + n) * HIST floats are dense in global memory and in general not 16-byte aligned, so the
@@ -566,23 +514,17 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
                         if (col >= R) { col -= R; ++row; }
                     }
                 }
-            } else {
-#if SHIPSIM_TMA_STORE
-            if (p.obs && leader) bulk_store(p.obs + ((size_t)k * p.N + e) * OBS4, EA(0), OBS4 * 16);
-#else
-            // lane -> (row lane / OBS4, column lane % OBS4), each further round moves 32 / OBS4 rows down.  A round is real
-            // iff its row belongs to an env of this batch, i.e. iff its address lies before the end of this step's rows
-            // (tested against the step's end pointer, which moves with k: a loop-invariant row limit was hoisted, spilled
-            // and reloaded from local memory right here in every iteration)
-            if (p.obs && lane < EPW * OBS4) {
+            } else if (p.obs && lane < EPW * OBS4) {
+                // lane -> (row lane / OBS4, column lane % OBS4), each further round moves 32 / OBS4 rows down.  A round is
+                // real iff its row belongs to an env of this batch, i.e. iff its address lies before the end of this step's
+                // rows (tested against the step's end pointer, which moves with k: a loop-invariant row limit was hoisted,
+                // spilled and reloaded from local memory right here in every iteration)
                 const unsigned cp_src = WA(lane / OBS4, lane % OBS4);
                 float4 *o = p.obs + ((size_t)k * p.N + (e - grp)) * OBS4 + lane;
                 const float4 *o_end = p.obs + (size_t)(k + 1) * p.N * OBS4;
 #pragma unroll
                 for (int i = 0; i < (EPW * OBS4 >= 32 ? EPW * OBS4 / 32 : 1); ++i)
                     if (o + i * 32 < o_end) __stcs(o + i * 32, lds4(cp_src + i * (32 / OBS4) * (EB4 * 16)));
-            }
-#endif
             }
             if (leader) {
                 const size_t row = (size_t)k * p.N + e;
@@ -593,25 +535,17 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
         __syncwarp();                           // copy-out done and plane rows complete before the next iteration
     }
     // the loop leaves the pose of the last step in r (no integration after it)
-    if (SHIPSIM_TMA_STORE) bulk_store_wait_read();
     if (leader) {
-        const float4 l1 = lds4(EA(NF + 1)), l2 = lds4(EA(NF + 2)), l3 = lds4(EA(NF + 3));
         r.episode = __float_as_int(lds1(EA(GOL + 2) + 12));
         r.alive = __float_as_int(lds1(EA(GOL + 2) + 8));
         r.rudder = (int)lds1(EA(NF) + 8);
-        store_env(p, e, r, make_float4(l1.z, l1.w, l2.x, l2.y), make_float4(l2.z, l2.w, l3.x, l3.y), l3.z, l3.w);
+        store_env_frame(p, e, r, RowSmem{EA(NF)});
         if (WIDE) {
             const int nx = extra_lidar_planes(nb);
             for (int q = 0; q < nx; ++q) p.state[(size_t)(kPlanes + q) * p.N + e] = lds4(EA(NF + 4 + q));
         }
     }
-
-    // episode statistics: one red.add per non-zero value per warp into a slot row
-    __syncwarp();
-    if (lane < 8 && p.stats) {
-        const float v = lds1(wb + STA * 16 + 4 * lane);
-        if (v != 0.f) atomicAdd(p.stats + (size_t)(blockIdx.x % kStatSlots) * kStatLen + lane, (double)v);
-    }
+    flush_stats(p, lane, RowSmem{wb + STA * 16});
 #undef EA
 #undef WA
 }
@@ -736,17 +670,15 @@ __global__ void __launch_bounds__(256) reset_kernel(const __grid_constant__ Step
     int scen = scenario ? scenario[e] : pick_scenario(p, p.env_id_offset + e, ep);
     scen = min(max(scen, 0), p.n_scen - 1);       // caller-supplied ids index the bank: never out of range (the host layer raises first)
     reset_env(p, r, scen, ep);
-    const float4 *rec = p.bank + (size_t)scen * p.scen_stride4;
-    g0 = __ldg(rec + 2); g1 = __ldg(rec + 3); g2 = __ldg(rec + 4);
+    float2 g[kGoals];
+    float gx, gy;
+    scenario_goals(p, scen, g0, g1, g2, g);
+    closest_goal(g, r.alive, r.x, r.y, gx, gy);
     const float4 neg4 = make_float4(-1.f, -1.f, -1.f, -1.f);      // models.py:36: LiDAR.vals start at -1
     store_env(p, e, r, neg4, neg4, -1.f, -1.f);
     for (int q = 0; q < extra_lidar_planes(p.n_beams); ++q) p.state[(size_t)(kPlanes + q) * p.N + e] = neg4;
     store_goals(p, e, g0, g1, g2);
-    if (obs && p.n_beams != kBeams) {           // rows of (6 + n) * history floats: [-1 x (6 + n) | x, y, 0, 0, gx, gy, -1 x n]
-        float gx, gy;
-        float2 g[kGoals];
-        unpack_goals(g0, g1, g2, g);
-        closest_goal(g, r.alive, r.x, r.y, gx, gy);
+    if (obs) {                                  // rows of (6 + n) * history floats: [-1 x (6 + n) | x, y, 0, 0, gx, gy, -1 x n]
         const int F = 6 + p.n_beams;
         float *o = reinterpret_cast<float *>(obs) + (size_t)e * F * p.history;
         if (p.history == 2) {
@@ -755,18 +687,6 @@ __global__ void __launch_bounds__(256) reset_kernel(const __grid_constant__ Step
         }
         o[0] = r.x; o[1] = r.y; o[2] = 0.f; o[3] = 0.f; o[4] = gx; o[5] = gy;
         for (int i = 6; i < F; ++i) o[i] = -1.f;
-    } else if (obs) {
-        float gx, gy;
-        float2 g[kGoals];
-        unpack_goals(g0, g1, g2, g);
-        closest_goal(g, r.alive, r.x, r.y, gx, gy);
-        float4 *o = obs + (size_t)e * (4 * p.history);
-        const float4 neg = make_float4(-1.f, -1.f, -1.f, -1.f);
-        if (p.history == 2) { o[0] = neg; o[1] = neg; o[2] = neg; o[3] = neg; o += 4; }
-        o[0] = make_float4(r.x, r.y, 0.f, 0.f);
-        o[1] = make_float4(gx, gy, -1.f, -1.f);
-        o[2] = neg;
-        o[3] = neg;
     }
 }
 
@@ -795,11 +715,7 @@ __global__ void __launch_bounds__(256) frame_kernel(const __grid_constant__ Step
     unpack_goals(g0, g1, g2, g);
     float gx, gy;
     closest_goal(g, r.alive, r.x, r.y, gx, gy);
-    float4 *o = out + (size_t)e * 4;
-    o[0] = make_float4(r.x, r.y, (float)r.rudder, r.th);
-    o[1] = make_float4(gx, gy, l0.x, l0.y);
-    o[2] = make_float4(l0.z, l0.w, l1.x, l1.y);
-    o[3] = make_float4(l1.z, l1.w, l2.x, l2.y);
+    store_frame(RowPtr{out + (size_t)e * 4}, r, gx, gy, l0, l1, l2);
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -964,17 +880,17 @@ static cudaError_t launch_g(const StepParams &p, cudaStream_t stream, LaunchShap
     cudaError_t err = cudaSuccess;
     if constexpr (G == 1) {
         if (blocks >= 148 * 8) {
-            threads = SHIPSIM_BIG_THREADS;
+            threads = kBigThreads;
             blocks = (p.N + threads - 1) / threads;
-            if (p.history == 2) err = launch_gh<G, 2, SHIPSIM_BIG_MIN_BLOCKS, SHIPSIM_BIG_THREADS, NB>(p, blocks, stream);
-            else err = launch_gh<G, 1, SHIPSIM_BIG_MIN_BLOCKS, SHIPSIM_BIG_THREADS, NB>(p, blocks, stream);
+            if (p.history == 2) err = launch_gh<G, 2, kBigMinBlocks, kBigThreads, NB>(p, blocks, stream);
+            else err = launch_gh<G, 1, kBigMinBlocks, kBigThreads, NB>(p, blocks, stream);
             launched = true;
         }
     }
     if (!launched) {
         // Grids that do not fill the machine: 64-thread CTAs (same 16 warps per SM at 128 registers), so that the few
         // CTAs spread evenly -- 65,536 envs are 512 CTAs of 128 threads, 3.46 per SM: every SM waits for the ones that got 4
-        constexpr int T = SHIPSIM_SMALL_THREADS, MB = SHIPSIM_MIN_BLOCKS * kThreads / SHIPSIM_SMALL_THREADS;
+        constexpr int T = kSmallThreads, MB = kMinBlocks * kThreads / kSmallThreads;
         threads = T;
         blocks = (p.N + T / G - 1) / (T / G);
         if (p.history == 2) err = launch_gh<G, 2, MB, T, NB>(p, blocks, stream);

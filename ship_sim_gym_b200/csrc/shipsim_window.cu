@@ -35,29 +35,17 @@
 
 namespace shipsim {
 
-// The two physics scans are unrolled over the whole window when it is short (every shuffle that feeds the chains is then
-// issued ahead of them: 4 -> 16 iterations per trip took the headline from 0.458 to 0.449 ms), by 4 for the longest
-// window (T = 32 fully unrolled is 9 % SLOWER at 2,048 envs: code size).
-#ifndef SHIPSIM_SCAN_UNROLL
-#define SHIPSIM_SCAN_UNROLL (T <= 16 ? T : 4)
-#endif
-#define SHIPSIM_PRAGMA_(x) _Pragma(#x)
-#define SHIPSIM_UNROLL(n) SHIPSIM_PRAGMA_(unroll n)
-#ifndef SHIPSIM_WIN_THREADS
-#define SHIPSIM_WIN_THREADS 32
-#endif
-constexpr int kWinThreads = SHIPSIM_WIN_THREADS;      // one-warp CTAs: a latency-bound batch is a few thousand warps, spread them evenly over the SMs (64 -> 32 threads: 0.460 -> 0.458 ms on the headline, -1.8 % at 2,048 envs)
-#ifdef SHIPSIM_WIN_MAXNREG
-#define SHIPSIM_WIN_BOUNDS __maxnreg__(SHIPSIM_WIN_MAXNREG)
-#else
-#define SHIPSIM_WIN_BOUNDS __launch_bounds__(kWinThreads, 512 / SHIPSIM_WIN_THREADS)
-#endif
+constexpr int kWinThreads = 32;      // one-warp CTAs: a latency-bound batch is a few thousand warps, spread them evenly over the SMs (64 -> 32 threads: 0.460 -> 0.458 ms on the headline, -1.8 % at 2,048 envs)
 
 // LOG: write the episode log (shipsim_episode_log_bind).  The log-free kernel is a separate instantiation: its registers
 // and spills are those of the kernel before the log existed (-Xptxas -v; this kernel sits at the 128-register wall).
 template <int T, int HIST, bool LOG>
-__global__ void SHIPSIM_WIN_BOUNDS window_kernel(const __grid_constant__ StepParams p)
+__global__ void __launch_bounds__(kWinThreads, 512 / kWinThreads) window_kernel(const __grid_constant__ StepParams p)
 {
+    // The two physics scans are unrolled over the whole window when it is short (every shuffle that feeds the chains is
+    // then issued ahead of them: 4 -> 16 iterations per trip took the headline from 0.458 to 0.449 ms), by 4 for the
+    // longest window (T = 32 fully unrolled is 9 % SLOWER at 2,048 envs: code size).
+    constexpr int kScanUnroll = T <= 16 ? T : 4;
     constexpr int E = 32 / T;                   // envs per warp
     constexpr int NW = kWinThreads / 32;
     constexpr int OBS4 = 4 * HIST;              // float4 per obs row
@@ -74,7 +62,7 @@ __global__ void SHIPSIM_WIN_BOUNDS window_kernel(const __grid_constant__ StepPar
     __shared__ int4 s_env[NW * E];              // per env, for the copy-out: step cursor, committed steps, (carry slot of the plane ring), reset?
     __shared__ float s_ray[2 * 32];
     __shared__ unsigned s_src[NW][32];          // ray pass: compacted (plane row | frame offset) of the needy steps
-    __shared__ float s_stat[NW][8];
+    __shared__ __align__(16) float s_stat[NW][8];   // (warp_stats reads and writes it as two float4)
 
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int el = lane / T, t = lane % T;
@@ -125,11 +113,7 @@ __global__ void SHIPSIM_WIN_BOUNDS window_kernel(const __grid_constant__ StepPar
         if (t == 0) {
 #pragma unroll
             for (int i = 0; i < kGoals; ++i) s_goal[goal0 + i] = g[i];
-            float4 *f = s_frame + fr0;          // carry frame = frame of the current state
-            f[0] = make_float4(r.x, r.y, (float)r.rudder, r.th);
-            f[1] = make_float4(gx, gy, l0.x, l0.y);
-            f[2] = make_float4(l0.z, l0.w, l1.x, l1.y);
-            f[3] = make_float4(l1.z, l1.w, l2.x, l2.y);
+            store_frame(RowPtr{s_frame + fr0}, r, gx, gy, l0, l1, l2);     // carry frame = frame of the current state
             float hx, hy;                       // carry row = planes of the current pose
             hull_half_extents(p, c0, s0, hx, hy);
             const uint4 cell = load_cell(p, r.scen, r.x + hx, r.y + hy);
@@ -201,7 +185,7 @@ __global__ void SHIPSIM_WIN_BOUNDS window_kernel(const __grid_constant__ StepPar
                 const float dw_t = a_my == 0 ? -p.ang_dt * (float)rud_t : 0.f;
                 float th = r.th, w = r.w;
                 float2 *po = reinterpret_cast<float2 *>(ph);
-SHIPSIM_UNROLL(SHIPSIM_SCAN_UNROLL)
+#pragma unroll kScanUnroll
                 for (int i = 0; i < T; ++i) {
                     const float dw = __shfl_sync(kFull, dw_t, i, T);
                     th += w * p.dt;
@@ -225,7 +209,7 @@ SHIPSIM_UNROLL(SHIPSIM_SCAN_UNROLL)
             {
                 float x = r.x, y = r.y, vx = r.vx, vy = r.vy;
                 float4 *po = ph + 1;
-SHIPSIM_UNROLL(SHIPSIM_SCAN_UNROLL)
+#pragma unroll kScanUnroll
                 for (int i = 0; i < T; ++i) {
                     const float dvx = __shfl_sync(kFull, dvx_t, i, T), dvy = __shfl_sync(kFull, dvy_t, i, T);
                     x += vx * p.dt;
@@ -277,17 +261,7 @@ SHIPSIM_UNROLL(SHIPSIM_SCAN_UNROLL)
 
         const bool near_any = active && (cell.x | cell.y | (cell.z & 3u)) != 0u;
         const bool staged = near_any && ((cell.z >> 8) & 0xffu) <= (unsigned)kMaxCand;
-        if (staged) {
-            const float4 *E4 = reinterpret_cast<const float4 *>(p.edges_d + (size_t)r.scen * (2 * kMaxHull));
-#pragma unroll
-            for (int n = 0; n < kMaxCand; ++n) {
-                const unsigned idx = (cell.w >> (8 * n)) & 0xffu;
-                if (idx != 0xffu) {
-                    cp_async16(myrow + 1 + 2 * n, E4 + 2 * idx);
-                    cp_async16(myrow + 2 + 2 * n, E4 + 2 * idx + 1);
-                }
-            }
-        }
+        if (staged) stage_candidates(p, r.scen, cell, RowPtr{myrow + 1});
         const bool oob = (mx < 0.f) || (mx > p.W) || (my < 0.f) || (my > p.H);
         // (while the candidate planes are in flight: the exact goal tests and everything that follows from them)
 #pragma unroll 1
@@ -457,25 +431,7 @@ SHIPSIM_UNROLL(SHIPSIM_SCAN_UNROLL)
                 for (int q = rslot; q < cnt; q += 3) {
                     if (rslot < 3) {
                         const unsigned sw = s_src[warp][q];
-                        const int rw = wsc0 + (int)(sw & 0xffffu);
-                        const float4 hdr = s_scr[rw];
-                        float dirx, diry;
-                        ray_dir(hdr.x, hdr.y, ray_c, ray_s, dirx, diry);
-                        const int hz = __float_as_int(hdr.z);
-                        const int n = hz & 0xff;
-                        float v0 = -1.f, v1 = -1.f;
-#pragma unroll 1
-                        for (int i = 0; i < n; ++i) {
-                            const float4 e0 = s_scr[rw + 1 + 2 * i];
-                            const float2 e1 = *reinterpret_cast<const float2 *>(s_scr + rw + 2 + 2 * i);
-                            float val;
-                            const bool ok = ray_vs_plane(e0.x, e0.y, e0.z, e0.w, e1.x, dirx, diry, L, val);
-                            if (ok && e1.y == 0.f) v0 = val;
-                            if (ok && e1.y != 0.f) v1 = val;
-                        }
-                        if (hz & kHdrIn0) v0 = L;
-                        if (hz & kHdrIn1) v1 = L;
-                        const float v = v0 >= 0.f ? v0 : v1;
+                        const float v = ray_vs_row(RowPtr{s_scr + wsc0 + (int)(sw & 0xffffu)}, ray_c, ray_s, L);
                         if (v >= 0.f) reinterpret_cast<float *>(s_frame + wfr0)[(sw >> 16) + rj] = v;
                     }
                 }
@@ -546,14 +502,13 @@ SHIPSIM_UNROLL(SHIPSIM_SCAN_UNROLL)
             const int ep = r.episode + 1;
             reset_env(p, rn, next_scen, ep);
             c0n = 1.f; s0n = 0.f;
-            const float4 *rec = p.bank + (size_t)rn.scen * p.scen_stride4;
             const float4 *sp = p.spawn_rows + (size_t)rn.scen * kScr4;
-            const float4 rg0 = __ldg(rec + 2), rg1 = __ldg(rec + 3), rg2 = __ldg(rec + 4);
+            float4 rg0, rg1, rg2;
+            float2 gn[kGoals];
+            scenario_goals(p, rn.scen, rg0, rg1, rg2, gn);
 #pragma unroll
             for (int i = 0; i < SPL; ++i) if (t + i * T < kScr4) spv[i] = __ldg(sp + t + i * T);
             next_scen = pick_scenario_keyed(p, pkey, ep + 1);
-            float2 gn[kGoals];
-            unpack_goals(rg0, rg1, rg2, gn);
             float rgx, rgy;
             closest_goal(gn, rn.alive, rn.x, rn.y, rgx, rgy);
             if (t == 0) {
@@ -642,19 +597,13 @@ SHIPSIM_UNROLL(SHIPSIM_SCAN_UNROLL)
     }
 
     if (valid && t == 0) {
-        const float4 *f = s_frame + fr0;
-        const float4 l1 = f[1], l2 = f[2], l3 = f[3];
-        store_env(p, e, r, make_float4(l1.z, l1.w, l2.x, l2.y), make_float4(l2.z, l2.w, l3.x, l3.y), l3.z, l3.w);
+        store_env_frame(p, e, r, RowPtr{s_frame + fr0});
         if (goals_dirty) {
             const float2 a0 = s_goal[goal0], a1 = s_goal[goal0 + 1], a2 = s_goal[goal0 + 2], a3 = s_goal[goal0 + 3], a4 = s_goal[goal0 + 4];
             store_goals(p, e, make_float4(a0.x, a0.y, a1.x, a1.y), make_float4(a2.x, a2.y, a3.x, a3.y), make_float4(a4.x, a4.y, 0.f, 0.f));
         }
     }
-    __syncwarp();
-    if (lane < 8 && p.stats) {
-        const float v = stat[lane];
-        if (v != 0.f) atomicAdd(p.stats + (size_t)(blockIdx.x % kStatSlots) * kStatLen + lane, (double)v);
-    }
+    flush_stats(p, lane, RowPtr{reinterpret_cast<float4 *>(s_stat[warp])});
 #undef stat
 }
 
