@@ -170,6 +170,18 @@ int shipsim_fresh_maps(shipsim_t *h, int32_t enable);
 /* info[8] = enabled, period, first scenario and size of the slice resets pick from, regeneration count of the 4 slices. */
 int shipsim_fresh_info(const shipsim_t *h, int32_t *info);
 
+/* Weighted scenario picks: resets (automatic and shipsim_reset without explicit scenarios) draw map i with probability
+ * w[i] / sum(w) instead of uniformly, e.g. to hold maps out of training (weight 0) or to replay the maps a policy still
+ * fails on.  dev_weights = uint32 w[n_scenarios] in DEVICE memory; the handle's table (prefix sums and a guide table, 8
+ * bytes per scenario, allocated with the bank) is rebuilt from it by one kernel enqueued on `stream`: no allocation, no
+ * synchronisation, so the call may sit between the replays of a captured CUDA graph, whose step launches then read the
+ * new table.  The pick stays keyed by (seed, global env id, episode): equal weights give exactly the uniform picks, and
+ * the draws do not depend on how the envs are sharded.  Where every weight is 0, or the weights sum to 2^32 or more,
+ * the picks are uniform.  dev_weights == NULL returns to uniform picks.  A new bank (shipsim_load_scenarios,
+ * shipsim_generate_scenarios) drops the weights.  Fresh maps (shipsim_fresh_maps) never replay a map, so the two exclude
+ * each other: weights while fresh maps are on, and fresh maps while weights are on, fail with SHIPSIM_ERR_STATE. */
+int shipsim_scenario_weights(shipsim_t *h, const uint32_t *dev_weights, void *stream);
+
 /* Read the device-generated bank back (validation / inspection): host_hull_xy[n][2][SHIPSIM_MAX_HULL][2] (CCW, zero
  * padded), host_hull_n[n][2], host_goals[n][5][2]; hull vertices are the fp32-rounded ones the kernels use. */
 int shipsim_read_scenarios(shipsim_t *h, double *host_hull_xy, int32_t *host_hull_n, double *host_goals);

@@ -5,7 +5,7 @@ behind the C ABI in include/shipsim.h).  There is no CPU fallback: constructing 
 library or without a B200 raises.
 """
 from .config import EnvConfig, GameConfig, LidarConfig  # noqa: F401
-from .curriculum import Curriculum, CurriculumDriver, Lesson, LessonCondition  # noqa: F401
+from .curriculum import Curriculum, CurriculumDriver, Lesson, LessonCondition, LevelReplay  # noqa: F401
 from .scenario import ScenarioBank  # noqa: F401
 
 

@@ -28,6 +28,7 @@ SYMBOLS = (
     "shipsim_launch_count", "shipsim_launch_shape", "shipsim_launch_window", "shipsim_set_max_steps",
     "shipsim_generate_scenarios", "shipsim_read_scenarios", "shipsim_render", "shipsim_assemble_history", "shipsim_expand_delta", "shipsim_host_traffic", "shipsim_host_threads",
     "shipsim_fresh_maps", "shipsim_fresh_info", "shipsim_mlp_policy_forward", "shipsim_gae", "shipsim_episode_log_bind",
+    "shipsim_scenario_weights",
 )
 
 
@@ -89,6 +90,7 @@ def load():
     L.shipsim_host_threads.argtypes = [vp, C.POINTER(i32)]
     L.shipsim_fresh_maps.argtypes = [vp, i32]
     L.shipsim_fresh_info.argtypes = [vp, C.POINTER(i32)]
+    L.shipsim_scenario_weights.argtypes = [vp, vp, vp]
     L.shipsim_mlp_policy_forward.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.shipsim_gae.argtypes = [vp, vp, vp, i32, i32, C.c_float, C.c_float, vp, vp, vp]
     L.shipsim_episode_log_bind.argtypes = [vp, vp, vp, i32, vp]

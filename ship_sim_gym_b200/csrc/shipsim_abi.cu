@@ -125,6 +125,7 @@ struct Bank {
     DeviceBuf<EdgeD> edges;                  // [n_scen][2][kMaxHull] two-float planes
     DeviceBuf<uint4> grid;                   // [n_scen][kGridN * kGridN] reach grid
     DeviceBuf<float4> spawn;                 // [n_scen][kScr4] plane rows at the spawn pose
+    DeviceBuf<unsigned> pick;                // [2][n_scen + 1] weighted-pick table (cdf, guide): shipsim_scenario_weights
     int n_scen = 0, maxv = 0, stride4 = 0, hull_max = 0;
     bool generated = false;                  // by shipsim_generate_scenarios: fresh maps may regenerate it in place
 
@@ -135,6 +136,7 @@ struct Bank {
         if (e == cudaSuccess) e = edges.ensure((size_t)n * 2 * kMaxHull);
         if (e == cudaSuccess) e = grid.ensure((size_t)n * kGridN * kGridN);
         if (e == cudaSuccess) e = spawn.ensure((size_t)n * kScr4);
+        if (e == cudaSuccess) e = pick.ensure(2 * ((size_t)n + 1));
         return e;
     }
 };
@@ -503,6 +505,7 @@ static int install(shipsim_t *h, Bank &&b, cudaStream_t s)
     p.bank = nb.rec; p.edges_d = nb.edges; p.grid = nb.grid; p.spawn_rows = nb.spawn;
     p.n_scen = nb.n_scen; p.maxv = nb.maxv; p.scen_stride4 = nb.stride4; p.hull_max = nb.hull_max;
     h->fresh.on = false; h->fresh.pending = false; p.pick_base = 0; p.pick_count = 0;
+    p.pick_cdf = nullptr; p.pick_guide = nullptr;              // weights belong to the old bank
     if (p.state && nb.n_scen < old_n) {
         CU(launch_clamp_scenarios(p.state, h->cfg.num_envs, nb.n_scen, s));
         CU(cudaStreamSynchronize(s));
@@ -695,6 +698,7 @@ extern "C" int shipsim_fresh_maps(shipsim_t *h, int32_t enable)
         return SHIPSIM_OK;
     }
     Bank &b = h->bank;
+    if (h->p.pick_cdf) return fail(SHIPSIM_ERR_STATE, "fresh maps replay no map: turn scenario weights off first (shipsim_scenario_weights NULL)");
     if (!b.generated) return fail(SHIPSIM_ERR_STATE, "fresh maps need a device-generated bank: call shipsim_generate_scenarios first");
     const int q = b.n_scen / 4;
     if (b.n_scen % 4 != 0 || q < 1 || (q & (q - 1)) != 0)
@@ -718,6 +722,23 @@ extern "C" int shipsim_fresh_info(const shipsim_t *h, int32_t *info)
     if (!h || !info) return fail(SHIPSIM_ERR_ARG, "NULL argument");
     info[0] = h->fresh.on ? 1 : 0; info[1] = h->fresh.period; info[2] = h->p.pick_base; info[3] = h->p.pick_count;
     for (int i = 0; i < 4; ++i) info[4 + i] = h->fresh.generation[i];
+    return SHIPSIM_OK;
+}
+
+extern "C" int shipsim_scenario_weights(shipsim_t *h, const uint32_t *dev_weights, void *stream)
+{
+    if (!h) return fail(SHIPSIM_ERR_ARG, "handle is NULL");
+    if (!h->p.bank) return fail(SHIPSIM_ERR_STATE, "shipsim_load_scenarios has not been called");
+    if (!dev_weights) {
+        h->p.pick_cdf = nullptr; h->p.pick_guide = nullptr;
+        return SHIPSIM_OK;
+    }
+    if (h->fresh.on) return fail(SHIPSIM_ERR_STATE, "scenario weights replay maps: fresh maps are on (shipsim_fresh_maps 0 first)");
+    DeviceGuard g(h->device);
+    Bank &b = h->bank;
+    CU(launch_build_pick_table(dev_weights, b.n_scen, b.pick, (cudaStream_t)stream));
+    h->launches++;
+    h->p.pick_cdf = b.pick; h->p.pick_guide = b.pick + b.n_scen + 1;
     return SHIPSIM_OK;
 }
 

@@ -111,6 +111,11 @@ struct StepParams {
     // parameter offsets in the tuned kernels)
     int n_beams;                                     // 1 .. kMaxBeams
     float ray_cw[kMaxBeams], ray_sw[kMaxBeams];      // the whole fan's ray table (entries past n_beams: unused)
+    // weighted scenario picks (shipsim_scenario_weights; pick_cdf == nullptr: uniform picks, and the step kernels run their
+    // pick-free instantiation).
+    // Appended for the same reason as the beam fields.  Built on the stream by build_pick_table_kernel.
+    const unsigned *pick_cdf;                        // [n_scen + 1]: inclusive prefix sums of the weights, then the total (0: uniform)
+    const unsigned *pick_guide;                      // [n_scen + 1]: first i with cdf[i] > floor(j * total / n_scen); [n_scen] = n_scen - 1
 };
 
 // State planes [kPlanes, kPlanes + extra_lidar_planes(n)) hold lidar[10 .. n-1], four readings per plane.
@@ -185,17 +190,43 @@ __device__ __forceinline__ unsigned pick_key(const StepParams &p, long long gid)
     k = mix32(k ^ (unsigned)(unsigned long long)gid);
     return mix32(k ^ (unsigned)((unsigned long long)gid >> 32));
 }
+// Weighted pick from the hash h (shipsim_scenario_weights): with t = umulhi(h, total), the first i with cdf[i] > t.  The
+// answer lies in [guide[j], guide[j + 1]] for the bucket j = umulhi(h, n_scen) (floor(j * total / n) <= t <
+// floor((j + 1) * total / n) + 1), so a binary search over that range ends it: a run of zero weights costs no linear scan.
+// With equal weights w the pick is floor(umulhi(h, n * w) / w) == umulhi(h, n), the uniform pick; total == 0 (all weights
+// zero, or a sum of 2^32 or more) falls back to it as well.
+__device__ __forceinline__ int pick_weighted(const StepParams &p, unsigned h)
+{
+    const unsigned n = (unsigned)p.n_scen;
+    const unsigned j = __umulhi(h, n);
+    const unsigned total = __ldg(p.pick_cdf + n);
+    unsigned lo = __ldg(p.pick_guide + j), hi = __ldg(p.pick_guide + j + 1);
+    if (total == 0u) return (int)j;
+    const unsigned t = __umulhi(h, total);
+    while (lo < hi) {
+        const unsigned mid = (lo + hi) >> 1;
+        if (__ldg(p.pick_cdf + mid) > t) hi = mid;
+        else lo = mid + 1u;
+    }
+    return (int)lo;
+}
+// PICK: weighted picks (p.pick_cdf != nullptr).  The step kernels take it as a template flag, like the episode log's LOG,
+// so that their weight-free instantiations are the kernels as they were.
+template <bool PICK>
 __device__ __forceinline__ int pick_scenario_keyed(const StepParams &p, unsigned key, int episode)
 {
     if (p.pick_count > 0) {
         const unsigned stride = mix32(key ^ 0x5bd1e995u) | 1u;
         return p.pick_base + (int)((key + (unsigned)episode * stride) & (unsigned)(p.pick_count - 1));
     }
-    return (int)__umulhi(mix32(key + (unsigned)episode * 0x9E3779B9u), (unsigned)p.n_scen);
+    const unsigned h = mix32(key + (unsigned)episode * 0x9E3779B9u);
+    if (PICK) return pick_weighted(p, h);
+    return (int)__umulhi(h, (unsigned)p.n_scen);
 }
+template <bool PICK>
 __device__ __forceinline__ int pick_scenario(const StepParams &p, long long gid, int episode)
 {
-    return pick_scenario_keyed(p, pick_key(p, gid), episode);
+    return pick_scenario_keyed<PICK>(p, pick_key(p, gid), episode);
 }
 
 __device__ __forceinline__ int random_action(const StepParams &p, long long gid, unsigned step)

@@ -39,6 +39,7 @@ constexpr float kDeadGoal = 3.0e19f;        // coordinate of a goal that has bee
 // in their registers.)
 // LOG: write the episode log (shipsim_episode_log_bind).  The log-free kernel is a separate instantiation: its registers
 // and spills are those of the kernel before the log existed (-Xptxas -v).
+// PICK: weighted scenario picks (shipsim_scenario_weights), a separate instantiation for the same reason.
 // NB: lidar capacity.  kBeams (10) is the tuned kernel of the reference's fan, with the beam count a compile-time constant;
 // kMaxBeams (32) is the wide kernel: a 32-reading frame slot, p.n_beams (1..32) rays at run time, and its shared memory
 // allocated dynamically (StepLayout::BYTES; the G = 1 blocks exceed the 48 KB of a static allocation).  Everything else --
@@ -69,7 +70,7 @@ __device__ __forceinline__ float4 *step_smem()
     }
 }
 
-template <int G, int HIST, int MINB, int THREADS, bool LOG, int NB>
+template <int G, int HIST, int MINB, int THREADS, bool LOG, int NB, bool PICK>
 __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_constant__ StepParams p)
 {
     using LY = StepLayout<G, HIST, NB, THREADS>;
@@ -434,7 +435,7 @@ __global__ void __launch_bounds__(THREADS, MINB) step_kernel(const __grid_consta
             }
             if (do_reset) {
                 const int ep = G > 1 ? ep_g : __float_as_int(lds1(EA(GOL + 2) + 12)) + 1;    // (only a reset needs the episode number: kept in shared memory)
-                reset_env(p, r, pick_scenario(p, p.env_id_offset + e, ep), ep);
+                reset_env(p, r, pick_scenario<PICK>(p, p.env_id_offset + e, ep), ep);
                 c = 1.f; s = 0.f;
                 hx = 0.5f * (p.ship_aabb[2] - p.ship_aabb[0]); hy = 0.5f * (p.ship_aabb[3] - p.ship_aabb[1]);
                 {
@@ -667,7 +668,7 @@ __global__ void __launch_bounds__(256) reset_kernel(const __grid_constant__ Step
     float4 l0, l1, l2, g0, g1, g2;
     load_env(p, e, r, l0, l1, l2, g0, g1, g2);
     const int ep = first ? 0 : r.episode + 1;
-    int scen = scenario ? scenario[e] : pick_scenario(p, p.env_id_offset + e, ep);
+    int scen = scenario ? scenario[e] : p.pick_cdf ? pick_scenario<true>(p, p.env_id_offset + e, ep) : pick_scenario<false>(p, p.env_id_offset + e, ep);
     scen = min(max(scen, 0), p.n_scen - 1);       // caller-supplied ids index the bank: never out of range (the host layer raises first)
     reset_env(p, r, scen, ep);
     float2 g[kGoals];
@@ -839,30 +840,104 @@ __global__ void stats_reduce_kernel(double *slots, double *out, int clear)
     if (lane == 0) out[col] = acc;
 }
 
+// Table of the weighted scenario picks (pick_weighted) from w[n]: cdf[0, n) = inclusive prefix sums, cdf[n] = total, and
+// guide[j] = first i with cdf[i] > floor(j * total / n), guide[n] = n - 1.  A total of 0 or of 2^32 and more is stored as
+// 0 ("uniform"), and the rest is left as it was.  One CTA walks the bank a tile at a time (banks reach 2^28 maps): the
+// total in 64 bits first, then per tile a block-wide scan, and element i hands its guide entries -- the j with
+// floor(j * total / n) in [cdf[i - 1], cdf[i]), i.e. j in [ceil(cdf[i - 1] * n / total), ceil(cdf[i] * n / total)) -- to
+// its whole warp to write, so that one heavy weight does not leave a single thread filling most of the guide.
+constexpr int kPickThreads = 1024;
+__global__ void __launch_bounds__(kPickThreads) build_pick_table_kernel(const unsigned *w, int n, unsigned *cdf, unsigned *guide)
+{
+    __shared__ unsigned long long s_sum[kPickThreads / 32];
+    __shared__ unsigned s_scan[kPickThreads / 32];
+    __shared__ unsigned s_carry;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    unsigned long long acc = 0ull;
+    for (int i = tid; i < n; i += kPickThreads) acc += __ldg(w + i);
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) acc += __shfl_xor_sync(kFull, acc, off);
+    if (lane == 0) s_sum[warp] = acc;
+    __syncthreads();
+    if (warp == 0) {
+        acc = s_sum[lane];
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) acc += __shfl_xor_sync(kFull, acc, off);
+        if (lane == 0) { s_sum[0] = acc; s_carry = 0u; }
+    }
+    __syncthreads();
+    const unsigned long long total = s_sum[0];
+    if (total == 0ull || total >= (1ull << 32)) {
+        if (tid == 0) cdf[n] = 0u;
+        return;
+    }
+    if (tid == 0) { cdf[n] = (unsigned)total; guide[n] = (unsigned)(n - 1); }
+    for (int base = 0; base < n; base += kPickThreads) {
+        const int i = base + tid;
+        const unsigned v = i < n ? __ldg(w + i) : 0u;
+        unsigned x = v;                                          // inclusive scan within the warp ...
+#pragma unroll
+        for (int off = 1; off < 32; off <<= 1) {
+            const unsigned y = __shfl_up_sync(kFull, x, off);
+            if (lane >= off) x += y;
+        }
+        if (lane == 31) s_scan[warp] = x;
+        __syncthreads();
+        if (warp == 0) {                                         // ... of the warp totals ...
+            unsigned s = s_scan[lane];
+#pragma unroll
+            for (int off = 1; off < 32; off <<= 1) {
+                const unsigned y = __shfl_up_sync(kFull, s, off);
+                if (lane >= off) s += y;
+            }
+            s_scan[lane] = s;
+        }
+        __syncthreads();
+        const unsigned incl = s_carry + (warp ? s_scan[warp - 1] : 0u) + x;     // ... and of the tiles before (< 2^32)
+        const unsigned excl = incl - v;
+        __syncthreads();                                         // every thread has read s_carry and s_scan
+        if (tid == kPickThreads - 1) s_carry = incl;
+        if (i < n) cdf[i] = incl;
+        unsigned j0 = 0u, j1 = 0u;
+        if (i < n) {
+            j0 = (unsigned)(((unsigned long long)excl * (unsigned)n + total - 1ull) / total);
+            j1 = (unsigned)(((unsigned long long)incl * (unsigned)n + total - 1ull) / total);
+        }
+        for (unsigned m = __ballot_sync(kFull, j1 > j0); m; m &= m - 1u) {
+            const int src = __ffs(m) - 1;
+            const unsigned a = __shfl_sync(kFull, j0, src), b = __shfl_sync(kFull, j1, src);
+            const unsigned val = (unsigned)(base + warp * 32 + src);
+            for (unsigned k = a + lane; k < b; k += 32u) guide[k] = val;
+        }
+    }
+}
+
 // ------------------------------------------------------------------------------------------------------------
 // launch wrappers (called from the C ABI)
 // ------------------------------------------------------------------------------------------------------------
 template <int G, int HIST, int MB, int T, int NB>
 static cudaError_t launch_gh(const StepParams &p, int blocks, cudaStream_t stream)
 {
+    void (*const kern)(StepParams) =
+        p.log_count ? (p.pick_cdf ? step_kernel<G, HIST, MB, T, true, NB, true> : step_kernel<G, HIST, MB, T, true, NB, false>)
+                    : (p.pick_cdf ? step_kernel<G, HIST, MB, T, false, NB, true> : step_kernel<G, HIST, MB, T, false, NB, false>);
     if constexpr (NB == kBeams) {
-        if (p.log_count) step_kernel<G, HIST, MB, T, true, NB><<<blocks, T, 0, stream>>>(p);
-        else step_kernel<G, HIST, MB, T, false, NB><<<blocks, T, 0, stream>>>(p);
+        kern<<<blocks, T, 0, stream>>>(p);
     } else {
         // the wide kernel's shared memory is dynamic: up to 68 KB per CTA (G = 1, 128 threads, HISTORY_SIZE 2), beyond the
         // 48 KB a launch gets without asking -- the opt-in is made once per instantiation and device
         constexpr int bytes = StepLayout<G, HIST, NB, T>::BYTES;
-        void (*kern)(StepParams) = p.log_count ? step_kernel<G, HIST, MB, T, true, NB> : step_kernel<G, HIST, MB, T, false, NB>;
         if (bytes > 48 * 1024) {
-            static std::atomic<unsigned long long> opted[2] = {};
+            static std::atomic<unsigned long long> opted[4] = {};
+            const int which = (p.log_count ? 1 : 0) + (p.pick_cdf ? 2 : 0);
             int dev = 0;
             cudaError_t err = cudaGetDevice(&dev);
             if (err != cudaSuccess) return err;
             const unsigned long long bit = 1ull << (dev & 63);
-            if (!(opted[p.log_count ? 1 : 0].load() & bit)) {
+            if (!(opted[which].load() & bit)) {
                 err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
                 if (err != cudaSuccess) return err;
-                opted[p.log_count ? 1 : 0].fetch_or(bit);
+                opted[which].fetch_or(bit);
             }
         }
         kern<<<blocks, T, bytes, stream>>>(p);
@@ -981,6 +1056,12 @@ cudaError_t launch_log_prev_frames(const StepParams &p, const float4 *frames, co
 {
     const int blocks = p.log_cap < 1184 * 256 ? (p.log_cap + 255) / 256 : 1184;
     log_prev_frames_kernel<<<blocks, 256, 0, stream>>>(frames, prev0, p.N, k0, kc, p.log_call, p.log_rows, p.log_meta, p.log_count, p.log_cap);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_build_pick_table(const unsigned *weights, int n_scen, unsigned *table, cudaStream_t stream)
+{
+    build_pick_table_kernel<<<1, kPickThreads, 0, stream>>>(weights, n_scen, table, table + n_scen + 1);
     return cudaGetLastError();
 }
 

@@ -39,5 +39,7 @@ cudaError_t launch_render(const StepParams &p, int e, int img_w, int img_h, uint
 // episode log, frames-only host path: the previous frame of the records of chunk [k0, k0 + kc) of call p.log_call
 cudaError_t launch_log_prev_frames(const StepParams &p, const float4 *frames, const float4 *prev0, int k0, int kc, cudaStream_t stream);
 cudaError_t launch_stats_reduce(double *slots, double *out, int clear, cudaStream_t stream);
+// weighted scenario picks: table = [cdf: n_scen + 1][guide: n_scen + 1] built from the device array weights[n_scen]
+cudaError_t launch_build_pick_table(const unsigned *weights, int n_scen, unsigned *table, cudaStream_t stream);
 
 }  // namespace shipsim

@@ -39,7 +39,8 @@ constexpr int kWinThreads = 32;      // one-warp CTAs: a latency-bound batch is 
 
 // LOG: write the episode log (shipsim_episode_log_bind).  The log-free kernel is a separate instantiation: its registers
 // and spills are those of the kernel before the log existed (-Xptxas -v; this kernel sits at the 128-register wall).
-template <int T, int HIST, bool LOG>
+// PICK: weighted scenario picks (shipsim_scenario_weights), a separate instantiation for the same reason.
+template <int T, int HIST, bool LOG, bool PICK>
 __global__ void __launch_bounds__(kWinThreads, 512 / kWinThreads) window_kernel(const __grid_constant__ StepParams p)
 {
     // The two physics scans are unrolled over the whole window when it is short (every shuffle that feeds the chains is
@@ -130,7 +131,7 @@ __global__ void __launch_bounds__(kWinThreads, 512 / kWinThreads) window_kernel(
     // every window pulls those few lines towards L1 in case it ends in a reset.
     constexpr int SPL = (kScr4 + T - 1) / T;    // spawn-row float4s per lane
     const unsigned pkey = pick_key(p, gid);
-    int next_scen = pick_scenario_keyed(p, pkey, r.episode + 1);
+    int next_scen = pick_scenario_keyed<PICK>(p, pkey, r.episode + 1);
     int a_my = 3, a_nx = 3;
     if (valid && t < p.K) a_my = load_action(p, act0 + (size_t)t * act_stride, t, gid);
     if (valid && T + t < p.K) a_nx = load_action(p, act0 + (size_t)(T + t) * act_stride, T + t, gid);
@@ -508,7 +509,7 @@ __global__ void __launch_bounds__(kWinThreads, 512 / kWinThreads) window_kernel(
             scenario_goals(p, rn.scen, rg0, rg1, rg2, gn);
 #pragma unroll
             for (int i = 0; i < SPL; ++i) if (t + i * T < kScr4) spv[i] = __ldg(sp + t + i * T);
-            next_scen = pick_scenario_keyed(p, pkey, ep + 1);
+            next_scen = pick_scenario_keyed<PICK>(p, pkey, ep + 1);
             float rgx, rgy;
             closest_goal(gn, rn.alive, rn.x, rn.y, rgx, rgy);
             if (t == 0) {
@@ -607,19 +608,26 @@ __global__ void __launch_bounds__(kWinThreads, 512 / kWinThreads) window_kernel(
 #undef stat
 }
 
+template <int T, bool PICK>
+static void launch_th(const StepParams &p, int blocks, cudaStream_t stream)
+{
+    if (p.log_count) {
+        if (p.history == 2) window_kernel<T, 2, true, PICK><<<blocks, kWinThreads, 0, stream>>>(p);
+        else window_kernel<T, 1, true, PICK><<<blocks, kWinThreads, 0, stream>>>(p);
+    } else {
+        if (p.history == 2) window_kernel<T, 2, false, PICK><<<blocks, kWinThreads, 0, stream>>>(p);
+        else window_kernel<T, 1, false, PICK><<<blocks, kWinThreads, 0, stream>>>(p);
+    }
+}
+
 template <int T>
 static cudaError_t launch_t(const StepParams &p, cudaStream_t stream, LaunchShape *shape)
 {
     const int envs_per_cta = (kWinThreads / 32) * (32 / T);
     const int blocks = (p.N + envs_per_cta - 1) / envs_per_cta;
     if (shape) { shape->lanes_per_env = T; shape->threads = kWinThreads; shape->blocks = blocks; shape->window = T; }
-    if (p.log_count) {
-        if (p.history == 2) window_kernel<T, 2, true><<<blocks, kWinThreads, 0, stream>>>(p);
-        else window_kernel<T, 1, true><<<blocks, kWinThreads, 0, stream>>>(p);
-    } else {
-        if (p.history == 2) window_kernel<T, 2, false><<<blocks, kWinThreads, 0, stream>>>(p);
-        else window_kernel<T, 1, false><<<blocks, kWinThreads, 0, stream>>>(p);
-    }
+    if (p.pick_cdf) launch_th<T, true>(p, blocks, stream);
+    else launch_th<T, false>(p, blocks, stream);
     return cudaGetLastError();
 }
 

@@ -98,3 +98,79 @@ class CurriculumDriver(object):
         if advanced:
             self._apply()
         return advanced, mean_return
+
+
+def replay_distribution(score, played, last, clock, rho=0.1, beta=0.1):
+    """Prioritized Level Replay's replay distribution (Jiang et al., 2021) over the maps of a bank, as torch tensors on any
+    device: P = (1 - rho) * P_score + rho * P_stale, with P_score proportional to (1 / rank) ** (1 / beta) -- rank 1 = the
+    highest `score`; maps not `played` yet all share rank 1, ahead of every played map -- and P_stale proportional to
+    clock - last (the episodes played since the map was last played; uniform while that is 0 everywhere)."""
+    import torch
+    n = score.numel()
+    key = torch.where(played, score.double(), torch.full_like(score, float("inf"), dtype=torch.float64))
+    order = torch.sort(key, descending=True, stable=True).indices
+    pos = torch.empty(n, dtype=torch.float64, device=score.device)
+    pos.scatter_(0, order, torch.arange(1, n + 1, dtype=torch.float64, device=score.device))
+    rank = torch.where(played, pos, torch.ones_like(pos))
+    p_score = rank.pow(-1.0 / beta)
+    p_score = p_score / p_score.sum()
+    stale = (clock - last).double().clamp_min(0.0)
+    total = stale.sum()
+    p_stale = torch.where(total > 0, stale / total.clamp_min(1.0), torch.full_like(stale, 1.0 / n))
+    return (1.0 - rho) * p_score + rho * p_stale
+
+
+class LevelReplay(object):
+    """Prioritized Level Replay (Jiang et al., 2021) over the env's scenario bank: the maps the policy still does badly on
+    are replayed more often, through the env's scenario weights (BatchedShipEnv.set_scenario_weights).
+
+    After every rollout call `update()`: the env's episode log is folded into per-map outcomes
+    (BatchedShipEnv.scenario_outcomes, which empties the log), optionally summed over ranks by `all_reduce` (a callable
+    that takes the float64 [n_scenarios, 7] table and returns the global one, e.g. an all-reduce(SUM) -- so that every
+    rank holds the same weights and the picks stay independent of the sharding), and the replay distribution
+    (replay_distribution) becomes the env's pick weights.  No host synchronisation: with a captured RolloutCollector graph
+    the next replay plays the new weights.
+
+    Score of a map: minus the exponential moving average (factor `alpha`) of its per-rollout mean episode return -- low
+    returns, high priority.  PLR's own score (the mean GAE magnitude / value loss of the level's steps) needs the scenario
+    of every step, which the episode log does not record; the return-based score is what the log supports.
+    `table` accumulates the global per-map outcomes of every update (columns env.OUTCOME_COLUMNS)."""
+
+    def __init__(self, env, rho=0.1, beta=0.1, alpha=0.5, all_reduce=None):
+        import torch
+        if env._eplog is None:
+            raise ValueError("LevelReplay reads the episode log: call env.enable_episode_log() or use RolloutCollector(episode_log=True)")
+        if not (0.0 <= rho <= 1.0 and beta > 0.0 and 0.0 < alpha <= 1.0):
+            raise ValueError("need 0 <= rho <= 1, beta > 0 and 0 < alpha <= 1")
+        self.env, self.rho, self.beta, self.alpha, self.all_reduce = env, rho, beta, alpha, all_reduce
+        n, f64 = env.n_scenarios, dict(dtype=torch.float64, device=env.device)
+        self.table = torch.zeros(n, 7, **f64)
+        self.score = torch.zeros(n, **f64)
+        self.played = torch.zeros(n, dtype=torch.bool, device=env.device)
+        self.last = torch.zeros(n, **f64)              # value of `clock` when the map was last played
+        self.clock = torch.zeros((), **f64)            # episodes played so far (all ranks)
+
+    def observe(self, outcomes):
+        """Fold one global per-map outcome table (float64 [n_scenarios, 7]) into the scores and staleness."""
+        import torch
+        self.table += outcomes
+        ep = outcomes[:, 0]
+        hit = ep > 0
+        s = -outcomes[:, 1] / ep.clamp_min(1.0)
+        self.score = torch.where(hit, torch.where(self.played, (1.0 - self.alpha) * self.score + self.alpha * s, s), self.score)
+        self.played |= hit
+        self.clock += ep.sum()
+        self.last = torch.where(hit, self.clock, self.last)
+
+    def probabilities(self):
+        return replay_distribution(self.score, self.played, self.last, self.clock, self.rho, self.beta)
+
+    def update(self):
+        """Fold the rollout's episodes, set the env's scenario weights; returns the replay distribution (device tensor)."""
+        outcomes = self.env.scenario_outcomes(clear=True)
+        if self.all_reduce is not None:
+            outcomes = self.all_reduce(outcomes)
+        self.observe(outcomes)
+        p = self.probabilities()
+        self.env.set_scenario_weights(p)
+        return p

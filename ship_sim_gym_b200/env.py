@@ -95,6 +95,44 @@ def episode_dict(meta, rows, env_id_offset=0):
     }
 
 
+# columns of the per-scenario outcome table (fold_episode_log, BatchedShipEnv.scenario_outcomes)
+OUTCOME_COLUMNS = ("episodes", "return_sum", "length_sum", "collision", "all_goals", "oob", "timeout")
+
+
+def fold_episode_log(meta, count, n_scenarios, out=None):
+    """Per-scenario sums of the episode-log records meta[:count] (int32 [cap, 8], columns _abi.EP_*; `count` a 1-element
+    tensor, records past the capacity are lost): float64 [n_scenarios, len(OUTCOME_COLUMNS)] -- episodes, return sum,
+    length sum and the episodes that ended by collision, all goals, out of bounds and the step cap.  Added into `out`
+    when given.  Pure torch on meta's device, masked by the device-side count: no host synchronisation."""
+    cap = meta.shape[0]
+    dev = meta.device
+    valid = torch.arange(cap, device=dev) < count.to(dev)
+    end = meta[:, _abi.EP_END]
+    cols = torch.stack([torch.ones(cap, dtype=torch.float64, device=dev),
+                        meta[:, _abi.EP_RETURN].contiguous().view(torch.float32).double(),
+                        meta[:, _abi.EP_LENGTH].double()] +
+                       [((end & bit) != 0).double() for bit in (_abi.END_COLLISION, _abi.END_ALL_GOALS, _abi.END_OOB, _abi.END_TIMEOUT)], 1)
+    cols = torch.where(valid[:, None], cols, torch.zeros((), dtype=torch.float64, device=dev))
+    scen = meta[:, _abi.EP_SCENARIO].long().clamp(0, n_scenarios - 1)      # (rows past the count hold anything)
+    if out is None:
+        out = torch.zeros(n_scenarios, len(OUTCOME_COLUMNS), dtype=torch.float64, device=dev)
+    return out.index_add_(0, scen, cols)
+
+
+def quantize_scenario_weights(w):
+    """Float pick weights -> the uint32 weights shipsim_scenario_weights reads (as int32: every value is below 2^31), on
+    w's device with no host synchronisation: NaN and negative weights count as 0, +inf as the largest finite weight; the
+    weights are scaled so that their sum stays at most 2^31, and a positive weight is never rounded to 0 (it becomes at
+    least 1).  Equal weights stay equal (so the picks are the uniform ones), and all-zero weights stay zero (uniform
+    picks as well)."""
+    w = torch.nan_to_num(w.to(torch.float64), nan=0.0, posinf=torch.finfo(torch.float64).max, neginf=0.0).clamp_min(0.0)
+    n = w.numel()
+    w = w / w.amax().clamp_min(torch.finfo(torch.float64).tiny)            # in [0, 1], the largest is 1: no overflow below
+    # 2n of headroom: the rounding of the float64 sum (far below n) and the floor of positive weights at 1 (at most n)
+    q = torch.floor(w * ((2.0 ** 31 - 2 * n) / w.sum().clamp_min(1.0)))
+    return torch.where(w > 0, q.clamp_min(1.0), q).to(torch.int32)
+
+
 def long_history_terminal_rows(prev_rows, rows, k, env, frame):
     """HISTORY_SIZE > 2: the kernel logs the terminal FRAME; the terminal row is the env's row before the done step
     (`rows[k - 1]`, or `prev_rows` -- the rows before the call -- for k = 0) moved on by one frame, then that frame, i.e.
@@ -199,6 +237,7 @@ class BatchedShipEnv(object):
         self.graph_safe = True                 # False: kernel parameters change between launches (no CUDA-graph replay)
         self._calls = 0                        # shipsim_step / shipsim_step_host calls (mirrors the handle's SHIPSIM_EP_CALL)
         self._eplog = None                     # episode log: (rows, meta, count, capacity)
+        self._pick_w = None                    # scenario weights (set_scenario_weights): the quantized device copy, or None
         if fresh_maps:
             self.fresh_maps(True)
 
@@ -230,6 +269,7 @@ class BatchedShipEnv(object):
                                                      bank.goals.ctypes.data, len(bank), bank.maxv))
         self.params_epoch = getattr(self, "params_epoch", 0) + 1
         self.graph_safe = True                 # (a host bank leaves fresh-maps mode: shipsim_load_scenarios)
+        self._pick_w = None                    # (and drops the scenario weights)
         if getattr(self, "_state_bound", False) and not self._needs_reset:
             self.reset()
 
@@ -249,6 +289,7 @@ class BatchedShipEnv(object):
         self.params_epoch = getattr(self, "params_epoch", 0) + 1
         self._needs_reset = True
         self.graph_safe = True                 # (a new bank leaves fresh-maps mode: shipsim_generate_scenarios)
+        self._pick_w = None                    # (and drops the scenario weights)
 
     def fresh_maps(self, enable=True):
         """A new map for every episode, as ShipGame.reset builds one (game.py:271-272): the device-generated bank
@@ -258,6 +299,46 @@ class BatchedShipEnv(object):
             _abi.check(self.L.shipsim_fresh_maps(self._h, int(bool(enable))))
         self.graph_safe = not enable
         self.params_epoch += 1
+
+    @property
+    def n_scenarios(self):
+        """Size of the scenario bank the resets pick from."""
+        return self._n_scen
+
+    def set_scenario_weights(self, weights):
+        """Resets (automatic ones and reset() without explicit scenarios) pick map i with probability w[i] / sum(w)
+        instead of uniformly (shipsim_scenario_weights).  `weights`: n_scenarios floats (numpy, list or tensor); None
+        returns to uniform picks.  Weight 0 holds a map out; all-zero device weights fall back to uniform picks.  The
+        weights are quantized on the device (quantize_scenario_weights) and the pick table is rebuilt there: no host
+        synchronisation for device input, so the call may sit between the replays of a captured rollout graph, which
+        picks up the new weights (changing weights leaves `params_epoch` alone; turning them on or off moves it).  A new
+        bank drops the weights; fresh maps and weights exclude each other (ShipsimError)."""
+        if weights is None:
+            with torch.cuda.device(self.device):
+                _abi.check(self.L.shipsim_scenario_weights(self._h, None, self._stream()))
+            if self._pick_w is not None:
+                self._pick_w = None
+                self.params_epoch += 1
+            return
+        n = self._n_scen
+        if not (isinstance(weights, torch.Tensor) and weights.is_cuda):
+            a = np.asarray(weights.numpy() if isinstance(weights, torch.Tensor) else weights, dtype=np.float64)
+            if a.shape != (n,):
+                raise ValueError("scenario weights: need %d weights (one per scenario), got shape %s" % (n, a.shape))
+            if not (np.nan_to_num(a, nan=0.0) > 0).any():
+                raise ValueError("scenario weights: no positive weight (None returns to uniform picks)")
+            weights = torch.from_numpy(a)
+        elif tuple(weights.shape) != (n,):
+            raise ValueError("scenario weights: need %d weights (one per scenario), got shape %s" % (n, tuple(weights.shape)))
+        turning_on = self._pick_w is None
+        with torch.cuda.device(self.device):
+            q = quantize_scenario_weights(weights.to(self.device, non_blocking=True))
+            buf = torch.empty_like(q) if turning_on else self._pick_w
+            buf.copy_(q)                       # a fixed buffer: the table build reads it later in stream order
+            _abi.check(self.L.shipsim_scenario_weights(self._h, buf.data_ptr(), self._stream()))
+        self._pick_w = buf
+        if turning_on:
+            self.params_epoch += 1
 
     def fresh_info(self):
         """dict(enabled, period, pick_base, pick_count, generation[4]) of the fresh-maps rotation."""
@@ -548,6 +629,19 @@ class BatchedShipEnv(object):
             raise _abi.ShipsimError("episode log overflow: %d episodes finished, capacity %d: %d records lost" % (n, cap, n - cap))
         r = self._ep_term[:n] if self.history > 2 else rows[:n].to(self.device)
         return episode_dict(meta[:n].to(self.device), r, self.cfg.env_id_offset)
+
+    def scenario_outcomes(self, out=None, clear=True):
+        """Per-map outcomes of the episodes the log holds (fold_episode_log): float64 [n_scenarios, 7] device tensor with
+        columns OUTCOME_COLUMNS (episodes, return_sum, length_sum, collision, all_goals, oob, timeout), added into `out`
+        when given -- "which maps does the policy fail on".  `clear` empties the log.  No host synchronisation (an
+        overflowing log is not reported here: its lost records are simply missing)."""
+        if self._eplog is None:
+            raise _abi.ShipsimError("no episode log: call enable_episode_log() first")
+        _, meta, count, _ = self._eplog
+        out = fold_episode_log(meta.to(self.device, non_blocking=True), count, self._n_scen, out)
+        if clear:
+            count.zero_()
+        return out
 
     # ------------------------------------------------------------------------------------------ stats / state
     def stats_tensor(self, clear=False, out=None):
