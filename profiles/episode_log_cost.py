@@ -48,8 +48,8 @@ def kernel_case(name, env, K, reps, rounds):
             env.enable_episode_log(cap if mode == "on" else 0)
             t[mode].append(launch_ms(env, K, reps))
             if mode == "on":
-                eps = int(env._eplog[2].item())
-                env._eplog[2].zero_()
+                eps = int(env.episode_log.count.item())
+                env.episode_log.clear()
     env.enable_episode_log(0)
     info = env.launch_info()
     kern = "window_kernel<T=%d>" % info["steps_in_flight"] if info["steps_in_flight"] > 1 else "step_kernel<G=%d>" % info["lanes_per_env"]
@@ -94,19 +94,19 @@ def transport_case(n, steps, rounds):
     acts = rng.randint(0, 3, (steps, n))
     for _ in range(rounds):
         for m, env in envs.items():
-            rows, meta = (env._eplog[0], env._eplog[1]) if m != "none" else (None, None)
+            log = env.episode_log
             used = 0
             t0 = time.perf_counter()
             for i in range(steps):
                 if m != "none" and used + n > 64 * n:
-                    env._eplog[2].zero_()
+                    log.clear()
                     used = 0
                 obs, rew, done = env.step_np(acts[i])
                 k = int(np.count_nonzero(done))
                 if m == "mapped":
-                    got = (meta.numpy()[used:used + k].copy(), rows.numpy()[used:used + k].copy())
+                    got = (log.meta.numpy()[used:used + k].copy(), log.rows.numpy()[used:used + k].copy())
                 elif m == "copy" and k:
-                    got = (meta[used:used + k].cpu().numpy(), rows[used:used + k].cpu().numpy())
+                    got = (log.meta[used:used + k].cpu().numpy(), log.rows[used:used + k].cpu().numpy())
                 used += k
             t[m].append((time.perf_counter() - t0) / steps * 1e6)
     print("%-34s %s" % ("step_np %d envs + records" % n, "  ".join("%s %.1f us [%.1f-%.1f]" % (m, np.median(v), min(v), max(v)) for m, v in t.items())),

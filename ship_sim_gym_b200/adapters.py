@@ -16,7 +16,7 @@ import numpy as np
 import torch
 
 from . import _abi
-from .env import BatchedShipEnv
+from .env import BatchedShipEnv, end_truncated
 
 
 def tile_images(images):
@@ -46,9 +46,8 @@ def episode_infos(base, env, ret, length, truncated, rows):
 def log_infos(base, meta, rows):
     """episode_infos from raw episode-log records (int32 meta [n, 8], rows [n, D]; numpy; the rows are copied)."""
     meta = np.asarray(meta, dtype=np.int32)
-    reasons = meta[:, _abi.EP_END] & (_abi.END_COLLISION | _abi.END_ALL_GOALS | _abi.END_OOB | _abi.END_TIMEOUT)
     return episode_infos(base, meta[:, _abi.EP_ENV].tolist(), meta[:, _abi.EP_RETURN].view(np.float32).tolist(),
-                         meta[:, _abi.EP_LENGTH].tolist(), (reasons == _abi.END_TIMEOUT).tolist(), np.array(rows, dtype=np.float32))
+                         meta[:, _abi.EP_LENGTH].tolist(), end_truncated(meta[:, _abi.EP_END]).tolist(), np.array(rows, dtype=np.float32))
 
 
 class ShipVecEnv(object):
@@ -77,8 +76,8 @@ class ShipVecEnv(object):
             self.batch.enable_episode_log(self._log_cap, pinned=self._np_log)
             self._log_used = 0
             if self._np_log:
-                rows, meta, _, _ = self.batch._eplog
-                self._log_np = (rows.numpy(), meta.numpy())
+                log = self.batch.episode_log
+                self._log_np = (log.rows.numpy(), log.meta.numpy())
 
     def _out(self, t):
         return t if self.as_tensors else t.cpu().numpy()
@@ -92,7 +91,7 @@ class ShipVecEnv(object):
         if not self.as_tensors and not torch.is_tensor(actions) and self.batch.history <= 2:
             # a numpy caller: one call into the C ABI's host-buffer path (no torch ops; the work is done here)
             if self.episode_info and self._log_used + self.num_envs > self._log_cap:
-                self.batch._eplog[2].zero_()                # (enqueued ahead of the step on the same stream)
+                self.batch.episode_log.clear()             # (enqueued ahead of the step on the same stream)
                 self._log_used = 0
             obs, rew, done = self.batch.step_np(np.asarray(actions))
             infos = None

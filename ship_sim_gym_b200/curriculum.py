@@ -138,7 +138,7 @@ class LevelReplay(object):
 
     def __init__(self, env, rho=0.1, beta=0.1, alpha=0.5, all_reduce=None):
         import torch
-        if env._eplog is None:
+        if env.episode_log is None:
             raise ValueError("LevelReplay reads the episode log: call env.enable_episode_log() or use RolloutCollector(episode_log=True)")
         if not (0.0 <= rho <= 1.0 and beta > 0.0 and 0.0 < alpha <= 1.0):
             raise ValueError("need 0 <= rho <= 1, beta > 0 and 0 < alpha <= 1")

@@ -71,20 +71,42 @@ def _dtype_code(t):
     raise TypeError("actions must be int32, int64 or uint8, got %s" % t.dtype)
 
 
+# why an episode ended, in the order of the outcome table's columns (END_GOAL only says a goal was taken on the last step)
+END_REASONS = (_abi.END_COLLISION, _abi.END_ALL_GOALS, _abi.END_OOB, _abi.END_TIMEOUT)
+_END_REASON_BITS = _abi.END_COLLISION | _abi.END_ALL_GOALS | _abi.END_OOB | _abi.END_TIMEOUT
+
+
+def end_truncated(end):
+    """Episode-log end bits (column _abi.EP_END; numpy or torch integer array) -> truncated: the episode ended on the step
+    cap alone (SHIPSIM_END_TIMEOUT; a goal taken on that step does not change it)."""
+    return (end & _END_REASON_BITS) == _abi.END_TIMEOUT
+
+
+class EpisodeLog(object):
+    """The episode log's buffers (BatchedShipEnv.enable_episode_log): the kernels append terminal rows `rows` and metadata
+    `meta` (columns _abi.EP_*) and count the records in the device int32 `count` (those past `capacity` are lost).
+    HISTORY_SIZE > 2: the kernel logs terminal frames, and `term` holds the terminal rows assembled from them."""
+
+    def __init__(self, rows, meta, count, capacity, term=None):
+        self.rows, self.meta, self.count, self.capacity, self.term = rows, meta, count, capacity, term
+
+    def clear(self):
+        """Empty the log: zero the device count, in order on the current stream."""
+        self.count.zero_()
+
+
 def episode_dict(meta, rows, env_id_offset=0):
     """Episode-log records -> the dict `BatchedShipEnv.episodes()` returns, sorted by (call, k, env).
 
     meta: int32 [n, 8] (columns _abi.EP_*), rows: float32 [n, D] terminal observations.  Pure torch, any device.
-    `truncated` = the episode ended on the step cap alone (SHIPSIM_END_TIMEOUT; a goal taken on that step does not change
-    it), `terminated` = everything else: collision, out of bounds or all goals taken."""
+    `truncated` = end_truncated, `terminated` = everything else: collision, out of bounds or all goals taken."""
     meta = meta.to(torch.int32).contiguous()
     order = torch.arange(meta.shape[0], device=meta.device)
     for col in (_abi.EP_ENV, _abi.EP_K, _abi.EP_CALL):          # least significant key first, stable sorts
         order = order[torch.sort(meta[order, col], stable=True).indices]
     m = meta[order]
     end = m[:, _abi.EP_END]
-    reasons = end & (_abi.END_COLLISION | _abi.END_ALL_GOALS | _abi.END_OOB | _abi.END_TIMEOUT)
-    truncated = reasons == _abi.END_TIMEOUT
+    truncated = end_truncated(end)
     col = lambda c: m[:, c].long()      # noqa: E731
     return {
         "env": col(_abi.EP_ENV), "global_env": col(_abi.EP_ENV) + int(env_id_offset), "k": col(_abi.EP_K), "call": col(_abi.EP_CALL),
@@ -111,7 +133,7 @@ def fold_episode_log(meta, count, n_scenarios, out=None):
     cols = torch.stack([torch.ones(cap, dtype=torch.float64, device=dev),
                         meta[:, _abi.EP_RETURN].contiguous().view(torch.float32).double(),
                         meta[:, _abi.EP_LENGTH].double()] +
-                       [((end & bit) != 0).double() for bit in (_abi.END_COLLISION, _abi.END_ALL_GOALS, _abi.END_OOB, _abi.END_TIMEOUT)], 1)
+                       [((end & bit) != 0).double() for bit in END_REASONS], 1)
     cols = torch.where(valid[:, None], cols, torch.zeros((), dtype=torch.float64, device=dev))
     scen = meta[:, _abi.EP_SCENARIO].long().clamp(0, n_scenarios - 1)      # (rows past the count hold anything)
     if out is None:
@@ -133,10 +155,28 @@ def quantize_scenario_weights(w):
     return torch.where(w > 0, q.clamp_min(1.0), q).to(torch.int32)
 
 
+def long_history_rows(prev_rows, frames, done, auto_reset):
+    """HISTORY_SIZE > 2 (SURVEY App. A, N2): the rows [frame t-H+1 | ... | frame t] of K steps, put together from the
+    steps' frames and the rows before them, with -1 for everything older than an env's latest reset (under auto-reset the
+    frame of a done step IS the reset frame: ship_env.py:180-184).  Copies and -1 fills only.
+    prev_rows [N, H*F], frames [K, N, F], done [K, N] -> [K, N, H*F]."""
+    K, N, F = frames.shape
+    H = prev_rows.shape[1] // F
+    prev = prev_rows.view(N, H, F).permute(1, 0, 2)            # [H][N][F], oldest first
+    allf = torch.cat([prev, frames], dim=0)                   # frame of step k sits at index H + k
+    rows = allf.unfold(0, H, 1)[1:].permute(0, 1, 3, 2)       # [K][N][H][F]: rows[k] = frames k-H+1 .. k
+    if auto_reset:
+        k_idx = torch.arange(K, device=frames.device)[:, None]
+        last_reset = torch.where(done.bool(), k_idx, torch.full_like(k_idx, -(1 << 30))).cummax(dim=0).values      # [K][N]
+        slot_time = k_idx[:, :, None] - torch.arange(H - 1, -1, -1, device=frames.device)[None, None, :]           # [K][1][H]
+        rows = torch.where((slot_time < last_reset[:, :, None])[..., None], torch.full_like(rows, -1.0), rows)
+    return rows.reshape(K, N, H * F).contiguous()
+
+
 def long_history_terminal_rows(prev_rows, rows, k, env, frame):
     """HISTORY_SIZE > 2: the kernel logs the terminal FRAME; the terminal row is the env's row before the done step
     (`rows[k - 1]`, or `prev_rows` -- the rows before the call -- for k = 0) moved on by one frame, then that frame, i.e.
-    the H - 1 frames before the done step with -1 beyond the env's previous reset, as step() / rollout() build rows.
+    the H - 1 frames before the done step with -1 beyond the env's previous reset, as long_history_rows builds rows.
     prev_rows [N, H*F], rows [K, N, H*F], k / env [n] int64, frame [n, F] -> [n, H*F]."""
     F = frame.shape[1]
     before = torch.where((k > 0)[:, None], rows[(k - 1).clamp(min=0), env], prev_rows[env])
@@ -180,7 +220,6 @@ class BatchedShipEnv(object):
         self.auto_reset = bool(auto_reset)
         self.validate_actions = bool(validate_actions)
         self.seed_value = int(seed)
-        self._kernel_hist = min(self.history, 2)               # longer histories are assembled here from frames
 
         dt = BASE_DT * self.knobs["speed"]                     # game.py:194
         cfg = _abi.default_config()
@@ -191,7 +230,7 @@ class BatchedShipEnv(object):
         cfg.dt = dt
         cfg.damping = math.pow(SPACE_DAMPING, dt)              # cpSpaceStep: pow(space.damping, dt), in double
         cfg.max_steps = self.knobs["max_steps"]
-        cfg.history = self._kernel_hist if self.history <= 2 else 1
+        cfg.history = self.history if self.history <= 2 else 1         # longer rows are assembled here from frames
         cfg.auto_reset = int(self.auto_reset)
         cfg.lidar_spread_deg = self.knobs["lidar"]["ANGULAR_SPREAD"]
         cfg.lidar_distance = self.knobs["lidar"]["DISTANCE"]
@@ -208,11 +247,18 @@ class BatchedShipEnv(object):
         self.reset_epoch = 0
         self.last_reset_obs = None
         self.params_epoch = 0                  # bumped whenever kernel parameters change (captured CUDA graphs go stale)
+        self.graph_safe = True                 # False: kernel parameters change between launches (no CUDA-graph replay)
+        self._pick_w = None                    # scenario weights (set_scenario_weights): the quantized device copy, or None
+        self._n_generated = 0
+        self._hist = None                      # HISTORY_SIZE > 2: the latest rows [N, H*F] (long_history_rows)
+        self.total_steps = 0
+        self._calls = 0                        # shipsim_step / shipsim_step_host calls (mirrors the handle's SHIPSIM_EP_CALL)
+        self.episode_log = None                # EpisodeLog while the log is on (enable_episode_log)
+        self._np_bufs = None                   # step_np's page-locked buffers
         self._h = C.c_void_p()
         _abi.check(self.L.shipsim_create(C.byref(cfg), self.device.index, C.byref(self._h)))
         self._obs_dim_kernel = self.n_states * cfg.history
 
-        self._n_generated = 0
         if scenario_source not in ("host", "device"):
             raise ValueError("scenario_source must be 'host' or 'device'")
         if bank is None and scenario_source == "device":
@@ -231,13 +277,6 @@ class BatchedShipEnv(object):
             self._stats_slots = torch.zeros(self.L.shipsim_stats_bytes(self._h) // 8, dtype=torch.float64, device=self.device)
             self._stats_out = torch.zeros(_abi.STATS_LEN, dtype=torch.float64, device=self.device)
             _abi.check(self.L.shipsim_bind_state(self._h, self.state.data_ptr(), self._stats_slots.data_ptr(), self._stream()))
-        self._hist = None
-        self.total_steps = 0
-        self._state_bound = True
-        self.graph_safe = True                 # False: kernel parameters change between launches (no CUDA-graph replay)
-        self._calls = 0                        # shipsim_step / shipsim_step_host calls (mirrors the handle's SHIPSIM_EP_CALL)
-        self._eplog = None                     # episode log: (rows, meta, count, capacity)
-        self._pick_w = None                    # scenario weights (set_scenario_weights): the quantized device copy, or None
         if fresh_maps:
             self.fresh_maps(True)
 
@@ -262,19 +301,12 @@ class BatchedShipEnv(object):
         game.py:271-272); `last_reset_obs` holds the reset observations."""
         if tuple(bank.bounds) != tuple(self.bounds):
             raise ValueError("scenario bank was generated for bounds %s, env has %s" % (bank.bounds, self.bounds))
-        self.bank = bank
-        self._n_scen = len(bank)
         with torch.cuda.device(self.device):
             _abi.check(self.L.shipsim_load_scenarios(self._h, bank.hull_xy.ctypes.data, bank.hull_n.ctypes.data,
                                                      bank.goals.ctypes.data, len(bank), bank.maxv))
-        self.params_epoch = getattr(self, "params_epoch", 0) + 1
-        self.graph_safe = True                 # (a host bank leaves fresh-maps mode: shipsim_load_scenarios)
-        self._pick_w = None                    # (and drops the scenario weights)
-        if getattr(self, "_state_bound", False) and not self._needs_reset:
+        self._new_bank(bank, len(bank))
+        if not self._needs_reset:
             self.reset()
-
-    def _gen_count(self):
-        return self._n_generated
 
     def generate_scenarios(self, n_scenarios, seed=0, map_N=10, map_width_frac=0.5):
         """Replace the scenario bank by `n_scenarios` maps generated on the device (river banks, hulls, goal paths;
@@ -283,13 +315,18 @@ class BatchedShipEnv(object):
         with torch.cuda.device(self.device):
             _abi.check(self.L.shipsim_generate_scenarios(self._h, int(n_scenarios), int(seed) & 0xFFFFFFFFFFFFFFFF, int(map_N),
                                                          float(map_width_frac), self._stream()))
-        self.bank = None
         self._n_generated = int(n_scenarios)
-        self._n_scen = int(n_scenarios)
-        self.params_epoch = getattr(self, "params_epoch", 0) + 1
+        self._new_bank(None, self._n_generated)
         self._needs_reset = True
-        self.graph_safe = True                 # (a new bank leaves fresh-maps mode: shipsim_generate_scenarios)
-        self._pick_w = None                    # (and drops the scenario weights)
+
+    def _new_bank(self, bank, n_scenarios):
+        """Host-side state of a newly installed bank (`bank` None: generated on the device).  A new bank leaves fresh-maps
+        mode and drops the scenario weights (shipsim_load_scenarios / shipsim_generate_scenarios)."""
+        self.bank = bank
+        self._n_scen = n_scenarios
+        self.params_epoch += 1
+        self.graph_safe = True
+        self._pick_w = None
 
     def fresh_maps(self, enable=True):
         """A new map for every episode, as ShipGame.reset builds one (game.py:271-272): the device-generated bank
@@ -348,7 +385,7 @@ class BatchedShipEnv(object):
 
     def read_scenarios(self):
         """The device-generated bank as a host ScenarioBank (validation / inspection)."""
-        S = self._gen_count()
+        S = self._n_generated
         hull_xy = np.zeros((S, 2, _abi.MAX_HULL, 2))
         hull_n = np.zeros((S, 2), dtype=np.int32)
         goals = np.zeros((S, 5, 2))
@@ -409,16 +446,10 @@ class BatchedShipEnv(object):
         self._needs_reset = False
         self.reset_epoch += 1
         self.last_reset_obs = obs if mask is None else None
-        if self.history > 2:
-            frame = obs
-            if self._hist is None or mask is None:
-                self._hist = torch.full((N, self.states_history), -1.0, dtype=torch.float32, device=self.device)
-                self._hist[:, -self.n_states:] = frame
-            else:
-                mb = m.bool()
-                fresh = torch.full_like(self._hist, -1.0)
-                fresh[:, -self.n_states:] = frame
-                self._hist = torch.where(mb[:, None], fresh, self._hist)
+        if self.history > 2:                   # obs holds the reset frames: rows [-1 ... -1 | frame]
+            fresh = torch.full((N, self.states_history), -1.0, dtype=torch.float32, device=self.device)
+            fresh[:, -self.n_states:] = obs
+            self._hist = fresh if mask is None or self._hist is None else torch.where(m.bool()[:, None], fresh, self._hist)
             return self._hist.clone()
         return obs
 
@@ -438,19 +469,8 @@ class BatchedShipEnv(object):
         a = a.contiguous().view(-1)
         assert a.numel() == self.num_envs, "expected %d actions" % self.num_envs
         self._check_actions(a)
-        obs, rew, done = self._launch(a, 1)
-        obs, rew, done = obs[0], rew[0], done[0].bool()
-        if self.history > 2:
-            frame = obs
-            shifted = torch.cat([self._hist[:, self.n_states:], frame], dim=1)
-            if self.auto_reset:
-                fresh = torch.full_like(shifted, -1.0)
-                fresh[:, -self.n_states:] = frame
-                shifted = torch.where(done[:, None], fresh, shifted)
-            self._log_long_terminal(self._hist, shifted[None])
-            self._hist = shifted
-            obs = shifted.clone()
-        return obs, rew, done, {}
+        obs, rew, done = self._step_long(a, 1) if self.history > 2 else self._launch(a, 1)
+        return obs[0], rew[0], done[0].bool(), {}
 
     def rollout(self, actions=None, K=None, out=None):
         """K consecutive env-steps in one kernel launch.  actions: int tensor [K,N] on device, or None for the
@@ -469,29 +489,22 @@ class BatchedShipEnv(object):
             assert K is not None
             a = None
         if self.history > 2:
-            frames, rew, done = self._launch(a, K, None)          # the kernel runs in its one-frame mode
-            before = self._hist
-            rows = self._long_history_rows(frames, done)
-            self._log_long_terminal(before, rows)
-            return rows, rew, done
+            return self._step_long(a, K)
         return self._launch(a, K, out)
 
-    def _long_history_rows(self, frames, done):
-        """HISTORY_SIZE > 2 (SURVEY App. A, N2): rows [frame t-H+1 | ... | frame t] put together from the K frames of a
-        rollout and the running history, with -1 for everything older than an env's latest reset (under auto-reset the
-        frame of a done step IS the reset frame: ship_env.py:180-184)."""
-        K, N, H, F = frames.shape[0], self.num_envs, self.history, self.n_states
-        prev = self._hist.view(N, H, F).permute(1, 0, 2)          # [H][N][F], oldest first
-        allf = torch.cat([prev, frames], dim=0)                   # frame of step k sits at index H + k
-        rows = allf.unfold(0, H, 1)[1:].permute(0, 1, 3, 2)       # [K][N][H][F]: rows[k] = frames k-H+1 .. k
-        if self.auto_reset:
-            k_idx = torch.arange(K, device=self.device)[:, None]
-            last_reset = torch.where(done.bool(), k_idx, torch.full_like(k_idx, -(1 << 30))).cummax(dim=0).values      # [K][N]
-            slot_time = k_idx[:, :, None] - torch.arange(H - 1, -1, -1, device=self.device)[None, None, :]             # [K][1][H]
-            rows = torch.where((slot_time < last_reset[:, :, None])[..., None], torch.full_like(rows, -1.0), rows)
-        rows = rows.reshape(K, N, H * F).contiguous()
+    def _step_long(self, a, K):
+        """HISTORY_SIZE > 2: one launch in the kernel's one-frame mode; the rows come from long_history_rows, and the
+        records the launch logged get their terminal rows (no host sync).  -> rows [K, N, H*F], reward, done."""
+        frames, rew, done = self._launch(a, K)
+        rows = long_history_rows(self._hist, frames, done, self.auto_reset)
+        log = self.episode_log
+        if log is not None:
+            new = (torch.arange(log.capacity, device=self.device) < log.count) & (log.meta[:, _abi.EP_CALL] == self._calls - 1)
+            k = log.meta[:, _abi.EP_K].long().clamp(0, K - 1)
+            env = log.meta[:, _abi.EP_ENV].long().clamp(0, self.num_envs - 1)
+            log.term = torch.where(new[:, None], long_history_terminal_rows(self._hist, rows, k, env, log.rows), log.term)
         self._hist = rows[-1].clone()
-        return rows
+        return rows, rew, done
 
     def alloc_rollout(self, K):
         N = self.num_envs
@@ -517,27 +530,12 @@ class BatchedShipEnv(object):
     def step_host(self, actions, K=1, out=None):
         """The CPU-caller path: numpy/pinned int32 actions [K,N] in, numpy obs/reward/done out, with the
         host<->device copies inside (shipsim_step_host)."""
-        if self.history > 2:          # (rows assembled on the device, then copied: this path is not tuned for long histories)
-            o, r, d = self.rollout(torch.as_tensor(np.ascontiguousarray(actions, dtype=np.int32).reshape(K, self.num_envs)))
-            res = (o.cpu().numpy(), r.cpu().numpy(), d.cpu().numpy())
-            if out is not None:
-                for dst, src in zip(out, res):
-                    if dst is not None:
-                        dst[...] = src
-                return out
-            return res
         a = np.ascontiguousarray(actions, dtype=np.int32).reshape(K, self.num_envs)
-        if self.validate_actions:
-            assert ((a >= 0) & (a <= 2)).all(), "%r invalid" % (actions,)
         if out is None:
-            out = (np.empty((K, self.num_envs, self._obs_dim_kernel), dtype=np.float32),
+            out = (np.empty((K, self.num_envs, self.states_history), dtype=np.float32),
                    np.empty((K, self.num_envs), dtype=np.float32), np.empty((K, self.num_envs), dtype=np.uint8))
         obs, rew, done = out           # any of them may be None: that output is then not copied back
-        ptr = lambda x: None if x is None else x.ctypes.data    # noqa: E731
-        with torch.cuda.device(self.device):
-            _abi.check(self.L.shipsim_step_host(self._h, a.ctypes.data, K, ptr(obs), ptr(rew), ptr(done), self._stream()))
-        self._calls += 1
-        self.total_steps += K * self.num_envs
+        self._step_host(a, K, obs, rew, done)
         return obs, rew, done
 
     def step_np(self, actions):
@@ -545,23 +543,30 @@ class BatchedShipEnv(object):
         (obs [N, n_states * history] float32, reward [N] float32, done [N] bool) out -- ONE call into shipsim_step_host with
         page-locked buffers kept on the env; no torch ops, one stream wait.  The returned arrays are the env's buffers:
         valid until the next call (copy them to keep them)."""
-        if self.history > 2:
-            obs, rew, done, _ = self.step(torch.as_tensor(np.asarray(actions)))
-            return obs.cpu().numpy(), rew.cpu().numpy(), done.cpu().numpy()
-        if getattr(self, "_np_bufs", None) is None:
+        if self._np_bufs is None:
             pin = lambda *shape, dtype: torch.empty(*shape, dtype=dtype).pin_memory()      # noqa: E731
-            self._np_keep = (pin(1, self.num_envs, dtype=torch.int32), pin(1, self.num_envs, self._obs_dim_kernel, dtype=torch.float32),
+            self._np_keep = (pin(1, self.num_envs, dtype=torch.int32), pin(1, self.num_envs, self.states_history, dtype=torch.float32),
                              pin(1, self.num_envs, dtype=torch.float32), pin(1, self.num_envs, dtype=torch.uint8))
             self._np_bufs = tuple(t.numpy() for t in self._np_keep)
         a, obs, rew, done = self._np_bufs
         a[0, :] = actions
-        if self.validate_actions:
-            assert ((a >= 0) & (a <= 2)).all(), "%r invalid" % (actions,)
-        with torch.cuda.device(self.device):
-            _abi.check(self.L.shipsim_step_host(self._h, a.ctypes.data, 1, obs.ctypes.data, rew.ctypes.data, done.ctypes.data, self._stream()))
-        self._calls += 1
-        self.total_steps += self.num_envs
+        self._step_host(a, 1, obs, rew, done)
         return obs[0], rew[0], done[0].view(np.bool_)
+
+    def _step_host(self, a, K, obs, rew, done):
+        """step_host / step_np: int32 actions a [K, N] and numpy outputs (None: not copied back) through shipsim_step_host."""
+        if self.validate_actions:
+            assert ((a >= 0) & (a <= 2)).all(), "%r invalid" % (a,)       # ship_env.py:143
+        if self.history > 2:          # (rows assembled on the device, then copied: this path is not tuned for long histories)
+            for dst, src in zip((obs, rew, done), self._step_long(torch.from_numpy(a).to(self.device), K)):
+                if dst is not None:
+                    dst[...] = src.cpu().numpy()
+            return
+        with torch.cuda.device(self.device):
+            _abi.check(self.L.shipsim_step_host(self._h, a.ctypes.data, K, None if obs is None else obs.ctypes.data, None if rew is None
+                                                else rew.ctypes.data, None if done is None else done.ctypes.data, self._stream()))
+        self._calls += 1
+        self.total_steps += K * self.num_envs
 
     def host_threads(self):
         """Host threads step_host() uses to rebuild observation rows (0 before its first call)."""
@@ -587,31 +592,20 @@ class BatchedShipEnv(object):
         self.params_epoch += 1                 # (the buffers' addresses travel in the kernel parameters: captured graphs go stale)
         if capacity == 0:
             _abi.check(self.L.shipsim_episode_log_bind(self._h, None, None, 0, None))
-            self._eplog = None
+            self.episode_log = None
             return
-        if pinned and self.history > 2:
-            raise ValueError("pinned episode logs need HISTORY_SIZE <= 2 (longer terminal rows are assembled on the device)")
+        term = None
+        if self.history > 2:                   # the kernel logs frames: the terminal rows are assembled in _step_long
+            if pinned:
+                raise ValueError("pinned episode logs need HISTORY_SIZE <= 2 (longer terminal rows are assembled on the device)")
+            term = torch.full((capacity, self.states_history), -1.0, dtype=torch.float32, device=self.device)
         where = dict(pin_memory=True) if pinned else dict(device=self.device)
         rows = torch.zeros(capacity, self._obs_dim_kernel, dtype=torch.float32, **where)
         meta = torch.zeros(capacity, _abi.EPISODE_META, dtype=torch.int32, **where)
         count = torch.zeros(1, dtype=torch.int32, device=self.device)
         with torch.cuda.device(self.device):
             _abi.check(self.L.shipsim_episode_log_bind(self._h, rows.data_ptr(), meta.data_ptr(), capacity, count.data_ptr()))
-        self._eplog = (rows, meta, count, capacity)
-        if self.history > 2:
-            self._ep_term = torch.full((capacity, self.states_history), -1.0, dtype=torch.float32, device=self.device)
-
-    def _log_long_terminal(self, prev_rows, rows):
-        """HISTORY_SIZE > 2: complete the terminal rows of the records the last launch appended (no host sync)."""
-        if self._eplog is None:
-            return
-        _, meta, count, cap = self._eplog
-        K, N = rows.shape[0], self.num_envs
-        new = (torch.arange(cap, device=self.device) < count) & (meta[:, _abi.EP_CALL] == self._calls - 1)
-        k = meta[:, _abi.EP_K].long().clamp(0, K - 1)
-        env = meta[:, _abi.EP_ENV].long().clamp(0, N - 1)
-        term = long_history_terminal_rows(prev_rows, rows, k, env, self._eplog[0])
-        self._ep_term = torch.where(new[:, None], term, self._ep_term)
+        self.episode_log = EpisodeLog(rows, meta, count, capacity, term)
 
     def episodes(self, clear=True):
         """The records of the episodes that finished since the log was last cleared, as a dict of device tensors sorted by
@@ -619,28 +613,28 @@ class BatchedShipEnv(object):
         number of the step call), length, return, terminated, truncated (step cap alone), collision, oob, all_goals, goal,
         scenario, episode (of the finished episode) and terminal_obs.  `clear` empties the log.  Raises ShipsimError when
         more episodes finished than the log could hold."""
-        if self._eplog is None:
+        log = self.episode_log
+        if log is None:
             raise _abi.ShipsimError("no episode log: call enable_episode_log() first")
-        rows, meta, count, cap = self._eplog
-        n = int(count.item())                  # (waits for the stream: the records of every launch so far are in place)
+        n, cap = int(log.count.item()), log.capacity       # (waits for the stream: the records of every launch so far are in place)
         if clear:
-            count.zero_()
+            log.clear()
         if n > cap:
             raise _abi.ShipsimError("episode log overflow: %d episodes finished, capacity %d: %d records lost" % (n, cap, n - cap))
-        r = self._ep_term[:n] if self.history > 2 else rows[:n].to(self.device)
-        return episode_dict(meta[:n].to(self.device), r, self.cfg.env_id_offset)
+        r = log.rows[:n].to(self.device) if log.term is None else log.term[:n]
+        return episode_dict(log.meta[:n].to(self.device), r, self.cfg.env_id_offset)
 
     def scenario_outcomes(self, out=None, clear=True):
         """Per-map outcomes of the episodes the log holds (fold_episode_log): float64 [n_scenarios, 7] device tensor with
         columns OUTCOME_COLUMNS (episodes, return_sum, length_sum, collision, all_goals, oob, timeout), added into `out`
         when given -- "which maps does the policy fail on".  `clear` empties the log.  No host synchronisation (an
         overflowing log is not reported here: its lost records are simply missing)."""
-        if self._eplog is None:
+        log = self.episode_log
+        if log is None:
             raise _abi.ShipsimError("no episode log: call enable_episode_log() first")
-        _, meta, count, _ = self._eplog
-        out = fold_episode_log(meta.to(self.device, non_blocking=True), count, self._n_scen, out)
+        out = fold_episode_log(log.meta.to(self.device, non_blocking=True), log.count, self._n_scen, out)
         if clear:
-            count.zero_()
+            log.clear()
         return out
 
     # ------------------------------------------------------------------------------------------ stats / state

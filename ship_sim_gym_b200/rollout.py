@@ -130,7 +130,7 @@ class RolloutCollector(object):
     def _collect(self):
         env, T = self.env, self.T
         if self.episode_log:
-            env._eplog[2].zero_()
+            env.episode_log.clear()
             # (a replayed graph repeats the call numbers of its capture: this value is the capture's, like the records')
             self._call0 = env._calls
         # categorical sampling by Gumbel-max (no host sync, graph-capturable): the noise of the whole rollout at once
@@ -202,7 +202,7 @@ class RolloutCollector(object):
             if self.env.last_reset_obs is not None:
                 self.obs[0].copy_(self.env.last_reset_obs)
             self._seen_reset_epoch = self.env.reset_epoch
-        if not self.use_graph or not getattr(self.env, "graph_safe", True):     # (fresh maps: the pick slice moves between launches)
+        if not self.use_graph or not self.env.graph_safe:     # (fresh maps: the pick slice moves between launches)
             self._collect()
         else:
             if self._graph is not None and self._graph_epoch != self.env.params_epoch:

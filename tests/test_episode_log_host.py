@@ -1,6 +1,6 @@
 """CPU only: the host-side pieces of the episode log -- the header's record layout against the binding's constants, the
-record -> dict conversion of BatchedShipEnv.episodes(), the HISTORY_SIZE > 2 terminal-row assembly and the record ->
-info-dict conversion of ShipVecEnv(episode_info=True) -- on hand-made record tensors."""
+record -> dict conversion of BatchedShipEnv.episodes(), the HISTORY_SIZE > 2 row and terminal-row assembly and the
+record -> info-dict conversion of ShipVecEnv(episode_info=True) -- on hand-made record tensors."""
 import os
 import re
 
@@ -88,6 +88,34 @@ def test_long_history_terminal_rows():
     out2 = long_history_terminal_rows(prev, rows, torch.tensor([3]), torch.tensor([1]), frame[:1])
     assert torch.equal(out2[0, F:2 * F], rows[2, 1, 2 * F:]) and bool((long_history_terminal_rows(
         prev, rows.clone().fill_(-1.0), torch.tensor([1]), torch.tensor([0]), frame[:1])[0, :2 * F] == -1.0).all())
+
+
+@pytest.mark.parametrize("auto_reset", [False, True])
+@pytest.mark.parametrize("H", [3, 4])
+def test_long_history_rows_single_and_fused_steps(H, auto_reset):
+    """HISTORY_SIZE > 2 rows at K = 1 follow the one-step rule: the previous row shifted by one frame, then the new frame;
+    under auto-reset a done env's row is [-1 ... -1 | frame] instead.  One K-step call gives the rows of K one-step calls."""
+    from ship_sim_gym_b200.env import long_history_rows
+    F, N, K = 16, 8, 24
+    g = torch.Generator().manual_seed(10 * H + auto_reset)
+    prev = torch.rand(N, H * F, generator=g) * 600
+    prev[:3, :F] = -1.0                                         # envs reset less than H steps ago
+    frames = torch.rand(K, N, F, generator=g) * 600
+    done = (torch.rand(K, N, generator=g) < 0.3).to(torch.uint8)
+    assert ((done[1:] + done[:-1]) == 2).any()                  # done on consecutive steps: resets closer than H frames
+    rows = long_history_rows(prev, frames, done, auto_reset)
+    assert rows.shape == (K, N, H * F)
+    row = prev
+    for k in range(K):
+        expect = torch.cat([row[:, F:], frames[k]], dim=1)
+        if auto_reset:
+            fresh = torch.full_like(expect, -1.0)
+            fresh[:, -F:] = frames[k]
+            expect = torch.where(done[k].bool()[:, None], fresh, expect)
+        one = long_history_rows(row, frames[k:k + 1], done[k:k + 1], auto_reset)
+        assert torch.equal(one[0], expect), k
+        assert torch.equal(rows[k], expect), k
+        row = one[0]
 
 
 def test_vec_env_infos_from_records():

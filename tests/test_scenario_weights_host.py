@@ -205,7 +205,7 @@ class _FakeEnv(object):
     """What LevelReplay needs of a BatchedShipEnv, on the CPU: a per-map outcome table per update and the weights it sets."""
 
     def __init__(self, n, outcomes):
-        self.n_scenarios, self.device, self._eplog = n, torch.device("cpu"), object()
+        self.n_scenarios, self.device, self.episode_log = n, torch.device("cpu"), object()
         self._outcomes = list(outcomes)
         self.weights = None
 
