@@ -219,6 +219,20 @@ int shipsim_reset(shipsim_t *h, const uint8_t *dev_mask, const int32_t *dev_scen
 int shipsim_step(shipsim_t *h, const void *dev_actions, int action_dtype, int32_t K, float *dev_obs,
                  float *dev_reward, uint8_t *dev_done, void *stream);
 
+/* shipsim_step for back-to-back rollouts: same arguments, same results, but a window-kernel launch may start while the
+ * handle's previous launch still runs, each env waiting only for its own previous launch (a launch otherwise lasts as
+ * long as its slowest warp).  It chains -- and counts in shipsim_chained_count -- when all of these hold:
+ *   - the handle's previous call was a window-kernel launch on the same stream, and no ABI call of any handle enqueued
+ *     work since (every other call that enqueues work, shipsim_step_host included, starts a new chain);
+ *   - lidar_beams = 10, no episode log bound, fresh maps off;
+ *   - the stream is not being captured into a graph.
+ * Otherwise it is exactly shipsim_step.  Launch N + 1 still completes after launch N: whatever is enqueued later on the
+ * stream sees both finished.  The caller promises that nothing enqueued on `stream` since the handle's previous step call
+ * writes what this call reads (the actions), and that no kernel in between lets later launches start early (programmatic
+ * dependent launch) while it reads what this call writes. */
+int shipsim_step_chained(shipsim_t *h, const void *dev_actions, int action_dtype, int32_t K, float *dev_obs,
+                         float *dev_reward, uint8_t *dev_done, void *stream);
+
 /* Episode log.  With auto_reset a done env's observation is replaced by the reset observation; with a log bound, the
  * step kernels first append one record per finished episode: dev_meta[i][SHIPSIM_EPISODE_META] (SHIPSIM_EP_*) and
  * dev_rows[i][(6 + lidar_beams) * history] = exactly the row an auto_reset = 0 launch writes for that env at that step (terminal
@@ -310,6 +324,8 @@ int shipsim_host_traffic(const shipsim_t *h, int64_t *h2d_bytes, int64_t *d2h_by
 int shipsim_host_threads(const shipsim_t *h, int32_t *n_threads);
 /* steps of one env the last launch speculated together (1 = the serial-in-time kernel ran) */
 int shipsim_launch_window(const shipsim_t *h, int32_t *steps_in_flight);
+/* shipsim_step_chained calls that chained onto the previous launch */
+int shipsim_chained_count(const shipsim_t *h, int64_t *out);
 
 #ifdef __cplusplus
 }

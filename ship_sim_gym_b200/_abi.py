@@ -28,7 +28,7 @@ SYMBOLS = (
     "shipsim_launch_count", "shipsim_launch_shape", "shipsim_launch_window", "shipsim_set_max_steps",
     "shipsim_generate_scenarios", "shipsim_read_scenarios", "shipsim_render", "shipsim_assemble_history", "shipsim_expand_delta", "shipsim_host_traffic", "shipsim_host_threads",
     "shipsim_fresh_maps", "shipsim_fresh_info", "shipsim_mlp_policy_forward", "shipsim_gae", "shipsim_episode_log_bind",
-    "shipsim_scenario_weights",
+    "shipsim_scenario_weights", "shipsim_step_chained", "shipsim_chained_count",
 )
 
 
@@ -76,6 +76,7 @@ def load():
     L.shipsim_bind_state.argtypes = [vp, vp, vp, vp]
     L.shipsim_reset.argtypes = [vp, vp, vp, C.c_int, vp, vp]
     L.shipsim_step.argtypes = [vp, vp, C.c_int, i32, vp, vp, vp, vp]
+    L.shipsim_step_chained.argtypes = [vp, vp, C.c_int, i32, vp, vp, vp, vp]
     L.shipsim_step_host.argtypes = [vp, vp, i32, vp, vp, vp, vp]
     L.shipsim_stats_read.argtypes = [vp, vp, C.c_int, vp]
     L.shipsim_set_state.argtypes = [vp, vp, vp, vp, vp, vp]
@@ -95,6 +96,7 @@ def load():
     L.shipsim_gae.argtypes = [vp, vp, vp, i32, i32, C.c_float, C.c_float, vp, vp, vp]
     L.shipsim_episode_log_bind.argtypes = [vp, vp, vp, i32, vp]
     L.shipsim_launch_count.argtypes = [vp, C.POINTER(i64)]
+    L.shipsim_chained_count.argtypes = [vp, C.POINTER(i64)]
     L.shipsim_launch_shape.argtypes = [vp, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)]
     L.shipsim_launch_window.argtypes = [vp, C.POINTER(i32)]
     for name in SYMBOLS:

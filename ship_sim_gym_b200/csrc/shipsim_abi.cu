@@ -232,11 +232,29 @@ struct shipsim_handle {
     int64_t last_h2d = 0, last_d2h = 0;      // bytes the last shipsim_step_host moved over PCIe
     int64_t launches = 0;
     int32_t calls = 0;                       // shipsim_step / shipsim_step_host calls so far (SHIPSIM_EP_CALL)
+    // chained launches (shipsim_step_chained)
+    DeviceBuf<unsigned> chain_tickets;       // [2][N]: started, done (bound and zeroed with the state)
+    bool chain_open = false;                 // the handle's last enqueue was a window launch on chain_stream ...
+    cudaStream_t chain_stream = nullptr;
+    uint64_t chain_seq = 0;                  // ... and g_enqueues has not moved since
+    int64_t chained = 0;                     // chained launches so far
     LaunchShape shape{1, kThreads, 0, 1};
     __attribute__((visibility("hidden"))) ~shipsim_handle() = default;     // (not one of the library's exported symbols)
 };
 
 static thread_local std::string g_err;
+
+// Every ABI call that enqueues work (or changes what a launch reads) moves this counter, so that a chained launch also
+// sees work that another handle put on the stream in between -- e.g. two handles alternating on one stream and writing
+// one output buffer: overlapping those launches would race.
+static std::atomic<uint64_t> g_enqueues{0};
+
+// The next step call of the handle starts a new chain.
+static void unchain(shipsim_t *h)
+{
+    if (h) h->chain_open = false;
+    g_enqueues.fetch_add(1, std::memory_order_relaxed);
+}
 
 static int fail(int code, const std::string &msg)
 {
@@ -517,6 +535,7 @@ static int install(shipsim_t *h, Bank &&b, cudaStream_t s)
 extern "C" int shipsim_load_scenarios(shipsim_t *h, const double *hull_xy, const int32_t *hull_n, const double *goals_xy,
                                       int32_t n_scen, int32_t maxv)
 {
+    unchain(h);
     if (!h || !hull_xy || !hull_n || !goals_xy) return fail(SHIPSIM_ERR_ARG, "NULL argument");
     if (n_scen < 1 || maxv < 3) return fail(SHIPSIM_ERR_ARG, "need n_scenarios >= 1 and maxv >= 3");
     int dev_maxv = 0;
@@ -588,6 +607,7 @@ extern "C" int shipsim_load_scenarios(shipsim_t *h, const double *hull_xy, const
 // ---- scenario generation on the device (SURVEY.md §8 f2) ------------------------------------------------------
 extern "C" int shipsim_generate_scenarios(shipsim_t *h, int32_t n_scen, uint64_t seed, int32_t map_N, float width_frac, void *stream)
 {
+    unchain(h);
     if (!h) return fail(SHIPSIM_ERR_ARG, "handle is NULL");
     if (n_scen < 1 || n_scen >= (1 << 28)) return fail(SHIPSIM_ERR_ARG, "n_scenarios out of range");
     if (map_N < 1 || map_N > kMaxHull - 2) return fail(SHIPSIM_ERR_ARG, "map_N must be in [1, 30] (two wall corners are added; hulls hold 32 vertices)");
@@ -621,6 +641,7 @@ extern "C" int shipsim_generate_scenarios(shipsim_t *h, int32_t n_scen, uint64_t
 
 extern "C" int shipsim_read_scenarios(shipsim_t *h, double *host_hull_xy, int32_t *host_hull_n, double *host_goals)
 {
+    unchain(h);
     if (!h || !host_hull_xy || !host_hull_n || !host_goals) return fail(SHIPSIM_ERR_ARG, "NULL argument");
     if (!h->gen.count) return fail(SHIPSIM_ERR_STATE, "no device-generated bank: call shipsim_generate_scenarios first");
     DeviceGuard g(h->device);
@@ -688,6 +709,7 @@ static int fresh_tick(shipsim_t *h, int K, cudaStream_t s)
 
 extern "C" int shipsim_fresh_maps(shipsim_t *h, int32_t enable)
 {
+    unchain(h);
     if (!h) return fail(SHIPSIM_ERR_ARG, "handle is NULL");
     DeviceGuard g(h->device);
     auto &f = h->fresh;
@@ -727,6 +749,7 @@ extern "C" int shipsim_fresh_info(const shipsim_t *h, int32_t *info)
 
 extern "C" int shipsim_scenario_weights(shipsim_t *h, const uint32_t *dev_weights, void *stream)
 {
+    unchain(h);
     if (!h) return fail(SHIPSIM_ERR_ARG, "handle is NULL");
     if (!h->p.bank) return fail(SHIPSIM_ERR_STATE, "shipsim_load_scenarios has not been called");
     if (!dev_weights) {
@@ -759,9 +782,15 @@ extern "C" size_t shipsim_stats_bytes(const shipsim_t *) { return (size_t)kStatS
 
 extern "C" int shipsim_bind_state(shipsim_t *h, void *dev_state, void *dev_stats, void *stream)
 {
+    unchain(h);
     if (!h || !dev_state || !dev_stats) return fail(SHIPSIM_ERR_ARG, "NULL argument");
     if (((uintptr_t)dev_state & 15) || ((uintptr_t)dev_stats & 7)) return fail(SHIPSIM_ERR_ARG, "state must be 16-byte aligned");
     DeviceGuard g(h->device);
+    const size_t N = (size_t)h->cfg.num_envs;
+    CU(h->chain_tickets.ensure(2 * N));
+    CU(cudaMemsetAsync(h->chain_tickets, 0, 2 * N * sizeof(unsigned), (cudaStream_t)stream));
+    h->p.chain_started = h->chain_tickets;
+    h->p.chain_done = h->chain_tickets + N;
     h->p.state = (float4 *)dev_state;
     h->p.stats = (double *)dev_stats;
     CU(cudaMemsetAsync(dev_stats, 0, shipsim_stats_bytes(h), (cudaStream_t)stream));
@@ -778,6 +807,7 @@ static int ready(const shipsim_t *h)
 
 extern "C" int shipsim_reset(shipsim_t *h, const uint8_t *dev_mask, const int32_t *dev_scenario, int first, float *dev_obs, void *stream)
 {
+    unchain(h);
     TRY(ready(h));
     DeviceGuard g(h->device);
     CU(launch_reset(h->p, dev_mask, dev_scenario, first, (float4 *)dev_obs, (cudaStream_t)stream));
@@ -802,6 +832,7 @@ static PtrInfo pointer_info(const void *ptr)
 
 extern "C" int shipsim_episode_log_bind(shipsim_t *h, float *dev_rows, int32_t *dev_meta, int32_t capacity, int32_t *dev_count)
 {
+    unchain(h);
     if (!h) return fail(SHIPSIM_ERR_ARG, "handle is NULL");
     StepParams &p = h->p;
     if (capacity == 0) {
@@ -826,7 +857,7 @@ extern "C" int shipsim_episode_log_bind(shipsim_t *h, float *dev_rows, int32_t *
 }
 
 static int step_impl(shipsim_t *h, const void *dev_actions, int action_dtype, int32_t K, float *dev_obs, float *dev_reward,
-                     uint8_t *dev_done, void *stream, int history)
+                     uint8_t *dev_done, void *stream, int history, bool chain = false)
 {
     TRY(ready(h));
     if (K < 1) return fail(SHIPSIM_ERR_ARG, "K must be >= 1");
@@ -836,16 +867,22 @@ static int step_impl(shipsim_t *h, const void *dev_actions, int action_dtype, in
     if ((uintptr_t)dev_obs & (h->cfg.lidar_beams == SHIPSIM_N_BEAMS ? 15 : 3))
         return fail(SHIPSIM_ERR_ARG, h->cfg.lidar_beams == SHIPSIM_N_BEAMS ? "dev_obs must be 16-byte aligned" : "dev_obs must be 4-byte aligned");
     DeviceGuard g(h->device);
+    h->chain_open = false;                   // (until this launch is enqueued)
     TRY(fresh_tick(h, K, (cudaStream_t)stream));
     StepParams p = h->p;
     p.actions = dev_actions; p.action_dtype = action_dtype; p.K = K;
     p.obs = (float4 *)dev_obs; p.reward = dev_reward; p.done = dev_done;
     p.history = history;
     // the window kernel needs the actions of the whole rollout up front and at least one full window of steps
-    if (h->window > 1 && K >= h->window) CU(launch_window(p, h->window, (cudaStream_t)stream, &h->shape));
+    const bool window = h->window > 1 && K >= h->window;
+    if (window) CU(launch_window(p, h->window, (cudaStream_t)stream, &h->shape, chain));
     else CU(launch_step(p, h->lanes, (cudaStream_t)stream, &h->shape));
     h->p.step0 += (unsigned)K;
     h->launches++;
+    h->chained += chain;
+    h->chain_open = window;
+    h->chain_stream = (cudaStream_t)stream;
+    h->chain_seq = g_enqueues.fetch_add(1, std::memory_order_relaxed) + 1;
     return SHIPSIM_OK;
 }
 
@@ -854,6 +891,28 @@ extern "C" int shipsim_step(shipsim_t *h, const void *dev_actions, int action_dt
 {
     if (h) { h->p.log_call = h->calls++; h->p.log_k0 = 0; }
     return step_impl(h, dev_actions, action_dtype, K, dev_obs, dev_reward, dev_done, stream, h ? h->p.history : 1);
+}
+
+// Whether this window launch may overlap the handle's previous one: that launch was the last work any handle enqueued
+// and it went to the same stream, the configuration is one the CHAIN kernels cover (log-free, 10 beams, no fresh maps:
+// their bank regeneration runs on a side stream), and the stream is not being captured (a graph has no previous launch
+// to overlap).
+static bool chainable(const shipsim_t *h, int32_t K, cudaStream_t s)
+{
+    if (!h->chain_open || h->chain_stream != s || h->chain_seq != g_enqueues.load(std::memory_order_relaxed)) return false;
+    if (!(h->window > 1 && K >= h->window) || h->cfg.lidar_beams != SHIPSIM_N_BEAMS || h->p.log_count || h->fresh.on) return false;
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    return cudaStreamIsCapturing(s, &cs) == cudaSuccess && cs == cudaStreamCaptureStatusNone;
+}
+
+extern "C" int shipsim_step_chained(shipsim_t *h, const void *dev_actions, int action_dtype, int32_t K, float *dev_obs,
+                                    float *dev_reward, uint8_t *dev_done, void *stream)
+{
+    if (!h) return shipsim_step(h, dev_actions, action_dtype, K, dev_obs, dev_reward, dev_done, stream);
+    const bool chain = h->p.state && chainable(h, K, (cudaStream_t)stream);
+    h->p.log_call = h->calls++;
+    h->p.log_k0 = 0;
+    return step_impl(h, dev_actions, action_dtype, K, dev_obs, dev_reward, dev_done, stream, h->p.history, chain);
 }
 
 // ---- shipsim_step_host ------------------------------------------------------------------------------------------------
@@ -1115,8 +1174,8 @@ static int step_frames_only(shipsim_t *h, const HostCall &c)
     return SHIPSIM_OK;
 }
 
-extern "C" int shipsim_step_host(shipsim_t *h, const int32_t *host_actions, int32_t K, float *host_obs, float *host_reward,
-                                 uint8_t *host_done, void *stream)
+static int step_host_impl(shipsim_t *h, const int32_t *host_actions, int32_t K, float *host_obs, float *host_reward,
+                          uint8_t *host_done, void *stream)
 {
     TRY(ready(h));
     if (K < 1 || !host_actions) return fail(SHIPSIM_ERR_ARG, "K must be >= 1 and host_actions non-NULL");
@@ -1196,10 +1255,19 @@ extern "C" int shipsim_step_host(shipsim_t *h, const int32_t *host_actions, int3
     return SHIPSIM_OK;
 }
 
+extern "C" int shipsim_step_host(shipsim_t *h, const int32_t *host_actions, int32_t K, float *host_obs, float *host_reward,
+                                 uint8_t *host_done, void *stream)
+{
+    const int rc = step_host_impl(h, host_actions, K, host_obs, host_reward, host_done, stream);
+    unchain(h);                              // (its window launches, if any, are no anchor for a chain)
+    return rc;
+}
+
 extern "C" int shipsim_mlp_policy_forward(const float *dev_obs, int32_t num_envs, const float *dev_w1, const float *dev_b1, const float *dev_w2,
                                           const float *dev_b2, const float *dev_w3, const float *dev_b3, const float *dev_noise, float *dev_out,
                                           int64_t *dev_actions, void *stream)
 {
+    unchain(nullptr);
     if (!dev_obs || !dev_w1 || !dev_b1 || !dev_w2 || !dev_b2 || !dev_w3 || !dev_b3 || !dev_noise || !dev_out || !dev_actions || num_envs < 1)
         return fail(SHIPSIM_ERR_ARG, "NULL buffer or num_envs < 1");
     if (((uintptr_t)dev_obs & 15) != 0) return fail(SHIPSIM_ERR_ARG, "dev_obs must be 16-byte aligned");
@@ -1211,6 +1279,7 @@ extern "C" int shipsim_mlp_policy_forward(const float *dev_obs, int32_t num_envs
 extern "C" int shipsim_gae(const float *dev_rewards, const float *dev_values, const uint8_t *dev_dones, int32_t n_steps, int32_t num_envs, float gamma,
                            float lam, float *dev_adv, float *dev_returns, void *stream)
 {
+    unchain(nullptr);
     if (!dev_rewards || !dev_values || !dev_dones || !dev_adv || !dev_returns || n_steps < 1 || num_envs < 1)
         return fail(SHIPSIM_ERR_ARG, "NULL buffer or bad sizes");
     CU(launch_gae(dev_rewards, dev_values, dev_dones, n_steps, num_envs, gamma, lam, dev_adv, dev_returns, (cudaStream_t)stream));
@@ -1252,6 +1321,7 @@ extern "C" int shipsim_assemble_history(float *host_obs, const float *host_frame
 
 extern "C" int shipsim_stats_read(shipsim_t *h, double *dev_out, int clear, void *stream)
 {
+    unchain(h);
     TRY(ready(h));
     if (!dev_out) return fail(SHIPSIM_ERR_ARG, "dev_out is NULL");
     DeviceGuard g(h->device);
@@ -1269,6 +1339,7 @@ static int lidar_slot(int j) { return j < kBeams ? 8 + j : 4 * kPlanes + j - kBe
 extern "C" int shipsim_set_state(shipsim_t *h, const float *pose, const int32_t *ints, const float *lidar, const float *goals,
                                  const float *ep_return)
 {
+    unchain(h);
     TRY(ready(h));
     if (!pose || !ints || !lidar || !goals || !ep_return) return fail(SHIPSIM_ERR_ARG, "NULL argument");
     const size_t N = (size_t)h->cfg.num_envs;
@@ -1296,6 +1367,7 @@ extern "C" int shipsim_set_state(shipsim_t *h, const float *pose, const int32_t 
 
 extern "C" int shipsim_get_state(shipsim_t *h, float *pose, int32_t *ints, float *lidar, float *goals, float *ep_return)
 {
+    unchain(h);
     TRY(ready(h));
     const size_t N = (size_t)h->cfg.num_envs;
     const int nb = h->cfg.lidar_beams, planes = state_planes(h);
@@ -1323,6 +1395,7 @@ extern "C" int shipsim_get_state(shipsim_t *h, float *pose, int32_t *ints, float
 
 extern "C" int shipsim_render(shipsim_t *h, int32_t env_index, int32_t width, int32_t height, uint8_t *dev_rgb, void *stream)
 {
+    unchain(h);
     TRY(ready(h));
     if (env_index < 0 || env_index >= h->cfg.num_envs) return fail(SHIPSIM_ERR_ARG, "env_index out of range");
     if (width < 1 || height < 1 || !dev_rgb) return fail(SHIPSIM_ERR_ARG, "bad image size / NULL buffer");
@@ -1344,6 +1417,13 @@ extern "C" int shipsim_launch_shape(const shipsim_t *h, int32_t *lanes, int32_t 
     if (lanes) *lanes = h->shape.lanes_per_env;
     if (threads) *threads = h->shape.threads;
     if (ctas) *ctas = h->shape.blocks;
+    return SHIPSIM_OK;
+}
+
+extern "C" int shipsim_chained_count(const shipsim_t *h, int64_t *out)
+{
+    if (!h || !out) return fail(SHIPSIM_ERR_ARG, "NULL argument");
+    *out = h->chained;
     return SHIPSIM_OK;
 }
 

@@ -14,6 +14,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <cstdio>
 
 namespace shipsim {
 
@@ -116,6 +117,10 @@ struct StepParams {
     // Appended for the same reason as the beam fields.  Built on the stream by build_pick_table_kernel.
     const unsigned *pick_cdf;                        // [n_scen + 1]: inclusive prefix sums of the weights, then the total (0: uniform)
     const unsigned *pick_guide;                      // [n_scen + 1]: first i with cdf[i] > floor(j * total / n_scen); [n_scen] = n_scen - 1
+    // chained launches (shipsim_step_chained): per-env tickets, [N] each, owned by the handle and zeroed at
+    // shipsim_bind_state.  started[e] counts the chained launches that have claimed env e, done[e] those that have
+    // stored its state.  Appended for the same reason as the beam fields.
+    unsigned *chain_started, *chain_done;
 };
 
 // State planes [kPlanes, kPlanes + extra_lidar_planes(n)) hold lidar[10 .. n-1], four readings per plane.
@@ -308,6 +313,56 @@ __device__ __forceinline__ void store_goals(const StepParams &p, int e, float4 g
     float4 *s = p.state;
     const size_t N = (size_t)p.N;
     s[5 * N + e] = g0; s[6 * N + e] = g1; s[7 * N + e] = make_float4(g2.x, g2.y, 0.f, 0.f);
+}
+
+// ---------------------------------------------------------------------------------------------- chained launches
+// Programmatic dependent launch (PTX griddepcontrol): launch_dependents lets the next launch of the stream start once
+// every CTA of this one has executed it (or exited); wait blocks until the previous launch has completed and its
+// memory is visible.  Both are no-ops in a launch without the programmatic-serialization attribute.
+__device__ __forceinline__ void griddep_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+__device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+
+__device__ __forceinline__ unsigned long long global_ns()
+{
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+
+// A chained env waits this long at most for its previous launch: far beyond any launch a caller would make (a CTA of
+// the headline runs for under half a millisecond), so only a broken ticket sequence reaches it, and then the kernel
+// traps with a message instead of holding the GPU forever.
+constexpr unsigned long long kChainWaitNs = 120ull * 1000000000ull;
+
+static __device__ __noinline__ void chain_stuck(int e, unsigned ticket, unsigned done)
+{
+    printf("shipsim: chained launch, env %d: ticket %u still waits after %llu s (done = %u)\n", e, ticket, kChainWaitNs / 1000000000ull, done);
+    __trap();
+}
+
+// Spin until the launch that holds ticket - 1 of env e has stored the env's state: done[e] - ticket >= 0 (wrap-safe),
+// acquire at gpu scope so that the state loads after it see that launch's stores.
+__device__ __forceinline__ void chain_await(const unsigned *done, unsigned ticket, int e)
+{
+    unsigned d;
+    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(d) : "l"(done) : "memory");
+    if ((int)(d - ticket) >= 0) return;
+    const unsigned long long t0 = global_ns();
+    unsigned ns = 64;
+    for (;;) {
+        __nanosleep(ns);
+        if (ns < 1024) ns <<= 1;
+        asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(d) : "l"(done) : "memory");
+        if ((int)(d - ticket) >= 0) return;
+        if (global_ns() - t0 > kChainWaitNs) chain_stuck(e, ticket, d);
+    }
+}
+
+// Publish that the env's state for ticket `ticket` is stored (release at gpu scope).  max, not a plain store: the counter
+// stays monotonic even if a caller races chained launches of one handle across streams.
+__device__ __forceinline__ void chain_release(unsigned *done, unsigned ticket)
+{
+    asm volatile("red.release.gpu.global.max.u32 [%0], %1;" :: "l"(done), "r"(ticket + 1u) : "memory");
 }
 
 // ShipGame.reset + ShipEnv.reset for one env (game.py:260-277, ship_env.py:171-184); the goals come from the bank

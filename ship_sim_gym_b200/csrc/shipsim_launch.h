@@ -12,8 +12,9 @@ constexpr int kThreads = 128;
 struct LaunchShape { int lanes_per_env, threads, blocks, window; };
 
 cudaError_t launch_step(const StepParams &p, int lanes_per_env, cudaStream_t stream, LaunchShape *shape);
-// time-parallel variant (shipsim_window.cu): `window` = 4, 8, 16 or 32 speculated steps per env
-cudaError_t launch_window(const StepParams &p, int window, cudaStream_t stream, LaunchShape *shape);
+// time-parallel variant (shipsim_window.cu): `window` = 4, 8, 16 or 32 speculated steps per env; `chain`: a chained
+// launch (log-free, p.chain_* bound), which may overlap the previous kernel of the stream
+cudaError_t launch_window(const StepParams &p, int window, cudaStream_t stream, LaunchShape *shape, bool chain);
 cudaError_t launch_reset(const StepParams &p, const uint8_t *mask, const int *scenario, int first, float4 *obs,
                          cudaStream_t stream);
 cudaError_t launch_build_grid(const double *hull_xy, const int *hull_n, int n_scen, int maxv_in, double gx0, double gy0,

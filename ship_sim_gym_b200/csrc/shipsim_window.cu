@@ -40,7 +40,20 @@ constexpr int kWinThreads = 32;      // one-warp CTAs: a latency-bound batch is 
 // LOG: write the episode log (shipsim_episode_log_bind).  The log-free kernel is a separate instantiation: its registers
 // and spills are those of the kernel before the log existed (-Xptxas -v; this kernel sits at the 128-register wall).
 // PICK: weighted scenario picks (shipsim_scenario_weights), a separate instantiation for the same reason.
-template <int T, int HIST, bool LOG, bool PICK>
+// CHAIN: a chained launch (shipsim_step_chained, log-free only).  Back-to-back launches of one handle each last as long
+// as their slowest warp (a launch of the headline: CTA ends spread from 0.30 to 0.44 ms, a sixth of the warp-slot time
+// idle), so a chained launch starts while the previous one still runs and each env waits for its own previous launch
+// only, through two tickets per env:
+//   * start: the env-group leader takes t = started[e]++, then -- once every ticket of the CTA is taken -- the CTA lets
+//     the next launch start (griddepcontrol.launch_dependents), and the leader waits until done[e] reaches t before the
+//     env's state is loaded;
+//   * end: after the state, goal, obs, reward and done stores and the statistics flush, done[e] = max(done[e], t + 1)
+//     with release semantics; then griddepcontrol.wait, so that launch N + 1 completes after launch N and everything
+//     later on the stream sees both (by then N is long done: it costs nothing in steady state).
+// Deadlock-free: a waiting CTA waits only for tickets taken earlier; a ticket is taken only by a CTA that is already
+// running; that CTA waits only on smaller tickets; and launch N + 1 starts only after every CTA of launch N has triggered,
+// i.e. is resident.  So the CTA that holds the smallest outstanding ticket is running and waits for nobody.
+template <int T, int HIST, bool LOG, bool PICK, bool CHAIN>
 __global__ void __launch_bounds__(kWinThreads, 512 / kWinThreads) window_kernel(const __grid_constant__ StepParams p)
 {
     // The two physics scans are unrolled over the whole window when it is short (every shuffle that feeds the chains is
@@ -64,6 +77,7 @@ __global__ void __launch_bounds__(kWinThreads, 512 / kWinThreads) window_kernel(
     __shared__ float s_ray[2 * 32];
     __shared__ unsigned s_src[NW][32];          // ray pass: compacted (plane row | frame offset) of the needy steps
     __shared__ __align__(16) float s_stat[NW][8];   // (warp_stats reads and writes it as two float4)
+    __shared__ unsigned s_ticket[CHAIN ? NW * E : 1];   // CHAIN: the ticket of each env of the CTA
 
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int el = lane / T, t = lane % T;
@@ -97,6 +111,16 @@ __global__ void __launch_bounds__(kWinThreads, 512 / kWinThreads) window_kernel(
     const size_t act_esize = p.action_dtype == 1 ? 8 : (p.action_dtype == 2 ? 1 : 4);
     const char *act0 = reinterpret_cast<const char *>(p.actions) + (size_t)ec * act_esize;
     const size_t act_stride = (size_t)p.N * act_esize;
+
+    if constexpr (CHAIN) {
+        const bool lead = valid && t == 0;
+        // (the shared store waits for the atomic's result: the CTA triggers with all its tickets taken)
+        if (lead) s_ticket[warp * E + el] = atomicAdd(p.chain_started + e, 1u);
+        __syncwarp();
+        griddep_launch_dependents();
+        if (lead) chain_await(p.chain_done + e, s_ticket[warp * E + el], e);
+        __syncwarp();
+    }
 
     EnvRegs r;
     int cb = 0;                                 // ring slot of the carry
@@ -605,39 +629,62 @@ __global__ void __launch_bounds__(kWinThreads, 512 / kWinThreads) window_kernel(
         }
     }
     flush_stats(p, lane, RowPtr{reinterpret_cast<float4 *>(s_stat[warp])});
+    if constexpr (CHAIN) {
+        __threadfence();
+        __syncwarp();
+        if (valid && t == 0) chain_release(p.chain_done + e, s_ticket[warp * E + el]);
+        griddep_wait();
+    }
 #undef stat
 }
 
-template <int T, bool PICK>
-static void launch_th(const StepParams &p, int blocks, cudaStream_t stream)
+// A chained launch: programmatic stream serialization lets it start before the previous kernel of the stream has
+// completed (as soon as that kernel's CTAs have all executed griddepcontrol.launch_dependents).
+static cudaError_t launch_pdl(void (*kernel)(StepParams), const StepParams &p, int blocks, cudaStream_t stream)
 {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(blocks);
+    cfg.blockDim = dim3(kWinThreads);
+    cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, kernel, p);
+}
+
+template <int T, bool PICK>
+static cudaError_t launch_th(const StepParams &p, int blocks, cudaStream_t stream, bool chain)
+{
+    if (chain) return launch_pdl(p.history == 2 ? window_kernel<T, 2, false, PICK, true> : window_kernel<T, 1, false, PICK, true>, p, blocks, stream);
     if (p.log_count) {
-        if (p.history == 2) window_kernel<T, 2, true, PICK><<<blocks, kWinThreads, 0, stream>>>(p);
-        else window_kernel<T, 1, true, PICK><<<blocks, kWinThreads, 0, stream>>>(p);
+        if (p.history == 2) window_kernel<T, 2, true, PICK, false><<<blocks, kWinThreads, 0, stream>>>(p);
+        else window_kernel<T, 1, true, PICK, false><<<blocks, kWinThreads, 0, stream>>>(p);
     } else {
-        if (p.history == 2) window_kernel<T, 2, false, PICK><<<blocks, kWinThreads, 0, stream>>>(p);
-        else window_kernel<T, 1, false, PICK><<<blocks, kWinThreads, 0, stream>>>(p);
+        if (p.history == 2) window_kernel<T, 2, false, PICK, false><<<blocks, kWinThreads, 0, stream>>>(p);
+        else window_kernel<T, 1, false, PICK, false><<<blocks, kWinThreads, 0, stream>>>(p);
     }
+    return cudaGetLastError();
 }
 
 template <int T>
-static cudaError_t launch_t(const StepParams &p, cudaStream_t stream, LaunchShape *shape)
+static cudaError_t launch_t(const StepParams &p, cudaStream_t stream, LaunchShape *shape, bool chain)
 {
     const int envs_per_cta = (kWinThreads / 32) * (32 / T);
     const int blocks = (p.N + envs_per_cta - 1) / envs_per_cta;
     if (shape) { shape->lanes_per_env = T; shape->threads = kWinThreads; shape->blocks = blocks; shape->window = T; }
-    if (p.pick_cdf) launch_th<T, true>(p, blocks, stream);
-    else launch_th<T, false>(p, blocks, stream);
-    return cudaGetLastError();
+    return p.pick_cdf ? launch_th<T, true>(p, blocks, stream, chain) : launch_th<T, false>(p, blocks, stream, chain);
 }
 
-cudaError_t launch_window(const StepParams &p, int window, cudaStream_t stream, LaunchShape *shape)
+cudaError_t launch_window(const StepParams &p, int window, cudaStream_t stream, LaunchShape *shape, bool chain)
 {
+    if (chain && (p.log_count || !p.chain_started || !p.chain_done)) return cudaErrorInvalidValue;
     switch (window) {
-        case 4: return launch_t<4>(p, stream, shape);
-        case 8: return launch_t<8>(p, stream, shape);
-        case 16: return launch_t<16>(p, stream, shape);
-        case 32: return launch_t<32>(p, stream, shape);
+        case 4: return launch_t<4>(p, stream, shape, chain);
+        case 8: return launch_t<8>(p, stream, shape, chain);
+        case 16: return launch_t<16>(p, stream, shape, chain);
+        case 32: return launch_t<32>(p, stream, shape, chain);
         default: return cudaErrorInvalidValue;
     }
 }

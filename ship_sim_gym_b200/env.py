@@ -255,6 +255,10 @@ class BatchedShipEnv(object):
         self._calls = 0                        # shipsim_step / shipsim_step_host calls (mirrors the handle's SHIPSIM_EP_CALL)
         self.episode_log = None                # EpisodeLog while the log is on (enable_episode_log)
         self._np_bufs = None                   # step_np's page-locked buffers
+        # back-to-back rollouts may overlap (shipsim_step_chained): each env's next launch starts as soon as its own
+        # previous one is done.  False: every launch waits for the whole previous launch (shipsim_step).
+        self.chain_launches = True
+        self._chain_prev = None                # (stream, actions, their _version) of the last _launch while it is the env's last device work
         self._h = C.c_void_p()
         _abi.check(self.L.shipsim_create(C.byref(cfg), self.device.index, C.byref(self._h)))
         self._obs_dim_kernel = self.n_states * cfg.history
@@ -282,6 +286,9 @@ class BatchedShipEnv(object):
 
     # ------------------------------------------------------------------------------------------ plumbing
     def _stream(self):
+        """The current stream of the env's device, for a call that enqueues work through the handle: such work ends a
+        chain of launches (_chains_on)."""
+        self._chain_prev = None
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
     def close(self):
@@ -301,6 +308,7 @@ class BatchedShipEnv(object):
         game.py:271-272); `last_reset_obs` holds the reset observations."""
         if tuple(bank.bounds) != tuple(self.bounds):
             raise ValueError("scenario bank was generated for bounds %s, env has %s" % (bank.bounds, self.bounds))
+        self._chain_prev = None
         with torch.cuda.device(self.device):
             _abi.check(self.L.shipsim_load_scenarios(self._h, bank.hull_xy.ctypes.data, bank.hull_n.ctypes.data,
                                                      bank.goals.ctypes.data, len(bank), bank.maxv))
@@ -332,6 +340,7 @@ class BatchedShipEnv(object):
         """A new map for every episode, as ShipGame.reset builds one (game.py:271-272): the device-generated bank
         (`scenario_source="device"` or `generate_scenarios`; 4 * 2^k scenarios) is regenerated slice by slice on a side
         stream behind the envs, and resets only pick from the newest slice (shipsim_fresh_maps).  Needs auto_reset."""
+        self._chain_prev = None
         with torch.cuda.device(self.device):
             _abi.check(self.L.shipsim_fresh_maps(self._h, int(bool(enable))))
         self.graph_safe = not enable
@@ -389,6 +398,7 @@ class BatchedShipEnv(object):
         hull_xy = np.zeros((S, 2, _abi.MAX_HULL, 2))
         hull_n = np.zeros((S, 2), dtype=np.int32)
         goals = np.zeros((S, 5, 2))
+        self._chain_prev = None
         with torch.cuda.device(self.device):
             _abi.check(self.L.shipsim_read_scenarios(self._h, hull_xy.ctypes.data, hull_n.ctypes.data, goals.ctypes.data))
         return ScenarioBank(hull_xy, hull_n, goals, self.bounds)
@@ -519,13 +529,24 @@ class BatchedShipEnv(object):
         code = _abi.ACTION_RANDOM if a is None else _dtype_code(a)
         # (no torch.cuda.device() context here: shipsim_step selects the handle's device itself, and on the gym-style K = 1
         # path the two extra cudaSetDevice calls were a fifth of the per-launch host time)
-        rc = self.L.shipsim_step(self._h, None if a is None else a.data_ptr(), code, K, obs.data_ptr(), rew.data_ptr(), done.data_ptr(),
-                                 torch.cuda.current_stream(self.device).cuda_stream)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        step = self.L.shipsim_step_chained if self._chains_on(a, stream) else self.L.shipsim_step
+        rc = step(self._h, None if a is None else a.data_ptr(), code, K, obs.data_ptr(), rew.data_ptr(), done.data_ptr(), stream)
         if rc:
             _abi.check(rc)
         self._calls += 1
         self.total_steps += K * self.num_envs
         return obs, rew, done
+
+    def _chains_on(self, a, stream):
+        """Whether this launch may chain onto the previous one (shipsim_step_chained, which checks the rest): that launch
+        was the env's last device work, on the same stream, with the same actions -- the same tensor, not modified in place
+        since (its _version), or the in-kernel random agent both times -- and rows are at most two frames long (longer
+        ones are assembled by torch ops between the launches)."""
+        prev, self._chain_prev = self._chain_prev, (stream, a, None if a is None else a._version)
+        if not self.chain_launches or self.history > 2 or prev is None:
+            return False
+        return prev[0] == stream and prev[1] is a and (a is None or prev[2] == a._version)
 
     def step_host(self, actions, K=1, out=None):
         """The CPU-caller path: numpy/pinned int32 actions [K,N] in, numpy obs/reward/done out, with the
@@ -589,6 +610,7 @@ class BatchedShipEnv(object):
         (written over PCIe by the kernel: a numpy caller reads them after step_np's own wait, with no copy).  Needs
         auto_reset."""
         capacity = self.num_envs if capacity is None else int(capacity)
+        self._chain_prev = None
         self.params_epoch += 1                 # (the buffers' addresses travel in the kernel parameters: captured graphs go stale)
         if capacity == 0:
             _abi.check(self.L.shipsim_episode_log_bind(self._h, None, None, 0, None))
@@ -619,6 +641,7 @@ class BatchedShipEnv(object):
         n, cap = int(log.count.item()), log.capacity       # (waits for the stream: the records of every launch so far are in place)
         if clear:
             log.clear()
+            self._chain_prev = None
         if n > cap:
             raise _abi.ShipsimError("episode log overflow: %d episodes finished, capacity %d: %d records lost" % (n, cap, n - cap))
         r = log.rows[:n].to(self.device) if log.term is None else log.term[:n]
@@ -635,6 +658,7 @@ class BatchedShipEnv(object):
         out = fold_episode_log(log.meta.to(self.device, non_blocking=True), log.count, self._n_scen, out)
         if clear:
             log.clear()
+            self._chain_prev = None
         return out
 
     # ------------------------------------------------------------------------------------------ stats / state
@@ -662,6 +686,7 @@ class BatchedShipEnv(object):
         lidar = np.zeros((N, self.n_beams), dtype=np.float32)
         goals = np.zeros((N, 5, 2), dtype=np.float32)
         ret = np.zeros(N, dtype=np.float32)
+        self._chain_prev = None
         with torch.cuda.device(self.device):
             _abi.check(self.L.shipsim_get_state(self._h, pose.ctypes.data, ints.ctypes.data, lidar.ctypes.data,
                                                 goals.ctypes.data, ret.ctypes.data))
@@ -674,20 +699,24 @@ class BatchedShipEnv(object):
         lidar = np.ascontiguousarray(lidar, dtype=np.float32).reshape(N, self.n_beams)
         goals = np.ascontiguousarray(goals, dtype=np.float32).reshape(N, 10)
         ret = np.ascontiguousarray(ep_return, dtype=np.float32).reshape(N)
+        self._chain_prev = None
         with torch.cuda.device(self.device):
             _abi.check(self.L.shipsim_set_state(self._h, pose.ctypes.data, ints.ctypes.data, lidar.ctypes.data,
                                                 goals.ctypes.data, ret.ctypes.data))
         self._needs_reset = False
 
     def launch_info(self):
-        n = C.c_int64()
+        """Launches issued so far, of which `chained` overlapped their predecessor (shipsim_step_chained), and the shape of
+        the last one."""
+        n, chained = C.c_int64(), C.c_int64()
         lanes, thr, ctas = C.c_int32(), C.c_int32(), C.c_int32()
         _abi.check(self.L.shipsim_launch_count(self._h, C.byref(n)))
         _abi.check(self.L.shipsim_launch_shape(self._h, C.byref(lanes), C.byref(thr), C.byref(ctas)))
         win = C.c_int32()
         _abi.check(self.L.shipsim_launch_window(self._h, C.byref(win)))
+        _abi.check(self.L.shipsim_chained_count(self._h, C.byref(chained)))
         return dict(launches=n.value, lanes_per_env=lanes.value, threads_per_cta=thr.value, ctas=ctas.value,
-                    steps_in_flight=win.value)
+                    steps_in_flight=win.value, chained=chained.value)
 
 
 class ShipEnv(object):
