@@ -10,8 +10,8 @@
 // front (they are: shipsim_step takes the whole [K][N] action tensor), T consecutive steps of one env are SPECULATED:
 //   1. the sequential part runs as two short scans executed by every lane of the env's group in lockstep (no
 //      divergence, no waiting): rudder / angular velocity / angle from pre-decoded actions, then ONE sincos per lane,
-//      then velocity / position with the thrust terms broadcast by shuffles; the group's first lane drops each step's
-//      result into shared memory and lane t = lane % T picks up the pose of "its" step;
+//      then velocity / position with the thrust terms broadcast through shared memory; the group's first lane drops
+//      each step's result into shared memory and lane t = lane % T picks up the pose of "its" step;
 //   2. lane t does the pose-dependent work of step t -- reach-grid lookup, plane phase, goal tests, out-of-bounds --
 //      and the cooperative ray / separating-axis passes run over (env, step) pairs instead of envs;
 //   3. the sequential leftovers are resolved without loops over steps where possible: goals taken (one ballot per
@@ -56,7 +56,7 @@ constexpr int kWinThreads = 32;      // one-warp CTAs: a latency-bound batch is 
 template <int T, int HIST, bool LOG, bool PICK, bool CHAIN>
 __global__ void __launch_bounds__(kWinThreads, 512 / kWinThreads) window_kernel(const __grid_constant__ StepParams p)
 {
-    // The two physics scans are unrolled over the whole window when it is short (every shuffle that feeds the chains is
+    // The two physics scans are unrolled over the whole window when it is short (every load that feeds the chains is
     // then issued ahead of them: 4 -> 16 iterations per trip took the headline from 0.458 to 0.449 ms), by 4 for the
     // longest window (T = 32 fully unrolled is 9 % SLOWER at 2,048 envs: code size).
     constexpr int kScanUnroll = T <= 16 ? T : 4;
@@ -73,6 +73,9 @@ __global__ void __launch_bounds__(kWinThreads, 512 / kWinThreads) window_kernel(
     __shared__ float2 s_goal[NW * E * kGoals];
     __shared__ float4 s_rf[NW * E * 2];         // reset frame, first two float4 (the rest is -1)
     __shared__ float4 s_ph[NW * 32 * 2];        // physics scan -> lanes: (th, w, bits(rudder), -) and (x, y, vx, vy) per step
+    // lanes -> scans: every lane's torque term, thrust pair and reward, read back by its group as LDS.128 broadcasts
+    // (4 torque terms, 2 thrust pairs or 4 rewards per load instead of one shuffle per value)
+    __shared__ float4 s_dw[NW * 8], s_dv[NW * 16], s_rw[NW * 8];
     __shared__ int4 s_env[NW * E];              // per env, for the copy-out: step cursor, committed steps, (carry slot of the plane ring), reset?
     __shared__ float s_ray[2 * 32];
     __shared__ unsigned s_src[NW][32];          // ray pass: compacted (plane row | frame offset) of the needy steps
@@ -207,16 +210,26 @@ __global__ void __launch_bounds__(kWinThreads, 512 / kWinThreads) window_kernel(
             // scan 1b: angular velocity and angle.  Thrust (action 0) leaves the rudder alone, so the torque term of
             // step t uses rud_t; it is rounded to fp32 before the fused multiply-add, exactly as in step_kernel.
             {
-                const float dw_t = a_my == 0 ? -p.ang_dt * (float)rud_t : 0.f;
+                reinterpret_cast<float *>(s_dw)[warp * 32 + lane] = a_my == 0 ? -p.ang_dt * (float)rud_t : 0.f;
+                __syncwarp();
+                const float4 *dw4 = s_dw + (warp * 32 + gbase) / 4;
                 float th = r.th, w = r.w;
                 float2 *po = reinterpret_cast<float2 *>(ph);
-#pragma unroll kScanUnroll
-                for (int i = 0; i < T; ++i) {
-                    const float dw = __shfl_sync(kFull, dw_t, i, T);
-                    th += w * p.dt;
-                    w = w * p.damping + dw;
-                    if (t == 0) *po = make_float2(th, w);
-                    po += 4;
+#pragma unroll 1
+                for (int i0 = 0; i0 < T; i0 += kScanUnroll) {
+                    float dw[kScanUnroll];                      // the trip's torque terms, all loaded ahead of the chain
+#pragma unroll
+                    for (int j = 0; j < kScanUnroll; j += 4) {
+                        const float4 d = dw4[(i0 + j) / 4];
+                        dw[j] = d.x; dw[j + 1] = d.y; dw[j + 2] = d.z; dw[j + 3] = d.w;
+                    }
+#pragma unroll
+                    for (int u = 0; u < kScanUnroll; ++u) {
+                        th += w * p.dt;
+                        w = w * p.damping + dw[u];
+                        if (t == 0) *po = make_float2(th, w);
+                        po += 4;
+                    }
                 }
             }
             __syncwarp();
@@ -228,21 +241,35 @@ __global__ void __launch_bounds__(kWinThreads, 512 / kWinThreads) window_kernel(
             // thrust of step t acts along the heading the step STARTS from: the trig of step t-1 (or of the carry)
             float pc = __shfl_up_sync(kFull, mc, 1, T), ps = __shfl_up_sync(kFull, ms, 1, T);
             if (t == 0) { pc = c0; ps = s0; }
-            float dvx_t = 0.f, dvy_t = 0.f;
-            if (a_my == 0) { dvx_t = -p.acc_dt * ps; dvy_t = p.acc_dt * pc; }
-            // scan 2: velocity and position
+            float2 dv_t = make_float2(0.f, 0.f);
+            if (a_my == 0) dv_t = make_float2(-p.acc_dt * ps, p.acc_dt * pc);
+            reinterpret_cast<float2 *>(s_dv)[warp * 32 + lane] = dv_t;
+            __syncwarp();
+            // scan 2: velocity and position, x and y as one pair.  x += vx * dt and vx = vx * damping + dvx each compile to
+            // one contracted fma; __ffma2_rn (FFMA2) does two of them in one issue slot, each element rounded exactly as
+            // by the scalar fma, so the results stay bit for bit those of step_kernel.  (ptxas does not pair scalar fmas.)
             {
-                float x = r.x, y = r.y, vx = r.vx, vy = r.vy;
-                float4 *po = ph + 1;
-#pragma unroll kScanUnroll
-                for (int i = 0; i < T; ++i) {
-                    const float dvx = __shfl_sync(kFull, dvx_t, i, T), dvy = __shfl_sync(kFull, dvy_t, i, T);
-                    x += vx * p.dt;
-                    y += vy * p.dt;
-                    vx = vx * p.damping + dvx;
-                    vy = vy * p.damping + dvy;
-                    if (t == 0) *po = make_float4(x, y, vx, vy);
-                    po += 2;
+                const float4 *dv4 = s_dv + (warp * 32 + gbase) / 2;
+                const float2 dt2 = make_float2(p.dt, p.dt), damp2 = make_float2(p.damping, p.damping);
+                float2 xy = make_float2(r.x, r.y), v = make_float2(r.vx, r.vy);
+                unsigned po = smem_addr(ph + 1);
+#pragma unroll 1
+                for (int i0 = 0; i0 < T; i0 += kScanUnroll) {
+                    float2 dv[kScanUnroll];                     // the trip's thrust terms, all loaded ahead of the chain
+#pragma unroll
+                    for (int j = 0; j < kScanUnroll; j += 2) {
+                        const float4 d = dv4[(i0 + j) / 2];
+                        dv[j] = make_float2(d.x, d.y); dv[j + 1] = make_float2(d.z, d.w);
+                    }
+#pragma unroll
+                    for (int u = 0; u < kScanUnroll; ++u) {
+                        xy = __ffma2_rn(v, dt2, xy);
+                        v = __ffma2_rn(v, damp2, dv[u]);
+                        // (two 8-byte stores that ptxas cannot merge: a 16-byte one wants (xy, v) in one register
+                        // quad and costs four moves a step)
+                        if (t == 0) { sts2(po, xy); sts2(po + 8, v); }
+                        po += 32;
+                    }
                 }
             }
             __syncwarp();
@@ -466,10 +493,19 @@ __global__ void __launch_bounds__(kWinThreads, 512 / kWinThreads) window_kernel(
         // episode return after step t: ordered sum (lane t adds the rewards of steps 0..t one by one), same rounding
         // as one step at a time
         float my_ret = r.ret;
+        reinterpret_cast<float *>(s_rw)[warp * 32 + lane] = reward;
+        __syncwarp();
+        {
+            const float4 *rw4 = s_rw + (warp * 32 + gbase) / 4;
+            float rv[T];
 #pragma unroll
-        for (int i = 0; i < T; ++i) {
-            const float rv = __shfl_sync(kFull, reward, i, T);
-            if (i <= t) my_ret += rv;
+            for (int j = 0; j < T; j += 4) {
+                const float4 d = rw4[j / 4];
+                rv[j] = d.x; rv[j + 1] = d.y; rv[j + 2] = d.z; rv[j + 3] = d.w;
+            }
+#pragma unroll
+            for (int i = 0; i < T; ++i)
+                if (i <= t) my_ret += rv[i];
         }
         warp_stats(stat_s, lane, commit, goal_reached, done, colliding, oob, timeout, all_goals, my_ret, steps_t);
         // this step's frame: pose, rudder, nearest remaining goal (closest_goal, game.py:333-349), and the lidar
