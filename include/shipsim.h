@@ -79,6 +79,13 @@ enum {
     SHIPSIM_EP_EPISODE,          /* ... and episode number                                                   */
     SHIPSIM_EP_CALL              /* the handle's sequence number of the step call, taken at enqueue         */
 };
+/* Per-map level scores (shipsim_gae_scored): one row of doubles per scenario, then one row for steps of no known scenario. */
+enum {
+    SHIPSIM_SCORE_STEPS = 0,     /* rollout steps played on the map                                          */
+    SHIPSIM_SCORE_POS_ADV,       /* sum over those steps of max(GAE advantage, 0): PLR's positive value loss  */
+    SHIPSIM_SCORE_ABS_ADV,       /* sum over those steps of |GAE advantage|: the L1 value loss                */
+    SHIPSIM_SCORE_COLS
+};
 enum {
     SHIPSIM_END_COLLISION = 1,   /* game.colliding (ship_env.py:120)          */
     SHIPSIM_END_ALL_GOALS = 2,   /* no goals left (ship_env.py:122)           */
@@ -295,6 +302,23 @@ int shipsim_mlp_policy_forward(const float *dev_obs, int32_t num_envs, const flo
  * the rollout), dev_dones[T][N] -> dev_adv[T][N], dev_returns[T][N] = adv + V.  One launch, enqueued on `stream`. */
 int shipsim_gae(const float *dev_rewards, const float *dev_values, const uint8_t *dev_dones, int32_t n_steps, int32_t num_envs, float gamma,
                 float lam, float *dev_adv, float *dev_returns, void *stream);
+
+/* shipsim_gae over a rollout of the handle's envs (num_envs of them), plus the map every step played and Prioritized Level
+ * Replay's value-loss scores per map.  The rollout is the handle's step calls call0, call0 + 1, ... (SHIPSIM_EP_CALL), each
+ * of steps_per_call steps: the episode-log record of call c, step k is rollout step (c - call0) * steps_per_call + k.
+ * Walking each env backwards from the last step, the steps after its last done belong to the scenario of the bound state
+ * (the episode it plays now), and the steps up to and including a done at t to the scenario of the record of (t, env).
+ * dev_adv / dev_returns are bit-identical to shipsim_gae's.  dev_step_scenario[T][num_envs] receives the scenario of every
+ * step, -1 where the episode's record was lost (log capacity) -- those steps go to row n_scenarios of dev_scores.
+ * dev_scores[n_scenarios + 1][SHIPSIM_SCORE_COLS] (doubles, ADDED into: zero it to start a table) sums per map the steps,
+ * max(adv, 0) and |adv|; the sums are double atomics, so their last bits depend on the order the atomics land in.  The
+ * record count is read on the device: no synchronisation, enqueued on `stream`, CUDA-graph capturable.  A replayed graph
+ * repeats its captured call0, exactly as the records repeat their captured call numbers (SHIPSIM_EP_CALL), so the two stay
+ * consistent.  Records of other calls are ignored.  Needs a bound state, a bank, auto_reset and an episode log
+ * (SHIPSIM_ERR_STATE otherwise); the log must not be drained between the rollout's steps and this call. */
+int shipsim_gae_scored(shipsim_t *h, const float *dev_rewards, const float *dev_values, const uint8_t *dev_dones, int32_t n_steps, float gamma,
+                       float lam, int32_t call0, int32_t steps_per_call, float *dev_adv, float *dev_returns, int32_t *dev_step_scenario,
+                       double *dev_scores, void *stream);
 
 /* Reduce the per-CTA statistic slots into dev_out[SHIPSIM_STATS_LEN] doubles (device memory, e.g. the tensor
  * handed to ncclAllReduce); clear != 0 zeroes the slots afterwards.  Replaces the counters ShipEnv keeps on the

@@ -19,6 +19,8 @@ MAX_BEAMS = 32                  # lidar_beams in [1, MAX_BEAMS]; a frame is 6 + 
 EPISODE_META = 8
 EP_K, EP_ENV, EP_LENGTH, EP_RETURN, EP_END, EP_SCENARIO, EP_EPISODE, EP_CALL = range(8)
 END_COLLISION, END_ALL_GOALS, END_OOB, END_TIMEOUT, END_GOAL = 1, 2, 4, 8, 16
+# level scores (shipsim_gae_scored): columns of a map's row; the table has one more row for steps of no known map
+SCORE_STEPS, SCORE_POS_ADV, SCORE_ABS_ADV, SCORE_COLS = range(4)
 
 # every symbol include/shipsim.h declares (tests check the library exports all of them)
 SYMBOLS = (
@@ -28,7 +30,7 @@ SYMBOLS = (
     "shipsim_launch_count", "shipsim_launch_shape", "shipsim_launch_window", "shipsim_set_max_steps",
     "shipsim_generate_scenarios", "shipsim_read_scenarios", "shipsim_render", "shipsim_assemble_history", "shipsim_expand_delta", "shipsim_host_traffic", "shipsim_host_threads",
     "shipsim_fresh_maps", "shipsim_fresh_info", "shipsim_mlp_policy_forward", "shipsim_gae", "shipsim_episode_log_bind",
-    "shipsim_scenario_weights", "shipsim_step_chained", "shipsim_chained_count",
+    "shipsim_scenario_weights", "shipsim_step_chained", "shipsim_chained_count", "shipsim_gae_scored",
 )
 
 
@@ -94,6 +96,7 @@ def load():
     L.shipsim_scenario_weights.argtypes = [vp, vp, vp]
     L.shipsim_mlp_policy_forward.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     L.shipsim_gae.argtypes = [vp, vp, vp, i32, i32, C.c_float, C.c_float, vp, vp, vp]
+    L.shipsim_gae_scored.argtypes = [vp, vp, vp, vp, i32, C.c_float, C.c_float, i32, i32, vp, vp, vp, vp, vp]
     L.shipsim_episode_log_bind.argtypes = [vp, vp, vp, i32, vp]
     L.shipsim_launch_count.argtypes = [vp, C.POINTER(i64)]
     L.shipsim_chained_count.argtypes = [vp, C.POINTER(i64)]

@@ -1286,6 +1286,27 @@ extern "C" int shipsim_gae(const float *dev_rewards, const float *dev_values, co
     return SHIPSIM_OK;
 }
 
+extern "C" int shipsim_gae_scored(shipsim_t *h, const float *dev_rewards, const float *dev_values, const uint8_t *dev_dones, int32_t n_steps,
+                                  float gamma, float lam, int32_t call0, int32_t steps_per_call, float *dev_adv, float *dev_returns,
+                                  int32_t *dev_step_scenario, double *dev_scores, void *stream)
+{
+    unchain(h);
+    TRY(ready(h));
+    if (!h->cfg.auto_reset) return fail(SHIPSIM_ERR_STATE, "level scores need auto_reset (they attribute steps through the episode log)");
+    if (!h->p.log_count) return fail(SHIPSIM_ERR_STATE, "level scores need the episode log: call shipsim_episode_log_bind first");
+    if (!dev_rewards || !dev_values || !dev_dones || !dev_adv || !dev_returns || !dev_step_scenario || !dev_scores || n_steps < 1 || steps_per_call < 1)
+        return fail(SHIPSIM_ERR_ARG, "NULL buffer or bad sizes");
+    if (((uintptr_t)dev_scores & 7) || ((uintptr_t)dev_step_scenario & 3))
+        return fail(SHIPSIM_ERR_ARG, "dev_scores must be 8-byte and dev_step_scenario 4-byte aligned");
+    DeviceGuard g(h->device);
+    const StepParams &p = h->p;
+    CU(launch_gae_scored(dev_rewards, dev_values, dev_dones, n_steps, h->cfg.num_envs, gamma, lam, dev_adv, dev_returns, p.log_meta, p.log_count,
+                         p.log_cap, call0, steps_per_call, p.state + (size_t)4 * h->cfg.num_envs, p.n_scen, (int *)dev_step_scenario, dev_scores,
+                         (cudaStream_t)stream));
+    h->launches += 2;
+    return SHIPSIM_OK;
+}
+
 extern "C" int shipsim_host_traffic(const shipsim_t *h, int64_t *h2d_bytes, int64_t *d2h_bytes)
 {
     if (!h) return fail(SHIPSIM_ERR_ARG, "NULL argument");

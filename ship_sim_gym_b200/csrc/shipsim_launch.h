@@ -34,6 +34,11 @@ cudaError_t launch_history_rows(const float4 *frames, const float4 *prev0, const
 cudaError_t launch_frame(const StepParams &p, float4 *out, cudaStream_t stream);
 cudaError_t launch_gae(const float *rew, const float *val, const unsigned char *done, int T, int N, float gamma, float lam, float *adv, float *ret,
                        cudaStream_t stream);
+// launch_gae, plus the map of every step (step_scen[T][N], from the episode-log records and the bound state's plane 4) and
+// the per-map value-loss sums added into scores[n_scen + 1][3] (shipsim_gae_scored)
+cudaError_t launch_gae_scored(const float *rew, const float *val, const unsigned char *done, int T, int N, float gamma, float lam, float *adv,
+                              float *ret, const int4 *log_meta, const int *log_count, int log_cap, int call0, int steps_per_call,
+                              const float4 *plane4, int n_scen, int *step_scen, double *scores, cudaStream_t stream);
 cudaError_t launch_mlp_policy(const float *obs, int n, const float *w1, const float *b1, const float *w2, const float *b2, const float *w3,
                               const float *b3, const float *noise, float *out, long long *actions, cudaStream_t stream);
 cudaError_t launch_render(const StepParams &p, int e, int img_w, int img_h, uint8_t *rgb, cudaStream_t stream);

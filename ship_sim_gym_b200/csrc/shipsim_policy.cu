@@ -168,24 +168,81 @@ __global__ void __launch_bounds__(64 * kPolSlots, 1) mlp_policy_kernel(const flo
     cp_async_wait_all();
 }
 
+// Per-map scoring of a rollout's steps (gae_kernel<true>, shipsim_gae_scored).  Appended after the unscored kernel's
+// parameters, which the unscored instantiation never reads, so that instantiation keeps its parameter offsets and its code.
+struct GaeScoring {
+    const float4 *plane4;        // state plane 4 of the bound state: .z = bits(scenario) of the episode each env plays now
+    int *step_scen;              // [T][N]: in, the scenario of the episode that ended at (t, e) or -1; out, the scenario of every step
+    double *scores;              // [n_scen + 1][3] (SHIPSIM_SCORE_*), added into; row n_scen: steps of no known scenario
+    int n_scen;
+};
+
 // Generalised advantage estimation over a finished rollout, as PPO2's runner computes it (the reference trains with
 // stable-baselines PPO2: train/stable_baselines/ppo.py:88,104): adv[t] = delta[t] + gamma * lam * nonterminal[t] * adv[t + 1],
 // delta[t] = r[t] + gamma * V[t + 1] * nonterminal[t] - V[t], returns = adv + V.  One thread per env walks its T steps
 // backwards (coalesced across envs): one launch instead of ~T + 8 elementwise torch kernels.
+//
+// SCORE: the same walk also attributes every step to its map and sums Prioritized Level Replay's value-loss scores per map.
+// Going backwards, the steps after an env's last done belong to the episode it plays now (the bound state); a done at t
+// starts, going backwards, the episode that ended at t, whose map scatter_records_kernel put into step_scen[t].  Per run
+// of steps on one map the count, sum max(adv, 0) and sum |adv| stay in registers (double) and are flushed with double
+// atomics when the map changes and at the end -- so the table's last bits depend on the order in which the atomics land.
+// adv and ret are computed by the same operations in the same order as without SCORE.
+template <bool SCORE>
 __global__ void __launch_bounds__(256) gae_kernel(const float *__restrict__ rew, const float *__restrict__ val, const unsigned char *__restrict__ done,
-                                                  int T, int N, float gamma, float gl, float *__restrict__ adv, float *__restrict__ ret)
+                                                  int T, int N, float gamma, float gl, float *__restrict__ adv, float *__restrict__ ret, GaeScoring sc)
 {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= N) return;
+    int seg = 0, steps = 0;
+    double pos = 0.0, mag = 0.0;
+    auto flush = [&]() {
+        if (steps) {
+            double *s = sc.scores + (size_t)(seg >= 0 && seg < sc.n_scen ? seg : sc.n_scen) * 3;
+            atomicAdd(s + 0, (double)steps);
+            atomicAdd(s + 1, pos);
+            atomicAdd(s + 2, mag);
+        }
+        steps = 0; pos = 0.0; mag = 0.0;
+    };
+    if (SCORE) seg = __float_as_int(sc.plane4[e].z);
     float last = 0.f, vnext = __ldg(val + (size_t)T * N + e);
     for (int t = T - 1; t >= 0; --t) {
         const size_t i = (size_t)t * N + e;
-        const float nt = done[i] ? 0.f : 1.f, v = __ldg(val + i);
+        const bool d = done[i];
+        const float nt = d ? 0.f : 1.f, v = __ldg(val + i);
         const float delta = __ldg(rew + i) + gamma * vnext * nt - v;
         last = delta + gl * nt * last;
         adv[i] = last;
         ret[i] = last + v;
         vnext = v;
+        if (SCORE) {
+            if (d) {                                                    // step t belongs to the episode that ended at t
+                const int s = sc.step_scen[i];
+                if (s != seg) { flush(); seg = s; }
+            }
+            sc.step_scen[i] = seg;
+            ++steps;
+            pos += (double)fmaxf(last, 0.f);
+            mag += (double)fabsf(last);
+        }
+    }
+    if (SCORE) flush();
+}
+
+// One thread per episode-log record (slots < min(*count, cap)): the record of call c, step k within it, env e, scenario s
+// is rollout step t = (c - call0) * steps_per_call + k, and step_scen[t][e] = s.  Records outside the rollout (t, e or s
+// out of range) are skipped.
+__global__ void __launch_bounds__(256) scatter_records_kernel(const int4 *__restrict__ meta, const int *__restrict__ count, int cap, int call0,
+                                                              int steps_per_call, int T, int N, int n_scen, int *__restrict__ step_scen)
+{
+    const int n = min(*count, cap);
+    for (int r = blockIdx.x * blockDim.x + threadIdx.x; r < n; r += gridDim.x * blockDim.x) {
+        const int4 a = meta[2 * (size_t)r], b = meta[2 * (size_t)r + 1];      // {k, env, length, return}, {end, scenario, episode, call}
+        const int k = a.x, env = a.y, s = b.y;
+        const long long t = (long long)(b.w - call0) * steps_per_call + k;
+        if (k < 0 || k >= steps_per_call || t < 0 || t >= T || env < 0 || env >= N || s < 0 || s >= n_scen) continue;
+        step_scen[t * N + env] = s;
     }
 }
 
@@ -193,7 +250,24 @@ cudaError_t launch_gae(const float *rew, const float *val, const unsigned char *
                        cudaStream_t stream)
 {
     if (T <= 0 || N <= 0) return cudaSuccess;
-    gae_kernel<<<(N + 255) / 256, 256, 0, stream>>>(rew, val, done, T, N, gamma, gamma * lam, adv, ret);
+    gae_kernel<false><<<(N + 255) / 256, 256, 0, stream>>>(rew, val, done, T, N, gamma, gamma * lam, adv, ret, GaeScoring{});
+    return cudaGetLastError();
+}
+
+cudaError_t launch_gae_scored(const float *rew, const float *val, const unsigned char *done, int T, int N, float gamma, float lam, float *adv,
+                              float *ret, const int4 *log_meta, const int *log_count, int log_cap, int call0, int steps_per_call,
+                              const float4 *plane4, int n_scen, int *step_scen, double *scores, cudaStream_t stream)
+{
+    if (T <= 0 || N <= 0) return cudaSuccess;
+    cudaError_t err = cudaMemsetAsync(step_scen, 0xff, (size_t)T * N * sizeof(int), stream);         // -1: no record
+    if (err != cudaSuccess) return err;
+    if (log_cap > 0) {
+        const int blocks = std::min((log_cap + 255) / 256, 1184);
+        scatter_records_kernel<<<blocks, 256, 0, stream>>>(log_meta, log_count, log_cap, call0, steps_per_call, T, N, n_scen, step_scen);
+        if ((err = cudaGetLastError()) != cudaSuccess) return err;
+    }
+    gae_kernel<true><<<(N + 255) / 256, 256, 0, stream>>>(rew, val, done, T, N, gamma, gamma * lam, adv, ret,
+                                                          GaeScoring{plane4, step_scen, scores, n_scen});
     return cudaGetLastError();
 }
 

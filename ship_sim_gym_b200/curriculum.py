@@ -126,38 +126,57 @@ class LevelReplay(object):
 
     After every rollout call `update()`: the env's episode log is folded into per-map outcomes
     (BatchedShipEnv.scenario_outcomes, which empties the log), optionally summed over ranks by `all_reduce` (a callable
-    that takes the float64 [n_scenarios, 7] table and returns the global one, e.g. an all-reduce(SUM) -- so that every
-    rank holds the same weights and the picks stay independent of the sharding), and the replay distribution
-    (replay_distribution) becomes the env's pick weights.  No host synchronisation: with a captured RolloutCollector graph
-    the next replay plays the new weights.
+    that takes a float64 table -- the [n_scenarios, 7] outcomes, and for the value-loss scores also the [n_scenarios + 1,
+    3] level scores -- and returns the global one, e.g. an all-reduce(SUM) -- so that every rank holds the same weights
+    and the picks stay independent of the sharding), and the replay distribution (replay_distribution) becomes the env's
+    pick weights.  No host synchronisation: with a captured RolloutCollector graph the next replay plays the new weights.
 
-    Score of a map: minus the exponential moving average (factor `alpha`) of its per-rollout mean episode return -- low
-    returns, high priority.  PLR's own score (the mean GAE magnitude / value loss of the level's steps) needs the scenario
-    of every step, which the episode log does not record; the return-based score is what the log supports.
+    The score of a map is the exponential moving average (factor `alpha`) of a per-rollout score, chosen by `score`:
+      * "positive_value_loss": PLR's default, the mean over the map's steps of max(GAE advantage, 0) -- high where the
+        value function still underestimates what the policy achieves, i.e. where there is still something to learn;
+      * "l1_value_loss": the mean over the map's steps of |GAE advantage|;
+      * "return": minus the mean return of the map's finished episodes -- low returns, high priority.
+    The value-loss scores read `update(scores)`, the `level_scores` table of a RolloutCollector(level_scores=True), which
+    attributes every step of the rollout to its map, so a map played only by an episode that has not finished yet is
+    scored too.  Whether a map has been played, and its staleness, count finished episodes for every score.
     `table` accumulates the global per-map outcomes of every update (columns env.OUTCOME_COLUMNS)."""
 
-    def __init__(self, env, rho=0.1, beta=0.1, alpha=0.5, all_reduce=None):
+    SCORES = ("return", "positive_value_loss", "l1_value_loss")
+
+    def __init__(self, env, rho=0.1, beta=0.1, alpha=0.5, all_reduce=None, score="return"):
         import torch
         if env.episode_log is None:
             raise ValueError("LevelReplay reads the episode log: call env.enable_episode_log() or use RolloutCollector(episode_log=True)")
         if not (0.0 <= rho <= 1.0 and beta > 0.0 and 0.0 < alpha <= 1.0):
             raise ValueError("need 0 <= rho <= 1, beta > 0 and 0 < alpha <= 1")
+        if score not in self.SCORES:
+            raise ValueError("score must be one of %s" % (self.SCORES,))
         self.env, self.rho, self.beta, self.alpha, self.all_reduce = env, rho, beta, alpha, all_reduce
+        self.score_name = score
         n, f64 = env.n_scenarios, dict(dtype=torch.float64, device=env.device)
         self.table = torch.zeros(n, 7, **f64)
         self.score = torch.zeros(n, **f64)
+        self.scored = torch.zeros(n, dtype=torch.bool, device=env.device)     # `score` holds a value for the map
         self.played = torch.zeros(n, dtype=torch.bool, device=env.device)
         self.last = torch.zeros(n, **f64)              # value of `clock` when the map was last played
         self.clock = torch.zeros((), **f64)            # episodes played so far (all ranks)
 
-    def observe(self, outcomes):
-        """Fold one global per-map outcome table (float64 [n_scenarios, 7]) into the scores and staleness."""
+    def observe(self, outcomes, scores=None):
+        """Fold one global per-map outcome table (float64 [n_scenarios, 7]) and, for the value-loss scores, one global
+        level-score table (float64 [n_scenarios + 1, 3], RolloutCollector.level_scores) into the scores and staleness."""
         import torch
+        from . import _abi
         self.table += outcomes
         ep = outcomes[:, 0]
         hit = ep > 0
-        s = -outcomes[:, 1] / ep.clamp_min(1.0)
-        self.score = torch.where(hit, torch.where(self.played, (1.0 - self.alpha) * self.score + self.alpha * s, s), self.score)
+        if self.score_name == "return":
+            new, s = hit, -outcomes[:, 1] / ep.clamp_min(1.0)
+        else:
+            steps = scores[:ep.numel(), _abi.SCORE_STEPS]
+            col = _abi.SCORE_POS_ADV if self.score_name == "positive_value_loss" else _abi.SCORE_ABS_ADV
+            new, s = steps > 0, scores[:ep.numel(), col] / steps.clamp_min(1.0)
+        self.score = torch.where(new, torch.where(self.scored, (1.0 - self.alpha) * self.score + self.alpha * s, s), self.score)
+        self.scored |= new
         self.played |= hit
         self.clock += ep.sum()
         self.last = torch.where(hit, self.clock, self.last)
@@ -165,12 +184,20 @@ class LevelReplay(object):
     def probabilities(self):
         return replay_distribution(self.score, self.played, self.last, self.clock, self.rho, self.beta)
 
-    def update(self):
-        """Fold the rollout's episodes, set the env's scenario weights; returns the replay distribution (device tensor)."""
+    def update(self, scores=None):
+        """Fold the rollout's episodes -- and for the value-loss scores `scores`, the collector's level_scores -- and set
+        the env's scenario weights; returns the replay distribution (device tensor)."""
+        if self.score_name == "return":
+            scores = None
+        elif scores is None:
+            raise ValueError("score=%r needs the rollout's level scores: update(RolloutCollector(level_scores=True).level_scores)"
+                             % self.score_name)
         outcomes = self.env.scenario_outcomes(clear=True)
         if self.all_reduce is not None:
             outcomes = self.all_reduce(outcomes)
-        self.observe(outcomes)
+            if scores is not None:
+                scores = self.all_reduce(scores.clone())    # (an in-place all-reduce leaves the collector's table alone)
+        self.observe(outcomes, scores)
         p = self.probabilities()
         self.env.set_scenario_weights(p)
         return p

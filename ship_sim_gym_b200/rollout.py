@@ -10,7 +10,44 @@ and never synchronises, the whole rollout is captured once in a CUDA graph and r
 import torch
 import torch.nn as nn
 
+from . import _abi
 from .env import BatchedShipEnv
+
+
+def score_levels(adv, dones, meta, count, scenario_now, call0, n_scenarios, steps_per_call=1, scenarios=None, scores=None):
+    """The map of every rollout step and Prioritized Level Replay's value-loss sums per map -- shipsim_gae_scored's rule, in
+    torch, on any device, with no host synchronisation.
+
+    adv float [T, N], dones [T, N]; meta int32 [cap, 8] episode-log records (columns _abi.EP_*) of which the first `count`
+    (a 1-element tensor) are valid; scenario_now int [N]: the map each env plays after the rollout.  The record of call c,
+    step k is rollout step t = (c - call0) * steps_per_call + k; records whose t, env or scenario are out of range are
+    ignored.  Walking backwards from step T - 1, an env's steps after its last done belong to scenario_now, and a done at
+    t switches to the scenario of the record of (t, env) -- -1 if that record was lost.  Returns (scenarios int32 [T, N],
+    scores float64 [n_scenarios + 1, 3]); the columns are _abi.SCORE_STEPS / SCORE_POS_ADV / SCORE_ABS_ADV, row
+    n_scenarios collects the steps of no known map, and the sums are added into `scores` when given."""
+    T, N = adv.shape
+    dev = adv.device
+    meta = meta.to(dev)
+    k, env, scen = meta[:, _abi.EP_K].long(), meta[:, _abi.EP_ENV].long(), meta[:, _abi.EP_SCENARIO].long()
+    t = (meta[:, _abi.EP_CALL].long() - call0) * steps_per_call + k
+    ok = ((torch.arange(meta.shape[0], device=dev) < count.to(dev)) & (k >= 0) & (k < steps_per_call) & (t >= 0) & (t < T)
+          & (env >= 0) & (env < N) & (scen >= 0) & (scen < n_scenarios))
+    ended = torch.full((T * N + 1,), -1, dtype=torch.int32, device=dev)       # last slot: where the skipped records land
+    ended.scatter_(0, torch.where(ok, t * N + env, T * N), torch.where(ok, scen, -1).to(torch.int32))
+    ended = ended[:T * N].view(T, N)
+    if scenarios is None:
+        scenarios = torch.empty(T, N, dtype=torch.int32, device=dev)
+    done = dones.bool()
+    torch.where(done[T - 1], ended[T - 1], scenario_now.to(device=dev, dtype=torch.int32), out=scenarios[T - 1])
+    for s in range(T - 2, -1, -1):
+        torch.where(done[s], ended[s], scenarios[s + 1], out=scenarios[s])
+    row = torch.where((scenarios >= 0) & (scenarios < n_scenarios), scenarios, n_scenarios).long().reshape(-1)
+    a = adv.double().reshape(-1)
+    cols = torch.stack([torch.ones_like(a), a.clamp_min(0.0), a.abs()], 1)
+    if scores is None:
+        scores = torch.zeros(n_scenarios + 1, _abi.SCORE_COLS, dtype=torch.float64, device=dev)
+    scores.index_add_(0, row, cols)
+    return scenarios, scores
 
 
 class MlpPolicy(nn.Module):
@@ -45,9 +82,15 @@ class RolloutCollector(object):
 
     episode_log=True: the env's episode log (BatchedShipEnv.enable_episode_log, room for T * N records: every env-step
     could end an episode) is emptied at the start of every rollout, inside the graph; episodes() returns the rollout's
-    finished episodes with `t` = the rollout step -- what a PPO loop logs as ep_reward_mean / ep_len_mean."""
+    finished episodes with `t` = the rollout step -- what a PPO loop logs as ep_reward_mean / ep_len_mean.
 
-    def __init__(self, env, policy, T=128, gamma=0.99, lam=0.95, use_graph=True, use_kernel=True, episode_log=False):
+    level_scores=True (implies episode_log=True): after every rollout `scenarios` (int32 [T, N]) holds the map every step
+    played, and `level_scores` (float64 [n_scenarios + 1, 3], zeroed at the start of every rollout) per map the steps, the
+    sum of max(advantage, 0) and the sum of |advantage| (columns _abi.SCORE_*; the last row: steps whose episode record was
+    lost) -- Prioritized Level Replay's value-loss scores, for LevelReplay(score="positive_value_loss").  The kernel path
+    computes them inside its GAE launch (shipsim_gae_scored), the generic path with score_levels."""
+
+    def __init__(self, env, policy, T=128, gamma=0.99, lam=0.95, use_graph=True, use_kernel=True, episode_log=False, level_scores=False):
         assert isinstance(env, BatchedShipEnv) and env.history <= 2
         self.env, self.policy, self.T, self.gamma, self.lam = env, policy, int(T), gamma, lam
         N, D, dev = env.num_envs, env.states_history, env.device
@@ -79,12 +122,21 @@ class RolloutCollector(object):
         self._coef = torch.empty(T, N, **f32)
         self._delta = torch.empty(T, N, **f32)
         env.validate_actions = False                            # the range check would need a host sync per step
-        self.episode_log = bool(episode_log)
+        self._scored = bool(level_scores)
+        self.episode_log = bool(episode_log) or self._scored
         self._call0 = 0                                         # the env's step-call number of the rollout's first launch
+        self.scenarios = self.level_scores = None
+        if self._scored:
+            self.scenarios = torch.empty(T, N, dtype=torch.int32, device=dev)
+            self._alloc_scores()
         if self.episode_log:
             env.enable_episode_log(self.T * N)
         self.obs[0].copy_(env.reset())
         self._seen_reset_epoch = env.reset_epoch
+
+    def _alloc_scores(self):
+        """The level-score table of the env's current bank (a bank of another size replaces it)."""
+        self.level_scores = torch.zeros(self.env.n_scenarios + 1, _abi.SCORE_COLS, dtype=torch.float64, device=self.env.device)
 
     def _alloc_fused(self, N, D, H, A, T, f32):
         self._H, self._A = H, A
@@ -133,6 +185,8 @@ class RolloutCollector(object):
             env.episode_log.clear()
             # (a replayed graph repeats the call numbers of its capture: this value is the capture's, like the records')
             self._call0 = env._calls
+        if self._scored:
+            self.level_scores.zero_()
         # categorical sampling by Gumbel-max (no host sync, graph-capturable): the noise of the whole rollout at once
         self._noise.uniform_().clamp_(1e-10, 1.0).log_().neg_().log_().neg_()
         if self._fused:
@@ -162,13 +216,22 @@ class RolloutCollector(object):
                 env.rollout(self.actions[t:t + 1], out=(self.obs[t + 1:t + 2], self.rewards[t:t + 1], self.dones[t:t + 1]))
             _, v = self.policy(self.obs[T])
             self.values[T].copy_(v)
-        if self._kernel:                                # one launch (shipsim_gae) instead of ~T + 8 elementwise kernels
-            from . import _abi
+        if self._kernel and self._scored:               # GAE + the map of every step + the per-map sums, one GAE launch
+            with torch.cuda.device(env.device):
+                _abi.check(env.L.shipsim_gae_scored(env._h, self.rewards.data_ptr(), self.values.data_ptr(), self.dones.data_ptr(), T,
+                                                    float(self.gamma), float(self.lam), self._call0, 1, self.adv.data_ptr(),
+                                                    self.returns.data_ptr(), self.scenarios.data_ptr(), self.level_scores.data_ptr(),
+                                                    env._stream()))
+        elif self._kernel:                              # one launch (shipsim_gae) instead of ~T + 8 elementwise kernels
             with torch.cuda.device(env.device):
                 _abi.check(env.L.shipsim_gae(self.rewards.data_ptr(), self.values.data_ptr(), self.dones.data_ptr(), T, env.num_envs,
                                              float(self.gamma), float(self.lam), self.adv.data_ptr(), self.returns.data_ptr(), env._stream()))
         else:
             self._gae()
+            if self._scored:
+                log = env.episode_log
+                score_levels(self.adv, self.dones, log.meta, log.count, env.state[4, :, 2].view(torch.int32), self._call0, env.n_scenarios,
+                             scenarios=self.scenarios, scores=self.level_scores)
 
     def _gae(self):
         """GAE(lambda), as PPO2 computes it: adv[t] = delta[t] + gamma * lam * nonterminal[t] * adv[t + 1], with the deltas
@@ -202,6 +265,8 @@ class RolloutCollector(object):
             if self.env.last_reset_obs is not None:
                 self.obs[0].copy_(self.env.last_reset_obs)
             self._seen_reset_epoch = self.env.reset_epoch
+        if self._scored and self.level_scores.shape[0] != self.env.n_scenarios + 1:
+            self._alloc_scores()                        # (a new bank also moved params_epoch: the graph is captured again)
         if not self.use_graph or not self.env.graph_safe:     # (fresh maps: the pick slice moves between launches)
             self._collect()
         else:
