@@ -292,7 +292,9 @@ int shipsim_expand_delta(float *host_obs, float *host_reward, uint8_t *host_done
  * folded in), dev_b1[128]; dev_w2[2][64][64] = the trunks' second layers (in x out), dev_b2[128]; dev_w3[128][4] = policy head in
  * rows 0..63 x columns 0..2, value head in rows 64..127 x column 3 (the other entries are not read), dev_b3[4];
  * dev_noise[num_envs][3] Gumbel(0, 1) draws.  Outputs: dev_out[num_envs][4] = 3 logits | value, dev_actions[num_envs] =
- * argmax(logits + noise) as int64 -- the dtype shipsim_step takes as SHIPSIM_ACTION_I64.  Enqueued on `stream`. */
+ * argmax(logits + noise) as int64 -- the dtype shipsim_step takes as SHIPSIM_ACTION_I64; the first maximum wins a tie.
+ * Alignment: dev_obs, dev_w1, dev_b1, dev_w2, dev_b2, dev_w3 and dev_out 16 bytes, dev_actions 8 bytes (SHIPSIM_ERR_ARG
+ * otherwise; dev_b3 and dev_noise need only float alignment).  Enqueued on `stream` on the current device. */
 int shipsim_mlp_policy_forward(const float *dev_obs, int32_t num_envs, const float *dev_w1, const float *dev_b1, const float *dev_w2,
                                const float *dev_b2, const float *dev_w3, const float *dev_b3, const float *dev_noise, float *dev_out,
                                int64_t *dev_actions, void *stream);

@@ -1270,7 +1270,14 @@ extern "C" int shipsim_mlp_policy_forward(const float *dev_obs, int32_t num_envs
     unchain(nullptr);
     if (!dev_obs || !dev_w1 || !dev_b1 || !dev_w2 || !dev_b2 || !dev_w3 || !dev_b3 || !dev_noise || !dev_out || !dev_actions || num_envs < 1)
         return fail(SHIPSIM_ERR_ARG, "NULL buffer or num_envs < 1");
-    if (((uintptr_t)dev_obs & 15) != 0) return fail(SHIPSIM_ERR_ARG, "dev_obs must be 16-byte aligned");
+    // the kernel moves these in 16-byte units (cp.async of the weights, float4 loads and stores) and the actions as int64
+    const struct { const void *p; uintptr_t mask; const char *msg; } aligned[] = {
+        {dev_obs, 15, "dev_obs must be 16-byte aligned"}, {dev_w1, 15, "dev_w1 must be 16-byte aligned"},
+        {dev_b1, 15, "dev_b1 must be 16-byte aligned"},   {dev_w2, 15, "dev_w2 must be 16-byte aligned"},
+        {dev_b2, 15, "dev_b2 must be 16-byte aligned"},   {dev_w3, 15, "dev_w3 must be 16-byte aligned"},
+        {dev_out, 15, "dev_out must be 16-byte aligned"}, {dev_actions, 7, "dev_actions must be 8-byte aligned"}};
+    for (const auto &a : aligned)
+        if (((uintptr_t)a.p & a.mask) != 0) return fail(SHIPSIM_ERR_ARG, a.msg);
     CU(launch_mlp_policy(dev_obs, num_envs, dev_w1, dev_b1, dev_w2, dev_b2, dev_w3, dev_b3, dev_noise, dev_out, (long long *)dev_actions,
                          (cudaStream_t)stream));
     return SHIPSIM_OK;

@@ -21,6 +21,7 @@
 #include "shipsim_launch.h"
 
 #include <algorithm>
+#include <atomic>
 
 namespace shipsim {
 
@@ -275,13 +276,19 @@ cudaError_t launch_mlp_policy(const float *obs, int n, const float *w1, const fl
                               const float *b3, const float *noise, float *out, long long *actions, cudaStream_t stream)
 {
     if (n <= 0) return cudaSuccess;
-    static int sms = 0;
+    // the opt-in into more than 48 KB of dynamic shared memory holds for one device, and the SM count is one device's: both
+    // are kept per device (a process may run collectors on several GPUs, from several threads).  The count is published
+    // after the opt-in succeeded; a thread that still reads 0 repeats both, which is harmless.
+    static std::atomic<int> sms_of[64] = {};
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    int sms = dev < 64 ? sms_of[dev].load() : 0;
     if (!sms) {
-        int dev = 0;
-        cudaError_t e = cudaGetDevice(&dev);
-        if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+        e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(mlp_policy_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmem);
-        if (e != cudaSuccess) { sms = 0; return e; }
+        if (e != cudaSuccess) return e;
+        if (dev < 64) sms_of[dev].store(sms);
     }
     const int ntiles = (n + kPolE - 1) / kPolE;
     const int blocks = std::min(sms, ntiles);

@@ -12,55 +12,7 @@ torch = pytest.importorskip("torch")
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-
-def synthetic_rollout(rng, T, N, n_scen, call0, steps_per_call=1, p_done=0.25):
-    """Random dones (ends at t = 0 and t = T - 1 included) and the episode-log records of a rollout made of calls call0 ..
-    of steps_per_call steps each, shuffled, plus records of other calls and garbage rows past the count.  One record is
-    dropped (lost to the log's capacity).  -> dones uint8 [T, N], meta int32 [cap, 8], count, records {(t, e): scenario},
-    scenario_now [N], the lost (t, e)."""
-    from ship_sim_gym_b200 import _abi
-    done = (rng.rand(T, N) < p_done).astype(np.uint8)
-    done[0, 0] = done[T - 1, 1] = 1
-    done[:, 2] = 1                                              # an env that ends on every step
-    rec = {}
-    rows = []
-    for t, e in zip(*np.nonzero(done)):
-        s = int(rng.randint(n_scen))
-        rec[(int(t), int(e))] = s
-        m = np.zeros(_abi.EPISODE_META, np.int32)
-        m[_abi.EP_K], m[_abi.EP_ENV], m[_abi.EP_SCENARIO] = t % steps_per_call, e, s
-        m[_abi.EP_CALL] = call0 + t // steps_per_call
-        m[_abi.EP_LENGTH], m[_abi.EP_EPISODE] = rng.randint(1, 50), rng.randint(100)
-        rows.append(m)
-    lost = (int(np.nonzero(done[:, 3])[0][0]), 3) if done[:, 3].any() else (T - 1, 1)
-    rows = [r for r in rows if (int(r[_abi.EP_CALL] - call0) * steps_per_call + int(r[_abi.EP_K]), int(r[_abi.EP_ENV])) != lost]
-    for call in (call0 - 1, call0 + (T + steps_per_call - 1) // steps_per_call):     # records of the calls before and after
-        m = np.zeros(_abi.EPISODE_META, np.int32)
-        m[_abi.EP_ENV], m[_abi.EP_SCENARIO], m[_abi.EP_CALL] = 4, n_scen - 1, call
-        rows.append(m)
-    bad = np.zeros(_abi.EPISODE_META, np.int32)                 # in the rollout, but a scenario outside the bank
-    bad[_abi.EP_ENV], bad[_abi.EP_SCENARIO], bad[_abi.EP_CALL] = 5, n_scen, call0
-    rows.append(bad)
-    rows = [rows[i] for i in rng.permutation(len(rows))]
-    count = len(rows)
-    garbage = rng.randint(0, 3, (7, _abi.EPISODE_META)).astype(np.int32)   # past the count: must not be read
-    garbage[:, _abi.EP_CALL] = call0
-    meta = np.concatenate([np.stack(rows), garbage])
-    now = rng.randint(n_scen, size=N).astype(np.int32)
-    return done, meta, count, rec, now, lost
-
-
-def loop_attribution(done, rec, now):
-    """The rule, one env and one step at a time: backwards from T - 1, a done at t switches to the record of (t, e)."""
-    T, N = done.shape
-    want = np.empty((T, N), np.int64)
-    for e in range(N):
-        seg = int(now[e])
-        for t in range(T - 1, -1, -1):
-            if done[t, e]:
-                seg = rec.get((t, e), -1)
-            want[t, e] = seg
-    return want
+from references import loop_attribution, synthetic_rollout  # noqa: E402
 
 
 def numpy_fold(adv, scen, n_scen):
