@@ -154,8 +154,9 @@ int shipsim_destroy(shipsim_t *h);
  * models.py:158-196) and the goal list of gen_goal_path (game.py:300-330): the host generates scenarios in
  * float64 (ship_sim_gym_b200/scenario.py) and hands over, per scenario, the two bank hulls (CCW, convex,
  * <= SHIPSIM_MAX_HULL vertices, host_hull_xy[s][bank][maxv][2], host_hull_n[s][bank]) and the 5 goal centres
- * (host_goals_xy[s][5][2]).  Planes are derived in double, packed to fp32 and copied to the device (the copy
- * is owned by the handle).  Synchronous; call once per curriculum change, not per step. */
+ * (host_goals_xy[s][5][2]).  The vertices are rounded to fp32 and copied to the device, where the planes are derived
+ * from them in double and packed as for a device-generated bank (the copy is owned by the handle).  Synchronous; call
+ * once per curriculum change, not per step. */
 int shipsim_load_scenarios(shipsim_t *h, const double *host_hull_xy, const int32_t *host_hull_n,
                            const double *host_goals_xy, int32_t n_scenarios, int32_t maxv);
 

@@ -1,4 +1,4 @@
-// shipsim_abi.cu -- the C ABI of libshipsim.so (include/shipsim.h): handle management, scenario packing,
+// shipsim_abi.cu -- the C ABI of libshipsim.so (include/shipsim.h): handle management, scenario banks,
 // parameter derivation and kernel launches.  Host-side C++; no torch types anywhere.
 #include "../../include/shipsim.h"
 #include "shipsim_geom.cuh"
@@ -345,8 +345,6 @@ double moment_for_poly(double m, const std::vector<P2> &v)
     return m * s1 / (6.0 * s2);
 }
 
-float round_down(double v) { float f = (float)v; return (double)f > v ? std::nextafterf(f, -INFINITY) : f; }
-float round_up(double v) { float f = (float)v; return (double)f < v ? std::nextafterf(f, INFINITY) : f; }
 }  // namespace
 
 static int derive_params(shipsim_handle *h)
@@ -495,21 +493,28 @@ extern "C" int shipsim_destroy(shipsim_t *h)
     return SHIPSIM_OK;
 }
 
-// The reach grid (one thread per cell, in double) and the plane rows at the spawn pose (what an env that is reset inside
-// the kernel starts from) of the scenarios [s0, s0 + n) of bank b, from their double hull vertices: hull_stride per hull,
-// hull_xy and hull_n start at scenario s0.
-static cudaError_t build_reach_tables(const shipsim_t *h, const Bank &b, size_t s0, int n, const double *hull_xy, const int *hull_n,
-                                      int hull_stride, cudaStream_t s)
+// Everything the kernels read of the scenarios [s0, s0 + n) of bank b, from their double hull vertices (b.maxv per hull,
+// rounded to fp32 in place), hull sizes and goals, which start at scenario s0: the records (pack_bank_kernel), the reach
+// grid (one thread per cell, in double) and the plane rows at the spawn pose (what an env that is reset inside the kernel
+// starts from).  b.hull_max must be set already: the spawn rows' SAT pass lane layout depends on it.
+static int build_bank(shipsim_t *h, const Bank &b, size_t s0, int n, double *hull_xy, const int *hull_n, const double *goals,
+                      cudaStream_t s)
 {
     const auto &gg = h->grid_geom;
-    uint4 *grid = b.grid + s0 * kGridN * kGridN;
-    const cudaError_t e = launch_build_grid(hull_xy, hull_n, n, hull_stride, (double)h->p.gridp.x0, (double)h->p.gridp.y0, gg.cw, gg.ch,
-                                            gg.reach, gg.margin, grid, s);
-    if (e != cudaSuccess) return e;
     StepParams q = h->p;
-    q.bank = b.rec + s0 * b.stride4; q.edges_d = b.edges + s0 * 2 * kMaxHull; q.grid = grid; q.n_scen = n;
+    float4 *rec = b.rec + s0 * b.stride4;
+    EdgeD *edges = b.edges + s0 * 2 * kMaxHull;
+    uint4 *grid = b.grid + s0 * kGridN * kGridN;
+    q.bank = rec; q.edges_d = edges; q.grid = grid; q.n_scen = n;
     q.maxv = b.maxv; q.scen_stride4 = b.stride4; q.hull_max = b.hull_max;
-    return launch_build_spawn_rows(q, b.spawn + s0 * kScr4, s);
+    CU(cudaMemsetAsync(rec, 0, (size_t)n * b.stride4 * sizeof(float4), s));
+    CU(cudaMemsetAsync(edges, 0, (size_t)n * 2 * kMaxHull * sizeof(EdgeD), s));
+    CU(launch_pack_bank(hull_xy, hull_n, goals, n, b.maxv, b.stride4, rec, edges, s));
+    CU(launch_build_grid(hull_xy, hull_n, n, b.maxv, (double)h->p.gridp.x0, (double)h->p.gridp.y0, gg.cw, gg.ch, gg.reach, gg.margin,
+                         grid, s));
+    CU(launch_build_spawn_rows(q, b.spawn + s0 * kScr4, s));
+    h->launches += 3;
+    return SHIPSIM_OK;
 }
 
 // Make `b` the bank the kernels read; the device is idle, so no launch still reads the old one.  A new bank leaves
@@ -544,63 +549,43 @@ extern "C" int shipsim_load_scenarios(shipsim_t *h, const double *hull_xy, const
             return fail(SHIPSIM_ERR_ARG, "hull vertex count out of range [3, min(maxv, 32)]");
         dev_maxv = std::max(dev_maxv, (int)hull_n[i]);
     }
-    const int stride4 = kBankHeader4 + 2 * dev_maxv;
-    std::vector<float4> host((size_t)n_scen * stride4, make_float4(0.f, 0.f, 0.f, 0.f));
-    std::vector<EdgeD> edges((size_t)n_scen * 2 * kMaxHull);
-    std::memset(edges.data(), 0, edges.size() * sizeof(EdgeD));
     // the device geometry is the fp32-rounded polygon: every derived quantity (fp32 planes, double planes, reach
     // grid) is computed in double from the ROUNDED vertices, so the representations agree with each other
     std::vector<double> rxy((size_t)n_scen * 2 * dev_maxv * 2, 0.0);
     for (int s = 0; s < n_scen; ++s) {
-        float4 *rec = host.data() + (size_t)s * stride4;
         for (int b = 0; b < 2; ++b) {
             const double *vin = hull_xy + ((size_t)s * 2 + b) * maxv * 2;
             double *v = rxy.data() + ((size_t)s * 2 + b) * dev_maxv * 2;
             const int n = hull_n[s * 2 + b];
             for (int i = 0; i < 2 * n; ++i) v[i] = (double)(float)vin[i];
-            double l = 1e300, bo = 1e300, r = -1e300, t = -1e300, area2 = 0;
+            double area2 = 0;
             for (int i = 0; i < n; ++i) {
                 const double ax = v[2 * ((i + n - 1) % n)], ay = v[2 * ((i + n - 1) % n) + 1], bx = v[2 * i], by = v[2 * i + 1];
                 area2 += ax * by - ay * bx;
-                l = std::min(l, bx); r = std::max(r, bx); bo = std::min(bo, by); t = std::max(t, by);
             }
             if (!(area2 > 0)) return fail(SHIPSIM_ERR_ARG, "bank hulls must be convex and counter-clockwise");
-            rec[b] = make_float4(round_down(l), round_down(bo), round_up(r), round_up(t));
-            float4 *E = rec + kBankHeader4 + b * dev_maxv;
-            EdgeD *ED = edges.data() + ((size_t)s * 2 + b) * kMaxHull;
             for (int i = 0; i < n; ++i) {
-                const double ax = v[2 * ((i + n - 1) % n)], ay = v[2 * ((i + n - 1) % n) + 1], bx = v[2 * i], by = v[2 * i + 1];
-                const double ex = bx - ax, ey = by - ay, ln = std::sqrt(ex * ex + ey * ey);
-                if (!(ln > 0)) return fail(SHIPSIM_ERR_ARG, "degenerate hull edge");
-                E[i] = make_float4((float)(ey / ln), (float)(-ex / ln), (float)bx, (float)by);   // cpvrperp: outward for CCW
-                ED[i].set_normal(ey / ln, -ex / ln); ED[i].vx = (float)bx; ED[i].vy = (float)by; ED[i].len = (float)ln;
-                { const int self = b * kMaxHull + i; std::memcpy(&ED[i].pad, &self, 4); }
+                const int j = (i + n - 1) % n;
+                const double ex = v[2 * i] - v[2 * j], ey = v[2 * i + 1] - v[2 * j + 1];
+                if (!(std::sqrt(ex * ex + ey * ey) > 0)) return fail(SHIPSIM_ERR_ARG, "degenerate hull edge");
             }
         }
-        const double *g = goals_xy + (size_t)s * 10;
-        rec[2] = make_float4((float)g[0], (float)g[1], (float)g[2], (float)g[3]);
-        rec[3] = make_float4((float)g[4], (float)g[5], (float)g[6], (float)g[7]);
-        float4 g2 = make_float4((float)g[8], (float)g[9], 0.f, 0.f);
-        const int n0 = hull_n[s * 2], n1 = hull_n[s * 2 + 1];
-        std::memcpy(&g2.z, &n0, 4); std::memcpy(&g2.w, &n1, 4);
-        rec[4] = g2;
     }
     if (n_scen >= (1 << 28)) return fail(SHIPSIM_ERR_ARG, "too many scenarios");
     DeviceGuard g(h->device);
     Bank b;
-    DeviceBuf<double> dxy;
+    DeviceBuf<double> dxy, dgo;
     DeviceBuf<int> dn;
     CU(b.alloc(n_scen, dev_maxv));
     CU(dxy.ensure(rxy.size()));
     CU(dn.ensure((size_t)n_scen * 2));
-    CU(cudaMemcpy(b.rec, host.data(), host.size() * sizeof(float4), cudaMemcpyHostToDevice));
-    CU(cudaMemcpy(b.edges, edges.data(), edges.size() * sizeof(EdgeD), cudaMemcpyHostToDevice));
+    CU(dgo.ensure((size_t)n_scen * 10));
     CU(cudaMemcpy(dxy, rxy.data(), rxy.size() * sizeof(double), cudaMemcpyHostToDevice));
     CU(cudaMemcpy(dn, hull_n, (size_t)n_scen * 2 * sizeof(int), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(dgo, goals_xy, (size_t)n_scen * 10 * sizeof(double), cudaMemcpyHostToDevice));
     b.hull_max = dev_maxv;
-    CU(build_reach_tables(h, b, 0, n_scen, dxy, dn, dev_maxv, 0));
+    TRY(build_bank(h, b, 0, n_scen, dxy, dn, dgo, 0));
     CU(cudaDeviceSynchronize());                                 // also: no launch may still be reading the old bank
-    h->launches += 2;
     return install(h, std::move(b), 0);
 }
 
@@ -622,16 +607,13 @@ extern "C" int shipsim_generate_scenarios(shipsim_t *h, int32_t n_scen, uint64_t
     CU(gen.goals.ensure((size_t)n_scen * 10));
     CU(gen.n.ensure((size_t)n_scen * 2));
     CU(dmax.ensure(1));
-    CU(cudaMemsetAsync(b.rec, 0, (size_t)n_scen * b.stride4 * sizeof(float4), s));
-    CU(cudaMemsetAsync(b.edges, 0, (size_t)n_scen * 2 * kMaxHull * sizeof(EdgeD), s));
     CU(launch_gen_scenarios(seed, n_scen, h->cfg.bounds_w, h->cfg.bounds_h, map_N, width_frac, gen.xy, gen.n, gen.goals, s));
     CU(launch_max_hull(gen.n, n_scen * 2, dmax, s));
-    CU(launch_pack_bank(gen.xy, gen.n, gen.goals, n_scen, b.maxv, b.stride4, b.rec, b.edges, s));
     CU(cudaMemcpyAsync(&b.hull_max, dmax, sizeof(int), cudaMemcpyDeviceToHost, s));
     CU(cudaStreamSynchronize(s));                                // 4-byte read-back: the SAT pass lane layout depends on it
-    CU(build_reach_tables(h, b, 0, n_scen, gen.xy, gen.n, kMaxHull, s));
+    h->launches += 2;
+    TRY(build_bank(h, b, 0, n_scen, gen.xy, gen.n, gen.goals, s));
     CU(cudaDeviceSynchronize());                                 // no launch may still be reading the old bank
-    h->launches += 5;
     b.generated = true;
     gen.count = n_scen;
     h->gen = std::move(gen);
@@ -661,21 +643,14 @@ static uint64_t fresh_seed(uint64_t seed, int period) { return seed + 0x9E3779B9
 
 static int fresh_regenerate(shipsim_t *h, int slice, uint64_t seed)
 {
-    const Bank &b = h->bank;
-    const int q = b.n_scen / 4;
+    const int q = h->bank.n_scen / 4;
     const size_t s0 = (size_t)slice * q;
     cudaStream_t gs = h->fresh.stream;
     double *dxy = h->gen.xy + s0 * 2 * kMaxHull * 2, *dgo = h->gen.goals + s0 * 10;
     int *dn = h->gen.n + s0 * 2;
-    float4 *d = b.rec + s0 * b.stride4;
-    EdgeD *de = b.edges + s0 * 2 * kMaxHull;
-    CU(cudaMemsetAsync(d, 0, (size_t)q * b.stride4 * sizeof(float4), gs));
-    CU(cudaMemsetAsync(de, 0, (size_t)q * 2 * kMaxHull * sizeof(EdgeD), gs));
     CU(launch_gen_scenarios(seed, q, h->cfg.bounds_w, h->cfg.bounds_h, h->fresh.map_N, h->fresh.width_frac, dxy, dn, dgo, gs));
-    CU(launch_pack_bank(dxy, dn, dgo, q, b.maxv, b.stride4, d, de, gs));
-    CU(build_reach_tables(h, b, s0, q, dxy, dn, kMaxHull, gs));
-    h->launches += 4;
-    return SHIPSIM_OK;
+    h->launches++;
+    return build_bank(h, h->bank, s0, q, dxy, dn, dgo, gs);
 }
 
 // called before every step launch: moves on to the next period when the current one has lasted long enough

@@ -7,9 +7,10 @@
 // those streams cannot be reproduced on a GPU, so draws come from Philox4x32-10 keyed by (seed, scenario): the
 // DISTRIBUTIONS are the reference's (tests compare against the host generator, which is pinned to the reference's
 // fixtures), the individual maps are not.
-// pack_bank_kernel then derives, from the fp32-rounded vertices, the same records shipsim_load_scenarios builds on the
-// host (fp32 planes, double planes, header); the reach grid and spawn rows follow in shipsim_kernels.cu.  Everything
-// is enqueued on the caller's stream: a bank can be regenerated between rollouts without a host round trip.
+// pack_bank_kernel then derives, from the fp32-rounded vertices, the scenario records (fp32 planes, double planes,
+// header) of every bank, generated here or loaded from the host; the reach grid and spawn rows follow in
+// shipsim_kernels.cu.  Everything is enqueued on the caller's stream: a bank can be regenerated between rollouts without
+// a host round trip.
 #include "shipsim_device.cuh"
 #include "shipsim_launch.h"
 
@@ -203,9 +204,11 @@ __global__ void max_hull_kernel(const int *hull_n, int n, int *out)
     if ((threadIdx.x & 31) == 0) atomicMax(out, m);
 }
 
-// Same records shipsim_load_scenarios builds on the host; one thread per scenario.  `stride4` / `maxv` are the layout
-// of the fp32 bank (fixed at kMaxHull for device-generated banks).  hull_xy is rounded to fp32 IN PLACE so that the
-// reach-grid build that follows sees the polygon the kernels represent.
+// The only writer of the scenario records (the fp32 records and the EdgeD planes; layout in shipsim_device.cuh) of every
+// bank, loaded or generated; one thread per scenario.  `stride4` / `maxv` are the layout of the fp32 bank, and hull_xy
+// holds `maxv` vertices per hull.  hull_xy is rounded to fp32 IN PLACE so that the reach-grid build that follows sees the
+// polygon the kernels represent.  The squared edge length is two rounded products and a rounded sum, never a DFMA: the
+// planes are then those plain double arithmetic gives (the float64 oracle is compiled with -ffp-contract=off).
 __global__ void __launch_bounds__(128) pack_bank_kernel(double *hull_xy, const int *hull_n, const double *goals, int n_scen,
                                                         int maxv, int stride4, float4 *bank, EdgeD *edges)
 {
@@ -213,19 +216,21 @@ __global__ void __launch_bounds__(128) pack_bank_kernel(double *hull_xy, const i
     if (sidx >= n_scen) return;
     float4 *rec = bank + (size_t)sidx * stride4;
     for (int b = 0; b < 2; ++b) {
-        double *v = hull_xy + ((size_t)sidx * 2 + b) * kMaxHull * 2;
+        double *v = hull_xy + ((size_t)sidx * 2 + b) * maxv * 2;
         const int n = hull_n[sidx * 2 + b];
         double l = 1e300, bo = 1e300, r = -1e300, t = -1e300;
-        for (int i = 0; i < n; ++i) {
-            v[2 * i] = (double)(float)v[2 * i]; v[2 * i + 1] = (double)(float)v[2 * i + 1];
-            l = fmin(l, v[2 * i]); r = fmax(r, v[2 * i]); bo = fmin(bo, v[2 * i + 1]); t = fmax(t, v[2 * i + 1]);
+        for (int i = 0; i < n; ++i) {           // (not fmin / fmax: a tie such as -0 against +0 keeps the earlier vertex)
+            const double x = (double)(float)v[2 * i], y = (double)(float)v[2 * i + 1];
+            v[2 * i] = x; v[2 * i + 1] = y;
+            l = x < l ? x : l; r = r < x ? x : r; bo = y < bo ? y : bo; t = t < y ? y : t;
         }
         rec[b] = make_float4(__double2float_rd(l), __double2float_rd(bo), __double2float_ru(r), __double2float_ru(t));
         float4 *E = rec + kBankHeader4 + b * maxv;
         EdgeD *ED = edges + ((size_t)sidx * 2 + b) * kMaxHull;
         for (int i = 0; i < n; ++i) {
             const int j = i == 0 ? n - 1 : i - 1;
-            const double ex = v[2 * i] - v[2 * j], ey = v[2 * i + 1] - v[2 * j + 1], ln = sqrt(ex * ex + ey * ey);
+            const double ex = v[2 * i] - v[2 * j], ey = v[2 * i + 1] - v[2 * j + 1];
+            const double ln = sqrt(__dadd_rn(__dmul_rn(ex, ex), __dmul_rn(ey, ey)));
             E[i] = make_float4((float)(ey / ln), (float)(-ex / ln), (float)v[2 * i], (float)v[2 * i + 1]);
             EdgeD e;
             e.set_normal(ey / ln, -ex / ln); e.vx = (float)v[2 * i]; e.vy = (float)v[2 * i + 1]; e.len = (float)ln;
